@@ -6,9 +6,13 @@ cfg 3 full pipeline, cfg 4 MODE_HH 1080p D=256, cfg 5 4K D=256) are measured in 
 `configs` block of the same JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--configs LIST|none]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (mvsv_compute: prefilter -> BT cost -> box sums -> 5 path scans -> WTA/LR ->
-median -> speckle) over one batch of B stereo pairs per GPU.  `value` times K steps with inputs resident in HBM
+median -> speckle) over one batch of B stereo pairs per GPU; every configuration runs K timed steps.  With
+--dump-outputs, rank 0 writes what the last HBM-resident step of each configuration returns to a caller (disparities;
+for cfg 3 also the ROI means) as DIR/<config>_<array>.npy in float32, so that two builds can be compared output for
+output: the inputs are seeded, the same from run to run.  `value` times K steps with inputs resident in HBM
 (CUDA events on the engine's stream); `e2e` times the same K steps through the host-facing C-ABI call with pinned
 HOST buffers, host->device and device->host copies inside the timed region, pipelined inside ONE engine over two
 I/O slots (mvsv_set_io_slots).  For N > 1 the script runs under torchrun, one rank per GPU; frames are
@@ -65,6 +69,9 @@ KERNEL_BYTES_PER_CELL = {"sgbm_vsum": 2.0, "sgbm_h1": 6.0, "sgbm_td": 6.0, "sgbm
 # the same when the aggregated volume S is kept as one byte per cell (mvsv_info.sgbm_s8: npaths * P2 <= 255)
 KERNEL_BYTES_PER_CELL_S8 = dict(KERNEL_BYTES_PER_CELL, sgbm_h1=5.0, sgbm_td=4.0, sgbm_h2_wta=3.0)
 NCU_SUMMARY = os.path.join(ROOT, "profiles", "r02_ncu_traffic.json")
+# --dump-outputs: at most this many values per array (8 MiB of float32), so that the seven arrays of a run with every
+# configuration stay under 64 MB
+DUMP_VALUES_PER_ARRAY = 1 << 21
 
 
 def hbm_peak():
@@ -150,6 +157,15 @@ def cells_per_frame(spec, W=None):
     return w1_of(W, p) * spec["H"] * p["numDisp"]
 
 
+def dump_sample(a):
+    """`a` as float32; above DUMP_VALUES_PER_ARRAY values, the values at a fixed seeded sample of its flat indices
+    (ascending), the same sample for every run at the same shape."""
+    if a.size > DUMP_VALUES_PER_ARRAY:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_VALUES_PER_ARRAY, replace=False))
+        a = a.reshape(-1)[idx]
+    return a.astype(np.float32)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons sampled DURING the timed region (B200_PROFILING.md recipe)."""
     Q = ("index,clocks.sm,clocks.max.sm,power.draw,clocks_event_reasons.active,clocks_event_reasons.hw_slowdown,"
@@ -230,7 +246,7 @@ def _make_cv_matcher(cv2, spec):
 def load_rectification():
     """Maps cv2 derives from the reference's parameters/baseline_small calibration (committed fixture, generated by
     tests/golden/make_golden.py)."""
-    g = np.load(os.path.join(ROOT, "tests", "golden", "rectify_baseline_small.npz"))
+    g = synth.load_rectification(os.path.join(ROOT, "tests", "golden"))
     return g, tuple(int(v) for v in g["roi"])
 
 
@@ -340,9 +356,10 @@ def make_inputs(spec, ids, B):
     return gen, uniq
 
 
-def run_config(cx, key, batch, steps, warmup, detail=False):
+def run_config(cx, key, batch, steps, warmup, detail=False, dump=False):
     """Device-resident and end-to-end throughput of one configuration (this rank's share of the frames), plus a
-    one-frame bit-exactness check against cv2 on rank 0.  Returns a dict; `detail` adds per-kernel times."""
+    one-frame bit-exactness check against cv2 on rank 0.  Returns a dict; `detail` adds per-kernel times, `dump` the
+    outputs of the last device-resident step under "_dump" (dump_sample of each)."""
     torch, api = cx.torch, cx.api
     spec = CONFIGS[key]
     p, H, W, B = spec["params"], spec["H"], spec["W"], batch
@@ -402,6 +419,7 @@ def run_config(cx, key, batch, steps, warmup, detail=False):
     ms = eng.timer_stop()
     launches = eng.launch_count - l0
     fence()
+    dumped = {k: dump_sample(v) for k, v in eng.download(B, **extra_out).items()} if dump else None
     # Per-kernel CUDA-event durations come from a second pass over the same K steps: with per-kernel timing enabled the
     # engine runs its kernels one after the other (mvsv_profile_enable), while in the timed pass above the cost kernel
     # and the first row scan of different chunks of frames overlap on two streams -- a kernel's duration only means
@@ -480,6 +498,8 @@ def run_config(cx, key, batch, steps, warmup, detail=False):
     if spec["kind"] == "bm":
         # bytes the two volume kernels actually move per cell: the column sums written once and read once
         out["roofline_path"]["step_bytes_per_cell"] = 2.0 if eng.info.bm_col8 else 4.0
+    if dump:
+        out["_dump"] = dumped
     if detail:
         out["_detail"] = dict(s8=bool(eng.info.sgbm_s8), prof=prof, launches=launches, clocks=clocks, gen=gen, uniq=uniq, gpu_disp=gpu_disp,
                               cells=cells, fps=fps, fps_e2e=fps_e2e, ms_max=ms_max, ms_e2e_max=ms_e2e_max, d2h=d2h)
@@ -504,6 +524,8 @@ def main():
     ap.add_argument("--configs", default="all",
                     help="comma separated keys of the other BASELINE configurations to add to the line (%s), "
                          "'all' or 'none'" % ", ".join(k for k in CONFIGS if k != HEADLINE))
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of each configuration's last timed step to DIR/<config>_<array>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -530,21 +552,27 @@ def main():
 
     spec = CONFIGS[HEADLINE]
     p, H, W, B = spec["params"], spec["H"], spec["W"], args.batch
-    head = run_config(cx, HEADLINE, B, args.steps, args.warmup, detail=True)
+    dump = args.dump_outputs is not None and rank == 0
+    head = run_config(cx, HEADLINE, B, args.steps, args.warmup, detail=True, dump=dump)
     det = head.pop("_detail")
+    dumped = {HEADLINE: head.pop("_dump", None)}
 
-    # ---- the other BASELINE configurations (short runs; same measurement, same parity gate) ----------------------
+    # ---- the other BASELINE configurations (same measurement, same parity gate) ----------------------------------
     others = {}
     want = [k for k in CONFIGS if k != HEADLINE] if args.configs == "all" else (
         [] if args.configs == "none" else [k.strip() for k in args.configs.split(",") if k.strip()])
     for key in want:
-        # steps sized so that each configuration takes a few seconds
-        per_step_cells = cells_per_frame(CONFIGS[key]) * CONFIGS[key]["batch"]
-        st = int(min(20, max(3, 2.0e11 / max(per_step_cells, 1))))
         try:
-            others[key] = run_config(cx, key, CONFIGS[key]["batch"], st, 3)
+            others[key] = run_config(cx, key, CONFIGS[key]["batch"], args.steps, args.warmup, dump=dump)
+            dumped[key] = others[key].pop("_dump", None)
         except Exception as e:       # a configuration that cannot run must not take the headline down with it
             others[key] = {"workload": CONFIGS[key]["name"], "error": "%s: %s" % (type(e).__name__, e)}
+
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for key, arrays in dumped.items():
+            for name, a in (arrays or {}).items():
+                np.save(os.path.join(args.dump_outputs, "%s_%s.npy" % (key, name)), a)
 
     if rank != 0:
         if dist is not None:

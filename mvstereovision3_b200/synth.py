@@ -3,6 +3,8 @@
 The reference ships no images (only calibration YAMLs), so every test and bench
 input is made here, seeded and reproducible with numpy alone.
 """
+import os
+
 import numpy as np
 
 
@@ -44,3 +46,23 @@ def random_pair(height, width, seed=0):
     a = _blur3(rng.integers(0, 256, size=(height, width), dtype=np.uint8))
     b = _blur3(rng.integers(0, 256, size=(height, width), dtype=np.uint8))
     return a, b
+
+
+def encode_map(m):
+    """float32 map -> int32 second differences along rows of its bit patterns (wrapping).  The maps are smooth, so
+    these deflate about six times smaller than the floats themselves; decode_map restores them bit for bit."""
+    return np.diff(m.view(np.int32), n=2, axis=1, prepend=np.zeros((m.shape[0], 2), np.int32))
+
+
+def decode_map(d):
+    return np.cumsum(np.cumsum(d, axis=1, dtype=np.int32), axis=1, dtype=np.int32).view(np.float32)
+
+
+def load_rectification(golden_dir):
+    """The rectification fixture of the reference's parameters/baseline_small calibration (written by
+    tests/golden/make_golden.py): cv2's float maps m1x, m1y, m2x, m2y, the display ROI `roi`, Q, and the seed-7 pair
+    remapped and cropped by cv2 (rectL, rectR)."""
+    g = dict(np.load(os.path.join(golden_dir, "rectify_baseline_small.npz")))
+    with np.load(os.path.join(golden_dir, "rectify_baseline_small_maps.npz")) as maps:
+        g.update((k, decode_map(maps[k])) for k in maps.files)
+    return g

@@ -43,7 +43,7 @@ def test_remap_median_speckle_xyz_vs_golden(oracle, golden):
 
 
 def test_rectify_fixture(oracle):
-    g = np.load(os.path.join(cases.GOLDEN_DIR, "rectify_baseline_small.npz"))
+    g = cases.synth.load_rectification(cases.GOLDEN_DIR)
     roi = tuple(int(v) for v in g["roi"])
     assert roi == (0, 0, 752, 479)          # SURVEY.md 8c: baseline_small yields a 752x479 display ROI
     l, r, _ = cases.synth.stereogram(480, 752, 1, 64, seed=7)

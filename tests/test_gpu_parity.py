@@ -316,7 +316,7 @@ def test_bm_batches_full_size_vs_cv2(nd, bs, cap, uniq, H, W, B):
 
 def test_cfg3_pipeline(oracle):
     """remap(maps of parameters/baseline_small) -> crop -> SGBM cfg 2 -> XYZ -> 81 sub-image + sample-point means."""
-    g = np.load(os.path.join(cases.GOLDEN_DIR, "rectify_baseline_small.npz"))
+    g = synth.load_rectification(cases.GOLDEN_DIR)
     roi = tuple(int(v) for v in g["roi"])
     B = 3
     raws = [synth.stereogram(480, 752, 1, 64, seed=7 + b)[:2] for b in range(B)]

@@ -64,7 +64,7 @@ def test_oracle_maps_match_committed_crc(oracle, rig, mode):
 
 def test_oracle_maps_match_committed_float_maps(oracle):
     """the float maps committed for parameters/baseline_small (the fixture of the remap tests)"""
-    g = np.load(os.path.join(cases.GOLDEN_DIR, "rectify_baseline_small.npz"))
+    g = cases.synth.load_rectification(cases.GOLDEN_DIR)
     cams, size, _ = cameras("baseline_small", "full")
     for (K, D, R, P), kx, ky in zip(cams, ("m1x", "m2x"), ("m1y", "m2y")):
         mx, my = oracle.rectify_maps(K, D, R, P, size)
@@ -134,7 +134,7 @@ def test_pipeline_with_device_maps_equals_uploaded_maps():
     """raw pair -> rectify -> SGBM: building the maps on the device gives the same images and disparities as
     uploading the committed cv2 float maps (Stereosystem::getRectifiedImagepair, src/Stereosystem.cpp:244-277)."""
     from mvstereovision3_b200 import api, synth
-    g = np.load(os.path.join(cases.GOLDEN_DIR, "rectify_baseline_small.npz"))
+    g = synth.load_rectification(cases.GOLDEN_DIR)
     cams, size, m = cameras("baseline_small", "full")
     roi = tuple(int(v) for v in g["roi"])
     assert list(roi) == m["display_roi"]
@@ -202,7 +202,7 @@ def test_oracle_resize_matches_cv2(oracle, size):
 def test_rectify_resize_sgbm_pipeline(oracle, factor):
     """raw pair -> remap -> crop -> resize(factor) -> SGBM, against the oracle chain and (resize) live cv2"""
     from mvstereovision3_b200 import api, synth
-    g = np.load(os.path.join(cases.GOLDEN_DIR, "rectify_baseline_small.npz"))
+    g = synth.load_rectification(cases.GOLDEN_DIR)
     cams, size, m = cameras("baseline_small", "full")
     roi = m["display_roi"]
     B = 2
