@@ -17,7 +17,7 @@ STAGE_RECTIFY, STAGE_SGBM, STAGE_BM, STAGE_XYZ, STAGE_MEANS = 1, 2, 4, 8, 16
 ABI_SYMBOLS = (
     "mvsv_init", "mvsv_destroy", "mvsv_last_error", "mvsv_set_sgbm_params", "mvsv_set_bm_params",
     "mvsv_upload_rectify_maps", "mvsv_set_rectification", "mvsv_set_resize", "mvsv_reset_rectification", "mvsv_set_Q", "mvsv_set_mean_rois", "mvsv_compute",
-    "mvsv_compute_device", "mvsv_tm", "mvsv_order_after", "mvsv_download", "mvsv_sync", "mvsv_get_info", "mvsv_stream", "mvsv_launch_count",
+    "mvsv_compute_device", "mvsv_tm", "mvsv_download", "mvsv_sync", "mvsv_get_info", "mvsv_stream", "mvsv_launch_count",
     "mvsv_host_alloc", "mvsv_host_free", "mvsv_debug_set_flags", "mvsv_debug_read",
     "mvsv_download_minmax", "mvsv_download_age", "mvsv_set_io_slots", "mvsv_timer_start", "mvsv_timer_stop", "mvsv_profile_enable", "mvsv_profile_read", "mvsv_kernel_name",
 )
@@ -79,7 +79,6 @@ def load_library():
     lib.mvsv_download_age.argtypes = [vp, ci, vp, sz, vp, vp, sz, vp, vp]
     lib.mvsv_set_io_slots.argtypes = [vp, ci]
     lib.mvsv_sync.argtypes = [vp]
-    lib.mvsv_order_after.argtypes = [vp, vp]
     lib.mvsv_download_minmax.argtypes = [vp, vp]
     lib.mvsv_get_info.argtypes = [vp, C.POINTER(Info)]
     lib.mvsv_stream.argtypes = [vp]
@@ -262,10 +261,6 @@ class Engine:
         self._ck(self._lib.mvsv_tm(self._ctx, left.ctypes.data, left.strides[1], right.ctypes.data, right.strides[1],
                                    left.strides[0], left.shape[0], int(kernel_size), out.ctypes.data, out.strides[1]))
         return out
-
-    def order_after(self, other):
-        """Kernels submitted to this engine from now on start after everything already submitted to `other`."""
-        self._ck(self._lib.mvsv_order_after(self._ctx, other._ctx))
 
     def sync(self):
         self._ck(self._lib.mvsv_sync(self._ctx))

@@ -514,18 +514,15 @@ static int bm_wta_cta_warps(size_t warpBytes, int* warpsPerSm)
 }
 
 template <int OPL, bool RING, bool B8>
-static void launch_bm_wta(mvsv_ctx* c, const BmArgs& a, int ringSlots, int ctaWarps)
+static cudaError_t launch_bm_wta(mvsv_ctx* c, const BmArgs& a, int ringSlots, int ctaWarps)
 {
     const int NL = (a.D / 8) / OPL, rowsPerWarp = 32 / NL;
     const long long warps = ((long long)a.B * (a.H - 2 * a.w2) + rowsPerWarp - 1) / rowsPerWarp;
-    static bool configured[64] = {};            // per device: a process may drive several GPUs
-    if (c->device < 0 || c->device >= 64 || !configured[c->device]) {
-        cudaFuncSetAttribute(k_bm_wta<OPL, RING, B8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
-        if (c->device >= 0 && c->device < 64) configured[c->device] = true;
-    }
+    MVSV_TRY(smem_limit((const void*)k_bm_wta<OPL, RING, B8>, 226 * 1024));
     const size_t smem = ctaWarps * bm_wta_warp_smem(a.D, OPL, B8 ? 1 : OPL, RING ? ringSlots : 0);
     k_bm_wta<OPL, RING, B8><<<(unsigned)((warps + ctaWarps - 1) / ctaWarps), ctaWarps * 32, smem, c->stream>>>(
         a, ringSlots, bm_sums_per_warp(a.D, OPL));
+    return cudaGetLastError();
 }
 
 // n is a multiple of 8 pixels (the image buffers are padded to 16 bytes): one 128-bit store per thread
@@ -539,20 +536,20 @@ __global__ void k_fill16(int16_t* p, size_t n, int16_t v)
 
 }  // namespace
 
-void launch_bm(mvsv_ctx* c, int B)
+cudaError_t launch_bm(mvsv_ctx* c, int B)
 {
     const BmNorm& n = c->bm;
     const bool col8 = n.col8 && !(c->debug_flags & 2u);         // debug bit 1: never keep a volume as bytes
     const int W = c->W, H = c->H;
     const size_t npx = (size_t)B * W * H;
-    { KernelTimer kt(c, KID_FILL); k_fill16<<<(unsigned)((npx / 8 + 256) / 256), 256, 0, c->stream>>>(c->disp, npx, (int16_t)n.FILT); }
+    { KernelTimer kt(c, KID_FILL); k_fill16<<<(unsigned)((npx / 8 + 256) / 256), 256, 0, c->stream>>>(io(c).disp, npx, (int16_t)n.FILT); }
     {
         dim3 blk(128), grd((W + 127) / 128, (H + 4 * BM_PF_ROWS - 1) / (4 * BM_PF_ROWS), 2 * B);
         KernelTimer kt(c, KID_BM_PREFILTER);
-        k_bm_prefilter<<<grd, blk, 0, c->stream>>>(c->rect[0], c->rect[1], c->pitch, W, H, n.cap, c->bm_pre[0], c->bm_pre[1]);
+        k_bm_prefilter<<<grd, blk, 0, c->stream>>>(io(c).rect[0], io(c).rect[1], c->pitch, W, H, n.cap, c->bm_pre[0], c->bm_pre[1]);
     }
     const bool any = !(n.lofs >= W || n.width1 < 1) && (H - 2 * n.w2 > 0) && (n.width1 - 2 * n.w2 > 0);
-    if (!any) return;
+    if (!any) return cudaGetLastError();
     {
         KernelTimer kt(c, KID_BM_TEX);
         if (n.bs <= 63) {
@@ -570,18 +567,13 @@ void launch_bm(mvsv_ctx* c, int B)
         dim3 grd((unsigned)((threads + 127) / 128), B);
         // blockSize^2 * 2 * cap <= 65535 (contract) bounds blockSize by 181: the ring needs at most 181 KB
         const size_t ringBytes = (size_t)n.bs * 128 * sizeof(uint2);
-        static bool configured[64] = {};        // per device: a process may drive several GPUs
-        if (c->device < 0 || c->device >= 64 || !configured[c->device]) {
-            cudaFuncSetAttribute(k_bm_colsum<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-            cudaFuncSetAttribute(k_bm_colsum<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-            if (c->device >= 0 && c->device < 64) configured[c->device] = true;
-        }
+        const auto colsum = col8 ? k_bm_colsum<true> : k_bm_colsum<false>;
+        MVSV_TRY(smem_limit((const void*)colsum, 200 * 1024));
         KernelTimer kt(c, KID_BM_COLSUM);
-        if (col8) k_bm_colsum<true><<<grd, 128, ringBytes, c->stream>>>(c->bm_pre[0], c->bm_pre[1], c->pitch, H, n.width1, n.D, n.lofs, n.w2, c->bm_col);
-        else k_bm_colsum<false><<<grd, 128, ringBytes, c->stream>>>(c->bm_pre[0], c->bm_pre[1], c->pitch, H, n.width1, n.D, n.lofs, n.w2, c->bm_col);
+        colsum<<<grd, 128, ringBytes, c->stream>>>(c->bm_pre[0], c->bm_pre[1], c->pitch, H, n.width1, n.D, n.lofs, n.w2, c->bm_col);
     }
     BmArgs a;
-    a.col = c->bm_col; a.tex = c->bm_tex2; a.disp = c->disp; a.W = W; a.H = H; a.width1 = n.width1; a.D = n.D; a.Dp = n.Dp;
+    a.col = c->bm_col; a.tex = c->bm_tex2; a.disp = io(c).disp; a.W = W; a.H = H; a.width1 = n.width1; a.D = n.D; a.Dp = n.Dp;
     a.lofs = n.lofs; a.w2 = n.w2; a.texThr = n.tex; a.uniq = n.uniq; a.B = B;
     KernelTimer kt(c, KID_BM_WTA);
     // Two octets per lane (numDisp is a multiple of 16) with the window ring while at least eight warps fit an SM
@@ -590,13 +582,12 @@ void launch_bm(mvsv_ctx* c, int B)
     int wps = 0, nw;
     if (col8) {
         nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 1, slots), &wps);
-        if (wps >= 4) launch_bm_wta<2, true, true>(c, a, slots, nw);
-        else launch_bm_wta<2, false, true>(c, a, slots, 4);
-    } else {
-        nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 2, slots), &wps);
-        if (wps >= 8) { launch_bm_wta<2, true, false>(c, a, slots, nw); return; }
-        nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 1, 1, slots), &wps);
-        if (wps >= 4) launch_bm_wta<1, true, false>(c, a, slots, nw);
-        else launch_bm_wta<2, false, false>(c, a, slots, 4);
+        if (wps >= 4) return launch_bm_wta<2, true, true>(c, a, slots, nw);
+        return launch_bm_wta<2, false, true>(c, a, slots, 4);
     }
+    nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 2, slots), &wps);
+    if (wps >= 8) return launch_bm_wta<2, true, false>(c, a, slots, nw);
+    nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 1, 1, slots), &wps);
+    if (wps >= 4) return launch_bm_wta<1, true, false>(c, a, slots, nw);
+    return launch_bm_wta<2, false, false>(c, a, slots, 4);
 }

@@ -498,40 +498,44 @@ __global__ void k_minmax(const int16_t* __restrict__ disp, int* __restrict__ mm,
 
 }  // namespace
 
-void launch_minmax(mvsv_ctx* c, int B)
+cudaError_t launch_minmax(mvsv_ctx* c, int B)
 {
     { KernelTimer kt(c, KID_MINMAX); k_minmax_init<<<(2 * B + 127) / 128, 128, 0, c->stream>>>(c->minmax, 2 * B); }
     dim3 grd(32, B);
     KernelTimer kt(c, KID_MINMAX);
-    k_minmax<<<grd, 256, 0, c->stream>>>(c->disp, c->minmax, c->W * c->H);
+    k_minmax<<<grd, 256, 0, c->stream>>>(io(c).disp, c->minmax, c->W * c->H);
+    return cudaGetLastError();
 }
 
-void launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t strideElems)
+cudaError_t launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t strideElems)
 {
     dim3 blk(128), grd((c->roi[2] + 127) / 128, c->roi[3]);
     KernelTimer kt(c, KID_REMAP);
     k_convert_maps<<<grd, blk, 0, c->stream>>>(dmapx, dmapy, strideElems, c->roi[0], c->roi[1], c->roi[2], c->roi[3],
                                                c->map_xy[cam]);
+    return cudaGetLastError();
 }
 
-void launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q)
+cudaError_t launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q)
 {
     dim3 blk(128), grd((c->roi[2] + 127) / 128, c->roi[3]);
     KernelTimer kt(c, KID_REMAP);
     k_rectify_maps<<<grd, blk, 0, c->stream>>>(q, c->roi[0], c->roi[1], c->roi[2], c->roi[3], c->map_xy[cam]);
+    return cudaGetLastError();
 }
 
-void launch_remap(mvsv_ctx* c, int cam, int B)
+cudaError_t launch_remap(mvsv_ctx* c, int cam, int B)
 {
     const int rw = c->roi[2], rh = c->roi[3];
     const bool resized = c->resize_factor > 0.0;
     dim3 blk(128), grd((rw + 511) / 512, rh, (B + RM_FRAMES - 1) / RM_FRAMES);
     KernelTimer kt(c, KID_REMAP);
-    k_remap<<<grd, blk, 0, c->stream>>>(c->raw[cam], c->raw_pitch, c->fw, c->fh, c->map_xy[cam],
-                                        resized ? c->crop[cam] : c->rect[cam], resized ? c->crop_pitch : c->pitch, rw, rh, B);
+    k_remap<<<grd, blk, 0, c->stream>>>(io(c).raw[cam], c->raw_pitch, c->fw, c->fh, c->map_xy[cam],
+                                        resized ? c->crop[cam] : io(c).rect[cam], resized ? c->crop_pitch : c->pitch, rw, rh, B);
+    return cudaGetLastError();
 }
 
-void launch_resize(mvsv_ctx* c, int cam, int B)
+cudaError_t launch_resize(mvsv_ctx* c, int cam, int B)
 {
     const int rw = c->roi[2], rh = c->roi[3];
     const double scale = 1.0 / c->resize_factor;
@@ -539,29 +543,31 @@ void launch_resize(mvsv_ctx* c, int cam, int B)
     dim3 blk(128), grd((c->W + 127) / 128, c->H, B);
     KernelTimer kt(c, KID_REMAP);
     if (fabs(scale - (double)iscale) < DBL_EPSILON && iscale == 2)
-        k_resize_half<<<grd, blk, 0, c->stream>>>(c->crop[cam], c->crop_pitch, rw, rh, c->rect[cam], c->pitch, c->W, c->H);
+        k_resize_half<<<grd, blk, 0, c->stream>>>(c->crop[cam], c->crop_pitch, rw, rh, io(c).rect[cam], c->pitch, c->W, c->H);
     else
-        k_resize_linear<<<grd, blk, 0, c->stream>>>(c->crop[cam], c->crop_pitch, rw, rh, c->rect[cam], c->pitch, c->W, c->H, scale);
+        k_resize_linear<<<grd, blk, 0, c->stream>>>(c->crop[cam], c->crop_pitch, rw, rh, io(c).rect[cam], c->pitch, c->W, c->H, scale);
+    return cudaGetLastError();
 }
 
-void launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B)
+cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B)
 {
     KernelTimer kt(c, KID_MEDIAN);
     if (c->W % 4 == 0 && c->W >= 4 && (reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) % 8 == 0) {
         const int ncx = (c->W + MED4_COLS - 1) / MED4_COLS, nbands = (c->H + MED_ROWS - 1) / MED_ROWS;
         dim3 grd((ncx * nbands + MED_WARPS - 1) / MED_WARPS, B);
         k_median3_w4<<<grd, MED_WARPS * 32, 0, c->stream>>>(in, out, c->W, c->H, ncx, nbands);
-        return;
+        return cudaGetLastError();
     }
     dim3 blk(MED_WARPS * 32), grd((c->W + MED_WARPS * MED_COLS - 1) / (MED_WARPS * MED_COLS), (c->H + MED_ROWS - 1) / MED_ROWS, B);
     k_median3<<<grd, blk, 0, c->stream>>>(in, out, c->W, c->H);
+    return cudaGetLastError();
 }
 
-void launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff)
+cudaError_t launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff)
 {
     const int W = c->W, H = c->H;
     const size_t n = (size_t)B * W * H;
-    cudaMemsetAsync(c->sizes, 0, n * sizeof(int), c->stream);
+    MVSV_TRY(cudaMemsetAsync(c->sizes, 0, n * sizeof(int), c->stream));
     const int nrows = B * H;
     { KernelTimer kt(c, KID_CCL_ROWS); k_ccl_rows<<<(nrows * 32 + 127) / 128, 128, 0, c->stream>>>(img, c->labels, W, nrows, newVal, maxDiff); }
     dim3 blk(128), grd((W + 127) / 128, (H + CCL_ROWS - 1) / CCL_ROWS, B);
@@ -571,21 +577,24 @@ void launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int ne
     }
     { KernelTimer kt(c, KID_CCL_FLATTEN); k_ccl_flatten<<<grd, blk, 0, c->stream>>>(img, c->labels, c->sizes, W, H, newVal, maxDiff); }
     { KernelTimer kt(c, KID_CCL_APPLY); k_ccl_apply<<<(unsigned)((n + 2047) / 2048), 256, 0, c->stream>>>(img, out, c->labels, c->sizes, n, newVal, maxSize); }
+    return cudaGetLastError();
 }
 
-void launch_xyz(mvsv_ctx* c, int B)
+cudaError_t launch_xyz(mvsv_ctx* c, int B)
 {
     QMat Q;
     for (int i = 0; i < 16; ++i) Q.q[i] = (double)c->Q[i];
     const size_t npx = (size_t)B * c->H * c->W;
     KernelTimer kt(c, KID_XYZ);
-    k_xyz<<<(unsigned)((npx / 4 + 256) / 256), 256, 0, c->stream>>>(c->disp, c->xyz, c->W, c->H, npx, Q);
+    k_xyz<<<(unsigned)((npx / 4 + 256) / 256), 256, 0, c->stream>>>(io(c).disp, io(c).xyz, c->W, c->H, npx, Q);
+    return cudaGetLastError();
 }
 
-void launch_means(mvsv_ctx* c, int B)
+cudaError_t launch_means(mvsv_ctx* c, int B)
 {
-    if (c->nrois <= 0) return;
+    if (c->nrois <= 0) return cudaSuccess;
     dim3 grd((c->nrois + MEANS_WARPS * 4 - 1) / (MEANS_WARPS * 4), B);
     KernelTimer kt(c, KID_MEANS);
-    k_means<<<grd, MEANS_WARPS * 32, 0, c->stream>>>(c->disp, c->rois, c->means, c->W, c->H, c->nrois);
+    k_means<<<grd, MEANS_WARPS * 32, 0, c->stream>>>(io(c).disp, c->rois, io(c).means, c->W, c->H, c->nrois);
+    return cudaGetLastError();
 }

@@ -37,13 +37,28 @@ extern const char* const kKernelNames[KID_COUNT];
 
 struct ProfBracket { int kid; cudaEvent_t a, b; };
 
+// I/O slot (mvsv_set_io_slots): the buffers a compute call reads its inputs into and leaves its results in.  They
+// exist once or twice; with two, the host->device copy of the next batch and the device->host copy of the previous
+// one overlap the kernels of the current batch inside ONE engine (one set of cost volumes).  The slot is the only
+// owner of these buffers; the launchers reach the slot of the compute in progress through io(c).
+struct IoSlot {
+    uint8_t* rect[2] = {nullptr, nullptr};    // [B][H][pitch]
+    uint8_t* raw[2] = {nullptr, nullptr};     // [B][fh][raw_pitch], once rectification maps are installed
+    int16_t* disp = nullptr;                  // final disparities [B][H][W]
+    float* xyz = nullptr;                     // [B][H][W][3], allocated by the first compute with MVSV_STAGE_XYZ
+    float* means = nullptr;                   // [B][nrois], once mean-disparity ROIs are set
+    cudaEvent_t done = nullptr;               // all kernels of the slot's last compute have finished
+    int B = 0;                                // frames of the slot's last compute; 0: it holds no results
+    unsigned stages = 0;
+};
+
 struct mvsv_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
-    // host->device input copies run on their own stream so that they overlap kernels of another engine that
-    // mvsv_order_after() has placed in front of this engine's kernels
+    // host->device input copies run on their own stream so that they overlap the kernels of the other I/O slot's
+    // compute
     cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_h2d = nullptr, ev_done = nullptr, ev_order = nullptr;
+    cudaEvent_t ev_h2d = nullptr, ev_done = nullptr;
     // second kernel stream: the first row scan of one chunk of frames runs beside the cost kernel of the next chunk
     // (sgbm.cu, launch_sgbm_g); joined back into `stream` before the sweep
     cudaStream_t aux_stream = nullptr;
@@ -52,8 +67,6 @@ struct mvsv_ctx {
     int fw = 0, fh = 0;          // raw frame
     int W = 0, H = 0;            // rectified/cropped pair
     int maxB = 0;
-    int lastB = 0;
-    unsigned last_stages = 0;
     unsigned long long launches = 0;
     unsigned debug_flags = 0;   // bit0: h2 pass stores the final S volume (test hook); bit1: never use the byte form of S;
                                 // bits 8..15: sweep strips; bits 16..23: frames per chunk of the vsum / h1 overlap (mvsv.h)
@@ -68,7 +81,6 @@ struct mvsv_ctx {
     bool has_maps[2] = {false, false};
     int roi[4] = {0, 0, 0, 0};
     int2* map_xy[2] = {nullptr, nullptr};     // (ix, iy) = rint(map*32), saturated int32
-    uint8_t* raw[2] = {nullptr, nullptr};     // [B][fh][raw_pitch]
     size_t raw_pitch = 0;
     // cv::resize(.., factor, factor) after the crop (Stereosystem::getRectifiedImagepair(sip, factor),
     // reference src/Stereosystem.cpp:279-315); off when resize_factor == 0
@@ -77,24 +89,10 @@ struct mvsv_ctx {
     uint8_t* crop[2] = {nullptr, nullptr};    // [B][roi_h][crop_pitch]: remap output when a resize follows
     size_t crop_pitch = 0;
 
-    uint8_t* rect[2] = {nullptr, nullptr};    // [B][H][pitch] -- of the current I/O slot (see below)
-    size_t pitch = 0;
+    size_t pitch = 0;                         // row pitch of the rectified images
 
-    // I/O slots (mvsv_set_io_slots): the buffers a compute call reads its inputs into and leaves its results in exist
-    // once or twice; with two, the host->device copy of the next batch and the device->host copy of the previous
-    // one overlap the kernels of the current batch inside ONE engine (one set of cost volumes).  rect / raw / disp /
-    // xyz / means above and below always alias the slot of the compute in progress.
-    int nslots = 1, cur = 0;
-    struct IoSlot {
-        uint8_t* rect[2] = {nullptr, nullptr};
-        uint8_t* raw[2] = {nullptr, nullptr};
-        int16_t* disp = nullptr;
-        float* xyz = nullptr;
-        float* means = nullptr;
-        cudaEvent_t done = nullptr;           // all kernels of the slot's last compute have finished
-        int B = 0;
-        unsigned stages = 0;
-    } slot[2];
+    int nslots = 1, cur = 0;                  // I/O slots in use; the slot of the last (or current) compute
+    IoSlot slot[2];
     cudaStream_t dl_stream = nullptr;         // device->host result copies
 
     bool has_sgbm = false, has_bm = false;
@@ -116,7 +114,6 @@ struct mvsv_ctx {
     int* d2 = nullptr;                        // [B][H][W] (disp2cost<<16 | disp2)
     int16_t* disp_raw = nullptr;              // [B][H][W]
     int16_t* disp_med = nullptr;              // [B][H][W]
-    int16_t* disp = nullptr;                  // final [B][H][W]
     int* labels = nullptr;                    // [B][H][W]
     int* sizes = nullptr;                     // [B][H][W]
 
@@ -127,12 +124,13 @@ struct mvsv_ctx {
 
     bool has_Q = false;
     float Q[16];
-    float* xyz = nullptr;                     // [B][H][W][3]
     int nrois = 0;
     int* rois = nullptr;                      // device [n][4]
-    float* means = nullptr;                   // device [B][n]
     int* minmax = nullptr;                    // device [B][2]
 };
+
+// the I/O slot of the compute in progress (or of the last one)
+inline IoSlot& io(mvsv_ctx* c) { return c->slot[c->cur]; }
 
 // RAII bracket: records CUDA events on the ctx stream around one kernel launch when profiling is on.
 struct KernelTimer {
@@ -155,23 +153,31 @@ struct KernelTimer {
 };
 
 // ---- kernel launchers (launch counting happens in KernelTimer) ------------------------------------------
-void launch_remap(mvsv_ctx* c, int cam, int B);
-void launch_resize(mvsv_ctx* c, int cam, int B);
+// Each returns the first error of its launches and of the CUDA calls it makes on the way; MVSV_TRY passes one on.
+#define MVSV_TRY(call)                                                                          \
+    do {                                                                                        \
+        cudaError_t e_ = (call);                                                                \
+        if (e_ != cudaSuccess) return e_;                                                       \
+    } while (0)
+// Sets a kernel's cudaFuncAttributeMaxDynamicSharedMemorySize on the current device when it differs from the value set
+// there before (function attributes are per device; engines on several devices and threads share this state).
+cudaError_t smem_limit(const void* kernel, int bytes);
+cudaError_t launch_remap(mvsv_ctx* c, int cam, int B);
+cudaError_t launch_resize(mvsv_ctx* c, int cam, int B);
 // inverse of P[:, :3]*R, camera matrix and distortion of one camera (cv::initUndistortRectifyMap's inputs)
 struct RectifyCoef { double iR[9]; double k1, k2, p1, p2, k3; double fx, fy, cx, cy; };
-void launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q);
-void launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
-void launch_sgbm(mvsv_ctx* c, int B);
-void launch_bm(mvsv_ctx* c, int B);
+cudaError_t launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q);
+cudaError_t launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
+cudaError_t launch_sgbm(mvsv_ctx* c, int B);
+cudaError_t launch_bm(mvsv_ctx* c, int B);
 size_t tm_smem_bytes(int W, int k);
 int tm_max_width();
 cudaError_t launch_tm(mvsv_ctx* c, int B, int k, uint8_t* out, size_t opitch);
-void launch_xyz(mvsv_ctx* c, int B);
-void launch_means(mvsv_ctx* c, int B);
-void launch_minmax(mvsv_ctx* c, int B);
-void launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B);
-void launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
-cudaError_t sgbm_configure_kernels();
+cudaError_t launch_xyz(mvsv_ctx* c, int B);
+cudaError_t launch_means(mvsv_ctx* c, int B);
+cudaError_t launch_minmax(mvsv_ctx* c, int B);
+cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B);
+cudaError_t launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
 // fused previous-row sweep (csrc/sweep.cu): strip decomposition of a batch, scratch sizes, launch
 struct SweepPlan { int NS = 0, NF = 0, Mmax = 0, threads = 0, G = 0, NR = 0; size_t smem = 0; };
 void sweep_layout(int D, int* G, int* NR);

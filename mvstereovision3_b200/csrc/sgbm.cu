@@ -800,7 +800,7 @@ size_t vsum_smem_bytes(int bs, bool r8)
 }
 
 template <int G, bool PAD>
-void launch_sgbm_g(mvsv_ctx* c, int B)
+cudaError_t launch_sgbm_g(mvsv_ctx* c, int B)
 {
     const SgbmNorm& n = c->sg;
     cudaStream_t st = c->stream;
@@ -809,10 +809,10 @@ void launch_sgbm_g(mvsv_ctx* c, int B)
         const int ncx = (c->W + PF_COLS - 1) / PF_COLS, nbands = (c->H + PF_ROWS - 1) / PF_ROWS;
         dim3 blk(PF_WARPS * 32), grd((ncx * nbands + PF_WARPS - 1) / PF_WARPS, 2 * B);
         KernelTimer kt(c, KID_SGBM_PREFILTER);
-        k_sgbm_prefilter<<<grd, blk, 0, st>>>(c->rect[0], c->rect[1], c->pitch, c->W, c->H, n.ftzero, c->recL, c->plR,
+        k_sgbm_prefilter<<<grd, blk, 0, st>>>(io(c).rect[0], io(c).rect[1], c->pitch, c->W, c->H, n.ftzero, c->recL, c->plR,
                                               planeStrideR, c->vsRP, c->vsJOFF, ncx, nbands);
     }
-    std::function<void(int, int)> launch_vsum;
+    std::function<cudaError_t(int, int)> launch_vsum;
     int vsum_gx = 1;                                  // column strips (CTAs) of the cost kernel per frame
     auto make_vsum = [&](auto wideTag) {
         constexpr bool WIDE = decltype(wideTag)::value;
@@ -830,18 +830,16 @@ void launch_sgbm_g(mvsv_ctx* c, int B)
         int bands = 1;
         while (bands < 8 && (long long)gx * B * (bands * 2) <= c->num_sms && c->H / (bands * 2) >= 4 * bs) bands *= 2;
         a.bandRows = (c->H + bands - 1) / bands;
+        const auto kern = bands > 1 ? (r8 ? k_sgbm_vsum<G, true, true, WIDE> : k_sgbm_vsum<G, false, true, WIDE>)
+                                    : (r8 ? k_sgbm_vsum<G, true, false, WIDE> : k_sgbm_vsum<G, false, false, WIDE>);
         launch_vsum = [=](int f0, int nb) {
+            MVSV_TRY(smem_limit((const void*)kern, 200 * 1024));
             VsArgs v = a;
             v.recL += (size_t)f0 * c->H * c->W; v.plR += (size_t)f0 * c->H * c->vsRP; v.VS += (size_t)f0 * c->H * n.W1 * n.Dp;
             dim3 grd(gx, nb, (c->H + v.bandRows - 1) / v.bandRows);
             KernelTimer kt(c, KID_SGBM_VSUM);
-            if (bands > 1) {
-                if (r8) k_sgbm_vsum<G, true, true, WIDE><<<grd, GE::THREADS, smem, st>>>(v);
-                else k_sgbm_vsum<G, false, true, WIDE><<<grd, GE::THREADS, smem, st>>>(v);
-            } else {
-                if (r8) k_sgbm_vsum<G, true, false, WIDE><<<grd, GE::THREADS, smem, st>>>(v);
-                else k_sgbm_vsum<G, false, false, WIDE><<<grd, GE::THREADS, smem, st>>>(v);
-            }
+            kern<<<grd, GE::THREADS, smem, st>>>(v);
+            return cudaSuccess;
         };
     };
     if constexpr (G == 32) {
@@ -880,6 +878,8 @@ void launch_sgbm_g(mvsv_ctx* c, int B)
     // cfg 2, frames per chunk 13 / 15 / 19 / 26 / all: 12.26 / 12.13 / 11.73 / 11.93 / 12.29; cfg 4, 2 / 3 / 4 / 5 / all:
     // 35.9 / 36.3 / 36.0 / 37.0 / 37.2; cfg 5, 1 / 2 / 3 / all: 78.3 / 74.3 / 76.0 / 76.2; a higher stream priority for the
     // scan: slower).
+    const auto h1 = s8 ? k_sgbm_h1<G, PAD, true> : k_sgbm_h1<G, PAD, false>;
+    MVSV_TRY(smem_limit((const void*)h1, 200 * 1024));
     auto launch_h1 = [&](int f0, int nb, cudaStream_t on) {
         AggArgs h = a;
         const size_t off = (size_t)f0 * c->H * n.W1 * n.Dp;
@@ -887,8 +887,7 @@ void launch_sgbm_g(mvsv_ctx* c, int B)
         const unsigned blocks = (unsigned)(((long long)nb * c->H * G + TPB - 1) / TPB);
         KernelTimer kt(c, KID_SGBM_H1, on);
         const size_t sm = (size_t)(2 * n.SW2 + 1 + H1_PFD) * TPB * 16;
-        if (s8) k_sgbm_h1<G, PAD, true><<<blocks, TPB, sm, on>>>(h);
-        else k_sgbm_h1<G, PAD, false><<<blocks, TPB, sm, on>>>(h);
+        h1<<<blocks, TPB, sm, on>>>(h);
     };
     int fpc = std::max((B + 6) / 7, (int)(0.9 * c->num_sms / vsum_gx + 0.999));   // frames per chunk
     if ((c->debug_flags >> 16) & 0xffu) fpc = (int)((c->debug_flags >> 16) & 0xffu);     // test hook: frames per chunk
@@ -898,82 +897,37 @@ void launch_sgbm_g(mvsv_ctx* c, int B)
     static const bool serialEnv = [] { const char* e = getenv("MVSV_SERIAL"); return e && atoi(e) != 0; }();
     const int nchunks = (c->prof || serialEnv) ? 1 : std::min((B + fpc - 1) / fpc, (int)mvsv_ctx::kMaxChunks);
     if (nchunks <= 1) {
-        launch_vsum(0, B);
+        MVSV_TRY(launch_vsum(0, B));
         launch_h1(0, B, st);
     } else {
         for (int i = 0; i < nchunks; ++i) {
             const int f0 = i * fpc, f1 = (i + 1 == nchunks) ? B : f0 + fpc;
-            launch_vsum(f0, f1 - f0);
-            cudaEventRecord(c->ev_chunk[i], st);
-            cudaStreamWaitEvent(c->aux_stream, c->ev_chunk[i], 0);
+            MVSV_TRY(launch_vsum(f0, f1 - f0));
+            MVSV_TRY(cudaEventRecord(c->ev_chunk[i], st));
+            MVSV_TRY(cudaStreamWaitEvent(c->aux_stream, c->ev_chunk[i], 0));
             launch_h1(f0, f1 - f0, c->aux_stream);
         }
-        cudaEventRecord(c->ev_join, c->aux_stream);
-        cudaStreamWaitEvent(st, c->ev_join, 0);
+        MVSV_TRY(cudaEventRecord(c->ev_join, c->aux_stream));
+        MVSV_TRY(cudaStreamWaitEvent(st, c->ev_join, 0));
     }
     auto vdirs = [&](int bottomUp) {
-        if (plan.NS > 0) {
-            launch_sweep(c, B, plan, bottomUp, s8);
-        } else {
-            { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, -1, bottomUp); }
-            { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, 0, bottomUp); }
-            { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, +1, bottomUp); }
-        }
+        if (plan.NS > 0) return launch_sweep(c, B, plan, bottomUp, s8);
+        { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, -1, bottomUp); }
+        { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, 0, bottomUp); }
+        { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, +1, bottomUp); }
+        return cudaSuccess;
     };
-    vdirs(0);
-    if (n.mode == 1) vdirs(1);
+    MVSV_TRY(vdirs(0));
+    if (n.mode == 1) MVSV_TRY(vdirs(1));
     {
         KernelTimer kt(c, KID_SGBM_H2_WTA);
         if (s8) k_sgbm_h2_wta<G, PAD, true><<<rowBlocks, TPB, 0, st>>>(a);
         else k_sgbm_h2_wta<G, PAD, false><<<rowBlocks, TPB, 0, st>>>(a);
     }
-}
-
-template <int G>
-cudaError_t cfg_vsum()
-{
-    cudaError_t e = cudaFuncSetAttribute(k_sgbm_vsum<G, true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_sgbm_vsum<G, false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_sgbm_vsum<G, true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_sgbm_vsum<G, false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    if constexpr (G == 32) {
-        e = cudaFuncSetAttribute(k_sgbm_vsum<G, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_sgbm_vsum<G, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_sgbm_vsum<G, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_sgbm_vsum<G, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e != cudaSuccess) return e;
-    }
-    e = cudaFuncSetAttribute(k_sgbm_h1<G, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_sgbm_h1<G, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_sgbm_h1<G, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_sgbm_h1<G, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    if (e != cudaSuccess) return e;
-    return cudaSuccess;
+    return cudaGetLastError();
 }
 
 }  // namespace
-
-cudaError_t sgbm_configure_kernels()
-{
-    cudaError_t e;
-    if ((e = cfg_vsum<1>()) != cudaSuccess) return e;
-    if ((e = cfg_vsum<2>()) != cudaSuccess) return e;
-    if ((e = cfg_vsum<4>()) != cudaSuccess) return e;
-    if ((e = cfg_vsum<8>()) != cudaSuccess) return e;
-    if ((e = cfg_vsum<16>()) != cudaSuccess) return e;
-    if ((e = cfg_vsum<32>()) != cudaSuccess) return e;
-    return cudaSuccess;
-}
 
 // Strips per frame the fused previous-row sweep uses for a full batch (reported by mvsv_get_info);
 // 0 = it cannot run (volume stride differs from the sweep's lane layout, or forced off): independent passes.
@@ -1004,7 +958,7 @@ void sgbm_plane_geometry(const SgbmNorm& n, int W, int* NV, int* RP, int* JOFF)
     *NV = nv; *JOFF = joff; *RP = (joff + W + nv * 8 + 16 + 7) / 8 * 8;
 }
 
-void launch_sgbm(mvsv_ctx* c, int B)
+cudaError_t launch_sgbm(mvsv_ctx* c, int B)
 {
     const SgbmNorm& n = c->sg;
     const size_t npx = (size_t)B * c->H * c->W;
@@ -1013,19 +967,20 @@ void launch_sgbm(mvsv_ctx* c, int B)
         k_fill_i16<<<(unsigned)((npx + 255) / 256), 256, 0, c->stream>>>(c->disp_raw, npx, (int16_t)n.INV);
     } else {
         const bool pad = n.D != 8 * n.G;             // some lanes of a pixel's lane group hold no disparity
+        cudaError_t e;
         switch (n.G) {
-            case 1: if (pad) launch_sgbm_g<1, true>(c, B); else launch_sgbm_g<1, false>(c, B); break;
-            case 2: if (pad) launch_sgbm_g<2, true>(c, B); else launch_sgbm_g<2, false>(c, B); break;
-            case 4: if (pad) launch_sgbm_g<4, true>(c, B); else launch_sgbm_g<4, false>(c, B); break;
-            case 8: if (pad) launch_sgbm_g<8, true>(c, B); else launch_sgbm_g<8, false>(c, B); break;
-            case 16: if (pad) launch_sgbm_g<16, true>(c, B); else launch_sgbm_g<16, false>(c, B); break;
-            default: if (pad) launch_sgbm_g<32, true>(c, B); else launch_sgbm_g<32, false>(c, B); break;
+            case 1: e = pad ? launch_sgbm_g<1, true>(c, B) : launch_sgbm_g<1, false>(c, B); break;
+            case 2: e = pad ? launch_sgbm_g<2, true>(c, B) : launch_sgbm_g<2, false>(c, B); break;
+            case 4: e = pad ? launch_sgbm_g<4, true>(c, B) : launch_sgbm_g<4, false>(c, B); break;
+            case 8: e = pad ? launch_sgbm_g<8, true>(c, B) : launch_sgbm_g<8, false>(c, B); break;
+            case 16: e = pad ? launch_sgbm_g<16, true>(c, B) : launch_sgbm_g<16, false>(c, B); break;
+            default: e = pad ? launch_sgbm_g<32, true>(c, B) : launch_sgbm_g<32, false>(c, B); break;
         }
+        MVSV_TRY(e);
     }
     if (n.speckleWin > 0) {
-        launch_median(c, c->disp_raw, c->disp_med, B);
-        launch_speckle(c, c->disp_med, c->disp, B, n.INV, n.speckleWin, 16 * n.speckleRange);
-    } else {
-        launch_median(c, c->disp_raw, c->disp, B);
+        MVSV_TRY(launch_median(c, c->disp_raw, c->disp_med, B));
+        return launch_speckle(c, c->disp_med, io(c).disp, B, n.INV, n.speckleWin, 16 * n.speckleRange);
     }
+    return launch_median(c, c->disp_raw, io(c).disp, B);
 }

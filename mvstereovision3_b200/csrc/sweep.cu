@@ -541,15 +541,7 @@ size_t sweep_smem_bytes(int NR, int G, int Mmax, int nthr)
 template <int NR, int G, bool PAD, int MODE, bool DSM>
 cudaError_t launch_one(const SweepArgs& a, int nthr, size_t smem, cudaStream_t st, bool* fits)
 {
-    // function attributes are per device: a process may drive several GPUs with one engine each
-    static bool configured[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(k_sweep<NR, G, PAD, MODE, DSM>, cudaFuncAttributeMaxDynamicSharedMemorySize, SW_SMEM_LIMIT);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) configured[dev] = true;
-    }
+    MVSV_TRY(smem_limit((const void*)k_sweep<NR, G, PAD, MODE, DSM>, SW_SMEM_LIMIT));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(a.NS * a.NF, 1, 1); cfg.blockDim = dim3(nthr, 1, 1); cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute at[1];
@@ -558,7 +550,7 @@ cudaError_t launch_one(const SweepArgs& a, int nthr, size_t smem, cudaStream_t s
         at[0].val.clusterDim.x = a.NS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
         int nmax = 0;
-        if (cudaOccupancyMaxActiveClusters(&nmax, k_sweep<NR, G, PAD, MODE, DSM>, &cfg) != cudaSuccess) { cudaGetLastError(); nmax = 0; }
+        MVSV_TRY(cudaOccupancyMaxActiveClusters(&nmax, k_sweep<NR, G, PAD, MODE, DSM>, &cfg));
         *fits = nmax >= a.NF;
         if (!*fits) return cudaSuccess;
     } else {

@@ -112,10 +112,9 @@ int tm_max_width() { return TM_THREADS * TM_MAXC; }
 cudaError_t launch_tm(mvsv_ctx* c, int B, int k, uint8_t* out, size_t opitch)
 {
     const size_t smem = tm_smem_bytes(c->W, k);
-    cudaError_t e = cudaFuncSetAttribute(k_tm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
+    MVSV_TRY(smem_limit((const void*)k_tm, (int)smem));
     dim3 grd(c->H - k, B);
     KernelTimer kt(c, KID_TM);
-    k_tm<<<grd, TM_THREADS, smem, c->stream>>>(c->rect[0], c->rect[1], c->pitch, c->W, c->H, k, out, opitch);
+    k_tm<<<grd, TM_THREADS, smem, c->stream>>>(io(c).rect[0], io(c).rect[1], c->pitch, c->W, c->H, k, out, opitch);
     return cudaGetLastError();
 }

@@ -441,34 +441,6 @@ def test_fused_sweep_degenerate_strips(oracle, H, nc):
         check("H=%d nc=%d" % (H, nc), e.download(1)["disp"][0], oracle.sgbm(l, r, p))
 
 
-def test_pipelined_engines_order_after(oracle):
-    """two engines submitting alternately with mvsv_order_after (the e2e pipeline of bench.py): same bits as one"""
-    p = cases.sgbm_params(minDisp=1, numDisp=32, blockSize=5, P1=20, P2=90, uniquenessRatio=5, speckleWindowSize=30, speckleRange=2)
-    H, W, B = 60, 200, 6
-    batches = []
-    for k in range(5):
-        ls, rs = zip(*[synth.random_pair(H, W, seed=100 * k + b) for b in range(B)])
-        batches.append((np.stack(ls), np.stack(rs)))
-    want = [np.stack([oracle.sgbm(L[b], R[b], p) for b in range(B)]) for L, R in batches]
-    engines = [api.Engine(W, H, max_batch=B) for _ in range(2)]
-    try:
-        for e in engines:
-            e.set_sgbm_params(**gpu_params(p))
-        got = [None] * len(batches)
-        engines[0].compute(batches[0][0], batches[0][1], api.STAGE_SGBM)
-        for k in range(1, len(batches)):
-            engines[k & 1].order_after(engines[(k - 1) & 1])
-            engines[k & 1].compute(batches[k][0], batches[k][1], api.STAGE_SGBM)
-            got[k - 1] = engines[(k - 1) & 1].download(B)["disp"]
-        got[-1] = engines[(len(batches) - 1) & 1].download(B)["disp"]
-        engines[0].order_after(engines[0])             # self-ordering is a no-op
-    finally:
-        for e in engines:
-            e.close()
-    for k in range(len(batches)):
-        check("batch %d" % k, got[k], want[k])
-
-
 def test_io_slots_pipeline_in_one_engine(oracle):
     """mvsv_set_io_slots(2): compute k+1 is submitted before the results of compute k are fetched (age 1); the
     copies overlap the kernels inside ONE engine and every batch still equals the oracle (bench.py's e2e loop)."""
@@ -503,6 +475,81 @@ def test_io_slots_pipeline_in_one_engine(oracle):
         for b in range(B):
             m = np.array([oracle.mean(want[k][b], roi) for roi in [(40, 5, 50, 40), (100, 10, 20, 20)]], np.float32)
             np.testing.assert_array_equal(means[k][b], m)
+
+
+def test_rejected_compute_keeps_the_last_results(oracle):
+    """Two I/O slots, three computes, the third rejected (row stride below the width): the rejected call takes no slot,
+    so download() still returns the second batch and age 1 the first, never the frames of an older compute."""
+    p = cases.sgbm_params(numDisp=16, blockSize=5)
+    H, W, B = 40, 96, 2
+    batches = []
+    for k in range(3):
+        ls, rs = zip(*[synth.random_pair(H, W, seed=500 + 10 * k + b) for b in range(B)])
+        batches.append((np.stack(ls), np.stack(rs)))
+    with api.Engine(W, H, max_batch=B) as e:
+        e.set_sgbm_params(**gpu_params(p))
+        e.set_io_slots(2)
+        for L, R in batches[:2]:
+            e.compute(L, R, api.STAGE_SGBM)
+        L, R = batches[2]
+        rc = e._lib.mvsv_compute(e._ctx, L.ctypes.data, W - 1, R.ctypes.data, W, L.strides[0], B, api.STAGE_SGBM)
+        assert rc == -1, rc                                  # MVSV_ERR_INVALID
+        got = e.download(B)["disp"], e.download(B, age=1)["disp"]
+    for b in range(B):
+        check("second batch/%d" % b, got[0][b], oracle.sgbm(batches[1][0][b], batches[1][1][b], p))
+        check("first batch/%d" % b, got[1][b], oracle.sgbm(batches[0][0][b], batches[0][1][b], p))
+
+
+def test_io_slots_with_rectification_and_resize(oracle):
+    """Two I/O slots with the cfg-3 stage set (RECTIFY | SGBM | XYZ | MEANS), maps and ROIs installed before
+    set_io_slots(2) as bench.py does, then a geometry change (set_resize) while both slots are live: the change drops
+    the results the slots held, and every batch, fetched one call late, equals the oracle."""
+    H, W, B = 96, 140, 2
+    mx, my = cases.warp_maps(H, W, 2)
+    roi = (4, 2, W - 20, H - 10)
+    p = cases.sgbm_params(numDisp=16, blockSize=5)
+    stages = api.STAGE_RECTIFY | api.STAGE_SGBM | api.STAGE_XYZ | api.STAGE_MEANS
+    raws = []
+    for k in range(6):
+        ls, rs = zip(*[synth.random_pair(H, W, seed=600 + 10 * k + b) for b in range(B)])
+        raws.append((np.stack(ls), np.stack(rs)))
+    with api.Engine(W, H, max_batch=B) as e:
+        e.upload_rectify_maps(0, mx, my, roi)
+        e.upload_rectify_maps(1, mx, my, roi)
+        e.set_sgbm_params(**gpu_params(p))
+        e.set_Q(cases.Q_REFERENCE)
+        for factor, batches in ((0, raws[:3]), (0.5, raws[3:])):
+            if factor:
+                e.set_resize(factor)
+                with pytest.raises(api.MvsvError) as ex:
+                    e.download(B, age=1)
+                assert ex.value.code == -4
+            w, h = e.info.width, e.info.height
+            rois = [(w // 2, h // 4, w // 3, h // 2), (2, 2, 10, 10)]
+            e.set_mean_rois(rois)
+            if not factor:
+                e.set_io_slots(2)
+            got = []
+            e.compute(batches[0][0], batches[0][1], stages)
+            for L, R in batches[1:]:
+                e.compute(L, R, stages)
+                got.append(e.download(B, rect=True, xyz=True, means=True, age=1))
+            got.append(e.download(B, rect=True, xyz=True, means=True))
+            for k, (L, R) in enumerate(batches):
+                for b in range(B):
+                    rl, rr = oracle.remap(L[b], mx, my, roi), oracle.remap(R[b], mx, my, roi)
+                    if factor:
+                        rl, rr = oracle.resize(rl, factor), oracle.resize(rr, factor)
+                    tag = "x%s/batch %d/%d" % (factor, k, b)
+                    check(tag + "/rectL", got[k]["rectL"][b], rl)
+                    check(tag + "/rectR", got[k]["rectR"][b], rr)
+                    disp = oracle.sgbm(rl, rr, p)
+                    check(tag + "/disp", got[k]["disp"][b], disp)
+                    xyz, valid = oracle.reproject(disp, cases.Q_REFERENCE)
+                    v = valid.astype(bool)
+                    np.testing.assert_allclose(got[k]["xyz"][b][v], xyz[v], rtol=1e-5)
+                    want = np.array([oracle.mean(disp, r_) for r_ in rois], np.float32)
+                    np.testing.assert_array_equal(got[k]["means"][b], want)
 
 
 def test_mean_rois_dropped_on_geometry_change(oracle):
