@@ -83,6 +83,17 @@ const char* mvsv_last_error(const mvsv_ctx* ctx); /* ctx may be NULL: error of t
 int mvsv_set_sgbm_params(mvsv_ctx* ctx, const mvsv_sgbm_params* p);
 /* cv::StereoBM::create(numDisp, blockSize) + setters (trgt/disparityTest.cpp:268, configs/bm.yml). */
 int mvsv_set_bm_params(mvsv_ctx* ctx, const mvsv_bm_params* p);
+/* The post-filters of cv::StereoBM, in cv2's own units (cv::StereoBM::setDisp12MaxDiff / setSpeckleWindowSize /
+ * setSpeckleRange):
+ *   disp12MaxDiff     >= 0: left-right check, a pixel is FILTERED (-16) when the disparities seen from the right
+ *                     image at both of its integer neighbours differ from it by more than disp12MaxDiff pixels;
+ *                     0 is the strictest check, < 0 switches it off.  Needs width <= 4096.
+ *   speckleWindowSize > 0: cv::filterSpeckles(disp, -16, speckleWindowSize, speckleRange) after the check;
+ *                     speckleRange is compared with the x16 fixed-point values as given (StereoSGBM multiplies it
+ *                     by 16, StereoBM does not).  0 switches it off.
+ * Defaults -1 / 0 / 0 (cv::StereoBM's): the engine computes what it computes without this call.  The setting is kept
+ * across mvsv_set_bm_params and geometry changes.  Rejected: speckleWindowSize < 0, speckleRange < 0 with a window. */
+int mvsv_set_bm_filters(mvsv_ctx* ctx, int disp12MaxDiff, int speckleWindowSize, int speckleRange);
 
 /* Replaces Stereosystem::initRectification's map state (src/Stereosystem.cpp:214-220): float CV_32FC1
  * maps of one camera (cam 0 = left, 1 = right), frame-sized, plus mDisplayROI.  The maps are converted once
@@ -189,7 +200,7 @@ int mvsv_host_free(void* p);
 
 /* Test hooks: read an internal device buffer of the last compute into host memory.
  * which: 0 = cost volume C, 1 = aggregated S (before the final right-to-left pass), 2 = raw disparity
- * (after LR check, before median), 3 = vertical-sum volume, 4 = disparity after median (before speckle),
+ * (after LR check, before median; StereoBM with a speckle window: after the LR check, before speckle), 3 = vertical-sum volume, 4 = disparity after median (before speckle),
  * 5 = BM prefiltered left, 6 = BM prefiltered right, 7 / 8 = fixed-point rectification map of camera 0 / 1
  * (roi_h x roi_w int32 pairs: x*32, y*32 rounded).  Returns bytes written or a negative error. */
 /* bit 0: keep the complete aggregated S volume (all paths) readable through mvsv_debug_read(which=1).

@@ -79,7 +79,13 @@ public:
     Matcher& operator=(const Matcher&) = delete;
 
     void setSgbm(const mvsv_sgbm_params& p) { sg_ = p; have_sg_ = true; if (ctx_) applied_ = (mvsv_set_sgbm_params(ctx_, &sg_) == MVSV_OK); }
-    void setBm(const mvsv_bm_params& p) { bm_ = p; have_bm_ = true; if (ctx_) applied_bm_ = (mvsv_set_bm_params(ctx_, &bm_) == MVSV_OK); }
+    void setBm(const mvsv_bm_params& p) { bm_ = p; have_bm_ = true; if (ctx_) applied_bm_ = applyBm() == MVSV_OK; }
+    // cv::StereoBM::setDisp12MaxDiff / setSpeckleWindowSize / setSpeckleRange (mvsv_set_bm_filters); default -1 / 0 / 0
+    void setBmFilters(int disp12MaxDiff, int speckleWindowSize, int speckleRange)
+    {
+        bmf_[0] = disp12MaxDiff; bmf_[1] = speckleWindowSize; bmf_[2] = speckleRange;
+        if (ctx_ && have_bm_) applied_bm_ = applyBm() == MVSV_OK;
+    }
     const char* lastError() const { return err_.empty() ? mvsv_last_error(ctx_) : err_.c_str(); }
     mvsv_ctx* ctx() { return ctx_; }
 
@@ -103,7 +109,7 @@ public:
         }
         if (stage == MVSV_STAGE_BM && !applied_bm_) {
             if (!have_bm_) { err_ = "BM parameters not set"; return MVSV_ERR_STATE; }
-            if ((rc = mvsv_set_bm_params(ctx_, &bm_)) != MVSV_OK) return rc;
+            if ((rc = applyBm()) != MVSV_OK) return rc;
             applied_bm_ = true;
         }
         if ((rc = mvsv_compute(ctx_, left.data, left.step, right.data, right.step, 0, 1, stage)) != MVSV_OK) return rc;
@@ -136,11 +142,18 @@ public:
     }
 
 private:
+    int applyBm()
+    {
+        const int rc = mvsv_set_bm_params(ctx_, &bm_);
+        return rc != MVSV_OK ? rc : mvsv_set_bm_filters(ctx_, bmf_[0], bmf_[1], bmf_[2]);
+    }
+
     int device_;
     mvsv_ctx* ctx_ = nullptr;
     int w_ = 0, h_ = 0;
     mvsv_sgbm_params sg_{};
     mvsv_bm_params bm_{};
+    int bmf_[3] = {-1, 0, 0};
     bool have_sg_ = false, have_bm_ = false, applied_ = false, applied_bm_ = false;
     std::string err_;
 };

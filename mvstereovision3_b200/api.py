@@ -20,6 +20,7 @@ ABI_SYMBOLS = (
     "mvsv_compute_device", "mvsv_tm", "mvsv_download", "mvsv_sync", "mvsv_get_info", "mvsv_stream", "mvsv_launch_count",
     "mvsv_host_alloc", "mvsv_host_free", "mvsv_debug_set_flags", "mvsv_debug_read",
     "mvsv_download_minmax", "mvsv_download_age", "mvsv_set_io_slots", "mvsv_timer_start", "mvsv_timer_stop", "mvsv_profile_enable", "mvsv_profile_read", "mvsv_kernel_name",
+    "mvsv_set_bm_filters",
 )
 
 
@@ -66,6 +67,7 @@ def load_library():
     lib.mvsv_last_error.restype = C.c_char_p
     lib.mvsv_set_sgbm_params.argtypes = [vp, C.POINTER(SgbmParams)]
     lib.mvsv_set_bm_params.argtypes = [vp, C.POINTER(BmParams)]
+    lib.mvsv_set_bm_filters.argtypes = [vp, ci, ci, ci]
     lib.mvsv_upload_rectify_maps.argtypes = [vp, ci, vp, vp, sz, ci, ci, ci, ci]
     lib.mvsv_set_rectification.argtypes = [vp, ci, vp, vp, ci, vp, vp, ci, ci, ci, ci]
     lib.mvsv_set_resize.argtypes = [vp, C.c_double]
@@ -188,6 +190,10 @@ class Engine:
     def set_bm_params(self, **kw):
         p = BmParams(**{k: int(v) for k, v in kw.items()})
         self._ck(self._lib.mvsv_set_bm_params(self._ctx, C.byref(p)))
+
+    def set_bm_filters(self, disp12MaxDiff=-1, speckleWindowSize=0, speckleRange=0):
+        """cv::StereoBM::setDisp12MaxDiff / setSpeckleWindowSize / setSpeckleRange, in cv2's units (include/mvsv.h)."""
+        self._ck(self._lib.mvsv_set_bm_filters(self._ctx, int(disp12MaxDiff), int(speckleWindowSize), int(speckleRange)))
 
     def upload_rectify_maps(self, cam, mapx, mapy, roi):
         mapx = np.ascontiguousarray(mapx, np.float32)
@@ -411,7 +417,8 @@ def loadSGBMParameters(filename, engine, para):
 def loadBMParameters(filename, engine, para):
     """configs/bm.yml has no loader in the reference (SURVEY.md section 2 row 4); this one reads its keys the
     way trgt/disparityTest.cpp drives cv::StereoBM (numDisp, blockSize + setters); preFilterSize is ignored by
-    PREFILTER_XSOBEL."""
+    PREFILTER_XSOBEL.  The optional keys disp12MaxDiff, speckleWindowSize and speckleRange, when present, set the
+    post-filters (cv::StereoBM's defaults -1 / 0 / 0 for the ones left out)."""
     try:
         fs = _read_flat_yaml(filename)
     except OSError:
@@ -421,6 +428,8 @@ def loadBMParameters(filename, engine, para):
     para.update(numDisp=fs["numDisp"], blockSize=fs["blockSize"], preFilterCap=fs.get("preFilterCap", 31),
                 textureThreshold=fs.get("textureThreshold", 10), uniquenessRatio=fs.get("uniquenessRatio", 15))
     engine.set_bm_params(**para)
+    if any(k in fs for k in ("disp12MaxDiff", "speckleWindowSize", "speckleRange")):
+        engine.set_bm_filters(fs.get("disp12MaxDiff", -1), fs.get("speckleWindowSize", 0), fs.get("speckleRange", 0))
     return True
 
 

@@ -11,7 +11,8 @@
 
 const char* const kKernelNames[KID_COUNT] = {
     "remap", "sgbm_prefilter", "sgbm_vsum", "sgbm_h1", "sgbm_vdir", "sgbm_td", "sgbm_h2_wta", "median3", "ccl_rows", "ccl_vmerge",
-    "ccl_flatten", "ccl_apply", "bm_prefilter", "bm_tex", "bm_colsum", "bm_wta", "xyz", "means", "fill", "minmax", "tm"};
+    "ccl_flatten", "ccl_apply", "bm_prefilter", "bm_tex", "bm_colsum", "bm_wta", "xyz", "means", "fill", "minmax", "tm",
+    "bm_lrcheck"};
 
 cudaError_t smem_limit(const void* kernel, int bytes)
 {
@@ -287,6 +288,8 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
         return fail(c, MVSV_ERR_STATE, "no mean-disparity ROIs (mvsv_set_mean_rois; a geometry change drops them)");
     if (rectify && (!c->has_maps[0] || !c->has_maps[1]))
         return fail(c, MVSV_ERR_STATE, "rectify maps missing (mvsv_upload_rectify_maps)");
+    if ((stages & MVSV_STAGE_BM) && c->bm_d12 >= 0 && c->W > bm_lrcheck_max_width())
+        return fail(c, MVSV_ERR_UNSUPPORTED, "BM left-right check (disp12MaxDiff >= 0): image wider than 4096");
     const int iw = rectify ? c->fw : c->W, ih = rectify ? c->fh : c->H;
     if (lstride < (size_t)iw || rstride < (size_t)iw)
         return fail(c, MVSV_ERR_INVALID, rectify ? "stride smaller than frame width" : "stride smaller than image width");
@@ -481,6 +484,22 @@ int mvsv_set_bm_params(mvsv_ctx* c, const mvsv_bm_params* p)
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
     c->bm = n; c->bm_raw = *p; c->has_bm = true;
     return ensure_bm_volumes(c);
+}
+
+int mvsv_set_bm_filters(mvsv_ctx* c, int disp12MaxDiff, int speckleWindowSize, int speckleRange)
+{
+    if (!c) return MVSV_ERR_INVALID;
+    if (speckleWindowSize < 0) return fail(c, MVSV_ERR_INVALID, "BM speckleWindowSize must be >= 0");
+    if (speckleWindowSize > 0 && speckleRange < 0) return fail(c, MVSV_ERR_INVALID, "BM speckleRange must be >= 0");
+    if (disp12MaxDiff >= 0 && c->W > bm_lrcheck_max_width())
+        return fail(c, MVSV_ERR_UNSUPPORTED, "BM left-right check (disp12MaxDiff >= 0): image wider than 4096");
+    int rc = bind(c);
+    if (rc) return rc;
+    MVSV_CK(c, cudaStreamSynchronize(c->stream));
+    c->bm_d12 = disp12MaxDiff < 0 ? -1 : disp12MaxDiff;
+    c->bm_speckle_win = speckleWindowSize;
+    c->bm_speckle_range = speckleWindowSize > 0 ? speckleRange : 0;
+    return MVSV_OK;
 }
 
 static int resize_rectified(mvsv_ctx* c, int W, int H)

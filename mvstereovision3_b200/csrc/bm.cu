@@ -298,11 +298,12 @@ struct BmArgs {
 // address any disparity there, no register indexing; two copies used in turn: one warp barrier per step).  The
 // per-pixel epilogue (texture test, sub-pixel division, store) is identical on the lanes of a row, so it is deferred:
 // lane q keeps the winner of every NL-th step and the lanes of a row finish NL pixels at once; the texture value of a
-// lane's pixel is requested one round ahead.
+// lane's pixel is requested one round ahead.  COST: the epilogue also stores the winner's SAD in cost[B][H][W] (the
+// left-right check's cost; a parameter of its own after the others, so that the kernels without it stay as they were).
 constexpr int BM_PF = 3;       // columns in flight ahead of the window (RING)
 
-template <int OPL, bool RING, bool B8>
-__global__ void __launch_bounds__(256) k_bm_wta(BmArgs a, int ringSlots, int sumsPerWarp)
+template <int OPL, bool RING, bool B8, bool COST>
+__global__ void __launch_bounds__(256) k_bm_wta(BmArgs a, int ringSlots, int sumsPerWarp, int* __restrict__ cost)
 {
     static_assert(!B8 || OPL == 2, "byte volume: sixteen disparities per lane");
     constexpr int NR = 4 * OPL;                                // packed registers per lane
@@ -400,6 +401,7 @@ __global__ void __launch_bounds__(256) k_bm_wta(BmArgs a, int ringSlots, int sum
             const int p = (int)svP, n = (int)svN;
             const int den = p + n - 2 * minsad + abs(p - n);
             a.disp[outRow + svX] = (int16_t)((((a.D - 1 - mind) * 256) + (den != 0 ? (p - n) * 256 / den : 0) + 15) >> 4);
+            if (COST) cost[outRow + svX] = minsad;
         }
         svX = -1;
     };
@@ -514,15 +516,110 @@ static int bm_wta_cta_warps(size_t warpBytes, int* warpsPerSm)
 }
 
 template <int OPL, bool RING, bool B8>
-static cudaError_t launch_bm_wta(mvsv_ctx* c, const BmArgs& a, int ringSlots, int ctaWarps)
+static cudaError_t launch_bm_wta(mvsv_ctx* c, const BmArgs& a, int* cost, int ringSlots, int ctaWarps)
 {
     const int NL = (a.D / 8) / OPL, rowsPerWarp = 32 / NL;
     const long long warps = ((long long)a.B * (a.H - 2 * a.w2) + rowsPerWarp - 1) / rowsPerWarp;
-    MVSV_TRY(smem_limit((const void*)k_bm_wta<OPL, RING, B8>, 226 * 1024));
+    const auto k = cost ? k_bm_wta<OPL, RING, B8, true> : k_bm_wta<OPL, RING, B8, false>;
+    MVSV_TRY(smem_limit((const void*)k, 226 * 1024));
     const size_t smem = ctaWarps * bm_wta_warp_smem(a.D, OPL, B8 ? 1 : OPL, RING ? ringSlots : 0);
-    k_bm_wta<OPL, RING, B8><<<(unsigned)((warps + ctaWarps - 1) / ctaWarps), ctaWarps * 32, smem, c->stream>>>(
-        a, ringSlots, bm_sums_per_warp(a.D, OPL));
+    k<<<(unsigned)((warps + ctaWarps - 1) / ctaWarps), ctaWarps * 32, smem, c->stream>>>(a, ringSlots, bm_sums_per_warp(a.D, OPL), cost);
     return cudaGetLastError();
+}
+
+// Left-right check of cv::StereoBM (disp12MaxDiff >= 0; semantics SURVEY.md A.4), in place on the x16 map, one CTA per
+// row.  cv::StereoBM matches the whole width1 domain, X in [D - 1, W), and runs the check before it clears the columns
+// outside the valid rectangle, so the border pixels X in [D, D - 1 + w2) and [W - w2, W) take part in the scatter
+// although they end up FILTERED.  The WTA does not evaluate them: phase 1 does, one warp per pixel, from the column
+// sums (clamped at the right edge) and, left of column 0 of the volume, from column sums of the clamped left pixel
+// against R[0 .. D - 1].  The scatter "x ascending, keep the first strict minimum of the cost at x2" is an atomicMin
+// of the keys (cost << 12) | x in shared memory; after one barrier every valid pixel checks itself against the table.
+constexpr int BM_LR_THREADS = 256;
+constexpr int BM_LR_MAXW = 4096;                                // 12-bit x in the keys; 16 KB of keys
+
+template <bool B8>
+__global__ void __launch_bounds__(BM_LR_THREADS)
+k_bm_lrcheck(int16_t* __restrict__ disp, const int* __restrict__ cost, const uint16_t* __restrict__ col,
+             const uint8_t* __restrict__ preL, const uint8_t* __restrict__ preR, size_t pitch, int W, int H, int width1,
+             int D, int w2, int cap, int texThr, int uniq, int d12)
+{
+    __shared__ unsigned keys[BM_LR_MAXW];
+    __shared__ int16_t rowd[BM_LR_MAXW];
+    __shared__ int sads[BM_LR_THREADS / 32][256];
+    const int f = blockIdx.y, y = blockIdx.x + w2, lofs = D - 1;
+    const int xlo = lofs + w2, xhi = W - w2;                  // valid rectangle
+    const int FILT = -16;
+    const size_t row = ((size_t)f * H + y) * W;
+    int16_t* drow = disp + row;
+    for (int x = threadIdx.x; x < W; x += BM_LR_THREADS) { keys[x] = 0xffffffffu; rowd[x] = drow[x]; }
+    __syncthreads();
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    // phase 1: the border pixels (w2 - 1 on the left, w2 on the right); x is the column in the width1 domain
+    const int nLeft = w2 - 1, nb = nLeft + w2;
+    const unsigned char* vol = reinterpret_cast<const unsigned char*>(col);
+    const size_t volRow = ((size_t)f * H + y) * width1;
+    const uint8_t* pl = preL + (size_t)f * H * pitch;
+    const uint8_t* pr = preR + (size_t)f * H * pitch;
+    int* sad = sads[warp];
+    for (int i = warp; i < nb; i += BM_LR_THREADS / 32) {
+        const int X = i < nLeft ? D + i : xhi + (i - nLeft), x = X - lofs;
+        int tex = 0;
+        for (int t = lane; t < (2 * w2 + 1) * (2 * w2 + 1); t += 32) {
+            const int dy = t / (2 * w2 + 1) - w2, dx = t % (2 * w2 + 1) - w2;
+            tex += abs((int)pl[(size_t)(y + dy) * pitch + min(max(X + dx, 0), W - 1)] - cap);
+        }
+        tex = __reduce_add_sync(FULL, tex);
+        unsigned best = 0xffffffffu;
+        for (int k = lane; k < D; k += 32) {
+            int s = 0;
+            for (int j = x - w2; j <= x + w2; ++j) {
+                if (j >= 0) {
+                    const size_t cell = (volRow + min(j, width1 - 1)) * D + k;
+                    s += B8 ? (int)vol[cell] : (int)col[cell];
+                } else {
+                    const int cl = max(j + lofs, 0);
+                    for (int dy = -w2; dy <= w2; ++dy)
+                        s += abs((int)pl[(size_t)(y + dy) * pitch + cl] - (int)pr[(size_t)(y + dy) * pitch + k]);
+                }
+            }
+            sad[k] = s;
+            best = min(best, ((unsigned)s << 8) | (unsigned)k);   // first minimum: smallest k among equal sums
+        }
+        best = __reduce_min_sync(FULL, best);
+        const int minsad = (int)(best >> 8), mind = (int)(best & 0xffu);
+        bool reject = tex < texThr;
+        if (uniq > 0) {
+            const int thresh = minsad + (minsad * uniq / 100);
+            bool other = false;
+            for (int k = lane; k < D; k += 32) other |= (k < mind - 1 || k > mind + 1) && sad[k] <= thresh;
+            reject |= __any_sync(FULL, other);
+        }
+        __syncwarp();
+        if (lane == 0 && !reject) {
+            const int p = mind + 1 < D ? sad[mind + 1] : sad[D - 2], n = mind > 0 ? sad[mind - 1] : sad[1];
+            const int den = p + n - 2 * minsad + abs(p - n);
+            const int d = ((D - 1 - mind) * 256 + (den != 0 ? (p - n) * 256 / den : 0) + 15) >> 4;
+            rowd[X] = (int16_t)d;
+            atomicMin(&keys[X - ((d + 8) >> 4)], ((unsigned)minsad << 12) | (unsigned)X);
+        }
+        __syncwarp();
+    }
+    // phase 2: the valid pixels the WTA matched (FILTERED ones take no part)
+    const int* crow = cost + row;
+    for (int X = xlo + threadIdx.x; X < xhi; X += BM_LR_THREADS) {
+        const int d = rowd[X];
+        if (d != FILT) atomicMin(&keys[X - ((d + 8) >> 4)], ((unsigned)crow[X] << 12) | (unsigned)X);
+    }
+    __syncthreads();
+    const int lim = 16 * d12;
+    auto inconsistent = [&](int x2, int d) {
+        if (x2 < 0 || x2 >= W || keys[x2] == 0xffffffffu) return false;
+        return abs((int)rowd[keys[x2] & 0xfffu] - d) > lim;
+    };
+    for (int X = xlo + threadIdx.x; X < xhi; X += BM_LR_THREADS) {
+        const int d = rowd[X];
+        if (d != FILT && inconsistent(X - (d >> 4), d) && inconsistent(X - ((d + 15) >> 4), d)) drow[X] = (int16_t)FILT;
+    }
 }
 
 // n is a multiple of 8 pixels (the image buffers are padded to 16 bytes): one 128-bit store per thread
@@ -536,20 +633,35 @@ __global__ void k_fill16(int16_t* p, size_t n, int16_t v)
 
 }  // namespace
 
+int bm_lrcheck_max_width() { return BM_LR_MAXW; }
+
+// the map after the matcher (and the left-right check) -> the speckle filter -> the slot's disparities
+static cudaError_t bm_speckle(mvsv_ctx* c, int B)
+{
+    if (c->bm_speckle_win <= 0) return cudaSuccess;
+    return launch_speckle(c, c->disp_raw, io(c).disp, B, c->bm.FILT, c->bm_speckle_win, c->bm_speckle_range);
+}
+
 cudaError_t launch_bm(mvsv_ctx* c, int B)
 {
     const BmNorm& n = c->bm;
     const bool col8 = n.col8 && !(c->debug_flags & 2u);         // debug bit 1: never keep a volume as bytes
     const int W = c->W, H = c->H;
     const size_t npx = (size_t)B * W * H;
-    { KernelTimer kt(c, KID_FILL); k_fill16<<<(unsigned)((npx / 8 + 256) / 256), 256, 0, c->stream>>>(io(c).disp, npx, (int16_t)n.FILT); }
+    // with the speckle filter the matcher's map is an intermediate (disp_raw, debug_read 2)
+    int16_t* const out = c->bm_speckle_win > 0 ? c->disp_raw : io(c).disp;
+    const bool lr = c->bm_d12 >= 0;
+    { KernelTimer kt(c, KID_FILL); k_fill16<<<(unsigned)((npx / 8 + 256) / 256), 256, 0, c->stream>>>(out, npx, (int16_t)n.FILT); }
     {
         dim3 blk(128), grd((W + 127) / 128, (H + 4 * BM_PF_ROWS - 1) / (4 * BM_PF_ROWS), 2 * B);
         KernelTimer kt(c, KID_BM_PREFILTER);
         k_bm_prefilter<<<grd, blk, 0, c->stream>>>(io(c).rect[0], io(c).rect[1], c->pitch, W, H, n.cap, c->bm_pre[0], c->bm_pre[1]);
     }
     const bool any = !(n.lofs >= W || n.width1 < 1) && (H - 2 * n.w2 > 0) && (n.width1 - 2 * n.w2 > 0);
-    if (!any) return cudaGetLastError();
+    if (!any) {
+        MVSV_TRY(cudaGetLastError());
+        return bm_speckle(c, B);
+    }
     {
         KernelTimer kt(c, KID_BM_TEX);
         if (n.bs <= 63) {
@@ -573,21 +685,33 @@ cudaError_t launch_bm(mvsv_ctx* c, int B)
         colsum<<<grd, 128, ringBytes, c->stream>>>(c->bm_pre[0], c->bm_pre[1], c->pitch, H, n.width1, n.D, n.lofs, n.w2, c->bm_col);
     }
     BmArgs a;
-    a.col = c->bm_col; a.tex = c->bm_tex2; a.disp = io(c).disp; a.W = W; a.H = H; a.width1 = n.width1; a.D = n.D; a.Dp = n.Dp;
+    a.col = c->bm_col; a.tex = c->bm_tex2; a.disp = out; a.W = W; a.H = H; a.width1 = n.width1; a.D = n.D; a.Dp = n.Dp;
     a.lofs = n.lofs; a.w2 = n.w2; a.texThr = n.tex; a.uniq = n.uniq; a.B = B;
-    KernelTimer kt(c, KID_BM_WTA);
-    // Two octets per lane (numDisp is a multiple of 16) with the window ring while at least eight warps fit an SM
-    // (four with the byte volume's smaller ring), one octet per lane while four do, else (blockSize > ~100) no ring.
-    const int slots = n.bs + 1 + BM_PF;
-    int wps = 0, nw;
-    if (col8) {
-        nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 1, slots), &wps);
-        if (wps >= 4) return launch_bm_wta<2, true, true>(c, a, slots, nw);
-        return launch_bm_wta<2, false, true>(c, a, slots, 4);
+    int* const cost = lr ? c->d2 : nullptr;                   // the SGBM's disp2 keys buffer: same shape, idle here
+    {
+        KernelTimer kt(c, KID_BM_WTA);
+        // Two octets per lane (numDisp is a multiple of 16) with the window ring while at least eight warps fit an SM
+        // (four with the byte volume's smaller ring), one octet per lane while four do, else (blockSize > ~100) no ring.
+        const int slots = n.bs + 1 + BM_PF;
+        int wps = 0, nw;
+        if (col8) {
+            nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 1, slots), &wps);
+            if (wps >= 4) MVSV_TRY((launch_bm_wta<2, true, true>(c, a, cost, slots, nw)));
+            else MVSV_TRY((launch_bm_wta<2, false, true>(c, a, cost, slots, 4)));
+        } else if (nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 2, slots), &wps), wps >= 8) {
+            MVSV_TRY((launch_bm_wta<2, true, false>(c, a, cost, slots, nw)));
+        } else if (nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 1, 1, slots), &wps), wps >= 4) {
+            MVSV_TRY((launch_bm_wta<1, true, false>(c, a, cost, slots, nw)));
+        } else {
+            MVSV_TRY((launch_bm_wta<2, false, false>(c, a, cost, slots, 4)));
+        }
     }
-    nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 2, 2, slots), &wps);
-    if (wps >= 8) return launch_bm_wta<2, true, false>(c, a, slots, nw);
-    nw = bm_wta_cta_warps(bm_wta_warp_smem(n.D, 1, 1, slots), &wps);
-    if (wps >= 4) return launch_bm_wta<1, true, false>(c, a, slots, nw);
-    return launch_bm_wta<2, false, false>(c, a, slots, 4);
+    if (lr) {
+        KernelTimer kt(c, KID_BM_LRCHECK);
+        const auto k = col8 ? k_bm_lrcheck<true> : k_bm_lrcheck<false>;
+        k<<<dim3(H - 2 * n.w2, B), BM_LR_THREADS, 0, c->stream>>>(out, c->d2, c->bm_col, c->bm_pre[0], c->bm_pre[1], c->pitch, W, H,
+                                                                  n.width1, n.D, n.w2, n.cap, n.tex, n.uniq, c->bm_d12);
+        MVSV_TRY(cudaGetLastError());
+    }
+    return bm_speckle(c, B);
 }

@@ -31,7 +31,7 @@ struct BmNorm {
 enum KernelId {
     KID_REMAP = 0, KID_SGBM_PREFILTER, KID_SGBM_VSUM, KID_SGBM_H1, KID_SGBM_VDIR, KID_SGBM_TD, KID_SGBM_H2_WTA, KID_MEDIAN,
     KID_CCL_ROWS, KID_CCL_VMERGE, KID_CCL_FLATTEN, KID_CCL_APPLY, KID_BM_PREFILTER, KID_BM_TEX, KID_BM_COLSUM,
-    KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_COUNT
+    KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_BM_LRCHECK, KID_COUNT
 };
 extern const char* const kKernelNames[KID_COUNT];
 
@@ -103,6 +103,8 @@ struct mvsv_ctx {
     int num_sms = 148;
     mvsv_bm_params bm_raw{};
     BmNorm bm{};
+    // mvsv_set_bm_filters, kept across mvsv_set_bm_params and geometry changes: -1 / 0 = off
+    int bm_d12 = -1, bm_speckle_win = 0, bm_speckle_range = 0;
 
     uint2* recL = nullptr;                    // left prefilter records [B][H][W] (a_s,lo_s,hi_s,a_r,lo_r,hi_r)
     uint16_t* plR = nullptr;                  // right prefilter planes, reversed + padded: [6][B][H][vsRP]
@@ -170,6 +172,7 @@ cudaError_t launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q);
 cudaError_t launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
 cudaError_t launch_sgbm(mvsv_ctx* c, int B);
 cudaError_t launch_bm(mvsv_ctx* c, int B);
+int bm_lrcheck_max_width();
 size_t tm_smem_bytes(int W, int k);
 int tm_max_width();
 cudaError_t launch_tm(mvsv_ctx* c, int B, int k, uint8_t* out, size_t opitch);
