@@ -205,6 +205,8 @@ int mvsv_host_free(void* p);
  * (roi_h x roi_w int32 pairs: x*32, y*32 rounded).  Returns bytes written or a negative error. */
 /* bit 0: keep the complete aggregated S volume (all paths) readable through mvsv_debug_read(which=1).
  * bit 1: never keep a volume as bytes (mvsv_info.sgbm_s8, mvsv_info.bm_col8).
+ * bit 2: run the 3x3 median with its one-column-per-lane kernel also where the four-columns-per-lane kernel qualifies
+ * (width % 4 == 0).
  * bits 8..15: force the number of column strips per frame of the fused sweep (0xff = force the independent passes,
  * 0xfe = force the sweep with the usual choice of strips: small batches otherwise take the independent passes).
  * bits 16..23: force the number of frames per chunk of the overlapped cost kernel / first row scan (0 = chosen by the
@@ -214,6 +216,16 @@ int mvsv_host_free(void* p);
  * sends the sweep's border records through global memory also where a thread-block cluster would be used. */
 int mvsv_debug_set_flags(mvsv_ctx* ctx, unsigned flags);
 long long mvsv_debug_read(mvsv_ctx* ctx, int which, void* host, size_t capacity_bytes);
+/* Test hook: the post-filters and consumers of a compute, run on caller-supplied disparity maps instead of a matcher's
+ * output.  `batch` int16 maps of width x height of mvsv_get_info in HOST memory (row stride `stride` bytes, map b at
+ * maps + b*height*stride) become the raw disparity (mvsv_debug_read which=2); then, in the order cv::StereoSGBM applies
+ * them, medianBlur(3) when median != 0 and filterSpeckles(newVal, maxSpeckleSize, maxDiff) when maxSpeckleSize > 0
+ * (maxDiff in x16 units, as filterSpeckles takes it; neither: a plain copy) leave the final map in the next I/O slot,
+ * and `stages` (MVSV_STAGE_XYZ and / or MVSV_STAGE_MEANS only) run on it.  The slot is then read like that of a
+ * compute (mvsv_download, mvsv_download_age, mvsv_download_minmax, mvsv_debug_read 2 and 4).  Argument and state
+ * checks, and the handling of a failure, are those of mvsv_compute. */
+int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int batch, int median, int newVal,
+                          int maxSpeckleSize, int maxDiff, unsigned stages);
 
 #ifdef __cplusplus
 }

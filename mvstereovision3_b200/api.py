@@ -20,7 +20,7 @@ ABI_SYMBOLS = (
     "mvsv_compute_device", "mvsv_tm", "mvsv_download", "mvsv_sync", "mvsv_get_info", "mvsv_stream", "mvsv_launch_count",
     "mvsv_host_alloc", "mvsv_host_free", "mvsv_debug_set_flags", "mvsv_debug_read",
     "mvsv_download_minmax", "mvsv_download_age", "mvsv_set_io_slots", "mvsv_timer_start", "mvsv_timer_stop", "mvsv_profile_enable", "mvsv_profile_read", "mvsv_kernel_name",
-    "mvsv_set_bm_filters",
+    "mvsv_set_bm_filters", "mvsv_debug_postfilter",
 )
 
 
@@ -92,6 +92,7 @@ def load_library():
     lib.mvsv_debug_set_flags.argtypes = [vp, C.c_uint]
     lib.mvsv_debug_read.argtypes = [vp, ci, vp, sz]
     lib.mvsv_debug_read.restype = C.c_longlong
+    lib.mvsv_debug_postfilter.argtypes = [vp, vp, sz, ci, ci, ci, ci, ci, C.c_uint]
     lib.mvsv_timer_start.argtypes = [vp]
     lib.mvsv_timer_stop.argtypes = [vp, C.POINTER(C.c_float)]
     lib.mvsv_profile_enable.argtypes = [vp, ci]
@@ -335,6 +336,20 @@ class Engine:
     # -- test hooks -----------------------------------------------------------------------------
     def debug_set_flags(self, flags):
         self._ck(self._lib.mvsv_debug_set_flags(self._ctx, flags))
+
+    def debug_postfilter(self, maps, median=True, new_val=0, speckle_size=0, speckle_diff=0, stages=0):
+        """mvsv_debug_postfilter: int16 maps [B,]H,W (row stride may exceed W) through medianBlur(3) when `median`, then
+        filterSpeckles(new_val, speckle_size, speckle_diff) when speckle_size > 0, then `stages` (STAGE_XYZ |
+        STAGE_MEANS); the results are fetched with download / download_minmax / debug_read like those of a compute."""
+        m = np.asarray(maps)
+        if m.ndim == 2:
+            m = m[None]
+        if m.dtype != np.int16 or m.ndim != 3:
+            raise ValueError("maps must be int16 [B,]H,W")
+        if m.strides[2] != 2 or m.strides[0] != m.shape[1] * m.strides[1]:
+            m = np.ascontiguousarray(m)
+        self._ck(self._lib.mvsv_debug_postfilter(self._ctx, m.ctypes.data, m.strides[1], m.shape[0], 1 if median else 0,
+                                                 int(new_val), int(speckle_size), int(speckle_diff), stages))
 
     def debug_read(self, which, batch):
         i = self.info

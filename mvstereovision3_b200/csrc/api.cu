@@ -269,6 +269,15 @@ static int inputs_uploaded(mvsv_ctx* c, bool device_src)
     return MVSV_OK;
 }
 
+// what the XYZ and MEANS stages need of the ctx and of the slot they write to
+int check_consumers(mvsv_ctx* c, const IoSlot& slot, unsigned stages)
+{
+    if ((stages & MVSV_STAGE_XYZ) && !c->has_Q) return fail(c, MVSV_ERR_STATE, "mvsv_set_Q not called");
+    if ((stages & MVSV_STAGE_MEANS) && (c->nrois < 1 || !c->rois || !slot.means))
+        return fail(c, MVSV_ERR_STATE, "no mean-disparity ROIs (mvsv_set_mean_rois; a geometry change drops them)");
+    return MVSV_OK;
+}
+
 int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride, int batch,
         unsigned stages, bool device_src)
 {
@@ -283,9 +292,8 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
     if ((stages & MVSV_STAGE_SGBM) && (stages & MVSV_STAGE_BM)) return fail(c, MVSV_ERR_INVALID, "choose SGBM or BM, not both");
     if ((stages & MVSV_STAGE_SGBM) && !c->has_sgbm) return fail(c, MVSV_ERR_STATE, "mvsv_set_sgbm_params not called");
     if ((stages & MVSV_STAGE_BM) && !c->has_bm) return fail(c, MVSV_ERR_STATE, "mvsv_set_bm_params not called");
-    if ((stages & MVSV_STAGE_XYZ) && !c->has_Q) return fail(c, MVSV_ERR_STATE, "mvsv_set_Q not called");
-    if ((stages & MVSV_STAGE_MEANS) && (c->nrois < 1 || !c->rois || !slot.means))
-        return fail(c, MVSV_ERR_STATE, "no mean-disparity ROIs (mvsv_set_mean_rois; a geometry change drops them)");
+    rc = check_consumers(c, slot, stages);
+    if (rc) return rc;
     if (rectify && (!c->has_maps[0] || !c->has_maps[1]))
         return fail(c, MVSV_ERR_STATE, "rectify maps missing (mvsv_upload_rectify_maps)");
     if ((stages & MVSV_STAGE_BM) && c->bm_d12 >= 0 && c->W > bm_lrcheck_max_width())
@@ -876,6 +884,46 @@ int mvsv_debug_set_flags(mvsv_ctx* c, unsigned flags)
     c->debug_flags = flags;
     if (c->has_sgbm) c->td_nc = sgbm_choose_td_cluster(c);
     return MVSV_OK;
+}
+
+int mvsv_debug_postfilter(mvsv_ctx* c, const int16_t* maps, size_t stride, int batch, int median, int newVal,
+                          int maxSpeckleSize, int maxDiff, unsigned stages)
+{
+    if (!c) return MVSV_ERR_INVALID;
+    int rc = bind(c);
+    if (rc) return rc;
+    // the next I/O slot, taken as run() takes it
+    const int k = (c->cur + 1) % c->nslots;
+    IoSlot& slot = c->slot[k];
+    if (!maps || batch < 1 || batch > c->maxB) return fail(c, MVSV_ERR_INVALID, "bad map pointer or batch size");
+    if (stride < (size_t)c->W * sizeof(int16_t)) return fail(c, MVSV_ERR_INVALID, "stride smaller than the map width");
+    if (stages & ~(unsigned)(MVSV_STAGE_XYZ | MVSV_STAGE_MEANS))
+        return fail(c, MVSV_ERR_INVALID, "post-filter hook: only MVSV_STAGE_XYZ and MVSV_STAGE_MEANS");
+    if (maxSpeckleSize > 0 && (newVal < -32768 || newVal > 32767)) return fail(c, MVSV_ERR_INVALID, "newVal does not fit CV_16S");
+    rc = check_consumers(c, slot, stages);
+    if (rc) return rc;
+    if ((stages & MVSV_STAGE_XYZ) && !slot.xyz) MVSV_CK(c, cudaMalloc(&slot.xyz, (size_t)c->maxB * c->H * c->W * 3 * sizeof(float)));
+
+    c->cur = k;                 // the slot is taken: a failing step leaves it empty
+    auto submit = [&]() -> int {
+        const size_t row = (size_t)c->W * sizeof(int16_t), npx = (size_t)batch * c->H * c->W;
+        MVSV_CK(c, cudaMemcpy2DAsync(c->disp_raw, row, maps, stride, row, (size_t)c->H * batch, cudaMemcpyHostToDevice, c->stream));
+        const bool speckle = maxSpeckleSize > 0;
+        if (median) MVSV_CK(c, launch_median(c, c->disp_raw, speckle ? c->disp_med : slot.disp, batch));
+        if (speckle)
+            MVSV_CK(c, launch_speckle(c, median ? c->disp_med : c->disp_raw, slot.disp, batch, newVal, maxSpeckleSize, maxDiff));
+        if (!median && !speckle)
+            MVSV_CK(c, cudaMemcpyAsync(slot.disp, c->disp_raw, npx * sizeof(int16_t), cudaMemcpyDeviceToDevice, c->stream));
+        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, launch_xyz(c, batch));
+        if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
+        MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
+        MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
+        return MVSV_OK;
+    };
+    rc = submit();
+    slot.B = rc ? 0 : batch;
+    slot.stages = rc ? 0 : stages;
+    return rc;
 }
 
 long long mvsv_debug_read(mvsv_ctx* c, int which, void* host, size_t cap)

@@ -552,7 +552,8 @@ cudaError_t launch_resize(mvsv_ctx* c, int cam, int B)
 cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B)
 {
     KernelTimer kt(c, KID_MEDIAN);
-    if (c->W % 4 == 0 && c->W >= 4 && (reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) % 8 == 0) {
+    const bool scalar = c->debug_flags & 4u;        // debug bit 2: k_median3 also where k_median3_w4 qualifies
+    if (!scalar && c->W % 4 == 0 && c->W >= 4 && (reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out)) % 8 == 0) {
         const int ncx = (c->W + MED4_COLS - 1) / MED4_COLS, nbands = (c->H + MED_ROWS - 1) / MED_ROWS;
         dim3 grd((ncx * nbands + MED_WARPS - 1) / MED_WARPS, B);
         k_median3_w4<<<grd, MED_WARPS * 32, 0, c->stream>>>(in, out, c->W, c->H, ncx, nbands);

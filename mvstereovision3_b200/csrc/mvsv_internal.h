@@ -69,7 +69,8 @@ struct mvsv_ctx {
     int maxB = 0;
     unsigned long long launches = 0;
     unsigned debug_flags = 0;   // bit0: h2 pass stores the final S volume (test hook); bit1: never use the byte form of S;
-                                // bits 8..15: sweep strips; bits 16..23: frames per chunk of the vsum / h1 overlap (mvsv.h)
+                                // bit2: the scalar median kernel only; bits 8..15: sweep strips; bits 16..23: frames per
+                                // chunk of the vsum / h1 overlap (mvsv.h)
     bool last_s8 = false;       // the last SGBM compute kept S as bytes (S8)
     bool prof = false;
     std::vector<ProfBracket> brackets;      // pending (unread) timed launches
