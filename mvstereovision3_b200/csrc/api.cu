@@ -8,6 +8,7 @@
 #include <map>
 #include <mutex>
 #include <new>
+#include <numeric>
 
 const char* const kKernelNames[KID_COUNT] = {
     "remap", "sgbm_prefilter", "sgbm_vsum", "sgbm_h1", "sgbm_vdir", "sgbm_td", "sgbm_h2_wta", "median3", "ccl_rows", "ccl_vmerge",
@@ -56,6 +57,38 @@ int fail(mvsv_ctx* c, int code, const std::string& msg)
     return code;
 }
 
+// some rig holds (or is getting) a rectification map
+bool any_maps(const mvsv_ctx* c)
+{
+    for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+        if (c->has_maps[r][0] || c->has_maps[r][1] || c->map_xy[r][0] || c->map_xy[r][1]) return true;
+    return false;
+}
+
+// the rigs frames 0 .. B-1 of a compute come from (bit r = rig r; frames past the mvsv_set_frame_rigs table: rig 0)
+uint64_t rigs_of_batch(const mvsv_ctx* c, int B)
+{
+    const int n = std::min(B, (int)c->frame_rig.size());
+    uint64_t m = B > n ? 1u : 0u;
+    for (int i = 0; i < n; ++i) m |= (uint64_t)1 << c->frame_rig[i];
+    return m;
+}
+
+// The rig-aware kernels read every rig's map and Q from c->rig_tables.  The copy is queued on the ctx stream, so that a
+// compute sees the Q's set before it was submitted, as the single-rig k_xyz does with its by-value Q.
+int upload_rig_tables(mvsv_ctx* c)
+{
+    if (!c->rig_tables_dirty) return MVSV_OK;
+    RigTables t;
+    for (int r = 0; r < MVSV_MAX_RIGS; ++r) {
+        for (int cam = 0; cam < 2; ++cam) t.map[cam][r] = c->map_xy[r][cam];
+        for (int i = 0; i < 16; ++i) t.Q[r][i] = (double)c->Q[r][i];
+    }
+    MVSV_CK(c, cudaMemcpyAsync(c->rig_tables, &t, sizeof(t), cudaMemcpyHostToDevice, c->stream));   // pageable: staged before it returns
+    c->rig_tables_dirty = false;
+    return MVSV_OK;
+}
+
 // What free_slot releases; each level includes the ones before it.
 enum SlotBuffers {
     SLOT_MEANS,     // the ROI means (the ROIs change)
@@ -82,7 +115,7 @@ void free_slot(mvsv_ctx* c, int k, SlotBuffers what)
 int ensure_slots(mvsv_ctx* c)
 {
     const size_t B = (size_t)c->maxB, npx = B * c->H * c->W, nimg = B * c->H * c->pitch;
-    const bool maps = c->map_xy[0] || c->map_xy[1];
+    const bool maps = any_maps(c);
     for (int k = 0; k < c->nslots; ++k) {
         IoSlot& s = c->slot[k];
         for (int i = 0; i < 2; ++i) {
@@ -269,10 +302,13 @@ static int inputs_uploaded(mvsv_ctx* c, bool device_src)
     return MVSV_OK;
 }
 
-// what the XYZ and MEANS stages need of the ctx and of the slot they write to
-int check_consumers(mvsv_ctx* c, const IoSlot& slot, unsigned stages)
+// what the XYZ and MEANS stages need of the ctx and of the slot they write to; `rigs`: the rigs of the batch's frames
+int check_consumers(mvsv_ctx* c, const IoSlot& slot, unsigned stages, uint64_t rigs)
 {
-    if ((stages & MVSV_STAGE_XYZ) && !c->has_Q) return fail(c, MVSV_ERR_STATE, "mvsv_set_Q not called");
+    if (stages & MVSV_STAGE_XYZ)
+        for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+            if (((rigs >> r) & 1) && !c->has_Q[r])
+                return fail(c, MVSV_ERR_STATE, r == 0 ? "mvsv_set_Q not called" : "no Q for rig " + std::to_string(r) + " (mvsv_set_Q_rig)");
     if ((stages & MVSV_STAGE_MEANS) && (c->nrois < 1 || !c->rois || !slot.means))
         return fail(c, MVSV_ERR_STATE, "no mean-disparity ROIs (mvsv_set_mean_rois; a geometry change drops them)");
     return MVSV_OK;
@@ -292,10 +328,16 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
     if ((stages & MVSV_STAGE_SGBM) && (stages & MVSV_STAGE_BM)) return fail(c, MVSV_ERR_INVALID, "choose SGBM or BM, not both");
     if ((stages & MVSV_STAGE_SGBM) && !c->has_sgbm) return fail(c, MVSV_ERR_STATE, "mvsv_set_sgbm_params not called");
     if ((stages & MVSV_STAGE_BM) && !c->has_bm) return fail(c, MVSV_ERR_STATE, "mvsv_set_bm_params not called");
-    rc = check_consumers(c, slot, stages);
+    // frames of rigs other than 0: the rig-aware remap and XYZ kernels
+    const uint64_t rigs = rigs_of_batch(c, batch);
+    const bool multi = rigs != 1;
+    rc = check_consumers(c, slot, stages, rigs);
     if (rc) return rc;
-    if (rectify && (!c->has_maps[0] || !c->has_maps[1]))
-        return fail(c, MVSV_ERR_STATE, "rectify maps missing (mvsv_upload_rectify_maps)");
+    if (rectify)
+        for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+            if (((rigs >> r) & 1) && (!c->has_maps[r][0] || !c->has_maps[r][1]))
+                return fail(c, MVSV_ERR_STATE, r == 0 ? "rectify maps missing (mvsv_upload_rectify_maps)"
+                                                      : "rectify maps of rig " + std::to_string(r) + " missing (mvsv_upload_rectify_maps_rig)");
     if ((stages & MVSV_STAGE_BM) && c->bm_d12 >= 0 && c->W > bm_lrcheck_max_width())
         return fail(c, MVSV_ERR_UNSUPPORTED, "BM left-right check (disp12MaxDiff >= 0): image wider than 4096");
     const int iw = rectify ? c->fw : c->W, ih = rectify ? c->fh : c->H;
@@ -319,14 +361,18 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
         if (!r) r = upload_images(c, dst[1], dpitch, right, rstride, frame_stride, iw, ih, batch, device_src);
         if (!r) r = inputs_uploaded(c, device_src);
         if (r) return r;
+        if (multi && (rectify || (stages & MVSV_STAGE_XYZ))) {
+            r = upload_rig_tables(c);
+            if (r) return r;
+        }
         if (rectify)
             for (int cam = 0; cam < 2; ++cam) {
-                MVSV_CK(c, launch_remap(c, cam, batch));
+                MVSV_CK(c, multi ? launch_remap_rigs(c, cam, batch) : launch_remap(c, cam, batch));
                 if (c->resize_factor > 0.0) MVSV_CK(c, launch_resize(c, cam, batch));
             }
         if (stages & MVSV_STAGE_SGBM) MVSV_CK(c, launch_sgbm(c, batch));
         else if (stages & MVSV_STAGE_BM) MVSV_CK(c, launch_bm(c, batch));
-        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, launch_xyz(c, batch));
+        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
         if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
         MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
         MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
@@ -447,7 +493,11 @@ void mvsv_destroy(mvsv_ctx* c)
     }
     free_sgbm_volumes(c);
     free_bm_volumes(c);
-    for (int i = 0; i < 2; ++i) { dfree(c->map_xy[i]); dfree(c->crop[i]); }
+    for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+        for (int i = 0; i < 2; ++i) dfree(c->map_xy[r][i]);
+    for (int i = 0; i < 2; ++i) dfree(c->crop[i]);
+    dfree(c->rig_frames.chunk);
+    dfree(c->rig_tables);
     dfree(c->rois);
     for (auto& b : c->brackets) { cudaEventDestroy(b.a); cudaEventDestroy(b.b); }
     for (auto e : c->ev_free) cudaEventDestroy(e);
@@ -549,8 +599,8 @@ static int resize_rectified(mvsv_ctx* c, int W, int H)
 // mvsv_set_resize is active; (re)allocates everything that depends on it
 static int apply_geometry(mvsv_ctx* c)
 {
-    const bool maps = c->has_maps[0] || c->has_maps[1] || c->map_xy[0] || c->map_xy[1];
-    int W = maps ? c->roi[2] : c->fw, H = maps ? c->roi[3] : c->fh;
+    const bool maps = any_maps(c);
+    int W = maps ? c->roi_w : c->fw, H = maps ? c->roi_h : c->fh;
     const bool resized = maps && c->resize_factor > 0.0;
     if (resized) {
         // cv::resize: dsize = Size(saturate_cast<int>(w*fx), saturate_cast<int>(h*fy)), round half to even
@@ -562,26 +612,31 @@ static int apply_geometry(mvsv_ctx* c)
     if (rc) return rc;
     for (int i = 0; i < 2; ++i) dfree(c->crop[i]);
     if (resized) {
-        c->crop_pitch = round_up((size_t)c->roi[2], 16);
-        for (int i = 0; i < 2; ++i) MVSV_CK(c, cudaMalloc(&c->crop[i], (size_t)c->maxB * c->roi[3] * c->crop_pitch));
+        c->crop_pitch = round_up((size_t)c->roi_w, 16);
+        for (int i = 0; i < 2; ++i) MVSV_CK(c, cudaMalloc(&c->crop[i], (size_t)c->maxB * c->roi_h * c->crop_pitch));
     }
     return MVSV_OK;
 }
 
 // shared by the two ways of installing a camera's maps: checks the display ROI, sizes the rectified images and
 // the raw-frame staging, allocates the fixed-point map
-static int prepare_maps(mvsv_ctx* c, int cam, int roi_x, int roi_y, int roi_w, int roi_h)
+static int prepare_maps(mvsv_ctx* c, int rig, int cam, int roi_x, int roi_y, int roi_w, int roi_h)
 {
     if (roi_x < 0 || roi_y < 0 || roi_w < 2 || roi_h < 1 || roi_x + roi_w > c->fw || roi_y + roi_h > c->fh)
         return fail(c, MVSV_ERR_INVALID, "display ROI outside the frame");
     const int other = 1 - cam;
-    if (c->has_maps[other] && (c->roi[0] != roi_x || c->roi[1] != roi_y || c->roi[2] != roi_w || c->roi[3] != roi_h))
+    if (c->has_maps[rig][other] &&
+        (c->roi_xy[rig][0] != roi_x || c->roi_xy[rig][1] != roi_y || c->roi_w != roi_w || c->roi_h != roi_h))
         return fail(c, MVSV_ERR_INVALID, "both cameras must share one display ROI (mDisplayROI)");
+    for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+        if (r != rig && (c->has_maps[r][0] || c->has_maps[r][1]) && (c->roi_w != roi_w || c->roi_h != roi_h))
+            return fail(c, MVSV_ERR_INVALID, "all rigs share the display-ROI size (rig " + std::to_string(r) + " holds maps of another size)");
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
-    c->roi[0] = roi_x; c->roi[1] = roi_y; c->roi[2] = roi_w; c->roi[3] = roi_h;
-    c->has_maps[cam] = false;
-    dfree(c->map_xy[cam]);
-    MVSV_CK(c, cudaMalloc(&c->map_xy[cam], (size_t)roi_w * roi_h * sizeof(int2)));
+    c->roi_xy[rig][0] = roi_x; c->roi_xy[rig][1] = roi_y; c->roi_w = roi_w; c->roi_h = roi_h;
+    c->has_maps[rig][cam] = false;
+    c->rig_tables_dirty = true;
+    dfree(c->map_xy[rig][cam]);
+    MVSV_CK(c, cudaMalloc(&c->map_xy[rig][cam], (size_t)roi_w * roi_h * sizeof(int2)));
     int rc = apply_geometry(c);
     if (rc) return rc;
     return ensure_slots(c);
@@ -590,11 +645,18 @@ static int prepare_maps(mvsv_ctx* c, int cam, int roi_x, int roi_y, int roi_w, i
 int mvsv_upload_rectify_maps(mvsv_ctx* c, int cam, const float* mapx, const float* mapy, size_t stride_bytes, int roi_x,
                              int roi_y, int roi_w, int roi_h)
 {
+    return mvsv_upload_rectify_maps_rig(c, 0, cam, mapx, mapy, stride_bytes, roi_x, roi_y, roi_w, roi_h);
+}
+
+int mvsv_upload_rectify_maps_rig(mvsv_ctx* c, int rig, int cam, const float* mapx, const float* mapy, size_t stride_bytes,
+                                 int roi_x, int roi_y, int roi_w, int roi_h)
+{
     if (!c || !mapx || !mapy || cam < 0 || cam > 1) return MVSV_ERR_INVALID;
+    if (rig < 0 || rig >= MVSV_MAX_RIGS) return fail(c, MVSV_ERR_INVALID, "rig outside [0, MVSV_MAX_RIGS)");
     int rc = bind(c);
     if (rc) return rc;
     if (stride_bytes < (size_t)c->fw * sizeof(float) || stride_bytes % sizeof(float)) return fail(c, MVSV_ERR_INVALID, "bad map stride");
-    rc = prepare_maps(c, cam, roi_x, roi_y, roi_w, roi_h);
+    rc = prepare_maps(c, rig, cam, roi_x, roi_y, roi_w, roi_h);
     if (rc) return rc;
     float *dx = nullptr, *dy = nullptr;
     const size_t mbytes = (size_t)c->fw * c->fh * sizeof(float);
@@ -604,18 +666,25 @@ int mvsv_upload_rectify_maps(mvsv_ctx* c, int cam, const float* mapx, const floa
     const size_t w = (size_t)c->fw * sizeof(float);
     e = cudaMemcpy2DAsync(dx, w, mapx, stride_bytes, w, c->fh, cudaMemcpyHostToDevice, c->stream);
     if (e == cudaSuccess) e = cudaMemcpy2DAsync(dy, w, mapy, stride_bytes, w, c->fh, cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) e = launch_convert_maps(c, cam, dx, dy, (size_t)c->fw);
+    if (e == cudaSuccess) e = launch_convert_maps(c, rig, cam, dx, dy, (size_t)c->fw);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
     cudaFree(dx); cudaFree(dy);
     if (e != cudaSuccess) { c->err = std::string("map upload: ") + cudaGetErrorString(e); return MVSV_ERR_CUDA; }
-    c->has_maps[cam] = true;
+    c->has_maps[rig][cam] = true;
     return MVSV_OK;
 }
 
 int mvsv_set_rectification(mvsv_ctx* c, int cam, const double K[9], const double* dist, int n_dist, const double R[9],
                            const double P[12], int roi_x, int roi_y, int roi_w, int roi_h)
 {
+    return mvsv_set_rectification_rig(c, 0, cam, K, dist, n_dist, R, P, roi_x, roi_y, roi_w, roi_h);
+}
+
+int mvsv_set_rectification_rig(mvsv_ctx* c, int rig, int cam, const double K[9], const double* dist, int n_dist,
+                               const double R[9], const double P[12], int roi_x, int roi_y, int roi_w, int roi_h)
+{
     if (!c || !K || !R || !P || cam < 0 || cam > 1 || n_dist < 0 || (n_dist > 0 && !dist)) return MVSV_ERR_INVALID;
+    if (rig < 0 || rig >= MVSV_MAX_RIGS) return fail(c, MVSV_ERR_INVALID, "rig outside [0, MVSV_MAX_RIGS)");
     int rc = bind(c);
     if (rc) return rc;
     if (n_dist != 0 && n_dist != 4 && n_dist != 5)
@@ -639,11 +708,11 @@ int mvsv_set_rectification(mvsv_ctx* c, int cam, const double K[9], const double
     q.k1 = n_dist > 0 ? dist[0] : 0; q.k2 = n_dist > 1 ? dist[1] : 0; q.p1 = n_dist > 2 ? dist[2] : 0;
     q.p2 = n_dist > 3 ? dist[3] : 0; q.k3 = n_dist > 4 ? dist[4] : 0;
     q.fx = K[0]; q.fy = K[4]; q.cx = K[2]; q.cy = K[5];
-    rc = prepare_maps(c, cam, roi_x, roi_y, roi_w, roi_h);
+    rc = prepare_maps(c, rig, cam, roi_x, roi_y, roi_w, roi_h);
     if (rc) return rc;
-    MVSV_CK(c, launch_rectify_maps(c, cam, q));
+    MVSV_CK(c, launch_rectify_maps(c, rig, cam, q));
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
-    c->has_maps[cam] = true;
+    c->has_maps[rig][cam] = true;
     return MVSV_OK;
 }
 
@@ -653,8 +722,12 @@ int mvsv_reset_rectification(mvsv_ctx* c)
     int rc = bind(c);
     if (rc) return rc;
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
-    c->has_maps[0] = c->has_maps[1] = false;
-    for (int i = 0; i < 2; ++i) dfree(c->map_xy[i]);
+    for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+        for (int i = 0; i < 2; ++i) {
+            c->has_maps[r][i] = false;
+            dfree(c->map_xy[r][i]);
+        }
+    c->rig_tables_dirty = true;
     return apply_geometry(c);
 }
 
@@ -702,11 +775,57 @@ int mvsv_tm(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* rig
     return MVSV_OK;
 }
 
-int mvsv_set_Q(mvsv_ctx* c, const float q[16])
+int mvsv_set_Q(mvsv_ctx* c, const float q[16]) { return mvsv_set_Q_rig(c, 0, q); }
+
+int mvsv_set_Q_rig(mvsv_ctx* c, int rig, const float q[16])
 {
     if (!c || !q) return MVSV_ERR_INVALID;
-    std::memcpy(c->Q, q, sizeof(float) * 16);
-    c->has_Q = true;
+    if (rig < 0 || rig >= MVSV_MAX_RIGS) return fail(c, MVSV_ERR_INVALID, "rig outside [0, MVSV_MAX_RIGS)");
+    std::memcpy(c->Q[rig], q, sizeof(float) * 16);
+    c->has_Q[rig] = true;
+    c->rig_tables_dirty = true;
+    return MVSV_OK;
+}
+
+int mvsv_set_frame_rigs(mvsv_ctx* c, const int* rig_of_frame, int n)
+{
+    if (!c || n < 0 || (n > 0 && !rig_of_frame)) return MVSV_ERR_INVALID;
+    if (n > c->maxB) return fail(c, MVSV_ERR_INVALID, "more frames than max_batch");
+    for (int i = 0; i < n; ++i)
+        if (rig_of_frame[i] < 0 || rig_of_frame[i] >= MVSV_MAX_RIGS)
+            return fail(c, MVSV_ERR_INVALID, "rig of frame " + std::to_string(i) + " outside [0, MVSV_MAX_RIGS)");
+    int rc = bind(c);
+    if (rc) return rc;
+    // every frame of max_batch: the given rig, rig 0 past n; the order sorted by rig (stable), cut into remap chunks
+    const int B = c->maxB;
+    std::vector<int> rig(B, 0);
+    std::copy(rig_of_frame, rig_of_frame + n, rig.begin());
+    std::vector<int> order(B);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return rig[a] < rig[b]; });
+    std::vector<int4> chunk;
+    for (int i = 0; i < B; ++i) {
+        const int r = rig[order[i]];
+        if (chunk.empty() || chunk.back().x != r || chunk.back().z == RM_FRAMES) chunk.push_back(make_int4(r, i, 0, 0));
+        ++chunk.back().z;
+    }
+    MVSV_CK(c, cudaStreamSynchronize(c->stream));
+    RigFrames& t = c->rig_frames;
+    if (!t.chunk) {
+        MVSV_CK(c, cudaMalloc(&t.chunk, (size_t)B * (sizeof(int4) + 2 * sizeof(int))));
+        t.order = reinterpret_cast<int*>(t.chunk + B);
+        t.rig = t.order + B;
+    }
+    if (!c->rig_tables) {
+        MVSV_CK(c, cudaMalloc(&c->rig_tables, sizeof(RigTables)));
+        c->rig_tables_dirty = true;
+    }
+    MVSV_CK(c, cudaMemcpyAsync(t.chunk, chunk.data(), chunk.size() * sizeof(int4), cudaMemcpyHostToDevice, c->stream));
+    MVSV_CK(c, cudaMemcpyAsync(t.order, order.data(), (size_t)B * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    MVSV_CK(c, cudaMemcpyAsync(t.rig, rig.data(), (size_t)B * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    MVSV_CK(c, cudaStreamSynchronize(c->stream));
+    t.nchunks = (int)chunk.size();
+    c->frame_rig.assign(rig_of_frame, rig_of_frame + n);
     return MVSV_OK;
 }
 
@@ -900,7 +1019,9 @@ int mvsv_debug_postfilter(mvsv_ctx* c, const int16_t* maps, size_t stride, int b
     if (stages & ~(unsigned)(MVSV_STAGE_XYZ | MVSV_STAGE_MEANS))
         return fail(c, MVSV_ERR_INVALID, "post-filter hook: only MVSV_STAGE_XYZ and MVSV_STAGE_MEANS");
     if (maxSpeckleSize > 0 && (newVal < -32768 || newVal > 32767)) return fail(c, MVSV_ERR_INVALID, "newVal does not fit CV_16S");
-    rc = check_consumers(c, slot, stages);
+    const uint64_t rigs = rigs_of_batch(c, batch);
+    const bool multi = rigs != 1;
+    rc = check_consumers(c, slot, stages, rigs);
     if (rc) return rc;
     if ((stages & MVSV_STAGE_XYZ) && !slot.xyz) MVSV_CK(c, cudaMalloc(&slot.xyz, (size_t)c->maxB * c->H * c->W * 3 * sizeof(float)));
 
@@ -914,7 +1035,13 @@ int mvsv_debug_postfilter(mvsv_ctx* c, const int16_t* maps, size_t stride, int b
             MVSV_CK(c, launch_speckle(c, median ? c->disp_med : c->disp_raw, slot.disp, batch, newVal, maxSpeckleSize, maxDiff));
         if (!median && !speckle)
             MVSV_CK(c, cudaMemcpyAsync(slot.disp, c->disp_raw, npx * sizeof(int16_t), cudaMemcpyDeviceToDevice, c->stream));
-        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, launch_xyz(c, batch));
+        if (stages & MVSV_STAGE_XYZ) {
+            if (multi) {
+                const int r = upload_rig_tables(c);
+                if (r) return r;
+            }
+            MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
+        }
         if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
         MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
         MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
@@ -935,9 +1062,9 @@ long long mvsv_debug_read(mvsv_ctx* c, int which, void* host, size_t cap)
     size_t bytes = 0;
     if (which == 7 || which == 8) {
         const int cam = which - 7;
-        if (!c->has_maps[cam]) return fail(c, MVSV_ERR_STATE, "no rectification map for this camera");
-        src = c->map_xy[cam];
-        bytes = (size_t)c->roi[2] * c->roi[3] * sizeof(int2);
+        if (!c->has_maps[0][cam]) return fail(c, MVSV_ERR_STATE, "no rectification map for this camera");
+        src = c->map_xy[0][cam];
+        bytes = (size_t)c->roi_w * c->roi_h * sizeof(int2);
         if (bytes > cap) return fail(c, MVSV_ERR_INVALID, "host buffer too small");
         MVSV_CK(c, cudaMemcpyAsync(host, src, bytes, cudaMemcpyDeviceToHost, c->stream));
         MVSV_CK(c, cudaStreamSynchronize(c->stream));

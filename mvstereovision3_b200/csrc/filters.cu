@@ -46,16 +46,15 @@ __device__ __forceinline__ int sat16(int v) { return max(-32768, min(32767, v));
 
 // One thread = four neighbouring output pixels of up to RM_FRAMES frames: the map entries and the bilinear weights are
 // the same for every frame of the batch, so they are fetched and expanded once and only the four taps per pixel are
-// gathered per frame; the four results leave as one 32-bit store.
-constexpr int RM_FRAMES = 8;
+// gathered per frame; the four results leave as one 32-bit store.  RM_FRAMES: mvsv_internal.h
 
-__global__ void __launch_bounds__(128)
-k_remap(const uint8_t* __restrict__ src, size_t spitch, int fw, int fh, const int2* __restrict__ map,
-        uint8_t* __restrict__ dst, size_t dpitch, int W, int H, int B)
+// frames f0 .. f1-1 of the batch (single rig), or, ORDERED, the frames order[f0 .. f1-1] that are below B (one rig)
+template <bool ORDERED>
+__device__ __forceinline__ void
+remap_frames(const uint8_t* __restrict__ src, size_t spitch, int fw, int fh, const int2* __restrict__ map,
+             uint8_t* __restrict__ dst, size_t dpitch, int W, int H, int B, int x4, int y, int f0, int f1,
+             const int* __restrict__ order)
 {
-    const int x4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4, y = blockIdx.y;
-    if (x4 >= W) return;
-    const int f0 = blockIdx.z * RM_FRAMES, f1 = min(f0 + RM_FRAMES, B);
     int off[4][4];              // byte offsets of the four taps inside a frame, -1 = outside (BORDER_CONSTANT 0)
     int wgt[4][4];
 #pragma unroll
@@ -72,7 +71,9 @@ k_remap(const uint8_t* __restrict__ src, size_t spitch, int fw, int fh, const in
         wgt[k][0] = (32 - fx) * (32 - fy) * 32; wgt[k][1] = fx * (32 - fy) * 32;
         wgt[k][2] = (32 - fx) * fy * 32; wgt[k][3] = fx * fy * 32;
     }
-    for (int f = f0; f < f1; ++f) {
+    for (int i = f0; i < f1; ++i) {
+        const int f = ORDERED ? order[i] : i;
+        if (ORDERED && f >= B) break;                       // a chunk's frames ascend: the rest are past the batch too
         const uint8_t* s = src + (size_t)f * fh * spitch;
         unsigned out = 0;
 #pragma unroll
@@ -89,6 +90,30 @@ k_remap(const uint8_t* __restrict__ src, size_t spitch, int fw, int fh, const in
             for (int k = 0; x4 + k < W; ++k) d[k] = (uint8_t)(out >> (8 * k));
         }
     }
+}
+
+__global__ void __launch_bounds__(128)
+k_remap(const uint8_t* __restrict__ src, size_t spitch, int fw, int fh, const int2* __restrict__ map,
+        uint8_t* __restrict__ dst, size_t dpitch, int W, int H, int B)
+{
+    const int x4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4, y = blockIdx.y;
+    if (x4 >= W) return;
+    const int f0 = blockIdx.z * RM_FRAMES, f1 = min(f0 + RM_FRAMES, B);
+    remap_frames<false>(src, spitch, fw, fh, map, dst, dpitch, W, H, B, x4, y, f0, f1, nullptr);
+}
+
+// Frames of several rigs: blockIdx.z walks the chunks of mvsv_set_frame_rigs, each up to RM_FRAMES frames of one rig,
+// which read and write at their own batch index through their rig's map.
+__global__ void __launch_bounds__(128)
+k_remap_rigs(const uint8_t* __restrict__ src, size_t spitch, int fw, int fh, const RigTables* __restrict__ rigs, int cam,
+             const int4* __restrict__ chunks, const int* __restrict__ order, uint8_t* __restrict__ dst, size_t dpitch,
+             int W, int H, int B)
+{
+    const int x4 = (blockIdx.x * blockDim.x + threadIdx.x) * 4, y = blockIdx.y;
+    if (x4 >= W) return;
+    const int4 ch = chunks[blockIdx.z];                     // rig, first, count
+    if (order[ch.y] >= B) return;
+    remap_frames<true>(src, spitch, fw, fh, rigs->map[cam][ch.x], dst, dpitch, W, H, B, x4, y, ch.y, ch.y + ch.z, order);
 }
 
 // cv::resize(src, dst, Size(0,0), f, f) for CV_8UC1, default INTER_LINEAR (reference src/Stereosystem.cpp:294-295):
@@ -398,7 +423,9 @@ k_ccl_apply(const int16_t* __restrict__ img, int16_t* __restrict__ out, const in
 struct QMat { double q[16]; };     // the CV_32F matrix, widened on the host (cv::Mat_<float> products accumulate in double)
 
 // One thread = four consecutive pixels of the batch's linear pixel index: one 8-byte load, three 16-byte stores.
-__global__ void __launch_bounds__(256) k_xyz(const int16_t* __restrict__ disp, float* __restrict__ xyz, int W, int H, size_t npx, QMat Q)
+// q(f, i) is element i of the Q of frame f (the four pixels may cross a frame boundary).
+template <class QOf>
+__device__ __forceinline__ void xyz_pixels(const int16_t* __restrict__ disp, float* __restrict__ xyz, int W, int H, size_t npx, QOf q)
 {
     const size_t i0 = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) * 4;
     if (i0 >= npx) return;
@@ -411,6 +438,7 @@ __global__ void __launch_bounds__(256) k_xyz(const int16_t* __restrict__ disp, f
     }
     const size_t row = i0 / W;
     int x = (int)(i0 - row * W), y = (int)(row % H);
+    int f = (int)(row / H);
     double dx = (double)x, dy = (double)y;                  // exact: the reference's float coordinates are integers < 2^24
     float o[12];
 #pragma unroll
@@ -423,10 +451,10 @@ __global__ void __launch_bounds__(256) k_xyz(const int16_t* __restrict__ disp, f
 #pragma unroll
             for (int r = 0; r < 4; ++r) {
                 // ((((0 + q0 x) + q1 y) + q2 d) + q3 1): every product of two floats is exact in double, one rounding per add
-                double acc = Q.q[r * 4] * dx;
-                acc = __fma_rn(Q.q[r * 4 + 1], dy, acc);
-                acc = __fma_rn(Q.q[r * 4 + 2], dd, acc);
-                acc += Q.q[r * 4 + 3];
+                double acc = q(f, r * 4) * dx;
+                acc = __fma_rn(q(f, r * 4 + 1), dy, acc);
+                acc = __fma_rn(q(f, r * 4 + 2), dd, acc);
+                acc += q(f, r * 4 + 3);
                 cc[r] = (float)acc;
             }
             X = cc[0] / cc[3]; Y = cc[1] / cc[3]; Z = cc[2] / cc[3];
@@ -434,7 +462,7 @@ __global__ void __launch_bounds__(256) k_xyz(const int16_t* __restrict__ disp, f
         }
         o[3 * k] = X; o[3 * k + 1] = Y; o[3 * k + 2] = Z;
         dx += 1.0;
-        if (++x == W) { x = 0; dx = 0.0; if (++y == H) y = 0; dy = (double)y; }
+        if (++x == W) { x = 0; dx = 0.0; if (++y == H) { y = 0; ++f; } dy = (double)y; }
     }
     float* dst = xyz + i0 * 3;
     if (i0 + 3 < npx) {
@@ -443,6 +471,19 @@ __global__ void __launch_bounds__(256) k_xyz(const int16_t* __restrict__ disp, f
     } else {
         for (int k = 0; i0 + k < npx; ++k) { dst[3 * k] = o[3 * k]; dst[3 * k + 1] = o[3 * k + 1]; dst[3 * k + 2] = o[3 * k + 2]; }
     }
+}
+
+__global__ void __launch_bounds__(256) k_xyz(const int16_t* __restrict__ disp, float* __restrict__ xyz, int W, int H, size_t npx, QMat Q)
+{
+    xyz_pixels(disp, xyz, W, H, npx, [&](int, int i) { return Q.q[i]; });
+}
+
+// Frames of several rigs: each pixel reprojects with the Q of its frame's rig, with the same arithmetic as k_xyz.
+__global__ void __launch_bounds__(256)
+k_xyz_rigs(const int16_t* __restrict__ disp, float* __restrict__ xyz, int W, int H, size_t npx, const RigTables* __restrict__ rigs,
+           const int* __restrict__ rig_of_frame)
+{
+    xyz_pixels(disp, xyz, W, H, npx, [&](int f, int i) { return rigs->Q[rig_of_frame[f]][i]; });
 }
 
 // Eight lanes per ROI (and frame), four ROIs per warp: the reference's Samplepoint windows are 5 x 5 pixels (a whole warp
@@ -507,37 +548,49 @@ cudaError_t launch_minmax(mvsv_ctx* c, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t strideElems)
+cudaError_t launch_convert_maps(mvsv_ctx* c, int rig, int cam, const float* dmapx, const float* dmapy, size_t strideElems)
 {
-    dim3 blk(128), grd((c->roi[2] + 127) / 128, c->roi[3]);
+    dim3 blk(128), grd((c->roi_w + 127) / 128, c->roi_h);
     KernelTimer kt(c, KID_REMAP);
-    k_convert_maps<<<grd, blk, 0, c->stream>>>(dmapx, dmapy, strideElems, c->roi[0], c->roi[1], c->roi[2], c->roi[3],
-                                               c->map_xy[cam]);
+    k_convert_maps<<<grd, blk, 0, c->stream>>>(dmapx, dmapy, strideElems, c->roi_xy[rig][0], c->roi_xy[rig][1], c->roi_w, c->roi_h,
+                                               c->map_xy[rig][cam]);
     return cudaGetLastError();
 }
 
-cudaError_t launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q)
+cudaError_t launch_rectify_maps(mvsv_ctx* c, int rig, int cam, const RectifyCoef& q)
 {
-    dim3 blk(128), grd((c->roi[2] + 127) / 128, c->roi[3]);
+    dim3 blk(128), grd((c->roi_w + 127) / 128, c->roi_h);
     KernelTimer kt(c, KID_REMAP);
-    k_rectify_maps<<<grd, blk, 0, c->stream>>>(q, c->roi[0], c->roi[1], c->roi[2], c->roi[3], c->map_xy[cam]);
+    k_rectify_maps<<<grd, blk, 0, c->stream>>>(q, c->roi_xy[rig][0], c->roi_xy[rig][1], c->roi_w, c->roi_h, c->map_xy[rig][cam]);
     return cudaGetLastError();
 }
 
 cudaError_t launch_remap(mvsv_ctx* c, int cam, int B)
 {
-    const int rw = c->roi[2], rh = c->roi[3];
+    const int rw = c->roi_w, rh = c->roi_h;
     const bool resized = c->resize_factor > 0.0;
     dim3 blk(128), grd((rw + 511) / 512, rh, (B + RM_FRAMES - 1) / RM_FRAMES);
     KernelTimer kt(c, KID_REMAP);
-    k_remap<<<grd, blk, 0, c->stream>>>(io(c).raw[cam], c->raw_pitch, c->fw, c->fh, c->map_xy[cam],
+    k_remap<<<grd, blk, 0, c->stream>>>(io(c).raw[cam], c->raw_pitch, c->fw, c->fh, c->map_xy[0][cam],
                                         resized ? c->crop[cam] : io(c).rect[cam], resized ? c->crop_pitch : c->pitch, rw, rh, B);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_remap_rigs(mvsv_ctx* c, int cam, int B)
+{
+    const int rw = c->roi_w, rh = c->roi_h;
+    const bool resized = c->resize_factor > 0.0;
+    const RigFrames& t = c->rig_frames;
+    dim3 blk(128), grd((rw + 511) / 512, rh, t.nchunks);
+    KernelTimer kt(c, KID_REMAP);
+    k_remap_rigs<<<grd, blk, 0, c->stream>>>(io(c).raw[cam], c->raw_pitch, c->fw, c->fh, c->rig_tables, cam, t.chunk, t.order,
+                                             resized ? c->crop[cam] : io(c).rect[cam], resized ? c->crop_pitch : c->pitch, rw, rh, B);
     return cudaGetLastError();
 }
 
 cudaError_t launch_resize(mvsv_ctx* c, int cam, int B)
 {
-    const int rw = c->roi[2], rh = c->roi[3];
+    const int rw = c->roi_w, rh = c->roi_h;
     const double scale = 1.0 / c->resize_factor;
     const long iscale = lrint(scale);
     dim3 blk(128), grd((c->W + 127) / 128, c->H, B);
@@ -584,10 +637,19 @@ cudaError_t launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B,
 cudaError_t launch_xyz(mvsv_ctx* c, int B)
 {
     QMat Q;
-    for (int i = 0; i < 16; ++i) Q.q[i] = (double)c->Q[i];
+    for (int i = 0; i < 16; ++i) Q.q[i] = (double)c->Q[0][i];
     const size_t npx = (size_t)B * c->H * c->W;
     KernelTimer kt(c, KID_XYZ);
     k_xyz<<<(unsigned)((npx / 4 + 256) / 256), 256, 0, c->stream>>>(io(c).disp, io(c).xyz, c->W, c->H, npx, Q);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_xyz_rigs(mvsv_ctx* c, int B)
+{
+    const size_t npx = (size_t)B * c->H * c->W;
+    KernelTimer kt(c, KID_XYZ);
+    k_xyz_rigs<<<(unsigned)((npx / 4 + 256) / 256), 256, 0, c->stream>>>(io(c).disp, io(c).xyz, c->W, c->H, npx, c->rig_tables,
+                                                                         c->rig_frames.rig);
     return cudaGetLastError();
 }
 

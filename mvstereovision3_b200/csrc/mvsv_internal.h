@@ -52,6 +52,25 @@ struct IoSlot {
     unsigned stages = 0;
 };
 
+// frames per thread of the remap kernel (csrc/filters.cu), and the largest chunk of one rig's frames it takes
+constexpr int RM_FRAMES = 8;
+
+// Device tables of mvsv_set_frame_rigs (one allocation of max_batch entries each), built on the host from the frame ->
+// rig table.  The remap kernel expands a map entry once for up to RM_FRAMES frames, which must then share the rig: it
+// walks `chunk`, runs of at most RM_FRAMES frames of one rig in `order`.
+struct RigFrames {
+    int4* chunk = nullptr;                    // (rig, first index into order, count <= RM_FRAMES, 0)
+    int* order = nullptr;                     // frames sorted by rig, ascending within a rig
+    int* rig = nullptr;                       // rig of each frame
+    int nchunks = 0;
+};
+
+// What the rig-aware kernels read of every rig: the fixed-point maps and Q widened to double (k_xyz's QMat).
+struct RigTables {
+    const int2* map[2][MVSV_MAX_RIGS];
+    double Q[MVSV_MAX_RIGS][16];
+};
+
 struct mvsv_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;
@@ -78,10 +97,12 @@ struct mvsv_ctx {
     cudaEvent_t timer_a = nullptr, timer_b = nullptr;
     std::string err;
 
-    // rectification (device): per camera, fixed-point maps for the ROI only
-    bool has_maps[2] = {false, false};
-    int roi[4] = {0, 0, 0, 0};
-    int2* map_xy[2] = {nullptr, nullptr};     // (ix, iy) = rint(map*32), saturated int32
+    // rectification (device): per rig and camera, fixed-point maps for the rig's display ROI only.  All rigs share the
+    // ROI size; rig r's ROI starts at roi_xy[r] of the frame.  Rig 0 is the single-rig engine.
+    bool has_maps[MVSV_MAX_RIGS][2] = {};
+    int roi_w = 0, roi_h = 0;
+    int roi_xy[MVSV_MAX_RIGS][2] = {};
+    int2* map_xy[MVSV_MAX_RIGS][2] = {};      // (ix, iy) = rint(map*32), saturated int32
     size_t raw_pitch = 0;
     // cv::resize(.., factor, factor) after the crop (Stereosystem::getRectifiedImagepair(sip, factor),
     // reference src/Stereosystem.cpp:279-315); off when resize_factor == 0
@@ -125,8 +146,17 @@ struct mvsv_ctx {
     size_t bm_vol_elems = 0;
     uint16_t* bm_col = nullptr;               // [B][H][width1][Dp]
 
-    bool has_Q = false;
-    float Q[16];
+    bool has_Q[MVSV_MAX_RIGS] = {};
+    float Q[MVSV_MAX_RIGS][16];
+
+    // mvsv_set_frame_rigs: frame i of a compute comes from rig frame_rig[i] (frames past its end: rig 0).  While every
+    // frame of a compute comes from rig 0 the single-rig kernels run; otherwise the rig-aware ones, which read the
+    // device tables below.
+    std::vector<int> frame_rig;
+    RigFrames rig_frames;
+    RigTables* rig_tables = nullptr;          // device mirror of map_xy and Q; refreshed by a compute when rig_tables_dirty
+    bool rig_tables_dirty = true;
+
     int nrois = 0;
     int* rois = nullptr;                      // device [n][4]
     int* minmax = nullptr;                    // device [B][2]
@@ -166,11 +196,12 @@ struct KernelTimer {
 // there before (function attributes are per device; engines on several devices and threads share this state).
 cudaError_t smem_limit(const void* kernel, int bytes);
 cudaError_t launch_remap(mvsv_ctx* c, int cam, int B);
+cudaError_t launch_remap_rigs(mvsv_ctx* c, int cam, int B);      // frames of several rigs (mvsv_set_frame_rigs)
 cudaError_t launch_resize(mvsv_ctx* c, int cam, int B);
 // inverse of P[:, :3]*R, camera matrix and distortion of one camera (cv::initUndistortRectifyMap's inputs)
 struct RectifyCoef { double iR[9]; double k1, k2, p1, p2, k3; double fx, fy, cx, cy; };
-cudaError_t launch_rectify_maps(mvsv_ctx* c, int cam, const RectifyCoef& q);
-cudaError_t launch_convert_maps(mvsv_ctx* c, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
+cudaError_t launch_rectify_maps(mvsv_ctx* c, int rig, int cam, const RectifyCoef& q);
+cudaError_t launch_convert_maps(mvsv_ctx* c, int rig, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
 cudaError_t launch_sgbm(mvsv_ctx* c, int B);
 cudaError_t launch_bm(mvsv_ctx* c, int B);
 int bm_lrcheck_max_width();
@@ -178,6 +209,7 @@ size_t tm_smem_bytes(int W, int k);
 int tm_max_width();
 cudaError_t launch_tm(mvsv_ctx* c, int B, int k, uint8_t* out, size_t opitch);
 cudaError_t launch_xyz(mvsv_ctx* c, int B);
+cudaError_t launch_xyz_rigs(mvsv_ctx* c, int B);                 // frames of several rigs (mvsv_set_frame_rigs)
 cudaError_t launch_means(mvsv_ctx* c, int B);
 cudaError_t launch_minmax(mvsv_ctx* c, int B);
 cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B);
