@@ -10,6 +10,9 @@
  * Threading contract (reference: one worker std::thread calls Disparity::sgbm,
  * trgt/demo.cpp:68-77,195): a ctx is thread-compatible -- any thread may call, one at a time.
  * Several ctxs (one per GPU or stream) may run concurrently.
+ *
+ * Multi-device ctx (mvsv_init_devices): one ctx over several engines, each on one of the listed devices.  Every entry
+ * point accepts it; the comments below say where its behaviour differs from that of an mvsv_init ctx.
  */
 #ifndef MVSV_H_
 #define MVSV_H_
@@ -75,7 +78,39 @@ typedef struct mvsv_info {
  * objects the drivers create (trgt/demo.cpp:190-194) and Stereosystem's rectification state. */
 int mvsv_init(int device, int frame_width, int frame_height, int max_batch, mvsv_ctx** out);
 void mvsv_destroy(mvsv_ctx* ctx);
-const char* mvsv_last_error(const mvsv_ctx* ctx); /* ctx may be NULL: error of the last failed mvsv_init */
+const char* mvsv_last_error(const mvsv_ctx* ctx); /* ctx may be NULL: error of the last failed mvsv_init(_devices) */
+
+/* One ctx over the devices devices[0 .. n-1] (one engine per GPU of a box, behind one handle).  Part k is an engine of
+ * mvsv_init(devices[k], frame_width, frame_height, ceil(max_batch / n)); the ctx holds n * ceil(max_batch / n) frames.
+ * A device may be listed more than once: its parts are separate engines, each with its own volumes.  n == 1 is exactly
+ * mvsv_init(devices[0], ...).  Rejected with MVSV_ERR_INVALID: devices == NULL, n < 1, n > max_batch, and whatever
+ * mvsv_init rejects for one of the parts (also with its code, e.g. MVSV_ERR_CUDA without a device); a failure frees the
+ * parts already created, leaves *out == NULL and puts the text, prefixed with the part, in mvsv_last_error(NULL).
+ *   Compute: a batch of b frames gives part k the contiguous frames [floor(k*b/n), floor((k+1)*b/n)), read at
+ *     base + first*frame_stride (host or device memory; device inputs on another device are copied peer to peer).  When
+ *     b < n some parts get no frames.  Every part is checked (arguments, state, rigs, consumers, allocations) before any
+ *     part submits: a rejected compute leaves the results of earlier ones downloadable, as on one engine; a failure while
+ *     submitting leaves the compute's I/O slot empty on every part.  Every compute advances the I/O slot of every part,
+ *     so the slots of all parts always hold the same compute.
+ *   Setters (parameters, filters, maps, rectification, resize, Q, ROIs, I/O slots) are repeated on every part in order.
+ *     The parts hold the same state, so an argument or state rejection comes from part 0 before any part changed.  A
+ *     CUDA or allocation error of such a call (e.g. a device with less free memory than the others) can leave the parts
+ *     different and marks the ctx broken: every later call except mvsv_destroy, mvsv_last_error and mvsv_get_info then
+ *     returns MVSV_ERR_STATE.  A part's error text is prefixed with its index and device.
+ *   mvsv_set_frame_rigs keeps the whole table; a compute hands each part its slice for that batch when the slice differs
+ *     from the one the part holds (the part's mvsv_set_frame_rigs, which waits for that part's stream).  While the batch
+ *     size stays the same nothing is re-sent; changing the batch size with a rig table installed costs that wait.
+ *   Downloads queue the copies of every part (at out + first*height*stride, XYZ and means likewise) before they wait, so
+ *     that the parts' copies run side by side; mvsv_download_minmax launches on every part, then gathers.
+ *   mvsv_get_info: part 0's fields, except max_batch (all parts), last_batch (all frames of the last compute) and device
+ *     (devices[0]).  mvsv_sync: every part.  mvsv_launch_count: the sum.  mvsv_timer_start / stop: events on every part;
+ *     stop returns the longest part's interval.  mvsv_stream: NULL.
+ *   Not available (MVSV_ERR_UNSUPPORTED; use a single-device engine): mvsv_tm, mvsv_profile_enable / read and the test
+ *     hooks mvsv_debug_set_flags, mvsv_debug_read, mvsv_debug_postfilter.
+ * No reference counterpart (the reference runs one pair at a time on the CPU). */
+int mvsv_init_devices(const int* devices, int n, int frame_width, int frame_height, int max_batch, mvsv_ctx** out);
+/* The devices of a ctx: returns the number of parts (1 for an mvsv_init ctx) and writes up to n of their ids. */
+int mvsv_get_devices(const mvsv_ctx* ctx, int* devices, int n);
 
 /* Replaces the eight StereoSGBM setters + setMode of Disparity::loadSGBMParameters
  * (src/disparity.cpp:83-95).  Parameters outside the bit-exact contract are rejected:
@@ -161,7 +196,8 @@ int mvsv_set_mean_rois(mvsv_ctx* ctx, const int* xywh, int n);
  * MVSV_STAGE_RECTIFY the inputs are raw frames (frame size),
  * otherwise rectified pairs (width x height of mvsv_get_info).  Strides in bytes.  A call that fails before it submits
  * work (arguments, engine state, allocation) leaves the results of earlier calls as they were; one that fails while
- * submitting leaves no results (mvsv_download then returns MVSV_ERR_STATE). */
+ * submitting leaves no results (mvsv_download then returns MVSV_ERR_STATE).  Multi-device ctx: the batch is split
+ * across the parts (mvsv_init_devices). */
 int mvsv_compute(mvsv_ctx* ctx, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride,
                  size_t frame_stride, int batch, unsigned stages);
 /* Same, inputs already resident in device memory (used for the HBM-resident bench figure and pipelines
@@ -203,7 +239,8 @@ int mvsv_download_minmax(mvsv_ctx* ctx, int16_t* minmax);
 int mvsv_sync(mvsv_ctx* ctx);
 
 int mvsv_get_info(const mvsv_ctx* ctx, mvsv_info* info);
-/* The CUDA stream (cudaStream_t) all work of this ctx is issued on -- for CUDA-event timing by the caller. */
+/* The CUDA stream (cudaStream_t) all work of this ctx is issued on -- for CUDA-event timing by the caller.  NULL for a
+ * multi-device ctx, whose parts each have their own (time it with mvsv_timer_start / stop). */
 void* mvsv_stream(mvsv_ctx* ctx);
 /* Number of kernel launches issued by this ctx since creation (bench.py's gpu_launches). */
 unsigned long long mvsv_launch_count(const mvsv_ctx* ctx);
@@ -221,7 +258,8 @@ int mvsv_profile_enable(mvsv_ctx* ctx, int enable);
 int mvsv_profile_read(mvsv_ctx* ctx, float* ms, int* counts, int n);
 const char* mvsv_kernel_name(int kid);
 
-/* Pinned host memory for zero-staging async copies. */
+/* Pinned host memory for zero-staging async copies.  With unified addressing (every 64-bit platform CUDA supports) it
+ * counts as pinned on every device, so one buffer serves all parts of a multi-device ctx. */
 int mvsv_host_alloc(void** p, size_t bytes);
 int mvsv_host_free(void* p);
 

@@ -280,7 +280,9 @@ int bind(mvsv_ctx* c)
 int upload_images(mvsv_ctx* c, uint8_t* dst, size_t dpitch, const uint8_t* src, size_t sstride, size_t frame_stride, int w,
                   int h, int batch, bool device_src)
 {
-    const cudaMemcpyKind kind = device_src ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    // device inputs may live on another device than the ctx (the parts of a multi-device ctx all read one batch):
+    // cudaMemcpyDefault lets unified addressing find both ends, and copies peer to peer where they differ
+    const cudaMemcpyKind kind = device_src ? cudaMemcpyDefault : cudaMemcpyHostToDevice;
     cudaStream_t st = device_src ? c->stream : c->copy_stream;
     if (sstride == (size_t)w && dpitch == (size_t)w && (batch == 1 || frame_stride == (size_t)w * h)) {
         MVSV_CK(c, cudaMemcpyAsync(dst, src, (size_t)w * h * batch, kind, st));
@@ -314,23 +316,21 @@ int check_consumers(mvsv_ctx* c, const IoSlot& slot, unsigned stages, uint64_t r
     return MVSV_OK;
 }
 
-int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride, int batch,
-        unsigned stages, bool device_src)
+}  // namespace
+
+int compute_check(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, int batch,
+                  unsigned stages)
 {
-    if (!c) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
     // next I/O slot; its previous results must have been downloaded by now (mvsv_set_io_slots)
-    const int k = (c->cur + 1) % c->nslots;
-    IoSlot& slot = c->slot[k];
+    IoSlot& slot = c->slot[(c->cur + 1) % c->nslots];
     const bool rectify = stages & MVSV_STAGE_RECTIFY;
     if (!left || !right || batch < 1 || batch > c->maxB) return fail(c, MVSV_ERR_INVALID, "bad image pointers or batch size");
     if ((stages & MVSV_STAGE_SGBM) && (stages & MVSV_STAGE_BM)) return fail(c, MVSV_ERR_INVALID, "choose SGBM or BM, not both");
     if ((stages & MVSV_STAGE_SGBM) && !c->has_sgbm) return fail(c, MVSV_ERR_STATE, "mvsv_set_sgbm_params not called");
     if ((stages & MVSV_STAGE_BM) && !c->has_bm) return fail(c, MVSV_ERR_STATE, "mvsv_set_bm_params not called");
-    // frames of rigs other than 0: the rig-aware remap and XYZ kernels
     const uint64_t rigs = rigs_of_batch(c, batch);
-    const bool multi = rigs != 1;
     rc = check_consumers(c, slot, stages, rigs);
     if (rc) return rc;
     if (rectify)
@@ -340,24 +340,36 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
                                                       : "rectify maps of rig " + std::to_string(r) + " missing (mvsv_upload_rectify_maps_rig)");
     if ((stages & MVSV_STAGE_BM) && c->bm_d12 >= 0 && c->W > bm_lrcheck_max_width())
         return fail(c, MVSV_ERR_UNSUPPORTED, "BM left-right check (disp12MaxDiff >= 0): image wider than 4096");
-    const int iw = rectify ? c->fw : c->W, ih = rectify ? c->fh : c->H;
+    const int iw = rectify ? c->fw : c->W;
     if (lstride < (size_t)iw || rstride < (size_t)iw)
         return fail(c, MVSV_ERR_INVALID, rectify ? "stride smaller than frame width" : "stride smaller than image width");
     if (stages & MVSV_STAGE_SGBM) rc = ensure_sgbm_volumes(c);
     else if (stages & MVSV_STAGE_BM) rc = ensure_bm_volumes(c);
     if (rc) return rc;
     if ((stages & MVSV_STAGE_XYZ) && !slot.xyz) MVSV_CK(c, cudaMalloc(&slot.xyz, (size_t)c->maxB * c->H * c->W * 3 * sizeof(float)));
+    return MVSV_OK;
+}
 
+int compute_submit(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
+                   int batch, unsigned stages, bool device_src)
+{
     // From here on the slot is taken: if a step fails it is left empty, so that a download reports the failure instead
     // of returning the frames of an older compute.
-    c->cur = k;
+    c->cur = (c->cur + 1) % c->nslots;
+    IoSlot& slot = io(c);
+    const bool rectify = stages & MVSV_STAGE_RECTIFY;
+    const int iw = rectify ? c->fw : c->W, ih = rectify ? c->fh : c->H;
+    // frames of rigs other than 0: the rig-aware remap and XYZ kernels
+    const bool multi = rigs_of_batch(c, batch) != 1;
     auto submit = [&]() -> int {
+        int r = bind(c);
+        if (r) return r;
         // host inputs: the copies wait for the slot's previous compute (which may still read the input buffers), the
         // kernels wait for the copies
         if (!device_src) MVSV_CK(c, cudaStreamWaitEvent(c->copy_stream, slot.done, 0));
         uint8_t* const* dst = rectify ? slot.raw : slot.rect;
         const size_t dpitch = rectify ? c->raw_pitch : c->pitch;
-        int r = upload_images(c, dst[0], dpitch, left, lstride, frame_stride, iw, ih, batch, device_src);
+        r = upload_images(c, dst[0], dpitch, left, lstride, frame_stride, iw, ih, batch, device_src);
         if (!r) r = upload_images(c, dst[1], dpitch, right, rstride, frame_stride, iw, ih, batch, device_src);
         if (!r) r = inputs_uploaded(c, device_src);
         if (r) return r;
@@ -378,16 +390,23 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
         MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
         return MVSV_OK;
     };
-    rc = submit();
+    const int rc = submit();
     slot.B = rc ? 0 : batch;
     slot.stages = rc ? 0 : stages;
     return rc;
 }
 
-// Copies the results a compute left in I/O slot `k` to the host on the download stream (so that it overlaps kernels
-// submitted later) and waits for them.
-int download_slot(mvsv_ctx* c, int k, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride, float* xyz,
-                  float* means)
+void compute_skip(mvsv_ctx* c)
+{
+    c->cur = (c->cur + 1) % c->nslots;
+    io(c).B = 0;
+    io(c).stages = 0;
+}
+
+// Queues the copies of the results a compute left in I/O slot `k` to the host on the download stream (so that they
+// overlap kernels submitted later); download_wait waits for them.
+int download_enqueue(mvsv_ctx* c, int k, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
+                     float* xyz, float* means)
 {
     IoSlot& s = c->slot[k];
     const int B = s.B;
@@ -416,11 +435,53 @@ int download_slot(mvsv_ctx* c, int k, int16_t* disp, size_t dstride, uint8_t* re
         if (!s.means || !(s.stages & MVSV_STAGE_MEANS)) return fail(c, MVSV_ERR_STATE, "MEANS stage was not computed");
         MVSV_CK(c, cudaMemcpyAsync(means, s.means, (size_t)B * c->nrois * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
-    MVSV_CK(c, cudaStreamSynchronize(st));
     return MVSV_OK;
 }
 
+int download_wait(mvsv_ctx* c)
+{
+    MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));
+    return MVSV_OK;
+}
+
+int minmax_launch(mvsv_ctx* c)
+{
+    const int B = io(c).B;
+    if (B < 1) return fail(c, MVSV_ERR_STATE, "nothing computed yet");
+    if (!c->minmax) MVSV_CK(c, cudaMalloc(&c->minmax, (size_t)c->maxB * 2 * sizeof(int)));
+    MVSV_CK(c, launch_minmax(c, B));
+    return MVSV_OK;
+}
+
+int minmax_read(mvsv_ctx* c, int16_t* minmax)
+{
+    const int B = io(c).B;
+    std::vector<int> h((size_t)2 * B);
+    MVSV_CK(c, cudaMemcpyAsync(h.data(), c->minmax, h.size() * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    MVSV_CK(c, cudaStreamSynchronize(c->stream));
+    for (int i = 0; i < B; ++i) {
+        const bool none = h[2 * i + 1] <= 0;
+        minmax[2 * i] = none ? 0 : (int16_t)h[2 * i];
+        minmax[2 * i + 1] = none ? 0 : (int16_t)h[2 * i + 1];
+    }
+    return MVSV_OK;
+}
+
+namespace {
+
+int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride, int batch,
+        unsigned stages, bool device_src)
+{
+    if (!c) return MVSV_ERR_INVALID;
+    if (is_multi(c)) return parts_compute(c, left, lstride, right, rstride, frame_stride, batch, stages, device_src);
+    const int rc = compute_check(c, left, lstride, right, rstride, batch, stages);
+    if (rc) return rc;
+    return compute_submit(c, left, lstride, right, rstride, frame_stride, batch, stages, device_src);
+}
+
 }  // namespace
+
+std::string& init_error() { return g_init_error; }
 
 extern "C" {
 
@@ -482,6 +543,7 @@ int mvsv_init(int device, int frame_width, int frame_height, int max_batch, mvsv
 void mvsv_destroy(mvsv_ctx* c)
 {
     if (!c) return;
+    if (is_multi(c)) { parts_destroy(c); return; }
     cudaSetDevice(c->device);
     if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
     if (c->dl_stream) cudaStreamSynchronize(c->dl_stream);
@@ -519,6 +581,7 @@ const char* mvsv_last_error(const mvsv_ctx* c) { return c ? c->err.c_str() : g_i
 
 int mvsv_set_sgbm_params(mvsv_ctx* c, const mvsv_sgbm_params* p)
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_set_sgbm_params(q, p); });
     if (!c || !p) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -533,6 +596,7 @@ int mvsv_set_sgbm_params(mvsv_ctx* c, const mvsv_sgbm_params* p)
 
 int mvsv_set_bm_params(mvsv_ctx* c, const mvsv_bm_params* p)
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_set_bm_params(q, p); });
     if (!c || !p) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -546,6 +610,8 @@ int mvsv_set_bm_params(mvsv_ctx* c, const mvsv_bm_params* p)
 
 int mvsv_set_bm_filters(mvsv_ctx* c, int disp12MaxDiff, int speckleWindowSize, int speckleRange)
 {
+    if (is_multi(c))
+        return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_set_bm_filters(q, disp12MaxDiff, speckleWindowSize, speckleRange); });
     if (!c) return MVSV_ERR_INVALID;
     if (speckleWindowSize < 0) return fail(c, MVSV_ERR_INVALID, "BM speckleWindowSize must be >= 0");
     if (speckleWindowSize > 0 && speckleRange < 0) return fail(c, MVSV_ERR_INVALID, "BM speckleRange must be >= 0");
@@ -651,6 +717,10 @@ int mvsv_upload_rectify_maps(mvsv_ctx* c, int cam, const float* mapx, const floa
 int mvsv_upload_rectify_maps_rig(mvsv_ctx* c, int rig, int cam, const float* mapx, const float* mapy, size_t stride_bytes,
                                  int roi_x, int roi_y, int roi_w, int roi_h)
 {
+    if (is_multi(c))
+        return parts_each(c, true, [&](mvsv_ctx* q) {
+            return mvsv_upload_rectify_maps_rig(q, rig, cam, mapx, mapy, stride_bytes, roi_x, roi_y, roi_w, roi_h);
+        });
     if (!c || !mapx || !mapy || cam < 0 || cam > 1) return MVSV_ERR_INVALID;
     if (rig < 0 || rig >= MVSV_MAX_RIGS) return fail(c, MVSV_ERR_INVALID, "rig outside [0, MVSV_MAX_RIGS)");
     int rc = bind(c);
@@ -683,6 +753,10 @@ int mvsv_set_rectification(mvsv_ctx* c, int cam, const double K[9], const double
 int mvsv_set_rectification_rig(mvsv_ctx* c, int rig, int cam, const double K[9], const double* dist, int n_dist,
                                const double R[9], const double P[12], int roi_x, int roi_y, int roi_w, int roi_h)
 {
+    if (is_multi(c))
+        return parts_each(c, true, [&](mvsv_ctx* q) {
+            return mvsv_set_rectification_rig(q, rig, cam, K, dist, n_dist, R, P, roi_x, roi_y, roi_w, roi_h);
+        });
     if (!c || !K || !R || !P || cam < 0 || cam > 1 || n_dist < 0 || (n_dist > 0 && !dist)) return MVSV_ERR_INVALID;
     if (rig < 0 || rig >= MVSV_MAX_RIGS) return fail(c, MVSV_ERR_INVALID, "rig outside [0, MVSV_MAX_RIGS)");
     int rc = bind(c);
@@ -718,6 +792,7 @@ int mvsv_set_rectification_rig(mvsv_ctx* c, int rig, int cam, const double K[9],
 
 int mvsv_reset_rectification(mvsv_ctx* c)
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_reset_rectification(q); });
     if (!c) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -733,6 +808,7 @@ int mvsv_reset_rectification(mvsv_ctx* c)
 
 int mvsv_set_resize(mvsv_ctx* c, double factor)
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_set_resize(q, factor); });
     if (!c) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -750,6 +826,7 @@ int mvsv_set_resize(mvsv_ctx* c, double factor)
 int mvsv_tm(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
             int batch, unsigned kernel_size, uint8_t* out, size_t ostride)
 {
+    if (is_multi(c)) return parts_unsupported(c, "mvsv_tm");
     if (!c || !left || !right || !out) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -779,6 +856,7 @@ int mvsv_set_Q(mvsv_ctx* c, const float q[16]) { return mvsv_set_Q_rig(c, 0, q);
 
 int mvsv_set_Q_rig(mvsv_ctx* c, int rig, const float q[16])
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* p) { return mvsv_set_Q_rig(p, rig, q); });
     if (!c || !q) return MVSV_ERR_INVALID;
     if (rig < 0 || rig >= MVSV_MAX_RIGS) return fail(c, MVSV_ERR_INVALID, "rig outside [0, MVSV_MAX_RIGS)");
     std::memcpy(c->Q[rig], q, sizeof(float) * 16);
@@ -789,6 +867,7 @@ int mvsv_set_Q_rig(mvsv_ctx* c, int rig, const float q[16])
 
 int mvsv_set_frame_rigs(mvsv_ctx* c, const int* rig_of_frame, int n)
 {
+    if (is_multi(c)) return parts_set_frame_rigs(c, rig_of_frame, n);
     if (!c || n < 0 || (n > 0 && !rig_of_frame)) return MVSV_ERR_INVALID;
     if (n > c->maxB) return fail(c, MVSV_ERR_INVALID, "more frames than max_batch");
     for (int i = 0; i < n; ++i)
@@ -831,6 +910,7 @@ int mvsv_set_frame_rigs(mvsv_ctx* c, const int* rig_of_frame, int n)
 
 int mvsv_set_mean_rois(mvsv_ctx* c, const int* xywh, int n)
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_set_mean_rois(q, xywh, n); });
     if (!c || n < 0 || (n > 0 && !xywh)) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -873,14 +953,18 @@ int mvsv_download_age(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8
                       float* xyz, float* means)
 {
     if (!c) return MVSV_ERR_INVALID;
+    if (is_multi(c)) return parts_download(c, age, disp, dstride, rectL, rectR, rstride, xyz, means);
     int rc = bind(c);
     if (rc) return rc;
     if (age < 0 || age >= c->nslots) return fail(c, MVSV_ERR_INVALID, "age must be below the number of I/O slots");
-    return download_slot(c, (c->cur + c->nslots - age) % c->nslots, disp, dstride, rectL, rectR, rstride, xyz, means);
+    rc = download_enqueue(c, (c->cur + c->nslots - age) % c->nslots, disp, dstride, rectL, rectR, rstride, xyz, means);
+    if (rc) return rc;
+    return download_wait(c);
 }
 
 int mvsv_set_io_slots(mvsv_ctx* c, int n)
 {
+    if (is_multi(c)) return parts_each(c, true, [&](mvsv_ctx* q) { return mvsv_set_io_slots(q, n); });
     if (!c) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -899,26 +983,18 @@ int mvsv_set_io_slots(mvsv_ctx* c, int n)
 int mvsv_download_minmax(mvsv_ctx* c, int16_t* minmax)
 {
     if (!c || !minmax) return MVSV_ERR_INVALID;
+    if (is_multi(c)) return parts_download_minmax(c, minmax);
     int rc = bind(c);
     if (rc) return rc;
-    const int B = io(c).B;
-    if (B < 1) return fail(c, MVSV_ERR_STATE, "nothing computed yet");
-    if (!c->minmax) MVSV_CK(c, cudaMalloc(&c->minmax, (size_t)c->maxB * 2 * sizeof(int)));
-    MVSV_CK(c, launch_minmax(c, B));
-    std::vector<int> h((size_t)2 * B);
-    MVSV_CK(c, cudaMemcpyAsync(h.data(), c->minmax, h.size() * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    MVSV_CK(c, cudaStreamSynchronize(c->stream));
-    for (int i = 0; i < B; ++i) {
-        const bool none = h[2 * i + 1] <= 0;
-        minmax[2 * i] = none ? 0 : (int16_t)h[2 * i];
-        minmax[2 * i + 1] = none ? 0 : (int16_t)h[2 * i + 1];
-    }
-    return MVSV_OK;
+    rc = minmax_launch(c);
+    if (rc) return rc;
+    return minmax_read(c, minmax);
 }
 
 int mvsv_sync(mvsv_ctx* c)
 {
     if (!c) return MVSV_ERR_INVALID;
+    if (is_multi(c)) return parts_each(c, false, [&](mvsv_ctx* q) { return mvsv_sync(q); });
     int rc = bind(c);
     if (rc) return rc;
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
@@ -928,6 +1004,7 @@ int mvsv_sync(mvsv_ctx* c)
 int mvsv_get_info(const mvsv_ctx* c, mvsv_info* info)
 {
     if (!c || !info) return MVSV_ERR_INVALID;
+    if (is_multi(c)) return parts_get_info(c, info);
     std::memset(info, 0, sizeof(*info));
     info->frame_width = c->fw; info->frame_height = c->fh; info->width = c->W; info->height = c->H; info->max_batch = c->maxB;
     if (c->has_sgbm) {
@@ -941,8 +1018,12 @@ int mvsv_get_info(const mvsv_ctx* c, mvsv_info* info)
     return MVSV_OK;
 }
 
-void* mvsv_stream(mvsv_ctx* c) { return c ? (void*)c->stream : nullptr; }
-unsigned long long mvsv_launch_count(const mvsv_ctx* c) { return c ? c->launches : 0ull; }
+void* mvsv_stream(mvsv_ctx* c) { return c ? (void*)c->stream : nullptr; }   // NULL for a multi-device ctx
+unsigned long long mvsv_launch_count(const mvsv_ctx* c)
+{
+    if (is_multi(c)) return parts_launch_count(c);
+    return c ? c->launches : 0ull;
+}
 
 int mvsv_host_alloc(void** p, size_t bytes)
 {
@@ -954,6 +1035,7 @@ int mvsv_host_free(void* p) { return cudaFreeHost(p) == cudaSuccess ? MVSV_OK : 
 int mvsv_timer_start(mvsv_ctx* c)
 {
     if (!c) return MVSV_ERR_INVALID;
+    if (is_multi(c)) return parts_each(c, false, [&](mvsv_ctx* q) { return mvsv_timer_start(q); });
     int rc = bind(c);
     if (rc) return rc;
     if (!c->timer_a) { MVSV_CK(c, cudaEventCreate(&c->timer_a)); MVSV_CK(c, cudaEventCreate(&c->timer_b)); }
@@ -963,6 +1045,7 @@ int mvsv_timer_start(mvsv_ctx* c)
 
 int mvsv_timer_stop(mvsv_ctx* c, float* ms)
 {
+    if (is_multi(c)) return parts_timer_stop(c, ms);
     if (!c || !ms || !c->timer_a) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -974,6 +1057,7 @@ int mvsv_timer_stop(mvsv_ctx* c, float* ms)
 
 int mvsv_profile_enable(mvsv_ctx* c, int enable)
 {
+    if (is_multi(c)) return parts_unsupported(c, "mvsv_profile_enable");
     if (!c) return MVSV_ERR_INVALID;
     c->prof = enable != 0;
     return MVSV_OK;
@@ -981,6 +1065,7 @@ int mvsv_profile_enable(mvsv_ctx* c, int enable)
 
 int mvsv_profile_read(mvsv_ctx* c, float* ms, int* counts, int n)
 {
+    if (is_multi(c)) return parts_unsupported(c, "mvsv_profile_read");
     if (!c || !ms || !counts || n < KID_COUNT) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -999,6 +1084,7 @@ const char* mvsv_kernel_name(int kid) { return (kid >= 0 && kid < KID_COUNT) ? k
 
 int mvsv_debug_set_flags(mvsv_ctx* c, unsigned flags)
 {
+    if (is_multi(c)) return parts_unsupported(c, "mvsv_debug_set_flags");
     if (!c) return MVSV_ERR_INVALID;
     c->debug_flags = flags;
     if (c->has_sgbm) c->td_nc = sgbm_choose_td_cluster(c);
@@ -1008,6 +1094,7 @@ int mvsv_debug_set_flags(mvsv_ctx* c, unsigned flags)
 int mvsv_debug_postfilter(mvsv_ctx* c, const int16_t* maps, size_t stride, int batch, int median, int newVal,
                           int maxSpeckleSize, int maxDiff, unsigned stages)
 {
+    if (is_multi(c)) return parts_unsupported(c, "mvsv_debug_postfilter");
     if (!c) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;
@@ -1055,6 +1142,7 @@ int mvsv_debug_postfilter(mvsv_ctx* c, const int16_t* maps, size_t stride, int b
 
 long long mvsv_debug_read(mvsv_ctx* c, int which, void* host, size_t cap)
 {
+    if (is_multi(c)) return parts_unsupported(c, "mvsv_debug_read");
     if (!c || !host) return MVSV_ERR_INVALID;
     int rc = bind(c);
     if (rc) return rc;

@@ -71,7 +71,13 @@ struct RigTables {
     double Q[MVSV_MAX_RIGS][16];
 };
 
+struct Parts;   // csrc/devices.cpp
+
 struct mvsv_ctx {
+    // mvsv_init_devices: the engines this ctx splits its batches across (NULL for an mvsv_init ctx).  Such a ctx holds no
+    // device state of its own; of the fields below it uses device (the first part's), maxB (the parts' total), frame_rig
+    // (the whole table), nslots / cur / slot[k].B (the frames of each I/O slot's compute, all parts together) and err.
+    Parts* parts = nullptr;
     int device = 0;
     cudaStream_t stream = nullptr;
     // host->device input copies run on their own stream so that they overlap the kernels of the other I/O slot's
@@ -164,6 +170,48 @@ struct mvsv_ctx {
 
 // the I/O slot of the compute in progress (or of the last one)
 inline IoSlot& io(mvsv_ctx* c) { return c->slot[c->cur]; }
+
+// ---- host steps of a single-device ctx that a multi-device ctx runs on each of its parts (csrc/api.cu) ---------------
+// mvsv_compute = compute_check (arguments, state, allocations; takes no I/O slot) + compute_submit (takes the next slot,
+// queues copies and kernels; a failure leaves the slot empty).  compute_skip takes the next slot and leaves it empty.
+int compute_check(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, int batch,
+                  unsigned stages);
+int compute_submit(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
+                   int batch, unsigned stages, bool device_src);
+void compute_skip(mvsv_ctx* c);
+// mvsv_download_age = download_enqueue (copies of I/O slot k on the download stream) + download_wait
+int download_enqueue(mvsv_ctx* c, int k, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
+                     float* xyz, float* means);
+int download_wait(mvsv_ctx* c);
+// mvsv_download_minmax = minmax_launch + minmax_read
+int minmax_launch(mvsv_ctx* c);
+int minmax_read(mvsv_ctx* c, int16_t* minmax);
+
+// the text of the last failed mvsv_init / mvsv_init_devices of the calling thread (mvsv_last_error(NULL))
+std::string& init_error();
+
+// ---- multi-device ctx (mvsv_init_devices, csrc/devices.cpp) -----------------------------------------------------------
+inline bool is_multi(const mvsv_ctx* c) { return c && c->parts; }
+// Runs `call` on every part in order, stopping at the first failure, whose text it prefixes with the part's index and
+// device.  `setter`: the call changes engine state, so a failure that can leave the parts different (a CUDA or
+// allocation error, or any failure past part 0) marks the ctx broken.
+int parts_each(mvsv_ctx* c, bool setter, int (*call)(mvsv_ctx* part, const void* arg), const void* arg);
+template <class F>
+int parts_each(mvsv_ctx* c, bool setter, F&& f)
+{
+    return parts_each(c, setter, [](mvsv_ctx* p, const void* a) { return (*static_cast<const F*>(a))(p); }, &f);
+}
+int parts_unsupported(mvsv_ctx* c, const char* what);
+int parts_set_frame_rigs(mvsv_ctx* c, const int* rig_of_frame, int n);
+int parts_compute(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
+                  int batch, unsigned stages, bool device_src);
+int parts_download(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
+                   float* xyz, float* means);
+int parts_download_minmax(mvsv_ctx* c, int16_t* minmax);
+int parts_timer_stop(mvsv_ctx* c, float* ms);
+int parts_get_info(const mvsv_ctx* c, mvsv_info* info);
+unsigned long long parts_launch_count(const mvsv_ctx* c);
+void parts_destroy(mvsv_ctx* c);
 
 // RAII bracket: records CUDA events on the ctx stream around one kernel launch when profiling is on.
 struct KernelTimer {
