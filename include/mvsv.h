@@ -97,9 +97,10 @@ const char* mvsv_last_error(const mvsv_ctx* ctx); /* ctx may be NULL: error of t
  *     CUDA or allocation error of such a call (e.g. a device with less free memory than the others) can leave the parts
  *     different and marks the ctx broken: every later call except mvsv_destroy, mvsv_last_error and mvsv_get_info then
  *     returns MVSV_ERR_STATE.  A part's error text is prefixed with its index and device.
- *   mvsv_set_frame_rigs keeps the whole table; a compute hands each part its slice for that batch when the slice differs
- *     from the one the part holds (the part's mvsv_set_frame_rigs, which waits for that part's stream).  While the batch
- *     size stays the same nothing is re-sent; changing the batch size with a rig table installed costs that wait.
+ *   mvsv_set_frame_rigs keeps the whole table; a compute hands each part the table from the part's first frame on (as
+ *     far as the part's capacity reaches) when it differs from the one the part holds, which waits for that part's
+ *     stream.  While the batch size stays the same nothing is re-sent; a batch size that moves a part's first frame
+ *     costs that wait with a rig table installed.
  *   Downloads queue the copies of every part (at out + first*height*stride, XYZ and means likewise) before they wait, so
  *     that the parts' copies run side by side; mvsv_download_minmax launches on every part, then gathers.
  *   mvsv_get_info: part 0's fields, except max_batch (all parts), last_batch (all frames of the last compute) and device

@@ -516,7 +516,7 @@ static int bm_wta_cta_warps(size_t warpBytes, int* warpsPerSm)
 }
 
 template <int OPL, bool RING, bool B8>
-static cudaError_t launch_bm_wta(mvsv_ctx* c, const BmArgs& a, int* cost, int ringSlots, int ctaWarps)
+static cudaError_t launch_bm_wta(Engine* c, const BmArgs& a, int* cost, int ringSlots, int ctaWarps)
 {
     const int NL = (a.D / 8) / OPL, rowsPerWarp = 32 / NL;
     const long long warps = ((long long)a.B * (a.H - 2 * a.w2) + rowsPerWarp - 1) / rowsPerWarp;
@@ -636,13 +636,13 @@ __global__ void k_fill16(int16_t* p, size_t n, int16_t v)
 int bm_lrcheck_max_width() { return BM_LR_MAXW; }
 
 // the map after the matcher (and the left-right check) -> the speckle filter -> the slot's disparities
-static cudaError_t bm_speckle(mvsv_ctx* c, int B)
+static cudaError_t bm_speckle(Engine* c, int B)
 {
     if (c->bm_speckle_win <= 0) return cudaSuccess;
     return launch_speckle(c, c->disp_raw, io(c).disp, B, c->bm.FILT, c->bm_speckle_win, c->bm_speckle_range);
 }
 
-cudaError_t launch_bm(mvsv_ctx* c, int B)
+cudaError_t launch_bm(Engine* c, int B)
 {
     const BmNorm& n = c->bm;
     const bool col8 = n.col8 && !(c->debug_flags & 2u);         // debug bit 1: never keep a volume as bytes

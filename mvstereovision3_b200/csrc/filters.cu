@@ -539,7 +539,7 @@ __global__ void k_minmax(const int16_t* __restrict__ disp, int* __restrict__ mm,
 
 }  // namespace
 
-cudaError_t launch_minmax(mvsv_ctx* c, int B)
+cudaError_t launch_minmax(Engine* c, int B)
 {
     { KernelTimer kt(c, KID_MINMAX); k_minmax_init<<<(2 * B + 127) / 128, 128, 0, c->stream>>>(c->minmax, 2 * B); }
     dim3 grd(32, B);
@@ -548,7 +548,7 @@ cudaError_t launch_minmax(mvsv_ctx* c, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_convert_maps(mvsv_ctx* c, int rig, int cam, const float* dmapx, const float* dmapy, size_t strideElems)
+cudaError_t launch_convert_maps(Engine* c, int rig, int cam, const float* dmapx, const float* dmapy, size_t strideElems)
 {
     dim3 blk(128), grd((c->roi_w + 127) / 128, c->roi_h);
     KernelTimer kt(c, KID_REMAP);
@@ -557,7 +557,7 @@ cudaError_t launch_convert_maps(mvsv_ctx* c, int rig, int cam, const float* dmap
     return cudaGetLastError();
 }
 
-cudaError_t launch_rectify_maps(mvsv_ctx* c, int rig, int cam, const RectifyCoef& q)
+cudaError_t launch_rectify_maps(Engine* c, int rig, int cam, const RectifyCoef& q)
 {
     dim3 blk(128), grd((c->roi_w + 127) / 128, c->roi_h);
     KernelTimer kt(c, KID_REMAP);
@@ -565,7 +565,7 @@ cudaError_t launch_rectify_maps(mvsv_ctx* c, int rig, int cam, const RectifyCoef
     return cudaGetLastError();
 }
 
-cudaError_t launch_remap(mvsv_ctx* c, int cam, int B)
+cudaError_t launch_remap(Engine* c, int cam, int B)
 {
     const int rw = c->roi_w, rh = c->roi_h;
     const bool resized = c->resize_factor > 0.0;
@@ -576,7 +576,7 @@ cudaError_t launch_remap(mvsv_ctx* c, int cam, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_remap_rigs(mvsv_ctx* c, int cam, int B)
+cudaError_t launch_remap_rigs(Engine* c, int cam, int B)
 {
     const int rw = c->roi_w, rh = c->roi_h;
     const bool resized = c->resize_factor > 0.0;
@@ -588,7 +588,7 @@ cudaError_t launch_remap_rigs(mvsv_ctx* c, int cam, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_resize(mvsv_ctx* c, int cam, int B)
+cudaError_t launch_resize(Engine* c, int cam, int B)
 {
     const int rw = c->roi_w, rh = c->roi_h;
     const double scale = 1.0 / c->resize_factor;
@@ -602,7 +602,7 @@ cudaError_t launch_resize(mvsv_ctx* c, int cam, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B)
+cudaError_t launch_median(Engine* c, const int16_t* in, int16_t* out, int B)
 {
     KernelTimer kt(c, KID_MEDIAN);
     const bool scalar = c->debug_flags & 4u;        // debug bit 2: k_median3 also where k_median3_w4 qualifies
@@ -617,7 +617,7 @@ cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff)
+cudaError_t launch_speckle(Engine* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff)
 {
     const int W = c->W, H = c->H;
     const size_t n = (size_t)B * W * H;
@@ -634,7 +634,7 @@ cudaError_t launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B,
     return cudaGetLastError();
 }
 
-cudaError_t launch_xyz(mvsv_ctx* c, int B)
+cudaError_t launch_xyz(Engine* c, int B)
 {
     QMat Q;
     for (int i = 0; i < 16; ++i) Q.q[i] = (double)c->Q[0][i];
@@ -644,7 +644,7 @@ cudaError_t launch_xyz(mvsv_ctx* c, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_xyz_rigs(mvsv_ctx* c, int B)
+cudaError_t launch_xyz_rigs(Engine* c, int B)
 {
     const size_t npx = (size_t)B * c->H * c->W;
     KernelTimer kt(c, KID_XYZ);
@@ -653,7 +653,7 @@ cudaError_t launch_xyz_rigs(mvsv_ctx* c, int B)
     return cudaGetLastError();
 }
 
-cudaError_t launch_means(mvsv_ctx* c, int B)
+cudaError_t launch_means(Engine* c, int B)
 {
     if (c->nrois <= 0) return cudaSuccess;
     dim3 grd((c->nrois + MEANS_WARPS * 4 - 1) / (MEANS_WARPS * 4), B);

@@ -71,13 +71,9 @@ struct RigTables {
     double Q[MVSV_MAX_RIGS][16];
 };
 
-struct Parts;   // csrc/devices.cpp
-
-struct mvsv_ctx {
-    // mvsv_init_devices: the engines this ctx splits its batches across (NULL for an mvsv_init ctx).  Such a ctx holds no
-    // device state of its own; of the fields below it uses device (the first part's), maxB (the parts' total), frame_rig
-    // (the whole table), nslots / cur / slot[k].B (the frames of each I/O slot's compute, all parts together) and err.
-    Parts* parts = nullptr;
+// One engine on one device: its streams, events, volumes and I/O slots.  An mvsv_ctx (csrc/api.cu) splits every batch
+// across one or more of them.
+struct Engine {
     int device = 0;
     cudaStream_t stream = nullptr;
     // host->device input copies run on their own stream so that they overlap the kernels of the other I/O slot's
@@ -169,55 +165,13 @@ struct mvsv_ctx {
 };
 
 // the I/O slot of the compute in progress (or of the last one)
-inline IoSlot& io(mvsv_ctx* c) { return c->slot[c->cur]; }
+inline IoSlot& io(Engine* c) { return c->slot[c->cur]; }
 
-// ---- host steps of a single-device ctx that a multi-device ctx runs on each of its parts (csrc/api.cu) ---------------
-// mvsv_compute = compute_check (arguments, state, allocations; takes no I/O slot) + compute_submit (takes the next slot,
-// queues copies and kernels; a failure leaves the slot empty).  compute_skip takes the next slot and leaves it empty.
-int compute_check(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, int batch,
-                  unsigned stages);
-int compute_submit(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
-                   int batch, unsigned stages, bool device_src);
-void compute_skip(mvsv_ctx* c);
-// mvsv_download_age = download_enqueue (copies of I/O slot k on the download stream) + download_wait
-int download_enqueue(mvsv_ctx* c, int k, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
-                     float* xyz, float* means);
-int download_wait(mvsv_ctx* c);
-// mvsv_download_minmax = minmax_launch + minmax_read
-int minmax_launch(mvsv_ctx* c);
-int minmax_read(mvsv_ctx* c, int16_t* minmax);
-
-// the text of the last failed mvsv_init / mvsv_init_devices of the calling thread (mvsv_last_error(NULL))
-std::string& init_error();
-
-// ---- multi-device ctx (mvsv_init_devices, csrc/devices.cpp) -----------------------------------------------------------
-inline bool is_multi(const mvsv_ctx* c) { return c && c->parts; }
-// Runs `call` on every part in order, stopping at the first failure, whose text it prefixes with the part's index and
-// device.  `setter`: the call changes engine state, so a failure that can leave the parts different (a CUDA or
-// allocation error, or any failure past part 0) marks the ctx broken.
-int parts_each(mvsv_ctx* c, bool setter, int (*call)(mvsv_ctx* part, const void* arg), const void* arg);
-template <class F>
-int parts_each(mvsv_ctx* c, bool setter, F&& f)
-{
-    return parts_each(c, setter, [](mvsv_ctx* p, const void* a) { return (*static_cast<const F*>(a))(p); }, &f);
-}
-int parts_unsupported(mvsv_ctx* c, const char* what);
-int parts_set_frame_rigs(mvsv_ctx* c, const int* rig_of_frame, int n);
-int parts_compute(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
-                  int batch, unsigned stages, bool device_src);
-int parts_download(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
-                   float* xyz, float* means);
-int parts_download_minmax(mvsv_ctx* c, int16_t* minmax);
-int parts_timer_stop(mvsv_ctx* c, float* ms);
-int parts_get_info(const mvsv_ctx* c, mvsv_info* info);
-unsigned long long parts_launch_count(const mvsv_ctx* c);
-void parts_destroy(mvsv_ctx* c);
-
-// RAII bracket: records CUDA events on the ctx stream around one kernel launch when profiling is on.
+// RAII bracket: records CUDA events on the engine's stream around one kernel launch when profiling is on.
 struct KernelTimer {
-    mvsv_ctx* c; int idx;
+    Engine* c; int idx;
     cudaStream_t st;
-    KernelTimer(mvsv_ctx* ctx, int kid, cudaStream_t on = nullptr) : c(ctx), idx(-1), st(on ? on : ctx->stream)
+    KernelTimer(Engine* ctx, int kid, cudaStream_t on = nullptr) : c(ctx), idx(-1), st(on ? on : ctx->stream)
     {
         ++c->launches;
         if (!c->prof) return;
@@ -243,33 +197,33 @@ struct KernelTimer {
 // Sets a kernel's cudaFuncAttributeMaxDynamicSharedMemorySize on the current device when it differs from the value set
 // there before (function attributes are per device; engines on several devices and threads share this state).
 cudaError_t smem_limit(const void* kernel, int bytes);
-cudaError_t launch_remap(mvsv_ctx* c, int cam, int B);
-cudaError_t launch_remap_rigs(mvsv_ctx* c, int cam, int B);      // frames of several rigs (mvsv_set_frame_rigs)
-cudaError_t launch_resize(mvsv_ctx* c, int cam, int B);
+cudaError_t launch_remap(Engine* c, int cam, int B);
+cudaError_t launch_remap_rigs(Engine* c, int cam, int B);      // frames of several rigs (mvsv_set_frame_rigs)
+cudaError_t launch_resize(Engine* c, int cam, int B);
 // inverse of P[:, :3]*R, camera matrix and distortion of one camera (cv::initUndistortRectifyMap's inputs)
 struct RectifyCoef { double iR[9]; double k1, k2, p1, p2, k3; double fx, fy, cx, cy; };
-cudaError_t launch_rectify_maps(mvsv_ctx* c, int rig, int cam, const RectifyCoef& q);
-cudaError_t launch_convert_maps(mvsv_ctx* c, int rig, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
-cudaError_t launch_sgbm(mvsv_ctx* c, int B);
-cudaError_t launch_bm(mvsv_ctx* c, int B);
+cudaError_t launch_rectify_maps(Engine* c, int rig, int cam, const RectifyCoef& q);
+cudaError_t launch_convert_maps(Engine* c, int rig, int cam, const float* dmapx, const float* dmapy, size_t stride_elems);
+cudaError_t launch_sgbm(Engine* c, int B);
+cudaError_t launch_bm(Engine* c, int B);
 int bm_lrcheck_max_width();
 size_t tm_smem_bytes(int W, int k);
 int tm_max_width();
-cudaError_t launch_tm(mvsv_ctx* c, int B, int k, uint8_t* out, size_t opitch);
-cudaError_t launch_xyz(mvsv_ctx* c, int B);
-cudaError_t launch_xyz_rigs(mvsv_ctx* c, int B);                 // frames of several rigs (mvsv_set_frame_rigs)
-cudaError_t launch_means(mvsv_ctx* c, int B);
-cudaError_t launch_minmax(mvsv_ctx* c, int B);
-cudaError_t launch_median(mvsv_ctx* c, const int16_t* in, int16_t* out, int B);
-cudaError_t launch_speckle(mvsv_ctx* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
+cudaError_t launch_tm(Engine* c, int B, int k, uint8_t* out, size_t opitch);
+cudaError_t launch_xyz(Engine* c, int B);
+cudaError_t launch_xyz_rigs(Engine* c, int B);                 // frames of several rigs (mvsv_set_frame_rigs)
+cudaError_t launch_means(Engine* c, int B);
+cudaError_t launch_minmax(Engine* c, int B);
+cudaError_t launch_median(Engine* c, const int16_t* in, int16_t* out, int B);
+cudaError_t launch_speckle(Engine* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
 // fused previous-row sweep (csrc/sweep.cu): strip decomposition of a batch, scratch sizes, launch
 struct SweepPlan { int NS = 0, NF = 0, Mmax = 0, threads = 0, G = 0, NR = 0; size_t smem = 0; };
 void sweep_layout(int D, int* G, int* NR);
-void sweep_plan(const mvsv_ctx* c, int B, int forcedNS, SweepPlan* p);
-size_t sweep_scratch_bytes(const mvsv_ctx* c);
-bool sweep_s8_ok(const mvsv_ctx* c, const SweepPlan& p);
-cudaError_t launch_sweep(mvsv_ctx* c, int B, const SweepPlan& p, int bottomUp, bool s8);
-int sgbm_choose_td_cluster(mvsv_ctx* c);
+void sweep_plan(const Engine* c, int B, int forcedNS, SweepPlan* p);
+size_t sweep_scratch_bytes(const Engine* c);
+bool sweep_s8_ok(const Engine* c, const SweepPlan& p);
+cudaError_t launch_sweep(Engine* c, int B, const SweepPlan& p, int bottomUp, bool s8);
+int sgbm_choose_td_cluster(Engine* c);
 void sgbm_plane_geometry(const SgbmNorm& n, int W, int* NV, int* RP, int* JOFF);
 bool sgbm_vsum_wide(const SgbmNorm& n);
 

@@ -800,7 +800,7 @@ size_t vsum_smem_bytes(int bs, bool r8)
 }
 
 template <int G, bool PAD>
-cudaError_t launch_sgbm_g(mvsv_ctx* c, int B)
+cudaError_t launch_sgbm_g(Engine* c, int B)
 {
     const SgbmNorm& n = c->sg;
     cudaStream_t st = c->stream;
@@ -895,7 +895,7 @@ cudaError_t launch_sgbm_g(mvsv_ctx* c, int B)
     // (MVSV_SERIAL=1 does the same for a whole process: under ncu every kernel runs alone anyway, and the chunked cost
     // kernel then shows its partial waves without the scan that fills them)
     static const bool serialEnv = [] { const char* e = getenv("MVSV_SERIAL"); return e && atoi(e) != 0; }();
-    const int nchunks = (c->prof || serialEnv) ? 1 : std::min((B + fpc - 1) / fpc, (int)mvsv_ctx::kMaxChunks);
+    const int nchunks = (c->prof || serialEnv) ? 1 : std::min((B + fpc - 1) / fpc, (int)Engine::kMaxChunks);
     if (nchunks <= 1) {
         MVSV_TRY(launch_vsum(0, B));
         launch_h1(0, B, st);
@@ -931,7 +931,7 @@ cudaError_t launch_sgbm_g(mvsv_ctx* c, int B)
 
 // Strips per frame the fused previous-row sweep uses for a full batch (reported by mvsv_get_info);
 // 0 = it cannot run (volume stride differs from the sweep's lane layout, or forced off): independent passes.
-int sgbm_choose_td_cluster(mvsv_ctx* c)
+int sgbm_choose_td_cluster(Engine* c)
 {
     const int forced = (int)((c->debug_flags >> 8) & 0xff);
     if (forced == 0xff) return 0;
@@ -958,7 +958,7 @@ void sgbm_plane_geometry(const SgbmNorm& n, int W, int* NV, int* RP, int* JOFF)
     *NV = nv; *JOFF = joff; *RP = (joff + W + nv * 8 + 16 + 7) / 8 * 8;
 }
 
-cudaError_t launch_sgbm(mvsv_ctx* c, int B)
+cudaError_t launch_sgbm(Engine* c, int B)
 {
     const SgbmNorm& n = c->sg;
     const size_t npx = (size_t)B * c->H * c->W;

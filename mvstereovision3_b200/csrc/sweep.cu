@@ -614,7 +614,7 @@ void sweep_layout(int D, int* G, int* NR)
 // Chooses the strip decomposition for a batch of B frames: NS strips per frame (0 = the sweep cannot run: use the
 // independent passes), NF frames in flight, CTA size.  `forcedNS` > 0 pins the strip count, 0xfe only rules out the
 // independent passes (test hooks).
-void sweep_plan(const mvsv_ctx* c, int B, int forcedNS, SweepPlan* p)
+void sweep_plan(const Engine* c, int B, int forcedNS, SweepPlan* p)
 {
     const SgbmNorm& n = c->sg;
     *p = SweepPlan();
@@ -654,7 +654,7 @@ void sweep_plan(const mvsv_ctx* c, int B, int forcedNS, SweepPlan* p)
     }
 }
 
-size_t sweep_scratch_bytes(const mvsv_ctx* c)
+size_t sweep_scratch_bytes(const Engine* c)
 {
     // worst case over all plans and disparity ranges: NF * NS <= num_sms CTAs, 2 directions x NSLOT records each
     return (size_t)c->num_sms * 2 * NSLOT * (256 + 8) * sizeof(uint16_t);
@@ -668,13 +668,13 @@ static bool sweep_fast_ok(const SgbmNorm& n)
 }
 
 // S as bytes: all npaths excesses (each <= P2) fit a byte, plain 16-bit row sums, whole 16-byte chunks per lane
-bool sweep_s8_ok(const mvsv_ctx* c, const SweepPlan& p)
+bool sweep_s8_ok(const Engine* c, const SweepPlan& p)
 {
     const SgbmNorm& n = c->sg;
     return p.NS > 0 && p.NR % 8 == 0 && sweep_fast_ok(n) && (long long)n.npaths * n.P2 <= 255;
 }
 
-cudaError_t launch_sweep(mvsv_ctx* c, int B, const SweepPlan& p, int bottomUp, bool s8)
+cudaError_t launch_sweep(Engine* c, int B, const SweepPlan& p, int bottomUp, bool s8)
 {
     const SgbmNorm& n = c->sg;
     SweepArgs a;

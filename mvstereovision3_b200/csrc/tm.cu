@@ -109,7 +109,7 @@ size_t tm_smem_bytes(int W, int k)
 int tm_max_width() { return TM_THREADS * TM_MAXC; }
 
 // out: [B][H][opitch] bytes, zero-filled by the caller
-cudaError_t launch_tm(mvsv_ctx* c, int B, int k, uint8_t* out, size_t opitch)
+cudaError_t launch_tm(Engine* c, int B, int k, uint8_t* out, size_t opitch)
 {
     const size_t smem = tm_smem_bytes(c->W, k);
     MVSV_TRY(smem_limit((const void*)k_tm, (int)smem));
