@@ -44,13 +44,6 @@ inline size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
         }                                                                                       \
     } while (0)
 
-template <class T>
-void dfree(T*& p)
-{
-    if (p) cudaFree(p);
-    p = nullptr;
-}
-
 template <class C>    // an Engine, or the mvsv_ctx handle
 int fail(C* c, int code, const std::string& msg)
 {
@@ -90,24 +83,16 @@ int upload_rig_tables(Engine* c)
     return MVSV_OK;
 }
 
-// What free_slot releases; each level includes the ones before it.
-enum SlotBuffers {
-    SLOT_MEANS,     // the ROI means (the ROIs change)
-    SLOT_SIZED,     // + rectified images, disparities, XYZ (the image size changes): the slot then holds no results
-    SLOT_ALL        // + the raw-frame staging (the slot goes away)
-};
-
-void free_slot(Engine* c, int k, SlotBuffers what)
+// Releases the slot's buffers sized by the image geometry (rectified images, disparities, XYZ, ROI means), and with
+// `staging` the raw-frame staging too (the slot goes away).  The slot then holds no results.
+void release_slot(IoSlot& s, bool staging)
 {
-    IoSlot& s = c->slot[k];
-    dfree(s.means);
-    s.stages &= ~(unsigned)MVSV_STAGE_MEANS;
-    if (what == SLOT_MEANS) return;
-    for (int i = 0; i < 2; ++i) dfree(s.rect[i]);
-    dfree(s.disp); dfree(s.xyz);
+    for (int i = 0; i < 2; ++i) {
+        s.rect[i].reset();
+        if (staging) s.raw[i].reset();
+    }
+    s.disp.reset(); s.xyz.reset(); s.means.reset();
     s.B = 0; s.stages = 0;
-    if (what == SLOT_ALL)
-        for (int i = 0; i < 2; ++i) dfree(s.raw[i]);
 }
 
 // Allocates what each live slot needs in the engine's present state and does not have yet: the rectified images and
@@ -120,58 +105,20 @@ int ensure_slots(Engine* c)
     for (int k = 0; k < c->nslots; ++k) {
         IoSlot& s = c->slot[k];
         for (int i = 0; i < 2; ++i) {
-            if (!s.rect[i]) MVSV_CK(c, cudaMalloc(&s.rect[i], nimg));
-            if (maps && !s.raw[i]) MVSV_CK(c, cudaMalloc(&s.raw[i], B * c->fh * c->raw_pitch));
+            MVSV_CK(c, s.rect[i].ensure(nimg));
+            if (maps) MVSV_CK(c, s.raw[i].ensure(B * c->fh * c->raw_pitch));
         }
         if (!s.disp) {
-            MVSV_CK(c, cudaMalloc(&s.disp, npx * sizeof(int16_t)));
+            MVSV_CK(c, s.disp.alloc(npx));
             MVSV_CK(c, cudaMemsetAsync(s.disp, 0, npx * sizeof(int16_t), c->stream));
         }
-        if (c->nrois > 0 && !s.means) MVSV_CK(c, cudaMalloc(&s.means, (size_t)c->nrois * B * sizeof(float)));
+        if (c->nrois > 0) MVSV_CK(c, s.means.ensure((size_t)c->nrois * B));
     }
     return MVSV_OK;
 }
 
-void free_images(Engine* c)
-{
-    for (int k = 0; k < 2; ++k) free_slot(c, k, SLOT_SIZED);
-    for (int i = 0; i < 2; ++i) dfree(c->bm_pre[i]);
-    dfree(c->recL);
-    dfree(c->d2); dfree(c->disp_raw); dfree(c->disp_med); dfree(c->labels); dfree(c->sizes);
-    dfree(c->bm_tex2); dfree(c->minmax); dfree(c->tm_out);
-}
-void free_sgbm_volumes(Engine* c)
-{
-    dfree(c->VS); dfree(c->C); dfree(c->S); dfree(c->plR); dfree(c->sweep_halo);
-    c->vol_elems = 0;
-}
-void free_bm_volumes(Engine* c) { dfree(c->bm_col); c->bm_vol_elems = 0; }
-
-int alloc_images(Engine* c)
-{
-    free_images(c);
-    // 16-byte aligned rows; when the width already is (752, 1920, 3840, ...) a batch is one contiguous block and
-    // host <-> device transfers are single linear copies instead of strided 2-D copies of many short rows
-    c->pitch = round_up((size_t)c->W, 16);
-    const size_t B = (size_t)c->maxB, npx = B * c->H * c->W, nimg = B * c->H * c->pitch;
-    // the connected-components labels of the speckle filter are int indices over the whole batch
-    if (nimg >= ((size_t)1 << 31)) return fail(c, MVSV_ERR_UNSUPPORTED, "max_batch * height * width must stay below 2^31 pixels");
-    // the slot buffers first: allocated after the scratch buffers below, the StereoBM configuration ran 0.4 % slower
-    // (49.35 K against 49.55 K frames/s on a B200 at 1000 W)
-    const int rc = ensure_slots(c);
-    if (rc) return rc;
-    for (int i = 0; i < 2; ++i) MVSV_CK(c, cudaMalloc(&c->bm_pre[i], nimg + 64));   // the BM column-sum kernel reads whole aligned words
-    MVSV_CK(c, cudaMalloc(&c->recL, npx * sizeof(uint2)));
-    MVSV_CK(c, cudaMalloc(&c->d2, npx * sizeof(int)));
-    MVSV_CK(c, cudaMalloc(&c->disp_raw, npx * sizeof(int16_t)));
-    MVSV_CK(c, cudaMalloc(&c->disp_med, npx * sizeof(int16_t)));
-    MVSV_CK(c, cudaMalloc(&c->labels, npx * sizeof(int)));
-    MVSV_CK(c, cudaMalloc(&c->sizes, npx * sizeof(int)));
-    MVSV_CK(c, cudaMalloc(&c->bm_tex2, npx * sizeof(int)));
-    return MVSV_OK;
-}
-
-int normalise_sgbm(Engine* c, const mvsv_sgbm_params* p, SgbmNorm* n)
+// StereoSGBM parameters p normalised for W x H images
+int normalise_sgbm(Engine* c, const mvsv_sgbm_params* p, int W, int H, SgbmNorm* n)
 {
     n->minD = p->minDisp;
     n->D = p->numDisp;
@@ -196,7 +143,7 @@ int normalise_sgbm(Engine* c, const mvsv_sgbm_params* p, SgbmNorm* n)
     n->P2 = std::max(p->P2 > 0 ? p->P2 : 5, n->P1 + 1);
     n->maxD = n->minD + n->D;
     n->minX1 = std::max(n->maxD, 0);
-    n->maxX1 = c->W + std::min(n->minD, 0);
+    n->maxX1 = W + std::min(n->minD, 0);
     n->W1 = n->maxX1 - n->minX1;
     n->INV = (n->minD - 1) * 16;
     n->mode = p->disparityMode == 1 ? 1 : 0;   // reference src/disparity.cpp:92-95
@@ -212,7 +159,7 @@ int normalise_sgbm(Engine* c, const mvsv_sgbm_params* p, SgbmNorm* n)
                     "blockSize^2*(2*ftzero+63)+P2 > 32767: int16 overflow regime of OpenCV is outside the bit-exact contract");
     if (n->INV < -32768 || (n->maxD) * 16 > 32767) return fail(c, MVSV_ERR_INVALID, "disparity range does not fit CV_16S");
     n->vsWide = sgbm_vsum_wide(*n) ? 1 : 0;
-    if (n->W1 > 0 && (long long)c->H * n->W1 * n->Dp >= (1ll << 31))
+    if (n->W1 > 0 && (long long)H * n->W1 * n->Dp >= (1ll << 31))
         return fail(c, MVSV_ERR_UNSUPPORTED, "cost volume of one frame exceeds 2^31 cells");
     return MVSV_OK;
 }
@@ -224,26 +171,19 @@ int ensure_sgbm_volumes(Engine* c)
     int nv, rp, joff;
     sgbm_plane_geometry(n, c->W, &nv, &rp, &joff);
     const size_t need = (size_t)c->maxB * c->H * n.W1 * n.Dp;
-    if (!(need <= c->vol_elems && c->VS)) {
-        dfree(c->VS); dfree(c->C); dfree(c->S);
-        c->vol_elems = 0;
-        MVSV_CK(c, cudaMalloc(&c->VS, need * 2));
-        MVSV_CK(c, cudaMalloc(&c->C, need * 2));
-        MVSV_CK(c, cudaMalloc(&c->S, need * 2));
-        c->vol_elems = need;
-    }
-    if (!c->sweep_halo) MVSV_CK(c, cudaMalloc(&c->sweep_halo, sweep_scratch_bytes(c)));   // strip-border records of the fused sweep
+    for (DeviceBuffer<uint16_t>* v : {&c->VS, &c->C, &c->S}) MVSV_CK(c, v->ensure(need));
+    MVSV_CK(c, c->sweep_halo.ensure(sweep_scratch_bytes(c) / sizeof(uint16_t)));   // strip-border records of the fused sweep
     if (!c->plR || nv != c->vsNV || rp != c->vsRP || joff != c->vsJOFF) {
-        dfree(c->plR);
-        const size_t bytes = (size_t)6 * c->maxB * c->H * rp * sizeof(uint16_t);
-        MVSV_CK(c, cudaMalloc(&c->plR, bytes));
-        MVSV_CK(c, cudaMemsetAsync(c->plR, 0, bytes, c->stream));   // the padding around each row stays zero
+        const size_t elems = (size_t)6 * c->maxB * c->H * rp;
+        MVSV_CK(c, c->plR.alloc(elems));
+        MVSV_CK(c, cudaMemsetAsync(c->plR, 0, elems * sizeof(uint16_t), c->stream));   // the padding around each row stays zero
         c->vsNV = nv; c->vsRP = rp; c->vsJOFF = joff;
     }
     return MVSV_OK;
 }
 
-int normalise_bm(Engine* c, const mvsv_bm_params* p, BmNorm* n)
+// StereoBM parameters p normalised for images W wide
+int normalise_bm(Engine* c, const mvsv_bm_params* p, int W, BmNorm* n)
 {
     n->D = p->numDisp; n->bs = p->blockSize; n->cap = p->preFilterCap; n->tex = p->textureThreshold; n->uniq = p->uniquenessRatio;
     if (n->D <= 0 || n->D % 16 != 0 || n->D > 256) return fail(c, MVSV_ERR_INVALID, "BM numDisp must be a positive multiple of 16 and <= 256");
@@ -254,7 +194,7 @@ int normalise_bm(Engine* c, const mvsv_bm_params* p, BmNorm* n)
     int g = 2;
     while (g * 8 < n->D) g <<= 1;
     n->G = g; n->Dp = n->D; n->w2 = n->bs / 2;      // lanes: next power of two; storage stride: numDisp itself
-    n->lofs = n->D - 1; n->width1 = c->W - n->D + 1; n->FILT = -16;
+    n->lofs = n->D - 1; n->width1 = W - n->D + 1; n->FILT = -16;
     n->col8 = n->bs * 2 * n->cap <= 255;
     return MVSV_OK;
 }
@@ -263,11 +203,92 @@ int ensure_bm_volumes(Engine* c)
 {
     const BmNorm& n = c->bm;
     if (n.width1 < 1) return MVSV_OK;
-    const size_t need = (size_t)c->maxB * c->H * n.width1 * n.Dp;
-    if (need <= c->bm_vol_elems && c->bm_col) return MVSV_OK;
-    free_bm_volumes(c);
-    MVSV_CK(c, cudaMalloc(&c->bm_col, need * 2));
-    c->bm_vol_elems = need;
+    MVSV_CK(c, c->bm_col.ensure((size_t)c->maxB * c->H * n.width1 * n.Dp));
+    return MVSV_OK;
+}
+
+// What the matcher sees under a geometry (the frame, or the display ROI, possibly resized)
+struct Geometry {
+    int W, H;
+    SgbmNorm sg;     // the matcher parameters normalised for W x H (while set)
+    BmNorm bm;
+};
+
+// The size of the images the matcher would see with display ROI roi_w x roi_h once some rig holds maps (`maps`; the
+// frame otherwise), resized by `factor` when that is on, and the matcher parameters normalised for it.  Every check
+// that can reject a geometry runs here, before the caller changes anything: a rejected geometry leaves the engine as
+// it was.
+int plan_geometry(Engine* c, bool maps, int roi_w, int roi_h, double factor, Geometry* g)
+{
+    g->W = maps ? roi_w : c->fw;
+    g->H = maps ? roi_h : c->fh;
+    if (maps && factor > 0.0) {
+        // cv::resize: dsize = Size(saturate_cast<int>(w*fx), saturate_cast<int>(h*fy)), round half to even
+        g->W = (int)lrint((double)g->W * factor);
+        g->H = (int)lrint((double)g->H * factor);
+        if (g->W < 2 || g->H < 1 || g->W > 16384 || g->H > 16384) return fail(c, MVSV_ERR_INVALID, "resized image out of range");
+    }
+    g->sg = c->sg;
+    g->bm = c->bm;
+    int rc = MVSV_OK;
+    if (c->has_sgbm) rc = normalise_sgbm(c, &c->sgbm_raw, g->W, g->H, &g->sg);
+    if (!rc && c->has_bm) rc = normalise_bm(c, &c->bm_raw, g->W, &g->bm);
+    if (rc) return rc;
+    // the connected-components labels of the speckle filter are int indices over the whole batch
+    if ((size_t)c->maxB * g->H * round_up((size_t)g->W, 16) >= ((size_t)1 << 31))
+        return fail(c, MVSV_ERR_UNSUPPORTED, "max_batch * height * width must stay below 2^31 pixels");
+    return MVSV_OK;
+}
+
+// Installs geometry g (plan_geometry) once the engine's ROI, maps and resize factor describe it, with the engine's stream
+// synchronised.  A new image size reallocates every buffer sized by it and drops the mean-disparity ROIs; the crop
+// buffers follow the display ROI.
+int apply_geometry(Engine* c, const Geometry& g)
+{
+    if (g.W != c->W || g.H != c->H) {
+        c->W = g.W; c->H = g.H;
+        // mean-disparity ROIs are coordinates of the old map: drop them (run() asks for new ones)
+        c->rois.reset();
+        c->nrois = 0;
+        for (IoSlot& s : c->slot) release_slot(s, false);
+        for (auto& b : c->bm_pre) b.reset();
+        c->recL.reset(); c->d2.reset(); c->disp_raw.reset(); c->disp_med.reset(); c->labels.reset(); c->sizes.reset();
+        c->bm_tex2.reset(); c->minmax.reset(); c->tm_out.reset();
+        // 16-byte aligned rows; when the width already is (752, 1920, 3840, ...) a batch is one contiguous block and
+        // host <-> device transfers are single linear copies instead of strided 2-D copies of many short rows
+        c->pitch = round_up((size_t)c->W, 16);
+        const size_t B = (size_t)c->maxB, npx = B * c->H * c->W, nimg = B * c->H * c->pitch;
+        // the slot buffers first: allocated after the scratch buffers below, the StereoBM configuration ran 0.4 % slower
+        // (49.35 K against 49.55 K frames/s on a B200 at 1000 W)
+        int rc = ensure_slots(c);
+        if (rc) return rc;
+        for (auto& b : c->bm_pre) MVSV_CK(c, b.alloc(nimg + 64));   // the BM column-sum kernel reads whole aligned words
+        MVSV_CK(c, c->recL.alloc(npx));
+        MVSV_CK(c, c->d2.alloc(npx));
+        MVSV_CK(c, c->disp_raw.alloc(npx));
+        MVSV_CK(c, c->disp_med.alloc(npx));
+        MVSV_CK(c, c->labels.alloc(npx));
+        MVSV_CK(c, c->sizes.alloc(npx));
+        MVSV_CK(c, c->bm_tex2.alloc(npx));
+        // the volumes grow within one geometry; a new one starts them afresh
+        for (DeviceBuffer<uint16_t>* v : {&c->VS, &c->C, &c->S, &c->plR, &c->sweep_halo, &c->bm_col}) v->reset();
+        if (c->has_sgbm) {
+            c->sg = g.sg;
+            c->td_nc = sgbm_choose_td_cluster(c);
+            rc = ensure_sgbm_volumes(c);
+            if (rc) { c->has_sgbm = false; return rc; }
+        }
+        if (c->has_bm) {
+            c->bm = g.bm;
+            rc = ensure_bm_volumes(c);
+            if (rc) { c->has_bm = false; return rc; }
+        }
+    }
+    for (auto& b : c->crop) b.reset();
+    if (any_maps(c) && c->resize_factor > 0.0) {
+        c->crop_pitch = round_up((size_t)c->roi_w, 16);
+        for (auto& b : c->crop) MVSV_CK(c, b.alloc((size_t)c->maxB * c->roi_h * c->crop_pitch));
+    }
     return MVSV_OK;
 }
 
@@ -356,7 +377,7 @@ int compute_check(Engine* c, size_t lstride, size_t rstride, int batch, unsigned
     if (stages & MVSV_STAGE_SGBM) rc = ensure_sgbm_volumes(c);
     else if (stages & MVSV_STAGE_BM) rc = ensure_bm_volumes(c);
     if (rc) return rc;
-    if ((stages & MVSV_STAGE_XYZ) && !slot.xyz) MVSV_CK(c, cudaMalloc(&slot.xyz, (size_t)c->maxB * c->H * c->W * 3 * sizeof(float)));
+    if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, slot.xyz.ensure((size_t)c->maxB * c->H * c->W * 3));
     return MVSV_OK;
 }
 
@@ -374,7 +395,7 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     // host inputs: the copies wait for the slot's previous compute (which may still read the input buffers), the
     // kernels wait for the copies
     if (!device_src) MVSV_CK(c, cudaStreamWaitEvent(c->copy_stream, slot.done, 0));
-    uint8_t* const* dst = rectify ? slot.raw : slot.rect;
+    const DeviceBuffer<uint8_t>* dst = rectify ? slot.raw : slot.rect;
     const size_t dpitch = rectify ? c->raw_pitch : c->pitch;
     rc = upload_images(c, dst[0], dpitch, left, lstride, frame_stride, iw, ih, batch, device_src);
     if (!rc) rc = upload_images(c, dst[1], dpitch, right, rstride, frame_stride, iw, ih, batch, device_src);
@@ -445,7 +466,7 @@ int minmax_launch(Engine* c)
 {
     int rc = bind(c);
     if (rc) return rc;
-    if (!c->minmax) MVSV_CK(c, cudaMalloc(&c->minmax, (size_t)c->maxB * 2 * sizeof(int)));
+    MVSV_CK(c, c->minmax.ensure((size_t)c->maxB * 2));
     MVSV_CK(c, launch_minmax(c, io(c).B));
     return MVSV_OK;
 }
@@ -487,13 +508,11 @@ int set_rigs(Engine* c, const std::vector<int>& rig_of_frame)
     }
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
     RigFrames& t = c->rig_frames;
-    if (!t.chunk) {
-        MVSV_CK(c, cudaMalloc(&t.chunk, (size_t)B * (sizeof(int4) + 2 * sizeof(int))));
-        t.order = reinterpret_cast<int*>(t.chunk + B);
-        t.rig = t.order + B;
-    }
+    MVSV_CK(c, t.chunk.ensure(B));
+    MVSV_CK(c, t.order.ensure(B));
+    MVSV_CK(c, t.rig.ensure(B));
     if (!c->rig_tables) {
-        MVSV_CK(c, cudaMalloc(&c->rig_tables, sizeof(RigTables)));
+        MVSV_CK(c, c->rig_tables.alloc(1));
         c->rig_tables_dirty = true;
     }
     // Until the copies below have all been queued the engine holds a table longer than any it accepts, which its
@@ -637,9 +656,29 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
 
 }  // namespace
 
+Engine::~Engine()
+{
+    for (auto& b : brackets) { cudaEventDestroy(b.a); cudaEventDestroy(b.b); }
+    for (cudaEvent_t ev : ev_free) cudaEventDestroy(ev);
+    for (cudaEvent_t ev : ev_chunk)
+        if (ev) cudaEventDestroy(ev);
+    for (cudaEvent_t ev : {timer_a, timer_b, ev_h2d, ev_done, ev_join, slot[0].done, slot[1].done})
+        if (ev) cudaEventDestroy(ev);
+    for (cudaStream_t st : {aux_stream, copy_stream, dl_stream, stream})
+        if (st) cudaStreamDestroy(st);
+}
+
 extern "C" {
 
-static void destroy_engine(Engine* c);
+static void destroy_engine(Engine* c)
+{
+    if (!c) return;
+    cudaSetDevice(c->device);
+    if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
+    if (c->dl_stream) cudaStreamSynchronize(c->dl_stream);
+    if (c->stream) cudaStreamSynchronize(c->stream);
+    delete c;
+}
 
 // an engine on `device`; the text of a failure goes to mvsv_last_error(NULL)
 static int init_engine(int device, int frame_width, int frame_height, int max_batch, Engine** out)
@@ -660,7 +699,7 @@ static int init_engine(int device, int frame_width, int frame_height, int max_ba
     }
     Engine* c = new (std::nothrow) Engine();
     if (!c) return MVSV_ERR_NOMEM;
-    c->device = device; c->fw = frame_width; c->fh = frame_height; c->W = frame_width; c->H = frame_height; c->maxB = max_batch;
+    c->device = device; c->fw = frame_width; c->fh = frame_height; c->maxB = max_batch;
     c->raw_pitch = round_up((size_t)frame_width, 16);
     auto bail = [&](cudaError_t ee, const char* what) {
         g_init_error = std::string("mvsv_init: ") + what + ": " + cudaGetErrorString(ee);
@@ -689,46 +728,12 @@ static int init_engine(int device, int frame_width, int frame_height, int max_ba
         if ((e = cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
     for (cudaEvent_t* ev : {&c->ev_h2d, &c->ev_done})
         if ((e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
-    int rc = alloc_images(c);
+    Geometry g;
+    int rc = plan_geometry(c, false, 0, 0, 0.0, &g);
+    if (!rc) rc = apply_geometry(c, g);
     if (rc) { g_init_error = c->err; destroy_engine(c); return rc; }
     *out = c;
     return MVSV_OK;
-}
-
-static void destroy_engine(Engine* c)
-{
-    if (!c) return;
-    cudaSetDevice(c->device);
-    if (c->copy_stream) cudaStreamSynchronize(c->copy_stream);
-    if (c->dl_stream) cudaStreamSynchronize(c->dl_stream);
-    if (c->stream) cudaStreamSynchronize(c->stream);
-    free_images(c);
-    for (int k = 0; k < 2; ++k) {
-        free_slot(c, k, SLOT_ALL);
-        if (c->slot[k].done) cudaEventDestroy(c->slot[k].done);
-    }
-    free_sgbm_volumes(c);
-    free_bm_volumes(c);
-    for (int r = 0; r < MVSV_MAX_RIGS; ++r)
-        for (int i = 0; i < 2; ++i) dfree(c->map_xy[r][i]);
-    for (int i = 0; i < 2; ++i) dfree(c->crop[i]);
-    dfree(c->rig_frames.chunk);
-    dfree(c->rig_tables);
-    dfree(c->rois);
-    for (auto& b : c->brackets) { cudaEventDestroy(b.a); cudaEventDestroy(b.b); }
-    for (auto e : c->ev_free) cudaEventDestroy(e);
-    if (c->timer_a) cudaEventDestroy(c->timer_a);
-    if (c->timer_b) cudaEventDestroy(c->timer_b);
-    for (cudaEvent_t ev : {c->ev_h2d, c->ev_done})
-        if (ev) cudaEventDestroy(ev);
-    for (cudaEvent_t ev : c->ev_chunk)
-        if (ev) cudaEventDestroy(ev);
-    if (c->ev_join) cudaEventDestroy(c->ev_join);
-    if (c->aux_stream) cudaStreamDestroy(c->aux_stream);
-    if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-    if (c->dl_stream) cudaStreamDestroy(c->dl_stream);
-    if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
 }
 
 // a ctx of one part per listed device, each of ceil(max_batch / n) frames
@@ -796,7 +801,7 @@ int mvsv_set_sgbm_params(mvsv_ctx* ctx, const mvsv_sgbm_params* p)
         int rc = bind(c);
         if (rc) return rc;
         SgbmNorm n;
-        rc = normalise_sgbm(c, p, &n);
+        rc = normalise_sgbm(c, p, c->W, c->H, &n);
         if (rc) return rc;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
         c->sg = n; c->sgbm_raw = *p; c->has_sgbm = true;
@@ -812,7 +817,7 @@ int mvsv_set_bm_params(mvsv_ctx* ctx, const mvsv_bm_params* p)
         int rc = bind(c);
         if (rc) return rc;
         BmNorm n;
-        rc = normalise_bm(c, p, &n);
+        rc = normalise_bm(c, p, c->W, &n);
         if (rc) return rc;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
         c->bm = n; c->bm_raw = *p; c->has_bm = true;
@@ -837,64 +842,6 @@ int mvsv_set_bm_filters(mvsv_ctx* ctx, int disp12MaxDiff, int speckleWindowSize,
     });
 }
 
-static int resize_rectified(Engine* c, int W, int H)
-{
-    if (W == c->W && H == c->H) return MVSV_OK;
-    MVSV_CK(c, cudaStreamSynchronize(c->stream));
-    // the matcher parameters are re-normalised for the new geometry BEFORE anything is committed: a geometry the
-    // contract rejects (e.g. a frame volume of 2^31 cells) leaves the engine exactly as it was
-    const int oldW = c->W, oldH = c->H;
-    SgbmNorm sg = c->sg;
-    BmNorm bm = c->bm;
-    c->W = W; c->H = H;
-    int rc = MVSV_OK;
-    if (c->has_sgbm) rc = normalise_sgbm(c, &c->sgbm_raw, &sg);
-    if (!rc && c->has_bm) rc = normalise_bm(c, &c->bm_raw, &bm);
-    if (rc) { c->W = oldW; c->H = oldH; return rc; }
-    // mean-disparity ROIs are coordinates of the old map: drop them (run() asks for new ones)
-    dfree(c->rois);
-    c->nrois = 0;
-    rc = alloc_images(c);
-    if (rc) return rc;
-    free_sgbm_volumes(c);
-    free_bm_volumes(c);
-    if (c->has_sgbm) {
-        c->sg = sg;
-        c->td_nc = sgbm_choose_td_cluster(c);
-        rc = ensure_sgbm_volumes(c);
-        if (rc) { c->has_sgbm = false; return rc; }
-    }
-    if (c->has_bm) {
-        c->bm = bm;
-        rc = ensure_bm_volumes(c);
-        if (rc) { c->has_bm = false; return rc; }
-    }
-    return MVSV_OK;
-}
-
-// size of the images the matcher sees: the frame, the display ROI once maps are installed, the resized ROI when
-// mvsv_set_resize is active; (re)allocates everything that depends on it
-static int apply_geometry(Engine* c)
-{
-    const bool maps = any_maps(c);
-    int W = maps ? c->roi_w : c->fw, H = maps ? c->roi_h : c->fh;
-    const bool resized = maps && c->resize_factor > 0.0;
-    if (resized) {
-        // cv::resize: dsize = Size(saturate_cast<int>(w*fx), saturate_cast<int>(h*fy)), round half to even
-        W = (int)lrint((double)W * c->resize_factor);
-        H = (int)lrint((double)H * c->resize_factor);
-        if (W < 2 || H < 1 || W > 16384 || H > 16384) return fail(c, MVSV_ERR_INVALID, "resized image out of range");
-    }
-    int rc = resize_rectified(c, W, H);
-    if (rc) return rc;
-    for (int i = 0; i < 2; ++i) dfree(c->crop[i]);
-    if (resized) {
-        c->crop_pitch = round_up((size_t)c->roi_w, 16);
-        for (int i = 0; i < 2; ++i) MVSV_CK(c, cudaMalloc(&c->crop[i], (size_t)c->maxB * c->roi_h * c->crop_pitch));
-    }
-    return MVSV_OK;
-}
-
 // shared by the two ways of installing a camera's maps: checks the display ROI, sizes the rectified images and
 // the raw-frame staging, allocates the fixed-point map
 static int prepare_maps(Engine* c, int rig, int cam, int roi_x, int roi_y, int roi_w, int roi_h)
@@ -908,13 +855,15 @@ static int prepare_maps(Engine* c, int rig, int cam, int roi_x, int roi_y, int r
     for (int r = 0; r < MVSV_MAX_RIGS; ++r)
         if (r != rig && (c->has_maps[r][0] || c->has_maps[r][1]) && (c->roi_w != roi_w || c->roi_h != roi_h))
             return fail(c, MVSV_ERR_INVALID, "all rigs share the display-ROI size (rig " + std::to_string(r) + " holds maps of another size)");
+    Geometry g;
+    int rc = plan_geometry(c, true, roi_w, roi_h, c->resize_factor, &g);
+    if (rc) return rc;
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
     c->roi_xy[rig][0] = roi_x; c->roi_xy[rig][1] = roi_y; c->roi_w = roi_w; c->roi_h = roi_h;
     c->has_maps[rig][cam] = false;
     c->rig_tables_dirty = true;
-    dfree(c->map_xy[rig][cam]);
-    MVSV_CK(c, cudaMalloc(&c->map_xy[rig][cam], (size_t)roi_w * roi_h * sizeof(int2)));
-    int rc = apply_geometry(c);
+    MVSV_CK(c, c->map_xy[rig][cam].alloc((size_t)roi_w * roi_h));
+    rc = apply_geometry(c, g);
     if (rc) return rc;
     return ensure_slots(c);
 }
@@ -936,18 +885,15 @@ int mvsv_upload_rectify_maps_rig(mvsv_ctx* ctx, int rig, int cam, const float* m
         if (stride_bytes < (size_t)c->fw * sizeof(float) || stride_bytes % sizeof(float)) return fail(c, MVSV_ERR_INVALID, "bad map stride");
         rc = prepare_maps(c, rig, cam, roi_x, roi_y, roi_w, roi_h);
         if (rc) return rc;
-        float *dx = nullptr, *dy = nullptr;
-        const size_t mbytes = (size_t)c->fw * c->fh * sizeof(float);
-        MVSV_CK(c, cudaMalloc(&dx, mbytes));
-        cudaError_t e = cudaMalloc(&dy, mbytes);
-        if (e != cudaSuccess) { cudaFree(dx); c->err = "cudaMalloc(map)"; return MVSV_ERR_NOMEM; }
+        // the float maps, staged on the device for the conversion
+        DeviceBuffer<float> dx, dy;
+        MVSV_CK(c, dx.alloc((size_t)c->fw * c->fh));
+        MVSV_CK(c, dy.alloc((size_t)c->fw * c->fh));
         const size_t w = (size_t)c->fw * sizeof(float);
-        e = cudaMemcpy2DAsync(dx, w, mapx, stride_bytes, w, c->fh, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = cudaMemcpy2DAsync(dy, w, mapy, stride_bytes, w, c->fh, cudaMemcpyHostToDevice, c->stream);
-        if (e == cudaSuccess) e = launch_convert_maps(c, rig, cam, dx, dy, (size_t)c->fw);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-        cudaFree(dx); cudaFree(dy);
-        if (e != cudaSuccess) { c->err = std::string("map upload: ") + cudaGetErrorString(e); return MVSV_ERR_CUDA; }
+        MVSV_CK(c, cudaMemcpy2DAsync(dx, w, mapx, stride_bytes, w, c->fh, cudaMemcpyHostToDevice, c->stream));
+        MVSV_CK(c, cudaMemcpy2DAsync(dy, w, mapy, stride_bytes, w, c->fh, cudaMemcpyHostToDevice, c->stream));
+        MVSV_CK(c, launch_convert_maps(c, rig, cam, dx, dy, (size_t)c->fw));
+        MVSV_CK(c, cudaStreamSynchronize(c->stream));
         c->has_maps[rig][cam] = true;
         return MVSV_OK;
     });
@@ -1002,14 +948,17 @@ int mvsv_reset_rectification(mvsv_ctx* ctx)
     return each(ctx, true, [&](Engine* c) -> int {
         int rc = bind(c);
         if (rc) return rc;
+        Geometry g;
+        rc = plan_geometry(c, false, 0, 0, c->resize_factor, &g);
+        if (rc) return rc;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
         for (int r = 0; r < MVSV_MAX_RIGS; ++r)
             for (int i = 0; i < 2; ++i) {
                 c->has_maps[r][i] = false;
-                dfree(c->map_xy[r][i]);
+                c->map_xy[r][i].reset();
             }
         c->rig_tables_dirty = true;
-        return apply_geometry(c);
+        return apply_geometry(c, g);
     });
 }
 
@@ -1021,12 +970,12 @@ int mvsv_set_resize(mvsv_ctx* ctx, double factor)
         if (!(factor == factor) || factor > 8.0) return fail(c, MVSV_ERR_INVALID, "resize factor must be in (0, 8]");
         const double f = (factor <= 0.0 || factor == 1.0) ? 0.0 : factor;   // off: cv::resize by 1 is the identity
         if (f > 0.0 && f < 1.0 / 64) return fail(c, MVSV_ERR_INVALID, "resize factor must be in (0, 8]");
+        Geometry g;
+        rc = plan_geometry(c, any_maps(c), c->roi_w, c->roi_h, f, &g);
+        if (rc) return rc;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
-        const double old = c->resize_factor;
         c->resize_factor = f;
-        rc = apply_geometry(c);
-        if (rc) { c->resize_factor = old; apply_geometry(c); }
-        return rc;
+        return apply_geometry(c, g);
     });
 }
 
@@ -1050,7 +999,7 @@ int mvsv_tm(mvsv_ctx* ctx, const uint8_t* left, size_t lstride, const uint8_t* r
         if (rc) return rc;
         rc = inputs_uploaded(c, false);
         if (rc) return rc;
-        if (!c->tm_out) MVSV_CK(c, cudaMalloc(&c->tm_out, (size_t)c->maxB * H * c->pitch));
+        MVSV_CK(c, c->tm_out.ensure((size_t)c->maxB * H * c->pitch));
         MVSV_CK(c, cudaMemsetAsync(c->tm_out, 0, (size_t)batch * H * c->pitch, c->stream));   // cv::Scalar::all(0)
         // the reference's loops are `i < rows - kernelSize` in unsigned arithmetic: nothing to do unless k < rows, cols
         if ((int)kernel_size < H && (int)kernel_size < W) MVSV_CK(c, launch_tm(c, batch, (int)kernel_size, c->tm_out, c->pitch));
@@ -1106,11 +1055,14 @@ int mvsv_set_mean_rois(mvsv_ctx* ctx, const int* xywh, int n)
                 return fail(c, MVSV_ERR_INVALID, "ROI outside the disparity map");
         }
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
-        dfree(c->rois);
-        for (int k = 0; k < 2; ++k) free_slot(c, k, SLOT_MEANS);
+        c->rois.reset();
+        for (IoSlot& s : c->slot) {
+            s.means.reset();
+            s.stages &= ~(unsigned)MVSV_STAGE_MEANS;
+        }
         c->nrois = n;
         if (n == 0) return MVSV_OK;
-        MVSV_CK(c, cudaMalloc(&c->rois, (size_t)n * 4 * sizeof(int)));
+        MVSV_CK(c, c->rois.alloc((size_t)n * 4));
         rc = ensure_slots(c);
         if (rc) return rc;
         MVSV_CK(c, cudaMemcpy(c->rois, xywh, (size_t)n * 4 * sizeof(int), cudaMemcpyHostToDevice));
@@ -1175,11 +1127,11 @@ int mvsv_set_io_slots(mvsv_ctx* ctx, int n)
         if (n == c->nslots) return MVSV_OK;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
         MVSV_CK(c, cudaStreamSynchronize(c->copy_stream));
-        if (n < c->nslots) free_slot(c, 1, SLOT_ALL);
+        if (n < c->nslots) release_slot(c->slot[1], true);
         c->nslots = n;
         c->cur = 0;
         rc = ensure_slots(c);
-        if (rc) { free_slot(c, 1, SLOT_ALL); c->nslots = 1; }
+        if (rc) { release_slot(c->slot[1], true); c->nslots = 1; }
         return rc;
     });
 }
@@ -1332,7 +1284,7 @@ int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int
         IoSlot& slot = next_slot(c);
         rc = check_consumers(c, slot, stages, rigs);
         if (rc) return rc;
-        if ((stages & MVSV_STAGE_XYZ) && !slot.xyz) MVSV_CK(c, cudaMalloc(&slot.xyz, (size_t)c->maxB * c->H * c->W * 3 * sizeof(float)));
+        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, slot.xyz.ensure((size_t)c->maxB * c->H * c->W * 3));
 
         take_slot(c);
         const size_t row = (size_t)c->W * sizeof(int16_t), npx = (size_t)batch * c->H * c->W;

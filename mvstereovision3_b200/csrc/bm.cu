@@ -687,7 +687,7 @@ cudaError_t launch_bm(Engine* c, int B)
     BmArgs a;
     a.col = c->bm_col; a.tex = c->bm_tex2; a.disp = out; a.W = W; a.H = H; a.width1 = n.width1; a.D = n.D; a.Dp = n.Dp;
     a.lofs = n.lofs; a.w2 = n.w2; a.texThr = n.tex; a.uniq = n.uniq; a.B = B;
-    int* const cost = lr ? c->d2 : nullptr;                   // the SGBM's disp2 keys buffer: same shape, idle here
+    int* const cost = lr ? static_cast<int*>(c->d2) : nullptr;                 // the SGBM's disp2 keys buffer: same shape, idle here
     {
         KernelTimer kt(c, KID_BM_WTA);
         // Two octets per lane (numDisp is a multiple of 16) with the window ring while at least eight warps fit an SM

@@ -37,16 +37,54 @@ extern const char* const kKernelNames[KID_COUNT];
 
 struct ProfBracket { int kid; cudaEvent_t a, b; };
 
+// One device allocation of T elements, the only owner of it: freed by reset() and by the destructor, on the current
+// device (whoever releases an engine's buffer has made the engine's device current).  Converts to T* for the launchers.
+template <class T>
+class DeviceBuffer {
+public:
+    DeviceBuffer() = default;
+    DeviceBuffer(DeviceBuffer&& o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+    DeviceBuffer& operator=(DeviceBuffer&& o) noexcept
+    {
+        if (this != &o) { reset(); p_ = o.p_; n_ = o.n_; o.p_ = nullptr; o.n_ = 0; }
+        return *this;
+    }
+    ~DeviceBuffer() { reset(); }
+
+    // exactly n elements, in place of what it held
+    cudaError_t alloc(size_t n)
+    {
+        reset();
+        const cudaError_t e = cudaMalloc(&p_, n * sizeof(T));
+        if (e == cudaSuccess) n_ = n;
+        else p_ = nullptr;
+        return e;
+    }
+    // at least n elements: reallocates only when it holds fewer
+    cudaError_t ensure(size_t n) { return p_ && n_ >= n ? cudaSuccess : alloc(n); }
+    void reset()
+    {
+        if (p_) cudaFree(p_);
+        p_ = nullptr;
+        n_ = 0;
+    }
+    operator T*() const { return p_; }
+
+private:
+    T* p_ = nullptr;
+    size_t n_ = 0;
+};
+
 // I/O slot (mvsv_set_io_slots): the buffers a compute call reads its inputs into and leaves its results in.  They
 // exist once or twice; with two, the host->device copy of the next batch and the device->host copy of the previous
 // one overlap the kernels of the current batch inside ONE engine (one set of cost volumes).  The slot is the only
 // owner of these buffers; the launchers reach the slot of the compute in progress through io(c).
 struct IoSlot {
-    uint8_t* rect[2] = {nullptr, nullptr};    // [B][H][pitch]
-    uint8_t* raw[2] = {nullptr, nullptr};     // [B][fh][raw_pitch], once rectification maps are installed
-    int16_t* disp = nullptr;                  // final disparities [B][H][W]
-    float* xyz = nullptr;                     // [B][H][W][3], allocated by the first compute with MVSV_STAGE_XYZ
-    float* means = nullptr;                   // [B][nrois], once mean-disparity ROIs are set
+    DeviceBuffer<uint8_t> rect[2];            // [B][H][pitch]
+    DeviceBuffer<uint8_t> raw[2];             // [B][fh][raw_pitch], once rectification maps are installed
+    DeviceBuffer<int16_t> disp;               // final disparities [B][H][W]
+    DeviceBuffer<float> xyz;                  // [B][H][W][3], allocated by the first compute with MVSV_STAGE_XYZ
+    DeviceBuffer<float> means;                // [B][nrois], once mean-disparity ROIs are set
     cudaEvent_t done = nullptr;               // all kernels of the slot's last compute have finished
     int B = 0;                                // frames of the slot's last compute; 0: it holds no results
     unsigned stages = 0;
@@ -59,9 +97,9 @@ constexpr int RM_FRAMES = 8;
 // rig table.  The remap kernel expands a map entry once for up to RM_FRAMES frames, which must then share the rig: it
 // walks `chunk`, runs of at most RM_FRAMES frames of one rig in `order`.
 struct RigFrames {
-    int4* chunk = nullptr;                    // (rig, first index into order, count <= RM_FRAMES, 0)
-    int* order = nullptr;                     // frames sorted by rig, ascending within a rig
-    int* rig = nullptr;                       // rig of each frame
+    DeviceBuffer<int4> chunk;                 // (rig, first index into order, count <= RM_FRAMES, 0)
+    DeviceBuffer<int> order;                  // frames sorted by rig, ascending within a rig
+    DeviceBuffer<int> rig;                    // rig of each frame
     int nchunks = 0;
 };
 
@@ -74,6 +112,7 @@ struct RigTables {
 // One engine on one device: its streams, events, volumes and I/O slots.  An mvsv_ctx (csrc/api.cu) splits every batch
 // across one or more of them.
 struct Engine {
+    ~Engine();                                // destroys the streams and events; the buffers free themselves
     int device = 0;
     cudaStream_t stream = nullptr;
     // host->device input copies run on their own stream so that they overlap the kernels of the other I/O slot's
@@ -104,13 +143,13 @@ struct Engine {
     bool has_maps[MVSV_MAX_RIGS][2] = {};
     int roi_w = 0, roi_h = 0;
     int roi_xy[MVSV_MAX_RIGS][2] = {};
-    int2* map_xy[MVSV_MAX_RIGS][2] = {};      // (ix, iy) = rint(map*32), saturated int32
+    DeviceBuffer<int2> map_xy[MVSV_MAX_RIGS][2];   // (ix, iy) = rint(map*32), saturated int32
     size_t raw_pitch = 0;
     // cv::resize(.., factor, factor) after the crop (Stereosystem::getRectifiedImagepair(sip, factor),
     // reference src/Stereosystem.cpp:279-315); off when resize_factor == 0
     double resize_factor = 0.0;
-    uint8_t* tm_out = nullptr;                // [B][H][pitch], Disparity::tm
-    uint8_t* crop[2] = {nullptr, nullptr};    // [B][roi_h][crop_pitch]: remap output when a resize follows
+    DeviceBuffer<uint8_t> tm_out;             // [B][H][pitch], Disparity::tm
+    DeviceBuffer<uint8_t> crop[2];            // [B][roi_h][crop_pitch]: remap output when a resize follows
     size_t crop_pitch = 0;
 
     size_t pitch = 0;                         // row pitch of the rectified images
@@ -123,30 +162,28 @@ struct Engine {
     mvsv_sgbm_params sgbm_raw{};
     SgbmNorm sg{};
     int td_nc = 0;               // strips per frame of the fused previous-row sweep at max_batch (0: independent passes)
-    uint16_t* sweep_halo = nullptr;   // tagged border-pixel records of the strip hand-off (csrc/sweep.cu)
+    DeviceBuffer<uint16_t> sweep_halo;        // tagged border-pixel records of the strip hand-off (csrc/sweep.cu)
     int num_sms = 148;
     mvsv_bm_params bm_raw{};
     BmNorm bm{};
     // mvsv_set_bm_filters, kept across mvsv_set_bm_params and geometry changes: -1 / 0 = off
     int bm_d12 = -1, bm_speckle_win = 0, bm_speckle_range = 0;
 
-    uint2* recL = nullptr;                    // left prefilter records [B][H][W] (a_s,lo_s,hi_s,a_r,lo_r,hi_r)
-    uint16_t* plR = nullptr;                  // right prefilter planes, reversed + padded: [6][B][H][vsRP]
+    DeviceBuffer<uint2> recL;                 // left prefilter records [B][H][W] (a_s,lo_s,hi_s,a_r,lo_r,hi_r)
+    DeviceBuffer<uint16_t> plR;               // right prefilter planes, reversed + padded: [6][B][H][vsRP]
     int vsNV = 0, vsRP = 0, vsJOFF = 0;
-    uint16_t* VS = nullptr;                   // [B][H][W1][Dp] vertical box sums of the pixel cost
-    uint16_t* C = nullptr;                    // [B][H][W1][Dp] block cost
-    uint16_t* S = nullptr;                    // [B][H][W1][Dp] aggregated cost
-    size_t vol_elems = 0;                     // elements allocated per volume
-    int* d2 = nullptr;                        // [B][H][W] (disp2cost<<16 | disp2)
-    int16_t* disp_raw = nullptr;              // [B][H][W]
-    int16_t* disp_med = nullptr;              // [B][H][W]
-    int* labels = nullptr;                    // [B][H][W]
-    int* sizes = nullptr;                     // [B][H][W]
+    DeviceBuffer<uint16_t> VS;                // [B][H][W1][Dp] vertical box sums of the pixel cost
+    DeviceBuffer<uint16_t> C;                 // [B][H][W1][Dp] block cost
+    DeviceBuffer<uint16_t> S;                 // [B][H][W1][Dp] aggregated cost
+    DeviceBuffer<int> d2;                     // [B][H][W] (disp2cost<<16 | disp2)
+    DeviceBuffer<int16_t> disp_raw;           // [B][H][W]
+    DeviceBuffer<int16_t> disp_med;           // [B][H][W]
+    DeviceBuffer<int> labels;                 // [B][H][W]
+    DeviceBuffer<int> sizes;                  // [B][H][W]
 
-    uint8_t* bm_pre[2] = {nullptr, nullptr};  // [B][H][pitch]
-    int* bm_tex2 = nullptr;                   // [B][H][W] texture: window sums of |L - cap|
-    size_t bm_vol_elems = 0;
-    uint16_t* bm_col = nullptr;               // [B][H][width1][Dp]
+    DeviceBuffer<uint8_t> bm_pre[2];          // [B][H][pitch]
+    DeviceBuffer<int> bm_tex2;                // [B][H][W] texture: window sums of |L - cap|
+    DeviceBuffer<uint16_t> bm_col;            // [B][H][width1][Dp]
 
     bool has_Q[MVSV_MAX_RIGS] = {};
     float Q[MVSV_MAX_RIGS][16];
@@ -156,12 +193,12 @@ struct Engine {
     // device tables below.
     std::vector<int> frame_rig;
     RigFrames rig_frames;
-    RigTables* rig_tables = nullptr;          // device mirror of map_xy and Q; refreshed by a compute when rig_tables_dirty
+    DeviceBuffer<RigTables> rig_tables;       // device mirror of map_xy and Q; refreshed by a compute when rig_tables_dirty
     bool rig_tables_dirty = true;
 
     int nrois = 0;
-    int* rois = nullptr;                      // device [n][4]
-    int* minmax = nullptr;                    // device [B][2]
+    DeviceBuffer<int> rois;                   // [n][4]
+    DeviceBuffer<int> minmax;                 // [B][2]
 };
 
 // the I/O slot of the compute in progress (or of the last one)
