@@ -266,7 +266,8 @@ private:
 
 // src/ply.cpp: ASCII PLY; WITH_COLOR greys every vertex by (z - min)/(max - min)*255 with min/max the smallest and
 // largest positive DISPARITY value of the map (Utility::calcMinMaxDisparity, src/utility.cpp:287-304) -- the
-// reference mixes millimetres and disparity units there; reproduced as is.  minmax comes from mvsv_download_minmax.
+// reference mixes millimetres and disparity units there; reproduced as is.  minmax comes from mvsv_download_minmax; a
+// whole map's points (Utility::dmap2pcl, src/utility.cpp:242-262) from MVSV_STAGE_POINTS and mvsv_download_points.
 class ply {
 public:
     enum MODE { PLAIN, WITH_COLOR, WITH_COLOR_SHADING };
@@ -276,14 +277,40 @@ public:
 
     bool write(std::ostream& out, std::vector<Vec4> const& to_write, int mode) const
     {
+        return write_n(out, to_write.size(), [&](size_t i) { return to_write[i].v; }, mode);
+    }
+    bool write(std::string const& filename, std::vector<Vec4> const& to_write, int mode) const
+    {
+        if (mode != PLAIN && !mHaveMap) return false;
+        std::ofstream f(filename.c_str());
+        return f.is_open() && write(f, to_write, mode);
+    }
+    // n points of x, y, z floats one after the other: the layout mvsv_download_points writes, so that the point list of
+    // a whole map (Utility::dmap2pcl) goes to the file without a copy into Vec4.  The same bytes as the Vec4 overload.
+    bool write(std::ostream& out, const float* xyz, size_t n, int mode) const
+    {
+        return write_n(out, n, [&](size_t i) { return xyz + 3 * i; }, mode);
+    }
+    bool write(std::string const& filename, const float* xyz, size_t n, int mode) const
+    {
+        if (mode != PLAIN && !mHaveMap) return false;
+        std::ofstream f(filename.c_str());
+        return f.is_open() && write(f, xyz, n, mode);
+    }
+
+private:
+    // at(i): the x, y, z of vertex i
+    template <class At>
+    bool write_n(std::ostream& out, size_t n, At at, int mode) const
+    {
         if (mode != PLAIN && !mHaveMap) return false;
         out << "ply\nformat ascii 1.0\ncomment author: " << mAuthor << "\ncomment object:" << mObjectName << "\n";
-        out << "element vertex " << std::to_string(to_write.size()) << "\n";
+        out << "element vertex " << std::to_string(n) << "\n";
         out << "property float x\nproperty float y\nproperty float z\n";
         if (mode != PLAIN) out << "property uchar red\nproperty uchar green\nproperty uchar blue\n";
         out << "end_header\n";
-        for (size_t i = 0; i < to_write.size(); ++i) {
-            const float* t = to_write[i].v;
+        for (size_t i = 0; i < n; ++i) {
+            const float* t = at(i);
             out << t[0] << " " << t[1] << " " << t[2];
             if (mode == WITH_COLOR) {
                 const int g = int((t[2] - mMin) / (mMax - mMin) * 255.0);
@@ -293,14 +320,7 @@ public:
         }
         return true;
     }
-    bool write(std::string const& filename, std::vector<Vec4> const& to_write, int mode) const
-    {
-        if (mode != PLAIN && !mHaveMap) return false;
-        std::ofstream f(filename.c_str());
-        return f.is_open() && write(f, to_write, mode);
-    }
 
-private:
     std::string mAuthor, mObjectName;
     bool mHaveMap = false;
     short mMin = 0, mMax = 0;

@@ -11,7 +11,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvsv.so")
 
-STAGE_RECTIFY, STAGE_SGBM, STAGE_BM, STAGE_XYZ, STAGE_MEANS = 1, 2, 4, 8, 16
+STAGE_RECTIFY, STAGE_SGBM, STAGE_BM, STAGE_XYZ, STAGE_MEANS, STAGE_POINTS = 1, 2, 4, 8, 16, 32
 
 # every symbol include/mvsv.h declares (tests check the library exports all of them)
 ABI_SYMBOLS = (
@@ -22,7 +22,7 @@ ABI_SYMBOLS = (
     "mvsv_download_minmax", "mvsv_download_age", "mvsv_set_io_slots", "mvsv_timer_start", "mvsv_timer_stop", "mvsv_profile_enable", "mvsv_profile_read", "mvsv_kernel_name",
     "mvsv_set_bm_filters", "mvsv_debug_postfilter",
     "mvsv_upload_rectify_maps_rig", "mvsv_set_rectification_rig", "mvsv_set_Q_rig", "mvsv_set_frame_rigs",
-    "mvsv_init_devices", "mvsv_get_devices",
+    "mvsv_init_devices", "mvsv_get_devices", "mvsv_download_points",
 )
 MAX_RIGS = 64       # MVSV_MAX_RIGS
 
@@ -88,6 +88,7 @@ def load_library():
     lib.mvsv_tm.argtypes = [vp, vp, sz, vp, sz, sz, ci, C.c_uint, vp, sz]
     lib.mvsv_download.argtypes = [vp, vp, sz, vp, vp, sz, vp, vp]
     lib.mvsv_download_age.argtypes = [vp, ci, vp, sz, vp, vp, sz, vp, vp]
+    lib.mvsv_download_points.argtypes = [vp, ci, vp, vp, sz]
     lib.mvsv_set_io_slots.argtypes = [vp, ci]
     lib.mvsv_sync.argtypes = [vp]
     lib.mvsv_download_minmax.argtypes = [vp, vp]
@@ -335,6 +336,24 @@ class Engine:
             res["means"] = mn
         return res
 
+    def download_points(self, batch, age=0, out=None):
+        """The point list of STAGE_POINTS (Utility::dmap2pcl, reference src/utility.cpp:242-262) of the compute `age`
+        calls back: (offsets int64 [batch + 1], points float32 [n, 3]); frame f's points are
+        points[offsets[f]:offsets[f + 1]].  `out`: a float32 array (e.g. api.pinned((cap, 3), np.float32).array) the
+        points are copied into, so that a pipelined loop allocates nothing per step; the points returned are a view of it.
+        Without `out` the list is sized by a first call that fetches only the offsets."""
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        offs = np.empty(i.max_batch + 1, np.int64)         # the C call writes the compute's frames + 1 entries
+        if out is None:
+            self._ck(self._lib.mvsv_download_points(self._ctx, age, offs.ctypes.data, None, 0))
+            out = np.empty((int(offs[batch]), 3), np.float32)
+        elif out.dtype != np.float32 or not out.flags.c_contiguous:
+            raise ValueError("out must be a C-contiguous float32 array")
+        self._ck(self._lib.mvsv_download_points(self._ctx, age, offs.ctypes.data, out.ctypes.data, out.size // 3))
+        return offs[:batch + 1], out.reshape(-1)[:3 * int(offs[batch])].reshape(-1, 3)
+
     def download_minmax(self, batch):
         """Utility::calcMinMaxDisparity (reference src/utility.cpp:287-304) per frame, reduced on the GPU."""
         self._check_batch(batch, self.info)
@@ -369,7 +388,7 @@ class Engine:
     def debug_postfilter(self, maps, median=True, new_val=0, speckle_size=0, speckle_diff=0, stages=0):
         """mvsv_debug_postfilter: int16 maps [B,]H,W (row stride may exceed W) through medianBlur(3) when `median`, then
         filterSpeckles(new_val, speckle_size, speckle_diff) when speckle_size > 0, then `stages` (STAGE_XYZ |
-        STAGE_MEANS); the results are fetched with download / download_minmax / debug_read like those of a compute."""
+        STAGE_POINTS | STAGE_MEANS); the results are fetched with download / download_minmax / debug_read like those of a compute."""
         m = np.asarray(maps)
         if m.ndim == 2:
             m = m[None]

@@ -13,7 +13,7 @@
 const char* const kKernelNames[KID_COUNT] = {
     "remap", "sgbm_prefilter", "sgbm_vsum", "sgbm_h1", "sgbm_vdir", "sgbm_td", "sgbm_h2_wta", "median3", "ccl_rows", "ccl_vmerge",
     "ccl_flatten", "ccl_apply", "bm_prefilter", "bm_tex", "bm_colsum", "bm_wta", "xyz", "means", "fill", "minmax", "tm",
-    "bm_lrcheck"};
+    "bm_lrcheck", "points"};
 
 cudaError_t smem_limit(const void* kernel, int bytes)
 {
@@ -83,7 +83,7 @@ int upload_rig_tables(Engine* c)
     return MVSV_OK;
 }
 
-// Releases the slot's buffers sized by the image geometry (rectified images, disparities, XYZ, ROI means), and with
+// Releases the slot's buffers sized by the image geometry (rectified images, disparities, XYZ, points, ROI means), and with
 // `staging` the raw-frame staging too (the slot goes away).  The slot then holds no results.
 void release_slot(IoSlot& s, bool staging)
 {
@@ -91,13 +91,13 @@ void release_slot(IoSlot& s, bool staging)
         s.rect[i].reset();
         if (staging) s.raw[i].reset();
     }
-    s.disp.reset(); s.xyz.reset(); s.means.reset();
+    s.disp.reset(); s.xyz.reset(); s.points.reset(); s.offsets.reset(); s.means.reset();
     s.B = 0; s.stages = 0;
 }
 
 // Allocates what each live slot needs in the engine's present state and does not have yet: the rectified images and
 // the (zeroed) disparities always, the raw-frame staging once rectification maps are installed, the ROI means once ROIs
-// are set.  The XYZ buffer is left to the first compute that asks for it.
+// are set.  The XYZ and point buffers are left to the first compute that asks for them.
 int ensure_slots(Engine* c)
 {
     const size_t B = (size_t)c->maxB, npx = B * c->H * c->W, nimg = B * c->H * c->pitch;
@@ -253,7 +253,7 @@ int apply_geometry(Engine* c, const Geometry& g)
         for (IoSlot& s : c->slot) release_slot(s, false);
         for (auto& b : c->bm_pre) b.reset();
         c->recL.reset(); c->d2.reset(); c->disp_raw.reset(); c->disp_med.reset(); c->labels.reset(); c->sizes.reset();
-        c->bm_tex2.reset(); c->minmax.reset(); c->tm_out.reset();
+        c->bm_tex2.reset(); c->minmax.reset(); c->tm_out.reset(); c->pt_tiles.reset();
         // 16-byte aligned rows; when the width already is (752, 1920, 3840, ...) a batch is one contiguous block and
         // host <-> device transfers are single linear copies instead of strided 2-D copies of many short rows
         c->pitch = round_up((size_t)c->W, 16);
@@ -338,15 +338,29 @@ void take_slot(Engine* c)
     io(c).stages = 0;
 }
 
-// what the XYZ and MEANS stages need of the engine and of the slot they write to; `rigs`: the rigs of the batch's frames
+// what the XYZ, POINTS and MEANS stages need of the engine and of the slot they write to; `rigs`: the rigs of the batch's
+// frames
 int check_consumers(Engine* c, const IoSlot& slot, unsigned stages, uint64_t rigs)
 {
-    if (stages & MVSV_STAGE_XYZ)
+    if (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS))
         for (int r = 0; r < MVSV_MAX_RIGS; ++r)
             if (((rigs >> r) & 1) && !c->has_Q[r])
                 return fail(c, MVSV_ERR_STATE, r == 0 ? "mvsv_set_Q not called" : "no Q for rig " + std::to_string(r) + " (mvsv_set_Q_rig)");
     if ((stages & MVSV_STAGE_MEANS) && (c->nrois < 1 || !c->rois || !slot.means))
         return fail(c, MVSV_ERR_STATE, "no mean-disparity ROIs (mvsv_set_mean_rois; a geometry change drops them)");
+    return MVSV_OK;
+}
+
+// The buffers the XYZ and POINTS stages write, in the slot they write to (and the engine's point tiles)
+int ensure_consumers(Engine* c, IoSlot& slot, unsigned stages)
+{
+    const size_t npx = (size_t)c->maxB * c->H * c->W;
+    if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, slot.xyz.ensure(npx * 3));
+    if (stages & MVSV_STAGE_POINTS) {
+        MVSV_CK(c, slot.points.ensure(npx * 3));
+        MVSV_CK(c, slot.offsets.ensure((size_t)c->maxB + 1));
+        MVSV_CK(c, c->pt_tiles.ensure(points_tiles(c->W, c->H, c->maxB)));
+    }
     return MVSV_OK;
 }
 
@@ -377,8 +391,7 @@ int compute_check(Engine* c, size_t lstride, size_t rstride, int batch, unsigned
     if (stages & MVSV_STAGE_SGBM) rc = ensure_sgbm_volumes(c);
     else if (stages & MVSV_STAGE_BM) rc = ensure_bm_volumes(c);
     if (rc) return rc;
-    if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, slot.xyz.ensure((size_t)c->maxB * c->H * c->W * 3));
-    return MVSV_OK;
+    return ensure_consumers(c, slot, stages);
 }
 
 // Queues engine c's copies and kernels of a compute of `batch` frames; they fill the I/O slot it has taken (take_slot).
@@ -388,7 +401,7 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     const IoSlot& slot = io(c);
     const bool rectify = stages & MVSV_STAGE_RECTIFY;
     const int iw = rectify ? c->fw : c->W, ih = rectify ? c->fh : c->H;
-    // frames of rigs other than 0: the rig-aware remap and XYZ kernels
+    // frames of rigs other than 0: the rig-aware remap, XYZ and point kernels
     const bool multi = rigs_of_batch(c, batch) != 1;
     int rc = bind(c);
     if (rc) return rc;
@@ -401,7 +414,7 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     if (!rc) rc = upload_images(c, dst[1], dpitch, right, rstride, frame_stride, iw, ih, batch, device_src);
     if (!rc) rc = inputs_uploaded(c, device_src);
     if (rc) return rc;
-    if (multi && (rectify || (stages & MVSV_STAGE_XYZ))) {
+    if (multi && (rectify || (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS)))) {
         rc = upload_rig_tables(c);
         if (rc) return rc;
     }
@@ -413,6 +426,7 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     if (stages & MVSV_STAGE_SGBM) MVSV_CK(c, launch_sgbm(c, batch));
     else if (stages & MVSV_STAGE_BM) MVSV_CK(c, launch_bm(c, batch));
     if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
+    if (stages & MVSV_STAGE_POINTS) MVSV_CK(c, launch_points(c, batch, multi));
     if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
     MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
     MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
@@ -458,6 +472,28 @@ int download_enqueue(Engine* c, int k, int16_t* disp, size_t dstride, uint8_t* r
 int download_wait(Engine* c)
 {
     MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));
+    return MVSV_OK;
+}
+
+// mvsv_download_points, first phase: the frame offsets of the point list in I/O slot `k` (B + 1 values) into `offsets`.
+// The copy is a few bytes to pageable memory, which the CUDA runtime completes before it returns.
+int points_offsets(Engine* c, int k, std::vector<long long>& offsets)
+{
+    int rc = bind(c);
+    if (rc) return rc;
+    const IoSlot& s = c->slot[k];
+    offsets.resize((size_t)s.B + 1);
+    MVSV_CK(c, cudaStreamWaitEvent(c->dl_stream, s.done, 0));
+    MVSV_CK(c, cudaMemcpyAsync(offsets.data(), s.offsets, offsets.size() * sizeof(long long), cudaMemcpyDeviceToHost, c->dl_stream));
+    return download_wait(c);
+}
+
+// second phase: queues the copy of the slot's n points to `points` on the download stream (download_wait waits for it)
+int points_enqueue(Engine* c, int k, float* points, long long n)
+{
+    int rc = bind(c);
+    if (rc) return rc;
+    if (n > 0) MVSV_CK(c, cudaMemcpyAsync(points, c->slot[k].points, (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->dl_stream));
     return MVSV_OK;
 }
 
@@ -1118,6 +1154,50 @@ int mvsv_download_age(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8
     return rc;
 }
 
+int mvsv_download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points)
+{
+    int rc = usable(c);
+    if (rc) return rc;
+    if (!offsets) return fail(c, MVSV_ERR_INVALID, "offsets must not be NULL");
+    const Engine* p0 = c->parts[0];
+    if (age < 0 || age >= p0->nslots) return fail(c, MVSV_ERR_INVALID, "age must be below the number of I/O slots");
+    const int s = (p0->cur + p0->nslots - age) % p0->nslots, n = (int)c->parts.size();
+    const std::vector<int> first = firsts(c, s);
+    if (first[n] < 1) return fail(c, MVSV_ERR_STATE, "nothing computed yet");
+    for (int k = 0; k < n; ++k)
+        if (first[k] < first[k + 1] && (!c->parts[k]->slot[s].offsets || !(c->parts[k]->slot[s].stages & MVSV_STAGE_POINTS)))
+            return fail(c, MVSV_ERR_STATE, "POINTS stage was not computed");
+    // phase 1: every part's frame offsets; part k's list goes after the points of the parts before it
+    std::vector<std::vector<long long>> part(n);
+    std::vector<long long> base(n + 1, 0);
+    for (int k = 0; k < n; ++k) {
+        if (first[k] < first[k + 1]) {
+            rc = on_part(c, k, [&](Engine* p) { return points_offsets(p, s, part[k]); });
+            if (rc) return rc;
+        }
+        base[k + 1] = base[k] + (part[k].empty() ? 0 : part[k].back());
+    }
+    for (int k = 0; k < n; ++k)
+        for (int f = first[k]; f < first[k + 1]; ++f) offsets[f] = base[k] + part[k][f - first[k]];
+    offsets[first[n]] = base[n];
+    if (!points) return MVSV_OK;
+    if (capacity_points < (size_t)base[n])
+        return fail(c, MVSV_ERR_INVALID, "points buffer holds " + std::to_string(capacity_points) + " points, the list has " +
+                                             std::to_string(base[n]));
+    // phase 2: every part's copy is queued before the first wait, so that the parts' copies run side by side
+    int queued = 0;
+    for (; queued < n && !rc; ++queued)
+        if (first[queued] < first[queued + 1])
+            rc = on_part(c, queued, [&](Engine* p) { return points_enqueue(p, s, points + 3 * (size_t)base[queued], base[queued + 1] - base[queued]); });
+    // wait also after a failure: the caller's buffer must not be written once the call has returned
+    for (int k = 0; k < queued; ++k)
+        if (first[k] < first[k + 1]) {
+            if (rc) cudaStreamSynchronize(c->parts[k]->dl_stream);
+            else rc = on_part(c, k, download_wait);
+        }
+    return rc;
+}
+
 int mvsv_set_io_slots(mvsv_ctx* ctx, int n)
 {
     return each(ctx, true, [&](Engine* c) -> int {
@@ -1275,16 +1355,16 @@ int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int
         if (rc) return rc;
         if (!maps || batch < 1 || batch > c->maxB) return fail(c, MVSV_ERR_INVALID, "bad map pointer or batch size");
         if (stride < (size_t)c->W * sizeof(int16_t)) return fail(c, MVSV_ERR_INVALID, "stride smaller than the map width");
-        if (stages & ~(unsigned)(MVSV_STAGE_XYZ | MVSV_STAGE_MEANS))
-            return fail(c, MVSV_ERR_INVALID, "post-filter hook: only MVSV_STAGE_XYZ and MVSV_STAGE_MEANS");
+        if (stages & ~(unsigned)(MVSV_STAGE_XYZ | MVSV_STAGE_POINTS | MVSV_STAGE_MEANS))
+            return fail(c, MVSV_ERR_INVALID, "post-filter hook: only MVSV_STAGE_XYZ, MVSV_STAGE_POINTS and MVSV_STAGE_MEANS");
         if (maxSpeckleSize > 0 && (newVal < -32768 || newVal > 32767)) return fail(c, MVSV_ERR_INVALID, "newVal does not fit CV_16S");
         const uint64_t rigs = rigs_of_batch(c, batch);
         const bool multi = rigs != 1;
         // the next I/O slot, taken as a compute takes it
         IoSlot& slot = next_slot(c);
         rc = check_consumers(c, slot, stages, rigs);
+        if (!rc) rc = ensure_consumers(c, slot, stages);
         if (rc) return rc;
-        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, slot.xyz.ensure((size_t)c->maxB * c->H * c->W * 3));
 
         take_slot(c);
         const size_t row = (size_t)c->W * sizeof(int16_t), npx = (size_t)batch * c->H * c->W;
@@ -1295,13 +1375,12 @@ int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int
             MVSV_CK(c, launch_speckle(c, median ? c->disp_med : c->disp_raw, slot.disp, batch, newVal, maxSpeckleSize, maxDiff));
         if (!median && !speckle)
             MVSV_CK(c, cudaMemcpyAsync(slot.disp, c->disp_raw, npx * sizeof(int16_t), cudaMemcpyDeviceToDevice, c->stream));
-        if (stages & MVSV_STAGE_XYZ) {
-            if (multi) {
-                rc = upload_rig_tables(c);
-                if (rc) return rc;
-            }
-            MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
+        if (multi && (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS))) {
+            rc = upload_rig_tables(c);
+            if (rc) return rc;
         }
+        if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
+        if (stages & MVSV_STAGE_POINTS) MVSV_CK(c, launch_points(c, batch, multi));
         if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
         MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
         MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));

@@ -422,6 +422,26 @@ k_ccl_apply(const int16_t* __restrict__ img, int16_t* __restrict__ out, const in
 // ------------------------------------------------------------------------------------------------
 struct QMat { double q[16]; };     // the CV_32F matrix, widened on the host (cv::Mat_<float> products accumulate in double)
 
+// Utility::calcCoordinate of one pixel (x, y) of frame f with disparity value > 0; q(f, i) is element i of the frame's
+// Q.  dx, dy: the pixel's coordinates, exact in double (the reference's float coordinates are integers < 2^24).
+template <class QOf>
+__device__ __forceinline__ void reproject(QOf q, int f, double dx, double dy, float value, float& X, float& Y, float& Z)
+{
+    const double dd = (double)(value / 16.f);
+    float cc[4];
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+        // ((((0 + q0 x) + q1 y) + q2 d) + q3 1): every product of two floats is exact in double, one rounding per add
+        double acc = q(f, r * 4) * dx;
+        acc = __fma_rn(q(f, r * 4 + 1), dy, acc);
+        acc = __fma_rn(q(f, r * 4 + 2), dd, acc);
+        acc += q(f, r * 4 + 3);
+        cc[r] = (float)acc;
+    }
+    X = cc[0] / cc[3]; Y = cc[1] / cc[3]; Z = cc[2] / cc[3];
+    if (isinf(Z / 1000.f)) Z = 0.f;
+}
+
 // One thread = four consecutive pixels of the batch's linear pixel index: one 8-byte load, three 16-byte stores.
 // q(f, i) is element i of the Q of frame f (the four pixels may cross a frame boundary).
 template <class QOf>
@@ -445,21 +465,7 @@ __device__ __forceinline__ void xyz_pixels(const int16_t* __restrict__ disp, flo
     for (int k = 0; k < 4; ++k) {
         const float value = (float)v4[k];
         float X = 0.f, Y = 0.f, Z = 0.f;
-        if (value > 0.f) {
-            const double dd = (double)(value / 16.f);
-            float cc[4];
-#pragma unroll
-            for (int r = 0; r < 4; ++r) {
-                // ((((0 + q0 x) + q1 y) + q2 d) + q3 1): every product of two floats is exact in double, one rounding per add
-                double acc = q(f, r * 4) * dx;
-                acc = __fma_rn(q(f, r * 4 + 1), dy, acc);
-                acc = __fma_rn(q(f, r * 4 + 2), dd, acc);
-                acc += q(f, r * 4 + 3);
-                cc[r] = (float)acc;
-            }
-            X = cc[0] / cc[3]; Y = cc[1] / cc[3]; Z = cc[2] / cc[3];
-            if (isinf(Z / 1000.f)) Z = 0.f;
-        }
+        if (value > 0.f) reproject(q, f, dx, dy, value, X, Y, Z);
         o[3 * k] = X; o[3 * k + 1] = Y; o[3 * k + 2] = Z;
         dx += 1.0;
         if (++x == W) { x = 0; dx = 0.0; if (++y == H) { y = 0; ++f; } dy = (double)y; }
@@ -484,6 +490,147 @@ k_xyz_rigs(const int16_t* __restrict__ disp, float* __restrict__ xyz, int W, int
            const int* __restrict__ rig_of_frame)
 {
     xyz_pixels(disp, xyz, W, H, npx, [&](int f, int i) { return rigs->Q[rig_of_frame[f]][i]; });
+}
+
+// Point list (dmap2pcl's selection, reference src/utility.cpp:242-262): the pixels with disparity > 0 in (frame, row,
+// column) order, reprojected as k_xyz does.  Ordered stream compaction in three kernels, none of which waits for
+// another CTA: count the valid pixels of every tile, scan the counts in one CTA, then re-read each tile and write its
+// points at the tile's base.  A tile is PT_TILE pixels of one frame (PT_THREADS threads x 8 consecutive pixels), so
+// a frame's offset is the base of its first tile.  8 pixels per thread keep the emit kernel's staging at 32 KB: shared
+// memory admits seven CTAs per SM, the registers six of k_points_emit (40 per thread) and four of k_points_emit_rigs
+// (57), which is still 1024 threads per SM for a kernel bound by its 2-byte loads and 12-byte stores.
+constexpr int PT_THREADS = 256, PT_PIX = 8, PT_TILE = PT_THREADS * PT_PIX;
+
+// This thread's PT_PIX pixels of the tile starting at p0 of a frame of HW pixels: values in v (0 past the frame), bit k
+// of the result set when v[k] > 0.  One 16-byte load where frames start 16-byte aligned (HW % 8 == 0).
+__device__ __forceinline__ unsigned points_load(const int16_t* __restrict__ frame, int HW, int p0, short (&v)[PT_PIX])
+{
+    if (HW % 8 == 0 && p0 + PT_PIX <= HW) {
+        const uint4 r = ld128(frame + p0);
+        const unsigned w[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) { v[2 * k] = (short)(w[k] & 0xffffu); v[2 * k + 1] = (short)(w[k] >> 16); }
+    } else {
+#pragma unroll
+        for (int k = 0; k < PT_PIX; ++k) v[k] = p0 + k < HW ? frame[p0 + k] : (short)0;
+    }
+    unsigned m = 0;
+#pragma unroll
+    for (int k = 0; k < PT_PIX; ++k) m |= (v[k] > 0 ? 1u : 0u) << k;
+    return m;
+}
+
+// one CTA per tile: its number of valid pixels
+__global__ void __launch_bounds__(PT_THREADS)
+k_points_count(const int16_t* __restrict__ disp, int HW, int tpf, long long* __restrict__ tiles)
+{
+    __shared__ int s_warp[PT_THREADS / 32];
+    const int f = blockIdx.x / tpf, t = blockIdx.x - f * tpf;
+    short v[PT_PIX];
+    const int n = __popc(points_load(disp + (size_t)f * HW, HW, t * PT_TILE + threadIdx.x * PT_PIX, v));
+    const int sum = __reduce_add_sync(0xffffffffu, n);
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = sum;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int total = 0;
+#pragma unroll
+        for (int w = 0; w < PT_THREADS / 32; ++w) total += s_warp[w];
+        tiles[blockIdx.x] = total;
+    }
+}
+
+// One CTA: the counts of the ntiles tiles become their exclusive bases in place; offsets[f] = base of frame f's first
+// tile, offsets[B] = the total.  A thread scans a contiguous segment (26 tiles at 148 frames of 752 x 479).
+constexpr int PT_SCAN_THREADS = 1024;
+
+__global__ void __launch_bounds__(PT_SCAN_THREADS)
+k_points_scan(long long* __restrict__ tiles, int ntiles, int tpf, long long* __restrict__ offsets, int B)
+{
+    __shared__ long long s_warp[PT_SCAN_THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int seg = (ntiles + PT_SCAN_THREADS - 1) / PT_SCAN_THREADS;
+    const int i0 = min((int)threadIdx.x * seg, ntiles), i1 = min(i0 + seg, ntiles);
+    long long sum = 0;
+    for (int i = i0; i < i1; ++i) sum += tiles[i];
+    long long incl = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const long long u = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += u;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    long long run = incl - sum;
+    for (int w = 0; w < warp; ++w) run += s_warp[w];
+    if (threadIdx.x == PT_SCAN_THREADS - 1) offsets[B] = run + sum;
+    for (int i = i0; i < i1; ++i) {
+        const long long n = tiles[i];
+        tiles[i] = run;
+        if (i % tpf == 0) offsets[i / tpf] = run;
+        run += n;
+    }
+}
+
+// One CTA per tile: the valid pixels are ranked within the tile (per-thread prefix, then warp and CTA scans), listed
+// in shared memory in pixel order, reprojected one per thread with the arithmetic of k_xyz, and the tile's span of
+// floats leaves as coalesced 4-byte stores (the span starts at 12 * base bytes: only 4-byte aligned).
+template <class QOf>
+__device__ __forceinline__ void points_emit(const int16_t* __restrict__ disp, int W, int HW, int tpf,
+                                            const long long* __restrict__ tiles, float* __restrict__ points, QOf q)
+{
+    __shared__ unsigned s_pix[PT_TILE];          // value << 16 | pixel index within the tile, in pixel order
+    __shared__ float s_xyz[PT_TILE * 3];
+    __shared__ int s_warp[PT_THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int f = blockIdx.x / tpf, t = blockIdx.x - f * tpf;
+    const int local0 = threadIdx.x * PT_PIX;
+    short v[PT_PIX];
+    unsigned m = points_load(disp + (size_t)f * HW, HW, t * PT_TILE + local0, v);
+    const int n = __popc(m);
+    int incl = n;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int u = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += u;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    int rank = incl - n, total = 0;
+#pragma unroll
+    for (int w = 0; w < PT_THREADS / 32; ++w) {
+        const int s = s_warp[w];
+        rank += w < warp ? s : 0;
+        total += s;
+    }
+#pragma unroll
+    for (int k = 0; k < PT_PIX; ++k)
+        if ((m >> k) & 1u) s_pix[rank++] = (unsigned)(unsigned short)v[k] << 16 | (unsigned)(local0 + k);
+    __syncthreads();
+    for (int i = threadIdx.x; i < total; i += PT_THREADS) {
+        const unsigned e = s_pix[i];
+        const int p = t * PT_TILE + (int)(e & 0xffffu), y = p / W, x = p - y * W;
+        float X, Y, Z;
+        reproject(q, f, (double)x, (double)y, (float)(short)(e >> 16), X, Y, Z);
+        s_xyz[3 * i] = X; s_xyz[3 * i + 1] = Y; s_xyz[3 * i + 2] = Z;
+    }
+    __syncthreads();
+    float* dst = points + 3 * (size_t)tiles[blockIdx.x];
+    for (int j = threadIdx.x; j < 3 * total; j += PT_THREADS) dst[j] = s_xyz[j];
+}
+
+__global__ void __launch_bounds__(PT_THREADS)
+k_points_emit(const int16_t* __restrict__ disp, int W, int HW, int tpf, const long long* __restrict__ tiles,
+              float* __restrict__ points, QMat Q)
+{
+    points_emit(disp, W, HW, tpf, tiles, points, [&](int, int i) { return Q.q[i]; });
+}
+
+// Frames of several rigs: each frame's points reproject with the Q of its rig, as in k_xyz_rigs.
+__global__ void __launch_bounds__(PT_THREADS)
+k_points_emit_rigs(const int16_t* __restrict__ disp, int W, int HW, int tpf, const long long* __restrict__ tiles,
+                   float* __restrict__ points, const RigTables* __restrict__ rigs, const int* __restrict__ rig_of_frame)
+{
+    points_emit(disp, W, HW, tpf, tiles, points, [&](int f, int i) { return rigs->Q[rig_of_frame[f]][i]; });
 }
 
 // Eight lanes per ROI (and frame), four ROIs per warp: the reference's Samplepoint windows are 5 x 5 pixels (a whole warp
@@ -650,6 +797,26 @@ cudaError_t launch_xyz_rigs(Engine* c, int B)
     KernelTimer kt(c, KID_XYZ);
     k_xyz_rigs<<<(unsigned)((npx / 4 + 256) / 256), 256, 0, c->stream>>>(io(c).disp, io(c).xyz, c->W, c->H, npx, c->rig_tables,
                                                                          c->rig_frames.rig);
+    return cudaGetLastError();
+}
+
+size_t points_tiles(int W, int H, int B) { return (size_t)B * (((size_t)W * H + PT_TILE - 1) / PT_TILE); }
+
+cudaError_t launch_points(Engine* c, int B, bool rigs)
+{
+    const int HW = c->W * c->H, tpf = (int)points_tiles(c->W, c->H, 1), ntiles = (int)points_tiles(c->W, c->H, B);
+    const int16_t* disp = io(c).disp;
+    { KernelTimer kt(c, KID_POINTS); k_points_count<<<ntiles, PT_THREADS, 0, c->stream>>>(disp, HW, tpf, c->pt_tiles); }
+    { KernelTimer kt(c, KID_POINTS); k_points_scan<<<1, PT_SCAN_THREADS, 0, c->stream>>>(c->pt_tiles, ntiles, tpf, io(c).offsets, B); }
+    KernelTimer kt(c, KID_POINTS);
+    if (rigs) {
+        k_points_emit_rigs<<<ntiles, PT_THREADS, 0, c->stream>>>(disp, c->W, HW, tpf, c->pt_tiles, io(c).points, c->rig_tables,
+                                                                 c->rig_frames.rig);
+    } else {
+        QMat Q;
+        for (int i = 0; i < 16; ++i) Q.q[i] = (double)c->Q[0][i];
+        k_points_emit<<<ntiles, PT_THREADS, 0, c->stream>>>(disp, c->W, HW, tpf, c->pt_tiles, io(c).points, Q);
+    }
     return cudaGetLastError();
 }
 

@@ -31,7 +31,7 @@ struct BmNorm {
 enum KernelId {
     KID_REMAP = 0, KID_SGBM_PREFILTER, KID_SGBM_VSUM, KID_SGBM_H1, KID_SGBM_VDIR, KID_SGBM_TD, KID_SGBM_H2_WTA, KID_MEDIAN,
     KID_CCL_ROWS, KID_CCL_VMERGE, KID_CCL_FLATTEN, KID_CCL_APPLY, KID_BM_PREFILTER, KID_BM_TEX, KID_BM_COLSUM,
-    KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_BM_LRCHECK, KID_COUNT
+    KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_BM_LRCHECK, KID_POINTS, KID_COUNT
 };
 extern const char* const kKernelNames[KID_COUNT];
 
@@ -84,6 +84,10 @@ struct IoSlot {
     DeviceBuffer<uint8_t> raw[2];             // [B][fh][raw_pitch], once rectification maps are installed
     DeviceBuffer<int16_t> disp;               // final disparities [B][H][W]
     DeviceBuffer<float> xyz;                  // [B][H][W][3], allocated by the first compute with MVSV_STAGE_XYZ
+    // MVSV_STAGE_POINTS, allocated by the first compute with it: the packed point list ([B*H*W][3] at most) and the
+    // frame offsets into it ([B+1]).  In the slot, because a download at age 1 reads them while the next compute runs.
+    DeviceBuffer<float> points;
+    DeviceBuffer<long long> offsets;
     DeviceBuffer<float> means;                // [B][nrois], once mean-disparity ROIs are set
     cudaEvent_t done = nullptr;               // all kernels of the slot's last compute have finished
     int B = 0;                                // frames of the slot's last compute; 0: it holds no results
@@ -199,6 +203,7 @@ struct Engine {
     int nrois = 0;
     DeviceBuffer<int> rois;                   // [n][4]
     DeviceBuffer<int> minmax;                 // [B][2]
+    DeviceBuffer<long long> pt_tiles;         // MVSV_STAGE_POINTS: per tile, its count, then its base (points_tiles)
 };
 
 // the I/O slot of the compute in progress (or of the last one)
@@ -250,6 +255,10 @@ cudaError_t launch_tm(Engine* c, int B, int k, uint8_t* out, size_t opitch);
 cudaError_t launch_xyz(Engine* c, int B);
 cudaError_t launch_xyz_rigs(Engine* c, int B);                 // frames of several rigs (mvsv_set_frame_rigs)
 cudaError_t launch_means(Engine* c, int B);
+// MVSV_STAGE_POINTS of the current I/O slot: the point tiles of B frames of W x H (the size of Engine::pt_tiles), and the
+// launch; `rigs`: frames of several rigs (mvsv_set_frame_rigs)
+size_t points_tiles(int W, int H, int B);
+cudaError_t launch_points(Engine* c, int B, bool rigs);
 cudaError_t launch_minmax(Engine* c, int B);
 cudaError_t launch_median(Engine* c, const int16_t* in, int16_t* out, int B);
 cudaError_t launch_speckle(Engine* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
