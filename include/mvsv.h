@@ -122,7 +122,10 @@ int mvsv_get_devices(const mvsv_ctx* ctx, int* devices, int n);
 
 /* Replaces the eight StereoSGBM setters + setMode of Disparity::loadSGBMParameters
  * (src/disparity.cpp:83-95).  Parameters outside the bit-exact contract are rejected:
- * numDisp in [8,256] and a multiple of 8; blockSize^2*(2*ftzero+63)+P2 <= 32767 (SURVEY.md section 7). */
+ * numDisp in [8,512] and a multiple of 8; blockSize^2*(2*ftzero+63)+P2 <= 32767 (SURVEY.md section 7).
+ * numDisp > 256 also needs a non-empty cost domain, W + min(minDisp, 0) > max(minDisp + numDisp, 0) (MVSV_ERR_INVALID
+ * otherwise, also for a later geometry change that would empty it); a cost volume of one frame above 2^31 cells
+ * (H * W1 * padded numDisp, e.g. 3840x2160 at numDisp > 256) is MVSV_ERR_UNSUPPORTED. */
 int mvsv_set_sgbm_params(mvsv_ctx* ctx, const mvsv_sgbm_params* p);
 /* cv::StereoBM::create(numDisp, blockSize) + setters (trgt/disparityTest.cpp:268, configs/bm.yml). */
 int mvsv_set_bm_params(mvsv_ctx* ctx, const mvsv_bm_params* p);

@@ -122,17 +122,19 @@ int normalise_sgbm(Engine* c, const mvsv_sgbm_params* p, int W, int H, SgbmNorm*
 {
     n->minD = p->minDisp;
     n->D = p->numDisp;
-    if (n->D <= 0 || n->D % 8 != 0 || n->D > 256)
-        return fail(c, MVSV_ERR_INVALID, "numDisp must be a positive multiple of 8 and <= 256");
-    // pixel stride of the volumes = the sweep's lane layout (csrc/sweep.cu): numDisp rounded up to 8, 16 or 32;
-    // the row-scan and cost kernels spread a pixel over the next power of two of lanes (8 disparities each)
+    if (n->D <= 0 || n->D % 8 != 0 || n->D > 512)
+        return fail(c, MVSV_ERR_INVALID, "numDisp must be a positive multiple of 8 and <= 512");
+    // pixel stride of the volumes = the sweep's lane layout (csrc/sweep.cu): numDisp rounded up to 8, 16 or 32, or for
+    // D > 256 to one of 320 / 384 / 448 / 512; the row-scan and cost kernels spread a pixel over the next power of two
+    // of lanes, 8 disparities each (D > 256: one warp, 16 disparities per lane)
     {
         int sg, snr;
         sweep_layout(n->D, &sg, &snr);
         n->Dp = sg * 2 * snr;
     }
+    n->dpl = n->D > 256 ? 16 : 8;
     int g = 1;
-    while (g * 8 < n->Dp) g <<= 1;
+    while (g * n->dpl < n->Dp) g <<= 1;
     n->G = g;
     n->bs = p->blockSize > 0 ? p->blockSize : 5;
     n->SW2 = n->SH2 = n->bs / 2;
@@ -145,6 +147,10 @@ int normalise_sgbm(Engine* c, const mvsv_sgbm_params* p, int W, int H, SgbmNorm*
     n->minX1 = std::max(n->maxD, 0);
     n->maxX1 = W + std::min(n->minD, 0);
     n->W1 = n->maxX1 - n->minX1;
+    // a range wider than 256 must leave some pixel with every disparity inside the image (it would give an all-INVALID
+    // map otherwise)
+    if (n->D > 256 && n->W1 <= 0)
+        return fail(c, MVSV_ERR_INVALID, "numDisp > 256 needs a non-empty cost domain: W + min(minDisp, 0) > max(minDisp + numDisp, 0)");
     n->INV = (n->minD - 1) * 16;
     n->mode = p->disparityMode == 1 ? 1 : 0;   // reference src/disparity.cpp:92-95
     n->npaths = n->mode ? 8 : 5;

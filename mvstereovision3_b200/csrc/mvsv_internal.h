@@ -14,7 +14,8 @@
 // Normalised StereoSGBM parameters (SURVEY.md 8a-3; OpenCV's own normalisation of the values that
 // Disparity::loadSGBMParameters hands over, reference src/disparity.cpp:83-95).
 struct SgbmNorm {
-    int minD, D, Dp, G;          // Dp = G*8 padded disparity count, G = lanes per pixel (power of two)
+    int minD, D, Dp, G;          // Dp = padded disparity count (pixel stride), G = lanes per pixel (power of two)
+    int dpl;                     // disparities per lane in the row scans: 8, or 16 when D > 256 (G = 32, Dp <= 16 G)
     int bs, SW2, SH2, ftzero, uniq, d12, P1, P2;
     int maxD, minX1, maxX1, W1, INV, mode, npaths;
     int speckleWin, speckleRange;

@@ -4,7 +4,7 @@
 // lives in sweep.cu.
 //
 // Data layout in HBM (volumes: disparity innermost, pixel stride Dp = numDisp rounded up to 8 / 16 / 32 for
-// D <= 64 / 128 / 256):
+// D <= 64 / 128 / 256, and to the sweep's 8-lane layout, one of 320 / 384 / 448 / 512, for D <= 512):
 //   recL[B][H][W] 8-byte records, plR[6][B][H][RP] u16 : prefilter channels a/lo/hi of the clipped x-Sobel and the raw image
 //   VS[B][H][W1][Dp] u16            : vertical box sums of the Birchfield-Tomasi pixel cost
 //   C [B][H][W1][Dp] u16            : block cost (horizontal box sum of VS)
@@ -13,7 +13,9 @@
 // Lane mapping of the kernels in this file: a pixel's disparities are spread over G adjacent lanes (G = next power of
 // two >= Dp / 8), 8 disparities (four packed u16x2 registers) per lane; lanes beyond Dp hold padding and never touch
 // memory; the min over d is a width-G shuffle butterfly; all arithmetic is packed 16x2 (VIADD / VIMNMX.U16x2 /
-// VIMNMX3 / VIADDMNMX on the integer ALU pipe of sm_100a).
+// VIMNMX3 / VIADDMNMX on the integer ALU pipe of sm_100a).  numDisp > 256: the row scans keep a pixel in one warp with
+// 16 disparities (NH = 2 halves of 8, each all padding or none) per lane, and the cost kernel runs once per block of
+// 256 disparities.
 #include "mvsv_internal.h"
 
 #include <algorithm>
@@ -460,6 +462,50 @@ __device__ __forceinline__ void sat_acc(uint4& S, const unsigned (&L)[4])
     S.z = __viaddmin_u16x2(S.z, L[2], MVSV_PK_MAX); S.w = __viaddmin_u16x2(S.w, L[3], MVSV_PK_MAX);
 }
 
+// A lane's 8 * NH disparities: NH = 1 is the form above; NH = 2 (numDisp > 256, G = 32) runs the same recurrence over
+// eight registers, with the neighbour shuffles only at the two ends of the lane's run and the REDUX minimum over the
+// warp.  padH[h]: half h of the lane (disparities 8 (NH q + h) .. + 7) lies beyond numDisp and holds 0x7fff.
+template <int G, bool PAD, int NH>
+__device__ __forceinline__ void lane_step(unsigned (&L)[4 * NH], unsigned& mm, const uint4 (&C)[NH], unsigned P1P1,
+                                          unsigned P2P2, int q, const bool (&padH)[NH])
+{
+    if constexpr (NH == 1) {
+        sgm_step<G, PAD>(L, mm, C[0], P1P1, P2P2, q, padH[0]);
+    } else {
+        static_assert(G == 32 && NH == 2, "16 disparities per lane: a pixel is one warp");
+        unsigned P[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) P[j] = L[j] + P1P1;
+        const unsigned u = __shfl_up_sync(FULL, P[7], 1), d = __shfl_down_sync(FULL, P[0], 1);
+        const unsigned up = q != 0 ? u : 0xffffffffu, dn = q != G - 1 ? d : 0xffffffffu;
+        const unsigned Cw[8] = {C[0].x, C[0].y, C[0].z, C[0].w, C[1].x, C[1].y, C[1].z, C[1].w};
+        const unsigned mP2 = mm + P2P2;
+        unsigned Xj = __byte_perm(up, P[0], 0x5432), n[8];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            const unsigned Xn = __byte_perm(P[j], j + 1 < 8 ? P[j + 1] : dn, 0x5432);
+            n[j] = __vimin3_u16x2(Xj, Xn, __vminu2(L[j], mP2)) + Cw[j] - mm;
+            Xj = Xn;
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) L[j] = (PAD && padH[j >> 2]) ? MVSV_PK_MAX : n[j];
+        const unsigned m = __vminu2(__vimin3_u16x2(L[0], L[1], L[2]), __vimin3_u16x2(L[3], L[4], __vimin3_u16x2(L[5], L[6], L[7])));
+        mm = __reduce_min_sync(FULL, min(m & 0xffffu, m >> 16)) * 0x10001u;
+    }
+}
+
+template <bool PAD, int NH>
+__device__ __forceinline__ void lane_reset(unsigned (&L)[4 * NH], unsigned& mm, const bool (&padH)[NH])
+{
+    if constexpr (NH == 1) {
+        reset_state<PAD>(L, mm, padH[0]);
+    } else {
+#pragma unroll
+        for (int j = 0; j < 4 * NH; ++j) L[j] = (PAD && padH[j >> 2]) ? MVSV_PK_MAX : 0u;
+        mm = 0u;
+    }
+}
+
 struct AggArgs {
     const uint16_t* VS; uint16_t* C; uint16_t* S;
     int H, W, W1, D, Dp, SW2, B;
@@ -547,6 +593,93 @@ __global__ void __launch_bounds__(128) k_sgbm_h1(AggArgs a)
     cp_async_wait<0>();
 }
 
+// K3a for numDisp > 256: the same scan with a pixel in one warp and 16 disparities (NH = 2 halves) per lane.
+template <bool PAD, bool S8>
+__global__ void __launch_bounds__(128) k_sgbm_h1_w16(AggArgs a)
+{
+    constexpr int G = 32, NH = 2;
+    // a pixel's stride in the volumes is a.Dp <= 8*NH*G: lanes beyond it hold padding only and never touch memory
+    const int DP = a.Dp;
+    const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long nrows = (long long)a.B * a.H;
+    long long row = gtid / G;
+    const int q = (int)(gtid % G);
+    const bool mem = q * 8 * NH < DP;
+    const bool active = row < nrows && mem;
+    if (row >= nrows) row = nrows - 1;
+    bool padH[NH];
+#pragma unroll
+    for (int h = 0; h < NH; ++h) padH[h] = q * 8 * NH + 8 * h >= a.D;
+    const int W1 = a.W1, SW2 = a.SW2;
+    const size_t rowBase = (size_t)row * W1 * DP + (mem ? q * 8 * NH : 0);
+    const uint16_t* __restrict__ vs = a.VS + rowBase;
+    uint16_t* __restrict__ cp = a.C + rowBase;
+    uint16_t* __restrict__ sp = a.S + rowBase;
+    uint8_t* __restrict__ sp8 = reinterpret_cast<uint8_t*>(a.S) + rowBase;      // S8: one byte per cell, same indexing
+
+    // Stream element t = VS[clamp(t - SW2)], t >= 0.  The window of step xi is t in [xi, xi + bs): it gains
+    // t = xi + bs and loses t = xi.  Ring slot of t is t mod R with R = bs + PFD, so the element fetched at step
+    // xi (t = xi + bs + PFD) lands in the slot of the element that has just left.  A slot holds the lane's NH 16-byte
+    // chunks, 128 * 16 bytes apart.
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    uint4* ring = reinterpret_cast<uint4*>(smem_raw) + threadIdx.x;
+    const int bs = 2 * SW2 + 1, R = bs + H1_PFD;
+    auto src = [&](int t) { return vs + min(max(t - SW2, 0), W1 - 1) * DP; };
+    for (int t = 0; t < bs; ++t)
+#pragma unroll
+        for (int h = 0; h < NH; ++h) cp_async16(ring + (t * NH + h) * 128, src(t) + 8 * h);
+    cp_async_commit();
+#pragma unroll
+    for (int k = 0; k < H1_PFD; ++k) {
+#pragma unroll
+        for (int h = 0; h < NH; ++h) cp_async16(ring + ((bs + k) * NH + h) * 128, src(bs + k) + 8 * h);
+        cp_async_commit();
+    }
+    // (lanes beyond the pixel stride read the first lane's data: valid addresses, values unused)
+    cp_async_wait<H1_PFD>();
+    uint4 hs[NH] = {};
+    for (int t = 0; t < bs; ++t) {
+#pragma unroll
+        for (int h = 0; h < NH; ++h) {
+            const uint4 v = ring[(t * NH + h) * 128];
+            hs[h].x += v.x; hs[h].y += v.y; hs[h].z += v.z; hs[h].w += v.w;
+        }
+    }
+    unsigned L[4 * NH], mm;
+    lane_reset<PAD, NH>(L, mm, padH);
+    int sOut = 0, sIn = bs;                         // slots of t = xi and t = xi + bs
+    for (int xi = 0; xi < W1; ++xi) {
+        cp_async_wait<H1_PFD - 1>();                // the group issued H1_PFD steps ago (t = xi + bs) has landed
+        uint4 od[NH], nx[NH];
+#pragma unroll
+        for (int h = 0; h < NH; ++h) { od[h] = ring[(sOut * NH + h) * 128]; nx[h] = ring[(sIn * NH + h) * 128]; }
+#pragma unroll
+        for (int h = 0; h < NH; ++h) cp_async16(ring + (sOut * NH + h) * 128, src(xi + bs + H1_PFD) + 8 * h);
+        cp_async_commit();
+        if (++sOut == R) sOut = 0;
+        if (++sIn == R) sIn = 0;
+        lane_step<G, PAD, NH>(L, mm, hs, a.P1P1, a.P2P2, q, padH);
+        if (active) {
+#pragma unroll
+            for (int h = 0; h < NH; ++h) {
+                st128(cp + xi * DP + 8 * h, hs[h]);
+                if (S8) {
+                    // L - C is in [0, P2] for every disparity (no borrow between the halves): keep the low bytes
+                    const unsigned e0 = L[4 * h] - hs[h].x, e1 = L[4 * h + 1] - hs[h].y, e2 = L[4 * h + 2] - hs[h].z, e3 = L[4 * h + 3] - hs[h].w;
+                    *reinterpret_cast<uint2*>(sp8 + xi * DP + 8 * h) = make_uint2(__byte_perm(e0, e1, 0x6420), __byte_perm(e2, e3, 0x6420));
+                } else {
+                    st128(sp + xi * DP + 8 * h, make_uint4(L[4 * h], L[4 * h + 1], L[4 * h + 2], L[4 * h + 3]));
+                }
+            }
+        }
+#pragma unroll
+        for (int h = 0; h < NH; ++h) {
+            hs[h].x += nx[h].x - od[h].x; hs[h].y += nx[h].y - od[h].y; hs[h].z += nx[h].z - od[h].z; hs[h].w += nx[h].w - od[h].w;
+        }
+    }
+    cp_async_wait<0>();
+}
+
 // K3b: vertical / diagonal paths, one direction per launch (generic fallback when the fused sweep below does
 // not fit in shared memory).  One lane group follows one path line through the frame: the vertical line of
 // column g, or the diagonal that starts at column g and wraps around the cost domain (a wrap is exactly an
@@ -585,6 +718,48 @@ __global__ void __launch_bounds__(128) k_sgbm_vdir(AggArgs a, int dxs, int botto
     }
 }
 
+// K3b for numDisp > 256 (one warp per pixel, 16 disparities per lane).
+template <bool PAD>
+__global__ void __launch_bounds__(128) k_sgbm_vdir_w16(AggArgs a, int dxs, int bottomUp)
+{
+    constexpr int G = 32, NH = 2;
+    const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long ncols = (long long)a.B * a.W1;
+    long long col = gtid / G;
+    const int q = (int)(gtid % G);
+    const bool active = col < ncols;
+    if (!active) col = ncols - 1;
+    const int f = (int)(col / a.W1);
+    int x = (int)(col % a.W1);
+    bool padH[NH];
+#pragma unroll
+    for (int h = 0; h < NH; ++h) padH[h] = q * 8 * NH + 8 * h >= a.D;
+    const int DP = a.Dp;
+    const bool mem = q * 8 * NH < DP;
+    const size_t frameBase = (size_t)f * a.H * a.W1 * DP + (mem ? q * 8 * NH : 0);
+
+    unsigned L[4 * NH], mm;
+    lane_reset<PAD, NH>(L, mm, padH);
+    for (int yi = 0; yi < a.H; ++yi) {
+        const int y = bottomUp ? a.H - 1 - yi : yi;
+        const size_t off = frameBase + ((size_t)y * a.W1 + x) * DP;
+        uint4 Cc[NH], Sc[NH];
+#pragma unroll
+        for (int h = 0; h < NH; ++h) { Cc[h] = ld128(a.C + off + 8 * h); Sc[h] = ld128(a.S + off + 8 * h); }
+        if ((dxs < 0 && x == 0) || (dxs > 0 && x == a.W1 - 1)) lane_reset<PAD, NH>(L, mm, padH);
+        lane_step<G, PAD, NH>(L, mm, Cc, a.P1P1, a.P2P2, q, padH);
+#pragma unroll
+        for (int h = 0; h < NH; ++h) {
+            Sc[h].x = __viaddmin_u16x2(Sc[h].x, L[4 * h], MVSV_PK_MAX); Sc[h].y = __viaddmin_u16x2(Sc[h].y, L[4 * h + 1], MVSV_PK_MAX);
+            Sc[h].z = __viaddmin_u16x2(Sc[h].z, L[4 * h + 2], MVSV_PK_MAX); Sc[h].w = __viaddmin_u16x2(Sc[h].w, L[4 * h + 3], MVSV_PK_MAX);
+            if (active && mem) st128(a.S + off + 8 * h, Sc[h]);
+        }
+        x -= dxs;
+        if (x >= a.W1) x = 0;
+        if (x < 0) x = a.W1 - 1;
+    }
+}
+
 // K3c + K4: right-to-left path r=(+1,0) fused with winner-take-all, uniqueness, sub-pixel interpolation,
 // the disp2 scatter (sequential in x per row, exactly the reference order) and the left-right check.
 template <int G>
@@ -605,7 +780,7 @@ __device__ __forceinline__ int div_trunc_small(int n, int d)
     return n < 0 ? -qq : qq;
 }
 
-template <int G, bool PAD, bool S8>
+template <int G, bool PAD, bool S8, int NH>
 __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
 {
     const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -614,11 +789,13 @@ __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
     const int q = (int)(gtid % G);
     const bool active = row < nrows;
     if (!active) row = nrows - 1;
-    const bool padLane = q * 8 >= a.D;
-    const int Dp = a.Dp;                            // pixel stride of the volumes (<= 8*G; lanes beyond it hold padding)
-    const bool mem = q * 8 < Dp;
+    bool padH[NH];
+#pragma unroll
+    for (int h = 0; h < NH; ++h) padH[h] = q * 8 * NH + 8 * h >= a.D;
+    const int Dp = a.Dp;                            // pixel stride of the volumes (<= 8*NH*G; lanes beyond it hold padding)
+    const bool mem = q * 8 * NH < Dp;
     const int W1 = a.W1;
-    const size_t rowBase = (size_t)row * W1 * Dp + (mem ? q * 8 : 0);
+    const size_t rowBase = (size_t)row * W1 * Dp + (mem ? q * 8 * NH : 0);
     const uint16_t* __restrict__ cp = a.C + rowBase;
     uint16_t* __restrict__ sp = a.S + rowBase;
     const uint8_t* __restrict__ sp8 = reinterpret_cast<const uint8_t*>(a.S) + rowBase;
@@ -634,15 +811,15 @@ __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
         for (int x = q; x < a.W; x += G) { drow[x] = (int16_t)a.INV; d2row[x] = (int)D2_EMPTY; }
     __syncwarp();
 
-    unsigned L[4], mm;
-    reset_state<PAD>(L, mm, padLane);
+    unsigned L[4 * NH], mm;
+    lane_reset<PAD, NH>(L, mm, padH);
     const int umul = 100 - a.uniq;
-    const unsigned kb = (unsigned)q * 8u;
+    const unsigned kb = (unsigned)q * (8u * NH);
     // The winner's neighbours S[best -/+ 1] are read from a shared-memory copy of the pixel's sums (any lane can address
     // any disparity there: no register picks, no index shuffles); two copies used in turn, one warp barrier per step.
-    __shared__ __align__(16) uint16_t sS[2][128 * 8];
-    uint16_t* smine = &sS[0][0] + threadIdx.x * 8;
-    const uint16_t* spix = &sS[0][0] + (threadIdx.x / G) * G * 8;
+    __shared__ __align__(16) uint16_t sS[2][128 * 8 * NH];
+    uint16_t* smine = &sS[0][0] + threadIdx.x * 8 * NH;
+    const uint16_t* spix = &sS[0][0] + (threadIdx.x / G) * G * 8 * NH;
     int alt = 0;
     // The per-pixel epilogue (parabola, division, scatter, store) is identical on all G lanes of a pixel, so it is
     // deferred: lane q keeps the winner of every G-th step and the G lanes finish G pixels at once.
@@ -665,34 +842,49 @@ __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
         }
         svX = -1;
     };
-    auto step = [&](const uint4& Cq, const uint4& Sq, int xi) {
-        sgm_step<G, PAD>(L, mm, Cq, a.P1P1, a.P2P2, q, padLane);
-        unsigned Sf[4];
-        if (S8) {
-            // Sum of all paths = (n + 1) * C + byte + (L - C), n paths before this one.  With c' = min(C, ceil(32767 / (n+1)))
-            // the product (n + 1) * c' plus the small excess fits 16 bits and reaches 32767 exactly when the true sum does:
-            // one clamp, one multiply-add and one saturation per register instead of rebuilding S and adding L.
-            const unsigned b0 = __byte_perm(Sq.x, 0, 0x4140), b1 = __byte_perm(Sq.x, 0, 0x4342);
-            const unsigned b2 = __byte_perm(Sq.y, 0, 0x4140), b3 = __byte_perm(Sq.y, 0, 0x4342);
-            const unsigned n1 = a.nprevPk & 0xffffu;          // n + 1
-            Sf[0] = __vminu2(__vminu2(Cq.x, a.kclampPk) * n1 + (b0 + L[0] - Cq.x), MVSV_PK_MAX);
-            Sf[1] = __vminu2(__vminu2(Cq.y, a.kclampPk) * n1 + (b1 + L[1] - Cq.y), MVSV_PK_MAX);
-            Sf[2] = __vminu2(__vminu2(Cq.z, a.kclampPk) * n1 + (b2 + L[2] - Cq.z), MVSV_PK_MAX);
-            Sf[3] = __vminu2(__vminu2(Cq.w, a.kclampPk) * n1 + (b3 + L[3] - Cq.w), MVSV_PK_MAX);
-        } else {
-            Sf[0] = __viaddmin_u16x2(Sq.x, L[0], MVSV_PK_MAX);
-            Sf[1] = __viaddmin_u16x2(Sq.y, L[1], MVSV_PK_MAX);
-            Sf[2] = __viaddmin_u16x2(Sq.z, L[2], MVSV_PK_MAX);
-            Sf[3] = __viaddmin_u16x2(Sq.w, L[3], MVSV_PK_MAX);
+    auto step = [&](const uint4 (&Cq)[NH], const uint4 (&Sq)[NH], int xi) {
+        lane_step<G, PAD, NH>(L, mm, Cq, a.P1P1, a.P2P2, q, padH);
+        unsigned Sf[4 * NH];
+#pragma unroll
+        for (int h = 0; h < NH; ++h) {
+            const unsigned* Lh = L + 4 * h;     // (compile-time offsets: the arrays stay in registers)
+            unsigned* Sh = Sf + 4 * h;
+            if (S8) {
+                // Sum of all paths = (n + 1) * C + byte + (L - C), n paths before this one.  With c' = min(C, ceil(32767 / (n+1)))
+                // the product (n + 1) * c' plus the small excess fits 16 bits and reaches 32767 exactly when the true sum does:
+                // one clamp, one multiply-add and one saturation per register instead of rebuilding S and adding L.
+                const unsigned b0 = __byte_perm(Sq[h].x, 0, 0x4140), b1 = __byte_perm(Sq[h].x, 0, 0x4342);
+                const unsigned b2 = __byte_perm(Sq[h].y, 0, 0x4140), b3 = __byte_perm(Sq[h].y, 0, 0x4342);
+                const unsigned n1 = a.nprevPk & 0xffffu;          // n + 1
+                Sh[0] = __vminu2(__vminu2(Cq[h].x, a.kclampPk) * n1 + (b0 + Lh[0] - Cq[h].x), MVSV_PK_MAX);
+                Sh[1] = __vminu2(__vminu2(Cq[h].y, a.kclampPk) * n1 + (b1 + Lh[1] - Cq[h].y), MVSV_PK_MAX);
+                Sh[2] = __vminu2(__vminu2(Cq[h].z, a.kclampPk) * n1 + (b2 + Lh[2] - Cq[h].z), MVSV_PK_MAX);
+                Sh[3] = __vminu2(__vminu2(Cq[h].w, a.kclampPk) * n1 + (b3 + Lh[3] - Cq[h].w), MVSV_PK_MAX);
+            } else {
+                Sh[0] = __viaddmin_u16x2(Sq[h].x, Lh[0], MVSV_PK_MAX);
+                Sh[1] = __viaddmin_u16x2(Sq[h].y, Lh[1], MVSV_PK_MAX);
+                Sh[2] = __viaddmin_u16x2(Sq[h].z, Lh[2], MVSV_PK_MAX);
+                Sh[3] = __viaddmin_u16x2(Sq[h].w, Lh[3], MVSV_PK_MAX);
+            }
+            if (PAD && padH[h]) Sh[0] = Sh[1] = Sh[2] = Sh[3] = MVSV_PK_MAX;
         }
-        if (PAD && padLane) Sf[0] = Sf[1] = Sf[2] = Sf[3] = MVSV_PK_MAX;
-        st128(smine + alt, make_uint4(Sf[0], Sf[1], Sf[2], Sf[3]));
-        if (a.storeS && active && mem) st128(sdbg + xi * Dp, make_uint4(Sf[0], Sf[1], Sf[2], Sf[3]));
+#pragma unroll
+        for (int h = 0; h < NH; ++h) st128(smine + alt + 8 * h, make_uint4(Sf[4 * h], Sf[4 * h + 1], Sf[4 * h + 2], Sf[4 * h + 3]));
+        if (a.storeS && active && mem)
+#pragma unroll
+            for (int h = 0; h < NH; ++h) st128(sdbg + xi * Dp + 8 * h, make_uint4(Sf[4 * h], Sf[4 * h + 1], Sf[4 * h + 2], Sf[4 * h + 3]));
         // ---- first argmin via (S << 16 | k) keys
         unsigned key = min(min((Sf[0] << 16) | kb, (Sf[0] & 0xffff0000u) | (kb + 1)),
                            min((Sf[1] << 16) | (kb + 2), (Sf[1] & 0xffff0000u) | (kb + 3)));
         key = min(key, min(min((Sf[2] << 16) | (kb + 4), (Sf[2] & 0xffff0000u) | (kb + 5)),
                            min((Sf[3] << 16) | (kb + 6), (Sf[3] & 0xffff0000u) | (kb + 7))));
+        if constexpr (NH == 2) {
+            unsigned k2 = min(min((Sf[4] << 16) | (kb + 8), (Sf[4] & 0xffff0000u) | (kb + 9)),
+                              min((Sf[5] << 16) | (kb + 10), (Sf[5] & 0xffff0000u) | (kb + 11)));
+            k2 = min(k2, min(min((Sf[6] << 16) | (kb + 12), (Sf[6] & 0xffff0000u) | (kb + 13)),
+                             min((Sf[7] << 16) | (kb + 14), (Sf[7] & 0xffff0000u) | (kb + 15))));
+            key = min(key, k2);
+        }
         key = group_min_u32<G>(key);
         const int minS = (int)(key >> 16);
         const int best = (int)(key & 0xffffu);
@@ -701,7 +893,7 @@ __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
         const int im = max(best - 1, 0), ip = min(best + 1, a.D - 1);
         __syncwarp();
         const unsigned vm = spix[alt + im], vp = spix[alt + ip];
-        alt ^= 128 * 8;
+        alt ^= 128 * 8 * NH;
         if (a.uniq > 0) {
             // Rejected when some disparity further than 1 from the winner has S * (100 - uniq) < minS * 100.  The test is
             // monotone in S (100 - uniq > 0), so the lane only needs the smallest of its sums outside best-1..best+1:
@@ -711,21 +903,22 @@ __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
             // per step costs more than eight multiply-compares.)
             bool bad = false;
             if (umul > 0) {
-                if (!(PAD && padLane)) {
+                if (NH == 2 || !(PAD && padH[0])) {
                     const unsigned b1 = ((unsigned)(best - 1) & 0xffffu) * 0x10001u;    // best - 1 mod 2^16 in both halves (best may be 0)
                     unsigned mn = 0xffffffffu;
 #pragma unroll
-                    for (int r = 0; r < 4; ++r) {
+                    for (int r = 0; r < 4 * NH; ++r) {
                         const unsigned kk2 = (kb + 2u * r) * 0x10001u + 0x00010000u;    // (kb + 2r, kb + 2r + 1)
                         const unsigned ex = __vcmpleu2(__vsub2(kk2, b1), 0x00020002u);  // 0xffff where |k - best| <= 1
-                        mn = __vminu2(mn, Sf[r] | ex);
+                        // (NH = 2: a padding half is left out as a whole, like a padding lane)
+                        mn = __vminu2(mn, Sf[r] | ex | ((NH == 2 && PAD && padH[r >> 2]) ? 0xffffffffu : 0u));
                     }
                     const int s = (int)min(mn & 0xffffu, mn >> 16);
                     bad = s <= 0x7fff && s * umul < minS * 100;
                 }
             } else {
 #pragma unroll
-                for (int j = 0; j < 8; ++j) {
+                for (int j = 0; j < 8 * NH; ++j) {
                     const int kk = (int)kb + j;
                     const int s = (int)((j & 1) ? (Sf[j >> 1] >> 16) : (Sf[j >> 1] & 0xffffu));
                     bad |= (!PAD || kk < a.D) && (s * umul < minS * 100) && (abs(kk - best) > 1);
@@ -737,21 +930,24 @@ __global__ void __launch_bounds__(128) k_sgbm_h2_wta(AggArgs a)
         if (++sc == G) { flush(); sc = 0; }
     };
     // operands of two steps are held one pair of steps ahead, in two register sets used alternately
-    uint4 CA[HPF], SA[HPF], CB[HPF], SB[HPF];
-    auto fetch = [&](uint4 (&Cd)[HPF], uint4 (&Sd)[HPF], int xfirst) {
+    uint4 CA[HPF][NH], SA[HPF][NH], CB[HPF][NH], SB[HPF][NH];
+    auto fetch = [&](uint4 (&Cd)[HPF][NH], uint4 (&Sd)[HPF][NH], int xfirst) {
 #pragma unroll
         for (int k = 0; k < HPF; ++k) {
             const int xn = max(xfirst - k, 0);
-            Cd[k] = ld128(cp + xn * Dp);
-            if (S8) {
-                const uint2 e = *reinterpret_cast<const uint2*>(sp8 + xn * Dp);
-                Sd[k] = make_uint4(e.x, e.y, 0u, 0u);
-            } else {
-                Sd[k] = ld128(sp + xn * Dp);
+#pragma unroll
+            for (int h = 0; h < NH; ++h) {
+                Cd[k][h] = ld128(cp + xn * Dp + 8 * h);
+                if (S8) {
+                    const uint2 e = *reinterpret_cast<const uint2*>(sp8 + xn * Dp + 8 * h);
+                    Sd[k][h] = make_uint4(e.x, e.y, 0u, 0u);
+                } else {
+                    Sd[k][h] = ld128(sp + xn * Dp + 8 * h);
+                }
             }
         }
     };
-    auto run = [&](const uint4 (&Cs)[HPF], const uint4 (&Ss)[HPF], int xfirst) {
+    auto run = [&](const uint4 (&Cs)[HPF][NH], const uint4 (&Ss)[HPF][NH], int xfirst) {
 #pragma unroll
         for (int k = 0; k < HPF; ++k)
             if (xfirst - k >= 0) step(Cs[k], Ss[k], xfirst - k);
@@ -799,7 +995,7 @@ size_t vsum_smem_bytes(int bs, bool r8)
            (size_t)VS_RD * GE::IPL * 2 * GE::NPT * 16 + (size_t)VS_RD * GE::RPL * GE::NPT * 8;
 }
 
-template <int G, bool PAD>
+template <int G, bool PAD, int NH>
 cudaError_t launch_sgbm_g(Engine* c, int B)
 {
     const SgbmNorm& n = c->sg;
@@ -837,8 +1033,20 @@ cudaError_t launch_sgbm_g(Engine* c, int B)
             VsArgs v = a;
             v.recL += (size_t)f0 * c->H * c->W; v.plR += (size_t)f0 * c->H * c->vsRP; v.VS += (size_t)f0 * c->H * n.W1 * n.Dp;
             dim3 grd(gx, nb, (c->H + v.bandRows - 1) / v.bandRows);
-            KernelTimer kt(c, KID_SGBM_VSUM);
-            kern<<<grd, GE::THREADS, smem, st>>>(v);
+            if constexpr (NH == 1) {
+                KernelTimer kt(c, KID_SGBM_VSUM);
+                kern<<<grd, GE::THREADS, smem, st>>>(v);
+            } else {
+                // numDisp > 256: costs of different disparities do not interact, so the G = 32 kernel runs once per block
+                // of 256 disparities [256 k, 256 k + 256): its minD is minD + 256 k (the cost domain minX1 / W1 stays),
+                // and it writes at disparity offset 256 k of the pixel stride
+                for (int d0 = 0; d0 < n.D; d0 += 256) {
+                    VsArgs vb = v;
+                    vb.D = std::min(256, n.D - d0); vb.minD = n.minD + d0; vb.VS += d0;
+                    KernelTimer kt(c, KID_SGBM_VSUM);
+                    kern<<<grd, GE::THREADS, smem, st>>>(vb);
+                }
+            }
             return cudaSuccess;
         };
     };
@@ -878,7 +1086,8 @@ cudaError_t launch_sgbm_g(Engine* c, int B)
     // cfg 2, frames per chunk 13 / 15 / 19 / 26 / all: 12.26 / 12.13 / 11.73 / 11.93 / 12.29; cfg 4, 2 / 3 / 4 / 5 / all:
     // 35.9 / 36.3 / 36.0 / 37.0 / 37.2; cfg 5, 1 / 2 / 3 / all: 78.3 / 74.3 / 76.0 / 76.2; a higher stream priority for the
     // scan: slower).
-    const auto h1 = s8 ? k_sgbm_h1<G, PAD, true> : k_sgbm_h1<G, PAD, false>;
+    const auto h1 = NH == 2 ? (s8 ? k_sgbm_h1_w16<PAD, true> : k_sgbm_h1_w16<PAD, false>)
+                            : (s8 ? k_sgbm_h1<G, PAD, true> : k_sgbm_h1<G, PAD, false>);
     MVSV_TRY(smem_limit((const void*)h1, 200 * 1024));
     auto launch_h1 = [&](int f0, int nb, cudaStream_t on) {
         AggArgs h = a;
@@ -886,7 +1095,7 @@ cudaError_t launch_sgbm_g(Engine* c, int B)
         h.VS += off; h.C += off; h.S += s8 ? off / 2 : off; h.B = nb;
         const unsigned blocks = (unsigned)(((long long)nb * c->H * G + TPB - 1) / TPB);
         KernelTimer kt(c, KID_SGBM_H1, on);
-        const size_t sm = (size_t)(2 * n.SW2 + 1 + H1_PFD) * TPB * 16;
+        const size_t sm = (size_t)(2 * n.SW2 + 1 + H1_PFD) * TPB * 16 * NH;
         h1<<<blocks, TPB, sm, on>>>(h);
     };
     int fpc = std::max((B + 6) / 7, (int)(0.9 * c->num_sms / vsum_gx + 0.999));   // frames per chunk
@@ -912,17 +1121,18 @@ cudaError_t launch_sgbm_g(Engine* c, int B)
     }
     auto vdirs = [&](int bottomUp) {
         if (plan.NS > 0) return launch_sweep(c, B, plan, bottomUp, s8);
-        { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, -1, bottomUp); }
-        { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, 0, bottomUp); }
-        { KernelTimer kt(c, KID_SGBM_VDIR); k_sgbm_vdir<G, PAD><<<colBlocks, TPB, 0, st>>>(a, +1, bottomUp); }
+        const auto vdir = NH == 2 ? k_sgbm_vdir_w16<PAD> : k_sgbm_vdir<G, PAD>;
+        { KernelTimer kt(c, KID_SGBM_VDIR); vdir<<<colBlocks, TPB, 0, st>>>(a, -1, bottomUp); }
+        { KernelTimer kt(c, KID_SGBM_VDIR); vdir<<<colBlocks, TPB, 0, st>>>(a, 0, bottomUp); }
+        { KernelTimer kt(c, KID_SGBM_VDIR); vdir<<<colBlocks, TPB, 0, st>>>(a, +1, bottomUp); }
         return cudaSuccess;
     };
     MVSV_TRY(vdirs(0));
     if (n.mode == 1) MVSV_TRY(vdirs(1));
     {
         KernelTimer kt(c, KID_SGBM_H2_WTA);
-        if (s8) k_sgbm_h2_wta<G, PAD, true><<<rowBlocks, TPB, 0, st>>>(a);
-        else k_sgbm_h2_wta<G, PAD, false><<<rowBlocks, TPB, 0, st>>>(a);
+        if (s8) k_sgbm_h2_wta<G, PAD, true, NH><<<rowBlocks, TPB, 0, st>>>(a);
+        else k_sgbm_h2_wta<G, PAD, false, NH><<<rowBlocks, TPB, 0, st>>>(a);
     }
     return cudaGetLastError();
 }
@@ -948,6 +1158,8 @@ bool sgbm_vsum_wide(const SgbmNorm& n)
     return vsum_smem_bytes<32, true>(2 * n.SH2 + 1, 2 * n.ftzero + 63 <= 255) <= (size_t)200 * 1024;
 }
 
+// numDisp > 256 needs no more padding: the cost kernel's block k reads entry 0 at j0 + 256 k, and since
+// minX1 >= minD + numDisp its reach stays below JOFF + W + 8 NV - PX.
 void sgbm_plane_geometry(const SgbmNorm& n, int W, int* NV, int* RP, int* JOFF)
 {
     const int PX = (n.vsWide ? 768 : vs_compute_threads(n.G)) / n.G;
@@ -966,15 +1178,18 @@ cudaError_t launch_sgbm(Engine* c, int B)
         KernelTimer kt(c, KID_FILL);
         k_fill_i16<<<(unsigned)((npx + 255) / 256), 256, 0, c->stream>>>(c->disp_raw, npx, (int16_t)n.INV);
     } else {
-        const bool pad = n.D != 8 * n.G;             // some lanes of a pixel's lane group hold no disparity
+        const bool pad = n.D != n.dpl * n.G;         // some lanes of a pixel's lane group hold no disparity
         cudaError_t e;
         switch (n.G) {
-            case 1: e = pad ? launch_sgbm_g<1, true>(c, B) : launch_sgbm_g<1, false>(c, B); break;
-            case 2: e = pad ? launch_sgbm_g<2, true>(c, B) : launch_sgbm_g<2, false>(c, B); break;
-            case 4: e = pad ? launch_sgbm_g<4, true>(c, B) : launch_sgbm_g<4, false>(c, B); break;
-            case 8: e = pad ? launch_sgbm_g<8, true>(c, B) : launch_sgbm_g<8, false>(c, B); break;
-            case 16: e = pad ? launch_sgbm_g<16, true>(c, B) : launch_sgbm_g<16, false>(c, B); break;
-            default: e = pad ? launch_sgbm_g<32, true>(c, B) : launch_sgbm_g<32, false>(c, B); break;
+            case 1: e = pad ? launch_sgbm_g<1, true, 1>(c, B) : launch_sgbm_g<1, false, 1>(c, B); break;
+            case 2: e = pad ? launch_sgbm_g<2, true, 1>(c, B) : launch_sgbm_g<2, false, 1>(c, B); break;
+            case 4: e = pad ? launch_sgbm_g<4, true, 1>(c, B) : launch_sgbm_g<4, false, 1>(c, B); break;
+            case 8: e = pad ? launch_sgbm_g<8, true, 1>(c, B) : launch_sgbm_g<8, false, 1>(c, B); break;
+            case 16: e = pad ? launch_sgbm_g<16, true, 1>(c, B) : launch_sgbm_g<16, false, 1>(c, B); break;
+            default:
+                if (n.dpl == 16) e = pad ? launch_sgbm_g<32, true, 2>(c, B) : launch_sgbm_g<32, false, 2>(c, B);
+                else e = pad ? launch_sgbm_g<32, true, 1>(c, B) : launch_sgbm_g<32, false, 1>(c, B);
+                break;
         }
         MVSV_TRY(e);
     }

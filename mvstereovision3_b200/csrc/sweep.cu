@@ -3,8 +3,8 @@
 // r = (-1,dy), (0,dy), (+1,dy) with dy = -1 (top-down) or +1 (bottom-up, second sweep of MODE_HH,
 // reference src/disparity.cpp:92-95), added into S in one pass over C and S.
 //
-// Layout of the work ("disparities in registers"): a pixel's D disparities live in the registers of G = 1, 2 or 4
-// adjacent lanes, NR packed u16x2 registers (2*NR disparities) per lane, so that for D <= 64 one lane owns a whole
+// Layout of the work ("disparities in registers"): a pixel's D disparities live in the registers of G = 1, 2, 4 or 8
+// (D > 256) adjacent lanes, NR packed u16x2 registers (2*NR disparities) per lane, so that for D <= 64 one lane owns a whole
 // pixel: the d-1 / d+1 neighbours of the recurrence are register-to-register byte permutes, the minimum over d is
 // an in-register tree, and there are no shuffles at all (G > 1: two neighbour shuffles and log2 G butterfly steps).
 // A warp owns 32/G adjacent pixels of a row and marches down the rows of its frame; a CTA is a column strip of up
@@ -28,7 +28,7 @@
 // and the receiver polls the (four-deep) record itself until every chunk carries the number it expects (the
 // low-latency protocol of collective libraries).  With a release/acquire flag the hand-off through global memory
 // cost 3.6-4 us per hop and set the pace of the whole frame; with tagged data it is one L2 round trip.  Two
-// transports: for one lane per pixel and 2..8 strips the strips of a frame are launched as one thread-block cluster
+// transports: for one or eight lanes per pixel and 2..8 strips the strips of a frame are launched as one thread-block cluster
 // and the record is stored straight into the neighbour's shared memory (mapa + st.shared::cluster; template
 // parameter DSM); otherwise it goes through global memory (L2) and all CTAs are co-resident by a cooperative launch
 // (one CTA per SM).
@@ -123,7 +123,8 @@ constexpr int NSLOT = 4;
 // One step of the path recurrence (A.2 `step`) on the 2*NR disparities of a lane:
 //   L[k] = C[k] + min(Lp[k], Lp[k-1]+P1, Lp[k+1]+P1, m+P2) - m ;  mm = packed min_k L[k] (both halves)
 // "No predecessor" is the state (L = 0, m = 0), which yields L = C.  Registers j >= jpad of the last lane hold
-// padding disparities (numDisp < G*2*NR): they stay at 0x7fff, the out-of-range neighbour value.
+// padding disparities (numDisp < G*2*NR): they stay at 0x7fff, the out-of-range neighbour value.  With G = 8 the
+// padding can span the last two lanes: jpad is then the lane's own (NR for a lane without padding).
 // Pipe balance: the packed min / permute instructions (VIMNMX, VIMNMX3, PRMT) issue on the ALU pipe at one warp
 // instruction per two cycles per scheduler, and so does IADD3; IMAD has the same rate on the FMA pipe.  The plain
 // adds of the recurrence are therefore written as x * one + y with `one` a kernel argument (always 1), which ptxas
@@ -150,7 +151,7 @@ __device__ __forceinline__ void path_step(unsigned (&L)[NR], unsigned& mm, const
         const unsigned Pn = (j + 1 < NR) ? L[j + 1] * one + P1P1 : dn;
         const unsigned Xn = __byte_perm(Pj, Pn, 0x5432);  // (d+1 of the low half, d+1 of the high half)
         unsigned n = (__vimin3_u16x2(Xj, Xn, __vminu2(L[j], mP2)) * one + negm) * one + C[j];
-        if (PAD && q == G - 1 && j >= jpad) n = MVSV_PK_MAX;
+        if (PAD && (G == 8 || q == G - 1) && j >= jpad) n = MVSV_PK_MAX;
         L[j] = n;
         Xj = Xn; Pj = Pn;
     }
@@ -194,7 +195,7 @@ __device__ __forceinline__ void path_step2(unsigned (&L)[NR], unsigned& mm, unsi
         const unsigned XnL = __byte_perm(PjL, PnL, 0x5432), XnK = __byte_perm(PjK, PnK, 0x5432);
         unsigned nL = (__vimin3_u16x2(XjL, XnL, __vminu2(L[j], mP2L)) * one + negL) * one + C[j];
         unsigned nK = (__vimin3_u16x2(XjK, XnK, __vminu2(K[j], mP2K)) * one + negK) * one + C[j];
-        if (PAD && q == G - 1 && j >= jpad) { nL = MVSV_PK_MAX; nK = MVSV_PK_MAX; }
+        if (PAD && (G == 8 || q == G - 1) && j >= jpad) { nL = MVSV_PK_MAX; nK = MVSV_PK_MAX; }
         L[j] = nL; K[j] = nK;
         XjL = XnL; PjL = PnL; XjK = XnK; PjK = PnK;
     }
@@ -225,7 +226,7 @@ template <int NR, int G, bool PAD>
 __device__ __forceinline__ void reset_path(unsigned (&L)[NR], unsigned& mm, int q, int jpad)
 {
 #pragma unroll
-    for (int j = 0; j < NR; ++j) L[j] = (PAD && q == G - 1 && j >= jpad) ? MVSV_PK_MAX : 0u;
+    for (int j = 0; j < NR; ++j) L[j] = (PAD && (G == 8 || q == G - 1) && j >= jpad) ? MVSV_PK_MAX : 0u;
     mm = 0u;
 }
 
@@ -301,7 +302,7 @@ __global__ void __launch_bounds__(SW_MAX_THREADS, 1) k_sweep(SweepArgs a)
     const int nact = min(max(M * G - w * 32, 0), 32); // active lanes of this warp
     // (nact == 0 is only possible for trailing warps of a narrower strip: they skip the row loop)
     const int wl = (M * G - 1) >> 5;                  // warp holding the strip's last pixel
-    const int jpad = PAD ? (a.D - (G - 1) * 2 * NR) / 2 : NR;
+    const int jpad = !PAD ? NR : G == 8 ? min(max(a.D / 2 - q * NR, 0), NR) : (a.D - (G - 1) * 2 * NR) / 2;
     const int nfr = (a.B - fs + a.NF - 1) / a.NF;     // frames this CTA walks
     const int T = nact > 0 ? nfr * a.H : 0;
     const bool hasL = s > 0, hasR = s + 1 < a.NS;
@@ -563,8 +564,9 @@ cudaError_t launch_one(const SweepArgs& a, int nthr, size_t smem, cudaStream_t s
 template <int NR, int G, bool PAD, int MODE>
 cudaError_t launch_fast(const SweepArgs& a, int nthr, size_t smem, cudaStream_t st)
 {
-    // the cluster variant only exists for one lane per pixel (D <= 64: cfg 2 and the reference's other 752x480 uses)
-    if constexpr (G == 1) {
+    // the cluster variant exists for one lane per pixel (D <= 64: cfg 2 and the reference's other 752x480 uses) and for
+    // eight (D > 256, where the strips are narrowest)
+    if constexpr (G == 1 || G == 8) {
         if (a.dsm) {
             bool fits = false;
             const cudaError_t e = launch_one<NR, G, PAD, MODE, true>(a, nthr, smem, st, &fits);
@@ -606,7 +608,7 @@ cudaError_t launch_nr(int NR, const SweepArgs& a, int nthr, size_t smem, cudaStr
 // stride is Dp = G * 2 * NR >= D (a multiple of 8; equal to D whenever D is a multiple of 8 * G).
 void sweep_layout(int D, int* G, int* NR)
 {
-    const int g = D <= 64 ? 1 : D <= 128 ? 2 : 4;
+    const int g = D <= 64 ? 1 : D <= 128 ? 2 : D <= 256 ? 4 : 8;
     const int per = (D + g - 1) / g;                  // disparities per lane
     *G = g; *NR = (per + 7) / 8 * 4;
 }
@@ -638,7 +640,7 @@ void sweep_plan(const Engine* c, int B, int forcedNS, SweepPlan* p)
         if (smem > (size_t)SW_SMEM_LIMIT) continue;
         const int NF = std::min(B, c->num_sms / NS);
         const int waves = (B + NF - 1) / NF;
-        const double handoff = NS == 1 ? 0.0 : (G == 1 && NS <= 8 && NF * NS <= c->num_sms - 16) ? hoCluster : hoGlobal;
+        const double handoff = NS == 1 ? 0.0 : ((G == 1 || G == 8) && NS <= 8 && NF * NS <= c->num_sms - 16) ? hoCluster : hoGlobal;
         const double cost = waves * (c0 + c1 * (nthr / 32) + handoff) + 1e-6 * NS;   // us per row; ties: fewer strips
         if (cost < best) { best = cost; p->NS = NS; p->NF = NF; p->Mmax = Mmax; p->threads = nthr; p->smem = smem; }
     }
@@ -657,7 +659,7 @@ void sweep_plan(const Engine* c, int B, int forcedNS, SweepPlan* p)
 size_t sweep_scratch_bytes(const Engine* c)
 {
     // worst case over all plans and disparity ranges: NF * NS <= num_sms CTAs, 2 directions x NSLOT records each
-    return (size_t)c->num_sms * 2 * NSLOT * (256 + 8) * sizeof(uint16_t);
+    return (size_t)c->num_sms * 2 * NSLOT * (512 + 8) * sizeof(uint16_t);
 }
 
 // 3 * (largest possible path cost) <= 65535: the three paths of a row can be summed in 16 bits without saturation
@@ -693,6 +695,7 @@ cudaError_t launch_sweep(Engine* c, int B, const SweepPlan& p, int bottomUp, boo
     switch (p.G) {
         case 1: return launch_nr<1, false>(p.NR, a, p.threads, p.smem, c->stream);
         case 2: return pad ? launch_nr<2, true>(p.NR, a, p.threads, p.smem, c->stream) : launch_nr<2, false>(p.NR, a, p.threads, p.smem, c->stream);
-        default: return pad ? launch_nr<4, true>(p.NR, a, p.threads, p.smem, c->stream) : launch_nr<4, false>(p.NR, a, p.threads, p.smem, c->stream);
+        case 4: return pad ? launch_nr<4, true>(p.NR, a, p.threads, p.smem, c->stream) : launch_nr<4, false>(p.NR, a, p.threads, p.smem, c->stream);
+        default: return pad ? launch_nr<8, true>(p.NR, a, p.threads, p.smem, c->stream) : launch_nr<8, false>(p.NR, a, p.threads, p.smem, c->stream);
     }
 }
