@@ -216,6 +216,19 @@ int mvsv_compute(mvsv_ctx* ctx, const uint8_t* left, size_t lstride, const uint8
  * that produce frames on the GPU). */
 int mvsv_compute_device(mvsv_ctx* ctx, const uint8_t* dleft, size_t lstride, const uint8_t* dright, size_t rstride,
                         size_t frame_stride, int batch, unsigned stages);
+
+/* GPU producers and consumers: ordering against the caller's CUDA stream.
+ * `stream` of the three calls below is a cudaStream_t on any device; cudaStreamLegacy and cudaStreamPerThread name the
+ * stream of the device current on the calling thread when the call is entered.  NULL means no ordering with the caller.
+ * The ctx keeps one event per device of the streams it is given (created on first use, freed by mvsv_destroy).
+ *
+ * mvsv_compute_device with `stream`: the engine reads the inputs only after the work queued on `stream` before the
+ * call, and work queued on `stream` after the call starts once the engine has copied the inputs into its I/O slot (not
+ * after the whole compute): the caller may then overwrite or free the inputs on that stream.  The call does not wait on
+ * the host.  stream == NULL is exactly mvsv_compute_device, which is this call with NULL.  Multi-device ctx: every part
+ * waits for the caller's stream, and the stream waits for the input copies of every part. */
+int mvsv_compute_device_stream(mvsv_ctx* ctx, const uint8_t* dleft, size_t lstride, const uint8_t* dright, size_t rstride,
+                               size_t frame_stride, int batch, unsigned stages, void* stream);
 /* Disparity::tm(Stereopair const&, cv::Mat& output, unsigned kernelSize) (src/disparity.cpp:25-58): for every pixel
  * (i, j), i < rows-kernelSize, j < cols-kernelSize, the kernelSize x kernelSize block of the left image is matched
  * by normalised cross-correlation (cv::matchTemplate TM_CCORR_NORMED) against the right image's blocks at
@@ -254,6 +267,31 @@ int mvsv_download_age(mvsv_ctx* ctx, int age, int16_t* disp, size_t dstride, uin
  * Multi-device ctx: the offsets of every part are fetched first; part k's points then go right after those of the parts
  * before it, with its frame offsets rebased onto them, and the parts' copies run side by side. */
 int mvsv_download_points(mvsv_ctx* ctx, int age, int64_t* offsets, float* points, size_t capacity_points);
+/* mvsv_download_age into DEVICE memory, for consumers on the GPU.  Same buffers, strides, frames and offsets as
+ * mvsv_download_age (disp at disp + first*height*dstride for the frames of each part, XYZ and means likewise; the frames
+ * of that slot's compute), on any device: the copies use cudaMemcpyDefault, so that unified addressing finds both ends
+ * and copies peer to peer where the devices differ.  No kernel runs: the copy engines move the results.
+ *   stream != NULL: the copies start after the work queued on `stream` before the call, work queued on `stream` after
+ *     the call sees the results, and the call returns without a host wait.
+ *   stream == NULL: the call waits for the copies before it returns, as mvsv_download_age does.
+ * Rejected, with the results left downloadable: MVSV_ERR_INVALID for a non-NULL destination that
+ * cudaPointerGetAttributes does not report as device or managed memory (host memory: mvsv_download_age); everything
+ * mvsv_download_age rejects, with its code (strides below the row, an age outside the slots, nothing computed, a stage
+ * the compute did not run).  A failure while the copies of several parts are queued waits for the copies queued before
+ * it: no copy into the caller's memory is in flight after an error.
+ * Slot lifetime: copies still in flight hold their I/O slot.  A compute (or mvsv_debug_postfilter) that takes the slot
+ * writes it only after them, and mvsv_set_io_slots, mvsv_set_mean_rois, a geometry change (maps, rectification, resize)
+ * and mvsv_destroy wait for them before they free slot buffers. */
+int mvsv_download_device(mvsv_ctx* ctx, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR,
+                         size_t rstride, float* xyz, float* means, void* stream);
+/* mvsv_download_points with the points into DEVICE memory (offsets still to host memory).  The list's size depends on the
+ * data, so the frame offsets are fetched to `offsets` first, exactly as mvsv_download_points does (multi-device rebase
+ * included): this phase WAITS ON THE HOST until the compute has finished.  The point copies then run as in
+ * mvsv_download_device, ordered on `stream`.  points == NULL (the size query), capacity_points too small
+ * (MVSV_ERR_INVALID, offsets written, `points` untouched) and MVSV_ERR_STATE are those of mvsv_download_points; a
+ * non-NULL `points` that is not device or managed memory is MVSV_ERR_INVALID. */
+int mvsv_download_points_device(mvsv_ctx* ctx, int age, int64_t* offsets, float* points, size_t capacity_points,
+                                void* stream);
 /* Utility::calcMinMaxDisparity (src/utility.cpp:287-304) of the last computed maps as a GPU reduction: for every
  * frame the smallest and largest disparity value > 0, minmax[2*i], minmax[2*i+1]; (0, 0) when a map has none (the
  * reference dereferences an end iterator there).  Consumed by the PLY writer's grey ramp (src/ply.cpp:62-95). */

@@ -3,6 +3,7 @@ disparity interface (reference inc/disparity.h:17-35, src/disparity.cpp:6-22,60-
 
 No CPU fallback: if the CUDA library is missing or there is no GPU, construction raises.
 """
+import contextlib
 import ctypes as C
 import os
 
@@ -12,6 +13,13 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvsv.so")
 
 STAGE_RECTIFY, STAGE_SGBM, STAGE_BM, STAGE_XYZ, STAGE_MEANS, STAGE_POINTS = 1, 2, 4, 8, 16, 32
+CUDA_STREAM_LEGACY = 1      # cudaStreamLegacy: the legacy default stream of the current device
+
+
+def _torch():
+    # imported on first use: the module, its host calls and the CPU tests work without torch
+    import torch
+    return torch
 
 # every symbol include/mvsv.h declares (tests check the library exports all of them)
 ABI_SYMBOLS = (
@@ -23,6 +31,7 @@ ABI_SYMBOLS = (
     "mvsv_set_bm_filters", "mvsv_debug_postfilter",
     "mvsv_upload_rectify_maps_rig", "mvsv_set_rectification_rig", "mvsv_set_Q_rig", "mvsv_set_frame_rigs",
     "mvsv_init_devices", "mvsv_get_devices", "mvsv_download_points",
+    "mvsv_compute_device_stream", "mvsv_download_device", "mvsv_download_points_device",
 )
 MAX_RIGS = 64       # MVSV_MAX_RIGS
 
@@ -85,10 +94,13 @@ def load_library():
     lib.mvsv_set_mean_rois.argtypes = [vp, vp, ci]
     lib.mvsv_compute.argtypes = [vp, vp, sz, vp, sz, sz, ci, C.c_uint]
     lib.mvsv_compute_device.argtypes = [vp, vp, sz, vp, sz, sz, ci, C.c_uint]
+    lib.mvsv_compute_device_stream.argtypes = [vp, vp, sz, vp, sz, sz, ci, C.c_uint, vp]
     lib.mvsv_tm.argtypes = [vp, vp, sz, vp, sz, sz, ci, C.c_uint, vp, sz]
     lib.mvsv_download.argtypes = [vp, vp, sz, vp, vp, sz, vp, vp]
     lib.mvsv_download_age.argtypes = [vp, ci, vp, sz, vp, vp, sz, vp, vp]
     lib.mvsv_download_points.argtypes = [vp, ci, vp, vp, sz]
+    lib.mvsv_download_device.argtypes = [vp, ci, vp, sz, vp, vp, sz, vp, vp, vp]
+    lib.mvsv_download_points_device.argtypes = [vp, ci, vp, vp, sz, vp]
     lib.mvsv_set_io_slots.argtypes = [vp, ci]
     lib.mvsv_sync.argtypes = [vp]
     lib.mvsv_download_minmax.argtypes = [vp, vp]
@@ -284,8 +296,44 @@ class Engine:
                                         left.strides[0], left.shape[0], stages))
         self._keep = (left, right)
 
-    def compute_device(self, dleft_ptr, lstride, dright_ptr, rstride, frame_stride, batch, stages):
-        self._ck(self._lib.mvsv_compute_device(self._ctx, dleft_ptr, lstride, dright_ptr, rstride, frame_stride, batch, stages))
+    def compute_device(self, dleft_ptr, lstride, dright_ptr, rstride, frame_stride, batch, stages, stream=None):
+        """Inputs in device memory.  `stream` (a torch.cuda.Stream): the inputs are read after the work queued on it, and
+        work queued on it afterwards waits only for the input copies (mvsv_compute_device_stream); None: no ordering."""
+        self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_compute_device_stream(
+            self._ctx, dleft_ptr, lstride, dright_ptr, rstride, frame_stride, batch, stages, h)))
+
+    def compute_tensors(self, left, right, stages, stream=None):
+        """uint8 CUDA tensors [B,]H,W with unit column stride; the row and frame strides are the tensors' own."""
+        torch = _torch()
+
+        def batchify(t):
+            if t.dim() == 2:
+                t = t.unsqueeze(0)
+            if t.dtype != torch.uint8 or t.dim() != 3 or not t.is_cuda or t.stride(2) != 1:
+                raise ValueError("images must be uint8 CUDA tensors [B,]H,W with unit column stride")
+            return t
+        left, right = batchify(left), batchify(right)
+        if left.shape != right.shape:
+            raise ValueError("left/right shapes differ")
+        if left.stride(0) != right.stride(0) and left.shape[0] > 1:
+            raise ValueError("left/right frame strides differ")
+        self.compute_device(left.data_ptr(), left.stride(1), right.data_ptr(), right.stride(1), left.stride(0),
+                            left.shape[0], stages, stream)
+
+    def _on_stream(self, stream, call):
+        """call(handle) with the ABI's `stream` argument for a torch.cuda.Stream or None.  Torch reports its default stream
+        as handle 0, which the ABI reads as "no ordering": it goes as cudaStreamLegacy, with the stream's device current."""
+        if stream is None:
+            return call(None)
+        with _torch().cuda.device(stream.device):
+            return call(stream.cuda_stream or CUDA_STREAM_LEGACY)
+
+    def _device_out(self, stream, device):
+        """the device results are allocated on (default: the first part's), and the context that allocates them on
+        `stream`, so that their memory follows that stream's order"""
+        torch = _torch()
+        dev = torch.device("cuda", self.devices[0]) if device is None else torch.device(device)   # an int is a CUDA ordinal
+        return dev, (torch.cuda.stream(stream) if stream is not None else contextlib.nullcontext())
 
     def tm(self, left, right, kernel_size):
         """Disparity::tm (reference src/disparity.cpp:25-58) on host images [B,]H,W -> uint8 [B,H,W]."""
@@ -353,6 +401,71 @@ class Engine:
             raise ValueError("out must be a C-contiguous float32 array")
         self._ck(self._lib.mvsv_download_points(self._ctx, age, offs.ctypes.data, out.ctypes.data, out.size // 3))
         return offs[:batch + 1], out.reshape(-1)[:3 * int(offs[batch])].reshape(-1, 3)
+
+    def download_device(self, batch, disp=True, rect=False, xyz=False, means=False, out=None, age=0, stream=None,
+                        device=None):
+        """The results of download() as torch tensors in device memory (mvsv_download_device): disp int16 [batch, H, W],
+        rectL / rectR uint8 [batch, H, W], xyz float32 [batch, H, W, 3], means float32 [batch, num_rois].  They are
+        allocated on `device` (default: the engine's first device), or taken from `out` (a dict with those keys): disp and
+        rect may be pitched views (unit column stride, frame stride = H * row stride), xyz and means are contiguous.
+        `stream` (a torch.cuda.Stream): the copies are ordered on it and the call returns without waiting; None: the call
+        returns with the copies done."""
+        torch = _torch()
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        H, W = i.height, i.width
+        dev, on_stream = self._device_out(stream, device)
+        out = out or {}
+        spec = (("disp", disp, (batch, H, W), torch.int16, True), ("rectL", rect, (batch, H, W), torch.uint8, True),
+                ("rectR", rect, (batch, H, W), torch.uint8, True), ("xyz", xyz, (batch, H, W, 3), torch.float32, False),
+                ("means", means, (batch, i.num_rois), torch.float32, False))
+        res = {}
+        with on_stream:
+            for key, on, shape, dtype, pitched in spec:
+                if not on:
+                    continue
+                t = out.get(key)
+                if t is None:
+                    t = torch.empty(shape, dtype=dtype, device=dev)
+                elif t.dtype != dtype or tuple(t.shape) != shape or not t.is_cuda:
+                    raise ValueError("out[%r] must be a %s CUDA tensor of shape %s" % (key, dtype, shape))
+                elif (t.stride(-1) != 1 or t.stride(0) != H * t.stride(1)) if pitched else not t.is_contiguous():
+                    raise ValueError("out[%r]: %s" % (key, "unit column stride and frame stride = H * row stride" if pitched
+                                                      else "must be contiguous"))
+                res[key] = t
+        if rect and res["rectL"].stride(1) != res["rectR"].stride(1):
+            raise ValueError("rectL and rectR must share one row stride")
+
+        def ptr(key):
+            return res[key].data_ptr() if key in res else None
+        dstride = res["disp"].stride(1) * 2 if disp else 0
+        rstride = res["rectL"].stride(1) if rect else 0
+        self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_download_device(
+            self._ctx, age, ptr("disp"), dstride, ptr("rectL"), ptr("rectR"), rstride, ptr("xyz"), ptr("means"), h)))
+        return res
+
+    def download_points_device(self, batch, age=0, out=None, stream=None, device=None):
+        """The point list of download_points() with the points in device memory (mvsv_download_points_device):
+        (offsets int64 numpy [batch + 1], points float32 tensor [n, 3]).  Fetching the offsets waits on the host for the
+        compute; the point copy is then ordered on `stream` as in download_device.  `out`: a contiguous float32 CUDA
+        tensor the points are copied into (the points returned are a view of it); without it the list is allocated on
+        `device` (default: the engine's first device), sized by a first call that fetches only the offsets."""
+        torch = _torch()
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        offs = np.empty(i.max_batch + 1, np.int64)         # the C call writes the compute's frames + 1 entries
+        if out is None:
+            self._ck(self._lib.mvsv_download_points_device(self._ctx, age, offs.ctypes.data, None, 0, None))
+            dev, on_stream = self._device_out(stream, device)
+            with on_stream:
+                out = torch.empty((int(offs[batch]), 3), dtype=torch.float32, device=dev)
+        elif out.dtype != torch.float32 or not out.is_cuda or not out.is_contiguous():
+            raise ValueError("out must be a contiguous float32 CUDA tensor")
+        self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_download_points_device(
+            self._ctx, age, offs.ctypes.data, out.data_ptr() or None, out.numel() // 3, h)))
+        return offs[:batch + 1], out.view(-1)[:3 * int(offs[batch])].view(-1, 3)
 
     def download_minmax(self, batch):
         """Utility::calcMinMaxDisparity (reference src/utility.cpp:287-304) per frame, reduced on the GPU."""

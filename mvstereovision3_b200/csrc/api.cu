@@ -401,8 +401,10 @@ int compute_check(Engine* c, size_t lstride, size_t rstride, int batch, unsigned
 }
 
 // Queues engine c's copies and kernels of a compute of `batch` frames; they fill the I/O slot it has taken (take_slot).
+// Device inputs with a caller's stream: the input copies wait for `caller_ready` (recorded on that stream), and with
+// `signal_read` ev_h2d marks the end of the input copies for the caller's stream to wait on.
 int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride,
-                   int batch, unsigned stages, bool device_src)
+                   int batch, unsigned stages, bool device_src, cudaEvent_t caller_ready = nullptr, bool signal_read = false)
 {
     const IoSlot& slot = io(c);
     const bool rectify = stages & MVSV_STAGE_RECTIFY;
@@ -414,12 +416,17 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     // host inputs: the copies wait for the slot's previous compute (which may still read the input buffers), the
     // kernels wait for the copies
     if (!device_src) MVSV_CK(c, cudaStreamWaitEvent(c->copy_stream, slot.done, 0));
+    // a device download of the slot's previous results may still be copying out of it; the stream that copies the
+    // inputs writes the slot first, and the kernels follow that stream
+    MVSV_CK(c, cudaStreamWaitEvent(device_src ? c->stream : c->copy_stream, slot.dl_done, 0));
+    if (caller_ready) MVSV_CK(c, cudaStreamWaitEvent(c->stream, caller_ready, 0));
     const DeviceBuffer<uint8_t>* dst = rectify ? slot.raw : slot.rect;
     const size_t dpitch = rectify ? c->raw_pitch : c->pitch;
     rc = upload_images(c, dst[0], dpitch, left, lstride, frame_stride, iw, ih, batch, device_src);
     if (!rc) rc = upload_images(c, dst[1], dpitch, right, rstride, frame_stride, iw, ih, batch, device_src);
     if (!rc) rc = inputs_uploaded(c, device_src);
     if (rc) return rc;
+    if (signal_read) MVSV_CK(c, cudaEventRecord(c->ev_h2d, device_src ? c->stream : c->copy_stream));
     if (multi && (rectify || (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS)))) {
         rc = upload_rig_tables(c);
         if (rc) return rc;
@@ -439,10 +446,13 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     return MVSV_OK;
 }
 
-// Queues the copies of the results a compute left in I/O slot `k` to the host on the download stream (so that they
-// overlap kernels submitted later); download_wait waits for them.
+// Queues the copies of the results a compute left in I/O slot `k` on the download stream (so that they overlap kernels
+// submitted later), to host memory (kind cudaMemcpyDeviceToHost) or to device memory on any device (cudaMemcpyDefault:
+// unified addressing finds both ends and copies peer to peer where they differ); download_wait waits for them.  The
+// copies start after the compute and after `caller_ready` (recorded on a caller's stream, or none); the slot's dl_done
+// marks their end.
 int download_enqueue(Engine* c, int k, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
-                     float* xyz, float* means)
+                     float* xyz, float* means, cudaMemcpyKind kind, cudaEvent_t caller_ready)
 {
     int rc = bind(c);
     if (rc) return rc;
@@ -450,28 +460,29 @@ int download_enqueue(Engine* c, int k, int16_t* disp, size_t dstride, uint8_t* r
     const int B = s.B;
     cudaStream_t st = c->dl_stream;
     MVSV_CK(c, cudaStreamWaitEvent(st, s.done, 0));
+    if (caller_ready) MVSV_CK(c, cudaStreamWaitEvent(st, caller_ready, 0));
     if (disp) {
         if (dstride < (size_t)c->W * 2) return fail(c, MVSV_ERR_INVALID, "disparity stride too small");
         if (dstride == (size_t)c->W * 2)
-            MVSV_CK(c, cudaMemcpyAsync(disp, s.disp, (size_t)c->W * 2 * c->H * B, cudaMemcpyDeviceToHost, st));
+            MVSV_CK(c, cudaMemcpyAsync(disp, s.disp, (size_t)c->W * 2 * c->H * B, kind, st));
         else
-            MVSV_CK(c, cudaMemcpy2DAsync(disp, dstride, s.disp, (size_t)c->W * 2, (size_t)c->W * 2, (size_t)c->H * B,
-                                         cudaMemcpyDeviceToHost, st));
+            MVSV_CK(c, cudaMemcpy2DAsync(disp, dstride, s.disp, (size_t)c->W * 2, (size_t)c->W * 2, (size_t)c->H * B, kind, st));
     }
     uint8_t* r[2] = {rectL, rectR};
     for (int i = 0; i < 2; ++i)
         if (r[i]) {
             if (rstride < (size_t)c->W) return fail(c, MVSV_ERR_INVALID, "rectified stride too small");
-            MVSV_CK(c, cudaMemcpy2DAsync(r[i], rstride, s.rect[i], c->pitch, (size_t)c->W, (size_t)c->H * B, cudaMemcpyDeviceToHost, st));
+            MVSV_CK(c, cudaMemcpy2DAsync(r[i], rstride, s.rect[i], c->pitch, (size_t)c->W, (size_t)c->H * B, kind, st));
         }
     if (xyz) {
         if (!s.xyz || !(s.stages & MVSV_STAGE_XYZ)) return fail(c, MVSV_ERR_STATE, "XYZ stage was not computed");
-        MVSV_CK(c, cudaMemcpyAsync(xyz, s.xyz, (size_t)B * c->H * c->W * 3 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        MVSV_CK(c, cudaMemcpyAsync(xyz, s.xyz, (size_t)B * c->H * c->W * 3 * sizeof(float), kind, st));
     }
     if (means) {
         if (!s.means || !(s.stages & MVSV_STAGE_MEANS)) return fail(c, MVSV_ERR_STATE, "MEANS stage was not computed");
-        MVSV_CK(c, cudaMemcpyAsync(means, s.means, (size_t)B * c->nrois * sizeof(float), cudaMemcpyDeviceToHost, st));
+        MVSV_CK(c, cudaMemcpyAsync(means, s.means, (size_t)B * c->nrois * sizeof(float), kind, st));
     }
+    MVSV_CK(c, cudaEventRecord(s.dl_done, st));
     return MVSV_OK;
 }
 
@@ -494,12 +505,16 @@ int points_offsets(Engine* c, int k, std::vector<long long>& offsets)
     return download_wait(c);
 }
 
-// second phase: queues the copy of the slot's n points to `points` on the download stream (download_wait waits for it)
-int points_enqueue(Engine* c, int k, float* points, long long n)
+// second phase: queues the copy of the slot's n points to `points` on the download stream, as download_enqueue does
+// (download_wait waits for it)
+int points_enqueue(Engine* c, int k, float* points, long long n, cudaMemcpyKind kind, cudaEvent_t caller_ready)
 {
     int rc = bind(c);
     if (rc) return rc;
-    if (n > 0) MVSV_CK(c, cudaMemcpyAsync(points, c->slot[k].points, (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->dl_stream));
+    IoSlot& s = c->slot[k];
+    if (caller_ready) MVSV_CK(c, cudaStreamWaitEvent(c->dl_stream, caller_ready, 0));
+    if (n > 0) MVSV_CK(c, cudaMemcpyAsync(points, s.points, (size_t)n * 3 * sizeof(float), kind, c->dl_stream));
+    MVSV_CK(c, cudaEventRecord(s.dl_done, c->dl_stream));
     return MVSV_OK;
 }
 
@@ -580,10 +595,64 @@ struct mvsv_ctx {
     int maxB = 0;                            // frames of all parts
     std::vector<int> frame_rig;              // the whole frame -> rig table (mvsv_set_frame_rigs)
     bool broken = false;                     // a setter failed in a way that can have left the parts different
+    // per device of a caller's stream (mvsv_compute_device_stream, mvsv_download_device, mvsv_download_points_device):
+    // the event recorded on that stream for the parts' streams to wait on; created on first use, destroyed with the ctx.
+    // The other direction needs none of its own: the caller's stream waits on the part's ev_h2d or on the slot's dl_done.
+    std::map<int, cudaEvent_t> ev_caller;
     std::string err;
 };
 
 namespace {
+
+// A caller's stream and its device: that of the stream, or for the special handles cudaStreamLegacy and
+// cudaStreamPerThread the device current when the call was entered.  st == nullptr: no ordering with the caller.
+struct Caller {
+    cudaStream_t st = nullptr;
+    int dev = 0;
+};
+
+// Read before any part is bound, which changes the current device.
+int caller_of(mvsv_ctx* c, void* stream, Caller* k)
+{
+    k->st = (cudaStream_t)stream;
+    if (!k->st) return MVSV_OK;
+    if (k->st == cudaStreamLegacy || k->st == cudaStreamPerThread) MVSV_CK(c, cudaGetDevice(&k->dev));
+    else MVSV_CK(c, cudaStreamGetDevice(k->st, &k->dev));
+    return MVSV_OK;
+}
+
+// Records the caller's stream as it stands into *ready, for the parts' streams to wait on (nullptr without a stream).
+int caller_ready(mvsv_ctx* c, const Caller& k, cudaEvent_t* ready)
+{
+    *ready = nullptr;
+    if (!k.st) return MVSV_OK;
+    MVSV_CK(c, cudaSetDevice(k.dev));   // the special handles name the stream of the current device
+    cudaEvent_t& ev = c->ev_caller[k.dev];
+    if (!ev) MVSV_CK(c, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    MVSV_CK(c, cudaEventRecord(ev, k.st));
+    *ready = ev;
+    return MVSV_OK;
+}
+
+// Work queued on the caller's stream from now on waits for `ev`, an event of a part's stream (waits across devices are
+// legal).
+int caller_wait(mvsv_ctx* c, const Caller& k, cudaEvent_t ev)
+{
+    MVSV_CK(c, cudaSetDevice(k.dev));
+    MVSV_CK(c, cudaStreamWaitEvent(k.st, ev, 0));
+    return MVSV_OK;
+}
+
+// A destination of a device download: device or managed memory on any device (cudaPointerGetAttributes)
+bool device_memory(const void* p)
+{
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();   // not a sticky error: leave no trace of it for the next call
+        return false;
+    }
+    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+}
 
 int usable(mvsv_ctx* c)
 {
@@ -661,10 +730,14 @@ int send_rigs(mvsv_ctx* c, int k, int first)
 
 // Part k computes the frames [floor(k*b/n), floor((k+1)*b/n)) of a batch of b: contiguous shares keep every host copy
 // one bulk or 2-D copy per buffer and part.
+// `stream` (device inputs only): a caller's stream the input copies wait for, and which waits for them in turn.
 int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, size_t rstride, size_t frame_stride, int batch,
-        unsigned stages, bool device_src)
+        unsigned stages, bool device_src, void* stream = nullptr)
 {
     int rc = usable(c);
+    if (rc) return rc;
+    Caller caller;
+    rc = caller_of(c, stream, &caller);
     if (rc) return rc;
     if (!left || !right || batch < 1 || batch > c->maxB) return fail(c, MVSV_ERR_INVALID, "bad image pointers or batch size");
     const int n = (int)c->parts.size();
@@ -678,14 +751,19 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
                 rc = on_part(c, k, [&](Engine* p) { return compute_check(p, lstride, rstride, first[k + 1] - first[k], stages); });
         }
     if (rc) return rc;
+    cudaEvent_t ready = nullptr;
+    rc = caller_ready(c, caller, &ready);
+    if (rc) return rc;
     // every part takes its next slot, one without frames too, so that the slots of all parts hold the same compute
     for (Engine* p : c->parts) take_slot(p);
     for (int k = 0; k < n; ++k)
         if (first[k] < first[k + 1]) {
             rc = on_part(c, k, [&](Engine* p) {
                 return compute_submit(p, left + first[k] * frame_stride, lstride, right + first[k] * frame_stride, rstride,
-                                      frame_stride, first[k + 1] - first[k], stages, device_src);
+                                      frame_stride, first[k + 1] - first[k], stages, device_src, ready, caller.st != nullptr);
             });
+            // the caller's stream goes on once this part has copied its inputs, not after its kernels
+            if (!rc && caller.st) rc = caller_wait(c, caller, c->parts[k]->ev_h2d);
             if (rc) return rc;
         }
     for (int k = 0; k < n; ++k) {
@@ -704,7 +782,7 @@ Engine::~Engine()
     for (cudaEvent_t ev : ev_free) cudaEventDestroy(ev);
     for (cudaEvent_t ev : ev_chunk)
         if (ev) cudaEventDestroy(ev);
-    for (cudaEvent_t ev : {timer_a, timer_b, ev_h2d, ev_done, ev_join, slot[0].done, slot[1].done})
+    for (cudaEvent_t ev : {timer_a, timer_b, ev_h2d, ev_done, ev_join, slot[0].done, slot[1].done, slot[0].dl_done, slot[1].dl_done})
         if (ev) cudaEventDestroy(ev);
     for (cudaStream_t st : {aux_stream, copy_stream, dl_stream, stream})
         if (st) cudaStreamDestroy(st);
@@ -767,7 +845,8 @@ static int init_engine(int device, int frame_width, int frame_height, int max_ba
         if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
     if ((e = cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
     for (auto& sl : c->slot)
-        if ((e = cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
+        for (cudaEvent_t* ev : {&sl.done, &sl.dl_done})
+            if ((e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
     for (cudaEvent_t* ev : {&c->ev_h2d, &c->ev_done})
         if ((e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming)) != cudaSuccess) return bail(e, "cudaEventCreate");
     Geometry g;
@@ -824,6 +903,10 @@ void mvsv_destroy(mvsv_ctx* c)
 {
     if (!c) return;
     for (Engine* p : c->parts) destroy_engine(p);
+    for (auto& de : c->ev_caller) {
+        cudaSetDevice(de.first);
+        cudaEventDestroy(de.second);
+    }
     delete c;
 }
 
@@ -901,6 +984,7 @@ static int prepare_maps(Engine* c, int rig, int cam, int roi_x, int roi_y, int r
     int rc = plan_geometry(c, true, roi_w, roi_h, c->resize_factor, &g);
     if (rc) return rc;
     MVSV_CK(c, cudaStreamSynchronize(c->stream));
+    MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));   // device downloads still copying out of the slots apply_geometry frees
     c->roi_xy[rig][0] = roi_x; c->roi_xy[rig][1] = roi_y; c->roi_w = roi_w; c->roi_h = roi_h;
     c->has_maps[rig][cam] = false;
     c->rig_tables_dirty = true;
@@ -994,6 +1078,7 @@ int mvsv_reset_rectification(mvsv_ctx* ctx)
         rc = plan_geometry(c, false, 0, 0, c->resize_factor, &g);
         if (rc) return rc;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
+        MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));
         for (int r = 0; r < MVSV_MAX_RIGS; ++r)
             for (int i = 0; i < 2; ++i) {
                 c->has_maps[r][i] = false;
@@ -1016,6 +1101,7 @@ int mvsv_set_resize(mvsv_ctx* ctx, double factor)
         rc = plan_geometry(c, any_maps(c), c->roi_w, c->roi_h, f, &g);
         if (rc) return rc;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
+        MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));
         c->resize_factor = f;
         return apply_geometry(c, g);
     });
@@ -1035,6 +1121,7 @@ int mvsv_tm(mvsv_ctx* ctx, const uint8_t* left, size_t lstride, const uint8_t* r
         if (W > tm_max_width()) return fail(c, MVSV_ERR_UNSUPPORTED, "tm: image wider than 4096");
         if (tm_smem_bytes(W, (int)kernel_size) > 200 * 1024) return fail(c, MVSV_ERR_UNSUPPORTED, "tm: kernelSize x width exceeds shared memory");
         MVSV_CK(c, cudaStreamWaitEvent(c->copy_stream, c->ev_done, 0));
+        MVSV_CK(c, cudaStreamWaitEvent(c->copy_stream, io(c).dl_done, 0));   // it writes the slot's rectified images
         rc = upload_images(c, io(c).rect[0], c->pitch, left, lstride, frame_stride, W, H, batch, false);
         if (rc) return rc;
         rc = upload_images(c, io(c).rect[1], c->pitch, right, rstride, frame_stride, W, H, batch, false);
@@ -1097,6 +1184,7 @@ int mvsv_set_mean_rois(mvsv_ctx* ctx, const int* xywh, int n)
                 return fail(c, MVSV_ERR_INVALID, "ROI outside the disparity map");
         }
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
+        MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));   // a device download may still copy the means it frees
         c->rois.reset();
         for (IoSlot& s : c->slot) {
             s.means.reset();
@@ -1121,7 +1209,13 @@ int mvsv_compute(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t
 int mvsv_compute_device(mvsv_ctx* c, const uint8_t* dleft, size_t lstride, const uint8_t* dright, size_t rstride,
                         size_t frame_stride, int batch, unsigned stages)
 {
-    return run(c, dleft, lstride, dright, rstride, frame_stride, batch, stages, true);
+    return mvsv_compute_device_stream(c, dleft, lstride, dright, rstride, frame_stride, batch, stages, nullptr);
+}
+
+int mvsv_compute_device_stream(mvsv_ctx* c, const uint8_t* dleft, size_t lstride, const uint8_t* dright, size_t rstride,
+                               size_t frame_stride, int batch, unsigned stages, void* stream)
+{
+    return run(c, dleft, lstride, dright, rstride, frame_stride, batch, stages, true, stream);
 }
 
 int mvsv_download(mvsv_ctx* c, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride, float* xyz,
@@ -1130,41 +1224,74 @@ int mvsv_download(mvsv_ctx* c, int16_t* disp, size_t dstride, uint8_t* rectL, ui
     return mvsv_download_age(c, 0, disp, dstride, rectL, rectR, rstride, xyz, means);
 }
 
-int mvsv_download_age(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
-                      float* xyz, float* means)
+// mvsv_download_age (host memory, kind cudaMemcpyDeviceToHost) and mvsv_download_device (device memory, cudaMemcpyDefault):
+// without a caller's stream the call waits for the copies, with one the stream waits for them instead.
+static int download(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
+                    float* xyz, float* means, cudaMemcpyKind kind, void* stream)
 {
     int rc = usable(c);
     if (rc) return rc;
+    Caller caller;
+    rc = caller_of(c, stream, &caller);
+    if (rc) return rc;
+    if (kind == cudaMemcpyDefault)
+        for (const void* p : {(const void*)disp, (const void*)rectL, (const void*)rectR, (const void*)xyz, (const void*)means})
+            if (p && !device_memory(p))
+                return fail(c, MVSV_ERR_INVALID, "a destination is not device memory (copy to host memory with mvsv_download_age)");
     const Engine* p0 = c->parts[0];
     if (age < 0 || age >= p0->nslots) return fail(c, MVSV_ERR_INVALID, "age must be below the number of I/O slots");
     const int s = (p0->cur + p0->nslots - age) % p0->nslots, n = (int)c->parts.size();
     const std::vector<int> first = firsts(c, s);
     if (first[n] < 1) return fail(c, MVSV_ERR_STATE, "nothing computed yet");
+    cudaEvent_t ready = nullptr;
+    rc = caller_ready(c, caller, &ready);
+    if (rc) return rc;
     // every part's copies are queued before the first wait, so that the parts' downloads run side by side
     int queued = 0;
     for (; queued < n && !rc; ++queued)
-        if (first[queued] < first[queued + 1])
+        if (first[queued] < first[queued + 1]) {
             rc = on_part(c, queued, [&](Engine* p) {
                 const size_t rows = (size_t)first[queued] * p->H;
                 return download_enqueue(p, s, disp ? (int16_t*)((uint8_t*)disp + rows * dstride) : nullptr, dstride,
                                         rectL ? rectL + rows * rstride : nullptr, rectR ? rectR + rows * rstride : nullptr,
                                         rstride, xyz ? xyz + rows * p->W * 3 : nullptr,
-                                        means ? means + (size_t)first[queued] * p->nrois : nullptr);
+                                        means ? means + (size_t)first[queued] * p->nrois : nullptr, kind, ready);
             });
+            if (!rc && caller.st) rc = caller_wait(c, caller, c->parts[queued]->slot[s].dl_done);
+        }
     // wait also after a failure: the caller's buffers must not be written once the call has returned
     for (int k = 0; k < queued; ++k)
         if (first[k] < first[k + 1]) {
             if (rc) cudaStreamSynchronize(c->parts[k]->dl_stream);
-            else rc = on_part(c, k, download_wait);
+            else if (!caller.st) rc = on_part(c, k, download_wait);
         }
     return rc;
 }
 
-int mvsv_download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points)
+int mvsv_download_age(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
+                      float* xyz, float* means)
+{
+    return download(c, age, disp, dstride, rectL, rectR, rstride, xyz, means, cudaMemcpyDeviceToHost, nullptr);
+}
+
+int mvsv_download_device(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, uint8_t* rectL, uint8_t* rectR, size_t rstride,
+                         float* xyz, float* means, void* stream)
+{
+    return download(c, age, disp, dstride, rectL, rectR, rstride, xyz, means, cudaMemcpyDefault, stream);
+}
+
+// mvsv_download_points and mvsv_download_points_device, as download() above
+static int download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points, cudaMemcpyKind kind,
+                           void* stream)
 {
     int rc = usable(c);
     if (rc) return rc;
+    Caller caller;
+    rc = caller_of(c, stream, &caller);
+    if (rc) return rc;
     if (!offsets) return fail(c, MVSV_ERR_INVALID, "offsets must not be NULL");
+    if (kind == cudaMemcpyDefault && points && !device_memory(points))
+        return fail(c, MVSV_ERR_INVALID, "points is not device memory (copy to host memory with mvsv_download_points)");
     const Engine* p0 = c->parts[0];
     if (age < 0 || age >= p0->nslots) return fail(c, MVSV_ERR_INVALID, "age must be below the number of I/O slots");
     const int s = (p0->cur + p0->nslots - age) % p0->nslots, n = (int)c->parts.size();
@@ -1190,18 +1317,35 @@ int mvsv_download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points, 
     if (capacity_points < (size_t)base[n])
         return fail(c, MVSV_ERR_INVALID, "points buffer holds " + std::to_string(capacity_points) + " points, the list has " +
                                              std::to_string(base[n]));
+    cudaEvent_t ready = nullptr;
+    rc = caller_ready(c, caller, &ready);
+    if (rc) return rc;
     // phase 2: every part's copy is queued before the first wait, so that the parts' copies run side by side
     int queued = 0;
     for (; queued < n && !rc; ++queued)
-        if (first[queued] < first[queued + 1])
-            rc = on_part(c, queued, [&](Engine* p) { return points_enqueue(p, s, points + 3 * (size_t)base[queued], base[queued + 1] - base[queued]); });
+        if (first[queued] < first[queued + 1]) {
+            rc = on_part(c, queued, [&](Engine* p) {
+                return points_enqueue(p, s, points + 3 * (size_t)base[queued], base[queued + 1] - base[queued], kind, ready);
+            });
+            if (!rc && caller.st) rc = caller_wait(c, caller, c->parts[queued]->slot[s].dl_done);
+        }
     // wait also after a failure: the caller's buffer must not be written once the call has returned
     for (int k = 0; k < queued; ++k)
         if (first[k] < first[k + 1]) {
             if (rc) cudaStreamSynchronize(c->parts[k]->dl_stream);
-            else rc = on_part(c, k, download_wait);
+            else if (!caller.st) rc = on_part(c, k, download_wait);
         }
     return rc;
+}
+
+int mvsv_download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points)
+{
+    return download_points(c, age, offsets, points, capacity_points, cudaMemcpyDeviceToHost, nullptr);
+}
+
+int mvsv_download_points_device(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points, void* stream)
+{
+    return download_points(c, age, offsets, points, capacity_points, cudaMemcpyDefault, stream);
 }
 
 int mvsv_set_io_slots(mvsv_ctx* ctx, int n)
@@ -1213,6 +1357,7 @@ int mvsv_set_io_slots(mvsv_ctx* ctx, int n)
         if (n == c->nslots) return MVSV_OK;
         MVSV_CK(c, cudaStreamSynchronize(c->stream));
         MVSV_CK(c, cudaStreamSynchronize(c->copy_stream));
+        MVSV_CK(c, cudaStreamSynchronize(c->dl_stream));
         if (n < c->nslots) release_slot(c->slot[1], true);
         c->nslots = n;
         c->cur = 0;
@@ -1373,6 +1518,7 @@ int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int
         if (rc) return rc;
 
         take_slot(c);
+        MVSV_CK(c, cudaStreamWaitEvent(c->stream, slot.dl_done, 0));   // a device download may still copy out of the slot
         const size_t row = (size_t)c->W * sizeof(int16_t), npx = (size_t)batch * c->H * c->W;
         MVSV_CK(c, cudaMemcpy2DAsync(c->disp_raw, row, maps, stride, row, (size_t)c->H * batch, cudaMemcpyHostToDevice, c->stream));
         const bool speckle = maxSpeckleSize > 0;

@@ -91,6 +91,9 @@ struct IoSlot {
     DeviceBuffer<long long> offsets;
     DeviceBuffer<float> means;                // [B][nrois], once mean-disparity ROIs are set
     cudaEvent_t done = nullptr;               // all kernels of the slot's last compute have finished
+    // recorded on dl_stream after every download of the slot's results: a device download (mvsv_download_device) may
+    // still be copying when its call returns, so whatever writes the slot next waits for it
+    cudaEvent_t dl_done = nullptr;
     int B = 0;                                // frames of the slot's last compute; 0: it holds no results
     unsigned stages = 0;
 };
@@ -161,7 +164,7 @@ struct Engine {
 
     int nslots = 1, cur = 0;                  // I/O slots in use; the slot of the last (or current) compute
     IoSlot slot[2];
-    cudaStream_t dl_stream = nullptr;         // device->host result copies
+    cudaStream_t dl_stream = nullptr;         // result copies to host or device memory (mvsv_download*)
 
     bool has_sgbm = false, has_bm = false;
     mvsv_sgbm_params sgbm_raw{};
