@@ -292,10 +292,42 @@ int mvsv_download_device(mvsv_ctx* ctx, int age, int16_t* disp, size_t dstride, 
  * non-NULL `points` that is not device or managed memory is MVSV_ERR_INVALID. */
 int mvsv_download_points_device(mvsv_ctx* ctx, int age, int64_t* offsets, float* points, size_t capacity_points,
                                 void* stream);
+/* The point list of I/O slot `age` entirely in DEVICE memory, with no host wait: a kernel on the engine's download
+ * stream writes both the offsets and the points, so the host never needs the list's size.
+ *   offsets: device or managed memory, not NULL.  Receives batch + 1 values (batch: frames of that slot's compute),
+ *     exactly those mvsv_download_points writes, multi-device rebase included.
+ *   points: device or managed memory, or NULL (the offsets only).  Receives points[0 .. min(total, capacity_points)):
+ *     the list cut off at the capacity, in list order; nothing past it is written.  The host does not know the total
+ *     here, so a short buffer truncates instead of failing.  A consumer detects truncation on the device by
+ *     offsets[batch] > capacity_points; every frame f with offsets[f+1] <= capacity_points is complete.
+ *   stream != NULL: the writes start after the work queued on `stream` before the call, work queued on `stream` after
+ *     the call sees them, and the call never waits on the host (no stream or event synchronisation, no copy to pageable
+ *     memory).  stream == NULL: the call waits for its writes before it returns.  cudaStreamLegacy and
+ *     cudaStreamPerThread as in mvsv_download_device.
+ *   Multi-device ctx: part k's base (the points of the parts before it) is summed on the device from their totals,
+ *     which part k's download stream copies from them once their computes are done (cudaMemcpyPeerAsync).  Where a
+ *     destination is on another device than a part, the part writes it through peer access, which the call enables
+ *     for this process (cudaDeviceEnablePeerAccess) where cudaDeviceCanAccessPeer allows it.
+ * Rejected before anything is queued, with earlier results still downloadable: MVSV_ERR_INVALID for a NULL `offsets`,
+ * `offsets` or `points` that cudaPointerGetAttributes does not report as device or managed memory, or an age outside
+ * the slots; MVSV_ERR_STATE when nothing was computed or the compute did not run MVSV_STAGE_POINTS;
+ * MVSV_ERR_UNSUPPORTED for a destination on a device that some part cannot reach by peer access.
+ * Slot lifetime as in mvsv_download_device: the writes finish before the slot's pending downloads are, so a compute that
+ * takes the slot next, and the setters that free slot buffers, wait for them. */
+int mvsv_download_points_stream(mvsv_ctx* ctx, int age, int64_t* offsets, float* points, size_t capacity_points,
+                                void* stream);
 /* Utility::calcMinMaxDisparity (src/utility.cpp:287-304) of the last computed maps as a GPU reduction: for every
  * frame the smallest and largest disparity value > 0, minmax[2*i], minmax[2*i+1]; (0, 0) when a map has none (the
  * reference dereferences an end iterator there).  Consumed by the PLY writer's grey ramp (src/ply.cpp:62-95). */
 int mvsv_download_minmax(mvsv_ctx* ctx, int16_t* minmax);
+/* mvsv_download_minmax of I/O slot `age` (ages as in mvsv_download_age) into DEVICE memory: 2 * batch int16 values,
+ * minmax[2*i], minmax[2*i+1], (0, 0) for a frame without a value > 0; on a multi-device ctx part k's frames at
+ * minmax + 2 * (its first frame).  The reduction runs on the engine's download stream into buffers of the slot, so it
+ * never races with mvsv_download_minmax.  Ordering on `stream`, stream == NULL and the slot lifetime are those of
+ * mvsv_download_points_stream.  Rejected, with earlier results still downloadable: MVSV_ERR_INVALID for a NULL
+ * `minmax` or one that is not device or managed memory, or an age outside the slots; MVSV_ERR_STATE when nothing was
+ * computed. */
+int mvsv_download_minmax_device(mvsv_ctx* ctx, int age, int16_t* minmax, void* stream);
 int mvsv_sync(mvsv_ctx* ctx);
 
 int mvsv_get_info(const mvsv_ctx* ctx, mvsv_info* info);

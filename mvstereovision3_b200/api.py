@@ -32,6 +32,7 @@ ABI_SYMBOLS = (
     "mvsv_upload_rectify_maps_rig", "mvsv_set_rectification_rig", "mvsv_set_Q_rig", "mvsv_set_frame_rigs",
     "mvsv_init_devices", "mvsv_get_devices", "mvsv_download_points",
     "mvsv_compute_device_stream", "mvsv_download_device", "mvsv_download_points_device",
+    "mvsv_download_points_stream", "mvsv_download_minmax_device",
 )
 MAX_RIGS = 64       # MVSV_MAX_RIGS
 
@@ -101,6 +102,8 @@ def load_library():
     lib.mvsv_download_points.argtypes = [vp, ci, vp, vp, sz]
     lib.mvsv_download_device.argtypes = [vp, ci, vp, sz, vp, vp, sz, vp, vp, vp]
     lib.mvsv_download_points_device.argtypes = [vp, ci, vp, vp, sz, vp]
+    lib.mvsv_download_points_stream.argtypes = [vp, ci, vp, vp, sz, vp]
+    lib.mvsv_download_minmax_device.argtypes = [vp, ci, vp, vp]
     lib.mvsv_set_io_slots.argtypes = [vp, ci]
     lib.mvsv_sync.argtypes = [vp]
     lib.mvsv_download_minmax.argtypes = [vp, vp]
@@ -466,6 +469,49 @@ class Engine:
         self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_download_points_device(
             self._ctx, age, offs.ctypes.data, out.data_ptr() or None, out.numel() // 3, h)))
         return offs[:batch + 1], out.view(-1)[:3 * int(offs[batch])].view(-1, 3)
+
+    def download_points_stream(self, batch, age=0, out=None, stream=None, device=None):
+        """The point list of download_points() entirely in device memory, with no host wait (mvsv_download_points_stream):
+        (offsets int64 tensor [batch + 1], points float32 tensor [capacity, 3]); frame f's points are
+        points[offsets[f]:offsets[f + 1]].  Without `out` both are allocated on `device` (default: the engine's first
+        device) with capacity batch * H * W, every pixel, so the list is never cut off.  `out`: (offsets, points)
+        contiguous CUDA tensors; points past its capacity are not written, and offsets[batch] > capacity tells so.
+        `stream` (a torch.cuda.Stream): the writes are ordered on it; None: the call returns with them done."""
+        torch = _torch()
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        if out is None:
+            dev, on_stream = self._device_out(stream, device)
+            with on_stream:
+                offs = torch.empty(batch + 1, dtype=torch.int64, device=dev)
+                pts = torch.empty((batch * i.height * i.width, 3), dtype=torch.float32, device=dev)
+        else:
+            offs, pts = out
+            if offs.dtype != torch.int64 or tuple(offs.shape) != (batch + 1,) or not offs.is_cuda or not offs.is_contiguous():
+                raise ValueError("out[0] must be a contiguous int64 CUDA tensor of shape (%d,)" % (batch + 1))
+            if pts.dtype != torch.float32 or pts.dim() != 2 or pts.shape[1] != 3 or not pts.is_cuda or not pts.is_contiguous():
+                raise ValueError("out[1] must be a contiguous float32 CUDA tensor [capacity, 3]")
+        self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_download_points_stream(
+            self._ctx, age, offs.data_ptr(), pts.data_ptr() if pts.numel() else None, pts.shape[0], h)))
+        return offs, pts
+
+    def download_minmax_device(self, batch, age=0, out=None, stream=None, device=None):
+        """download_minmax() of the compute `age` calls back as an int16 CUDA tensor [batch, 2]
+        (mvsv_download_minmax_device), allocated on `device` (default: the engine's first device) or taken from `out`
+        (contiguous); ordered on `stream` as in download_points_stream."""
+        torch = _torch()
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        if out is None:
+            dev, on_stream = self._device_out(stream, device)
+            with on_stream:
+                out = torch.empty((batch, 2), dtype=torch.int16, device=dev)
+        elif out.dtype != torch.int16 or tuple(out.shape) != (batch, 2) or not out.is_cuda or not out.is_contiguous():
+            raise ValueError("out must be a contiguous int16 CUDA tensor of shape (%d, 2)" % batch)
+        self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_download_minmax_device(self._ctx, age, out.data_ptr(), h)))
+        return out
 
     def download_minmax(self, batch):
         """Utility::calcMinMaxDisparity (reference src/utility.cpp:287-304) per frame, reduced on the GPU."""

@@ -4,6 +4,7 @@
 
 #include <algorithm>
 #include <cstdio>
+#include <climits>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -91,6 +92,7 @@ void release_slot(IoSlot& s, bool staging)
         s.rect[i].reset();
         if (staging) s.raw[i].reset();
     }
+    if (staging) { s.minmax.reset(); s.minmax16.reset(); }
     s.disp.reset(); s.xyz.reset(); s.points.reset(); s.offsets.reset(); s.means.reset();
     s.B = 0; s.stages = 0;
 }
@@ -113,6 +115,9 @@ int ensure_slots(Engine* c)
             MVSV_CK(c, cudaMemsetAsync(s.disp, 0, npx * sizeof(int16_t), c->stream));
         }
         if (c->nrois > 0) MVSV_CK(c, s.means.ensure((size_t)c->nrois * B));
+        // mvsv_download_minmax_device's buffers exist before any call, so that the call never allocates
+        MVSV_CK(c, s.minmax.ensure(B * 2));
+        MVSV_CK(c, s.minmax16.ensure(B * 2));
     }
     return MVSV_OK;
 }
@@ -524,7 +529,7 @@ int minmax_launch(Engine* c)
     int rc = bind(c);
     if (rc) return rc;
     MVSV_CK(c, c->minmax.ensure((size_t)c->maxB * 2));
-    MVSV_CK(c, launch_minmax(c, io(c).B));
+    MVSV_CK(c, launch_minmax(c, io(c), c->minmax, c->stream));
     return MVSV_OK;
 }
 
@@ -643,14 +648,16 @@ int caller_wait(mvsv_ctx* c, const Caller& k, cudaEvent_t ev)
     return MVSV_OK;
 }
 
-// A destination of a device download: device or managed memory on any device (cudaPointerGetAttributes)
-bool device_memory(const void* p)
+// A destination of a device download: device or managed memory on any device (cudaPointerGetAttributes).  *dev: the
+// device of device memory, -1 for managed memory.
+bool device_memory(const void* p, int* dev = nullptr)
 {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
         cudaGetLastError();   // not a sticky error: leave no trace of it for the next call
         return false;
     }
+    if (dev) *dev = a.type == cudaMemoryTypeDevice ? a.device : -1;
     return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
 
@@ -772,6 +779,39 @@ int run(mvsv_ctx* c, const uint8_t* left, size_t lstride, const uint8_t* right, 
         s.stages = s.B ? stages : 0;
     }
     return MVSV_OK;
+}
+
+// mvsv_download_points_stream and mvsv_download_minmax_device: the I/O slot `age` names (*s) and the frames of every part
+// in it (first, as firsts())
+int results_slot(mvsv_ctx* c, int age, int* s, std::vector<int>* first)
+{
+    const Engine* p0 = c->parts[0];
+    if (age < 0 || age >= p0->nslots) return fail(c, MVSV_ERR_INVALID, "age must be below the number of I/O slots");
+    *s = (p0->cur + p0->nslots - age) % p0->nslots;
+    *first = firsts(c, *s);
+    if (first->back() < 1) return fail(c, MVSV_ERR_STATE, "nothing computed yet");
+    return MVSV_OK;
+}
+
+// Queues f(k, part) on every part k with frames in slot s: work on the part's download stream that ends with the slot's
+// dl_done.  Then work queued on the caller's stream waits for every part's dl_done, or without a stream the call waits
+// for the parts' download streams.  After a failure it waits for the parts already queued: nothing is written into the
+// caller's memory once the call has returned.
+template <class F>
+int on_download_streams(mvsv_ctx* c, const Caller& caller, int s, const std::vector<int>& first, F&& f)
+{
+    const int n = (int)c->parts.size();
+    int rc = MVSV_OK, queued = 0;
+    for (; queued < n && !rc; ++queued)
+        if (first[queued] < first[queued + 1]) rc = on_part(c, queued, [&](Engine* p) { return f(queued, p); });
+    for (int k = 0; k < queued && !rc && caller.st; ++k)
+        if (first[k] < first[k + 1]) rc = caller_wait(c, caller, c->parts[k]->slot[s].dl_done);
+    for (int k = 0; k < queued; ++k)
+        if (first[k] < first[k + 1]) {
+            if (rc) cudaStreamSynchronize(c->parts[k]->dl_stream);
+            else if (!caller.st) rc = on_part(c, k, download_wait);
+        }
+    return rc;
 }
 
 }  // namespace
@@ -1348,6 +1388,91 @@ int mvsv_download_points_device(mvsv_ctx* c, int age, int64_t* offsets, float* p
     return download_points(c, age, offsets, points, capacity_points, cudaMemcpyDefault, stream);
 }
 
+int mvsv_download_points_stream(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points, void* stream)
+{
+    int rc = usable(c);
+    if (rc) return rc;
+    Caller caller;
+    rc = caller_of(c, stream, &caller);
+    if (rc) return rc;
+    int odev = -1, pdev = -1;
+    if (!offsets) return fail(c, MVSV_ERR_INVALID, "offsets must not be NULL");
+    if (!device_memory(offsets, &odev) || (points && !device_memory(points, &pdev)))
+        return fail(c, MVSV_ERR_INVALID, "offsets and points must be device memory (copy to host memory with mvsv_download_points)");
+    int s = 0;
+    std::vector<int> first;
+    rc = results_slot(c, age, &s, &first);
+    if (rc) return rc;
+    const int n = (int)c->parts.size();
+    int last = 0;   // the part holding the last frame writes offsets[batch]
+    for (int k = 0; k < n; ++k)
+        if (first[k] < first[k + 1]) {
+            last = k;
+            if (!c->parts[k]->slot[s].offsets || !(c->parts[k]->slot[s].stages & MVSV_STAGE_POINTS))
+                return fail(c, MVSV_ERR_STATE, "POINTS stage was not computed");
+        }
+    // k_points_out writes the destinations from the part's device: one on another device needs peer access there
+    for (int pass = 0; pass < 2; ++pass)
+        for (int k = 0; k < n; ++k) {
+            Engine* p = c->parts[k];
+            if (first[k] == first[k + 1]) continue;
+            for (int d : {odev, points ? pdev : -1}) {
+                if (d < 0 || d == p->device) continue;
+                if (pass == 0) {
+                    int can = 0;
+                    MVSV_CK(c, cudaDeviceCanAccessPeer(&can, p->device, d));
+                    if (!can)
+                        return fail(c, MVSV_ERR_UNSUPPORTED, "device " + std::to_string(p->device) + " cannot access device " +
+                                                                 std::to_string(d) + " by peer access (destination there)");
+                    continue;
+                }
+                MVSV_CK(c, cudaSetDevice(p->device));
+                const cudaError_t e = cudaDeviceEnablePeerAccess(d, 0);
+                if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+                else MVSV_CK(c, e);
+            }
+            if (pass == 0 && k > 0) {
+                MVSV_CK(c, cudaSetDevice(p->device));
+                MVSV_CK(c, p->pt_base.ensure((size_t)n));
+            }
+        }
+    cudaEvent_t ready = nullptr;
+    rc = caller_ready(c, caller, &ready);
+    if (rc) return rc;
+    const long long cap = (long long)std::min(capacity_points, (size_t)LLONG_MAX);
+    return on_download_streams(c, caller, s, first, [&](int k, Engine* p) -> int {
+        int r = bind(p);
+        if (r) return r;
+        const IoSlot& sl = p->slot[s];
+        cudaStream_t st = p->dl_stream;
+        MVSV_CK(p, cudaStreamWaitEvent(st, sl.done, 0));
+        if (ready) MVSV_CK(p, cudaStreamWaitEvent(st, ready, 0));
+        // the base: the totals of the parts before, each copied once that part's compute is done
+        int nb = 0;
+        for (int j = 0; j < k; ++j)
+            if (first[j] < first[j + 1]) {
+                const Engine* q = c->parts[j];
+                MVSV_CK(p, cudaStreamWaitEvent(st, q->slot[s].done, 0));
+                MVSV_CK(p, cudaMemcpyPeerAsync((long long*)p->pt_base + nb, p->device,
+                                               (const long long*)q->slot[s].offsets + q->slot[s].B, q->device, sizeof(long long), st));
+                ++nb;
+            }
+        MVSV_CK(p, launch_points_out(p, sl, nb ? (const long long*)p->pt_base : nullptr, nb,
+                                     reinterpret_cast<long long*>(offsets) + first[k], first[k + 1] - first[k] + (k == last ? 1 : 0),
+                                     points, cap));
+        MVSV_CK(p, cudaEventRecord(sl.dl_done, st));
+        // the parts before hold their slot until this part has read their totals: their dl_done covers that read
+        for (int j = 0; j < k; ++j)
+            if (first[j] < first[j + 1]) {
+                Engine* q = c->parts[j];
+                MVSV_CK(p, cudaSetDevice(q->device));
+                MVSV_CK(p, cudaStreamWaitEvent(q->dl_stream, sl.dl_done, 0));
+                MVSV_CK(p, cudaEventRecord(q->slot[s].dl_done, q->dl_stream));
+            }
+        return MVSV_OK;
+    });
+}
+
 int mvsv_set_io_slots(mvsv_ctx* ctx, int n)
 {
     return each(ctx, true, [&](Engine* c) -> int {
@@ -1383,6 +1508,37 @@ int mvsv_download_minmax(mvsv_ctx* c, int16_t* minmax)
                     return pass == 0 ? minmax_launch(p) : minmax_read(p, minmax + 2 * (size_t)first[k]);
                 });
     return rc;
+}
+
+int mvsv_download_minmax_device(mvsv_ctx* c, int age, int16_t* minmax, void* stream)
+{
+    int rc = usable(c);
+    if (rc) return rc;
+    Caller caller;
+    rc = caller_of(c, stream, &caller);
+    if (rc) return rc;
+    if (!minmax || !device_memory(minmax))
+        return fail(c, MVSV_ERR_INVALID, "minmax must be device memory (copy to host memory with mvsv_download_minmax)");
+    int s = 0;
+    std::vector<int> first;
+    rc = results_slot(c, age, &s, &first);
+    if (rc) return rc;
+    cudaEvent_t ready = nullptr;
+    rc = caller_ready(c, caller, &ready);
+    if (rc) return rc;
+    return on_download_streams(c, caller, s, first, [&](int k, Engine* p) -> int {
+        int r = bind(p);
+        if (r) return r;
+        IoSlot& sl = p->slot[s];
+        cudaStream_t st = p->dl_stream;
+        MVSV_CK(p, cudaStreamWaitEvent(st, sl.done, 0));
+        if (ready) MVSV_CK(p, cudaStreamWaitEvent(st, ready, 0));
+        MVSV_CK(p, launch_minmax(p, sl, sl.minmax, st));
+        MVSV_CK(p, launch_minmax_fold(p, sl.minmax, sl.minmax16, sl.B, st));
+        MVSV_CK(p, cudaMemcpyAsync(minmax + 2 * (size_t)first[k], sl.minmax16, (size_t)sl.B * 2 * sizeof(int16_t), cudaMemcpyDefault, st));
+        MVSV_CK(p, cudaEventRecord(sl.dl_done, st));
+        return MVSV_OK;
+    });
 }
 
 int mvsv_sync(mvsv_ctx* ctx)

@@ -1,6 +1,7 @@
 // Rectification (K1), 3x3 median (K5), speckle filter (K6), reprojection + ROI means (K8) on sm_100a.
 #include "mvsv_internal.h"
 
+#include <algorithm>
 #include <cstdint>
 #include <cfloat>
 #include <cmath>
@@ -684,14 +685,72 @@ __global__ void k_minmax(const int16_t* __restrict__ disp, int* __restrict__ mm,
     }
 }
 
+// k_minmax's (lo, hi) of B frames as the int16 pairs of mvsv_download_minmax: (0, 0) for a frame without a value > 0
+__global__ void k_minmax_fold(const int* __restrict__ mm, int16_t* __restrict__ out, int B)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= B) return;
+    const int lo = mm[2 * i], hi = mm[2 * i + 1];
+    const bool none = hi <= 0;
+    out[2 * i] = none ? (int16_t)0 : (int16_t)lo;
+    out[2 * i + 1] = none ? (int16_t)0 : (int16_t)hi;
+}
+
+// One part's share of mvsv_download_points_stream.  Its base (the points of the parts before it) is the sum of `bases`;
+// it writes its nout frame offsets rebased onto that base, and copies its points i with base + i < capacity to
+// dst + 3 * (base + i).  The list's length is known only on the device, which is why this is a kernel and not a copy.
+// Grid-stride and coalesced; 16-byte accesses where the destination is 16-byte aligned (the source, a cudaMalloc
+// buffer, always is), 4-byte ones otherwise (the destination moves in steps of 12 bytes).
+__global__ void __launch_bounds__(256)
+k_points_out(const long long* __restrict__ offs, int nfr, int nout, const long long* __restrict__ bases, int nbases,
+             const float* __restrict__ src, long long* __restrict__ dst_offs, float* __restrict__ dst, long long capacity)
+{
+    long long base = 0;
+    for (int j = 0; j < nbases; ++j) base += bases[j];
+    const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x, nthr = (long long)gridDim.x * blockDim.x;
+    for (long long i = tid; i < nout; i += nthr) dst_offs[i] = base + offs[i];
+    const long long n = dst ? min(offs[nfr], capacity - base) : 0;
+    if (n <= 0) return;
+    float* d = dst + 3 * base;
+    const long long nf = 3 * n;
+    long long head = 0;
+    if ((reinterpret_cast<uintptr_t>(d) & 15) == 0) {
+        const long long n4 = nf >> 2;
+        for (long long i = tid; i < n4; i += nthr) st128(d + 4 * i, ld128(src + 4 * i));
+        head = 4 * n4;
+    }
+    for (long long i = head + tid; i < nf; i += nthr) d[i] = src[i];
+}
+
 }  // namespace
 
-cudaError_t launch_minmax(Engine* c, int B)
+cudaError_t launch_minmax(Engine* c, const IoSlot& s, int* mm, cudaStream_t st)
 {
-    { KernelTimer kt(c, KID_MINMAX); k_minmax_init<<<(2 * B + 127) / 128, 128, 0, c->stream>>>(c->minmax, 2 * B); }
+    // per-kernel timing brackets the ctx stream only: on another stream the launches are counted, not timed
+    const int kid = st == c->stream ? KID_MINMAX : KID_UNTIMED;
+    const int B = s.B;
+    { KernelTimer kt(c, kid, st); k_minmax_init<<<(2 * B + 127) / 128, 128, 0, st>>>(mm, 2 * B); }
     dim3 grd(32, B);
-    KernelTimer kt(c, KID_MINMAX);
-    k_minmax<<<grd, 256, 0, c->stream>>>(io(c).disp, c->minmax, c->W * c->H);
+    KernelTimer kt(c, kid, st);
+    k_minmax<<<grd, 256, 0, st>>>(s.disp, mm, c->W * c->H);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_minmax_fold(Engine* c, const int* mm, int16_t* out, int B, cudaStream_t st)
+{
+    KernelTimer kt(c, KID_UNTIMED, st);
+    k_minmax_fold<<<(B + 127) / 128, 128, 0, st>>>(mm, out, B);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_points_out(Engine* c, const IoSlot& s, const long long* bases, int nbases, long long* dst_offs, int nout,
+                              float* dst, long long capacity)
+{
+    // enough threads for the largest list the slot can hold (or for the offsets alone), at most 8 CTAs per SM
+    const long long work = dst ? (3LL * s.B * c->H * c->W + 3) / 4 : nout;
+    const int blocks = (int)std::max(1LL, std::min((work + 255) / 256, 8LL * c->num_sms));
+    KernelTimer kt(c, KID_UNTIMED, c->dl_stream);
+    k_points_out<<<blocks, 256, 0, c->dl_stream>>>(s.offsets, s.B, nout, bases, nbases, s.points, dst_offs, dst, capacity);
     return cudaGetLastError();
 }
 

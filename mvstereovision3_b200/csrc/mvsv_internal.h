@@ -34,6 +34,9 @@ enum KernelId {
     KID_CCL_ROWS, KID_CCL_VMERGE, KID_CCL_FLATTEN, KID_CCL_APPLY, KID_BM_PREFILTER, KID_BM_TEX, KID_BM_COLSUM,
     KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_BM_LRCHECK, KID_POINTS, KID_COUNT
 };
+// a launch counted in mvsv_launch_count but never timed: the per-kernel timing brackets the engine's stream only
+// (mvsv_profile_read waits for that stream), and the device downloads launch on the download stream
+constexpr int KID_UNTIMED = -1;
 extern const char* const kKernelNames[KID_COUNT];
 
 struct ProfBracket { int kid; cudaEvent_t a, b; };
@@ -94,6 +97,10 @@ struct IoSlot {
     // recorded on dl_stream after every download of the slot's results: a device download (mvsv_download_device) may
     // still be copying when its call returns, so whatever writes the slot next waits for it
     cudaEvent_t dl_done = nullptr;
+    // mvsv_download_minmax_device: the reduction of the slot's disparities ([maxB][2]) and its int16 pairs.  Per slot, so that it never races with mvsv_download_minmax (Engine::minmax, on the engine's
+    // stream) or with the download of the other slot.
+    DeviceBuffer<int> minmax;
+    DeviceBuffer<int16_t> minmax16;
     int B = 0;                                // frames of the slot's last compute; 0: it holds no results
     unsigned stages = 0;
 };
@@ -208,6 +215,9 @@ struct Engine {
     DeviceBuffer<int> rois;                   // [n][4]
     DeviceBuffer<int> minmax;                 // [B][2]
     DeviceBuffer<long long> pt_tiles;         // MVSV_STAGE_POINTS: per tile, its count, then its base (points_tiles)
+    // mvsv_download_points_stream on a multi-device ctx: the point totals of the parts before this one, copied from
+    // their slots on dl_stream (one entry per part of the ctx); k_points_out adds them up into this part's base
+    DeviceBuffer<long long> pt_base;
 };
 
 // the I/O slot of the compute in progress (or of the last one)
@@ -220,7 +230,7 @@ struct KernelTimer {
     KernelTimer(Engine* ctx, int kid, cudaStream_t on = nullptr) : c(ctx), idx(-1), st(on ? on : ctx->stream)
     {
         ++c->launches;
-        if (!c->prof) return;
+        if (!c->prof || kid == KID_UNTIMED) return;
         ProfBracket b; b.kid = kid;
         for (cudaEvent_t* e : {&b.a, &b.b}) {
             if (!c->ev_free.empty()) { *e = c->ev_free.back(); c->ev_free.pop_back(); }
@@ -263,7 +273,14 @@ cudaError_t launch_means(Engine* c, int B);
 // launch; `rigs`: frames of several rigs (mvsv_set_frame_rigs)
 size_t points_tiles(int W, int H, int B);
 cudaError_t launch_points(Engine* c, int B, bool rigs);
-cudaError_t launch_minmax(Engine* c, int B);
+// Utility::calcMinMaxDisparity of slot s's disparities into mm ([s.B][2] int: lo, hi) on stream st; the fold turns B
+// such pairs into the int16 pairs of mvsv_download_minmax
+cudaError_t launch_minmax(Engine* c, const IoSlot& s, int* mm, cudaStream_t st);
+cudaError_t launch_minmax_fold(Engine* c, const int* mm, int16_t* out, int B, cudaStream_t st);
+// mvsv_download_points_stream, one part: slot s's frame offsets (nout of them) rebased by the sum of bases[0 .. nbases)
+// into dst_offs, and the points that fit below `capacity` into dst (NULL: the offsets only), on dl_stream
+cudaError_t launch_points_out(Engine* c, const IoSlot& s, const long long* bases, int nbases, long long* dst_offs, int nout,
+                              float* dst, long long capacity);
 cudaError_t launch_median(Engine* c, const int16_t* in, int16_t* out, int B);
 cudaError_t launch_speckle(Engine* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
 // fused previous-row sweep (csrc/sweep.cu): strip decomposition of a batch, scratch sizes, launch
