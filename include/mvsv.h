@@ -46,7 +46,12 @@ enum {
      * every pixel of the final map with disparity > 0 gives the three floats MVSV_STAGE_XYZ writes for it (same
      * arithmetic, same Z = 0 where Z/1000 is infinite), packed one after the other; fetched with mvsv_download_points.
      * With or without MVSV_STAGE_XYZ, after either matcher; like XYZ it needs the Q of every frame's rig. */
-    MVSV_STAGE_POINTS = 32
+    MVSV_STAGE_POINTS = 32,
+    /* MeanDisparityDetection::detectObstacles and SamplepointDetection::detectObstacles  src/MeanDisparityDetection.cpp:
+     * 71-266, src/SamplePointDetection.cpp:29-178 (as mirrored by include/mvsv_detection.hpp): the range test and
+     * Utility::calcCoordinate of every ROI mean, on the device.  Needs MVSV_STAGE_MEANS in the same compute and a table
+     * from mvsv_set_detection; the found-obstacle lists are fetched with mvsv_download_obstacles. */
+    MVSV_STAGE_DETECT = 64
 };
 
 /* Field order of the first nine ints == struct Disparity::sgbmParameters (inc/disparity.h:17-27).
@@ -201,6 +206,37 @@ int mvsv_set_frame_rigs(mvsv_ctx* ctx, const int* rig_of_frame, int n);
  * MVSV_STAGE_MEANS then fails with MVSV_ERR_STATE until they are set again. */
 int mvsv_set_mean_rois(mvsv_ctx* ctx, const int* xywh, int n);
 
+/* Obstacle detection on the device (MVSV_STAGE_DETECT).  The host mirror include/mvsv_detection.hpp defines the result:
+ * for every frame f of a compute and every ROI i with a detector d = detector_of_roi[i] >= 0, with rig = the frame's rig
+ * (mvsv_set_frame_rigs), Q its Q and value = the ROI mean of MVSV_STAGE_MEANS,
+ *   first  = Utility::calcDMapValues({0, 0, min_distance[d] * 1000}, Q).dValue,
+ *   second = Utility::calcDMapValues({0, 0, max_distance[d] * 1000}, Q).dValue   (float arithmetic, as in the header),
+ * ROI i is a hit iff value < first && value > second (the reference's test, kept as is), and a
+ * hit gives the record {roi = i, value, xyzw = Utility::calcCoordinate({value, cx_i, cy_i}, Q)}: the Vec4 the detectors
+ * push to getFoundPoints(), bit for bit (products accumulated in double in the order k = 0..3, each component rounded
+ * to float, then multiplied by the double reciprocal of the fourth; z := 0 where z / 1000 is infinite).  A frame's
+ * records come in ascending ROI order, the detectors interleaved by ROI index as their two host loops visit them. */
+typedef struct mvsv_obstacle {
+    int32_t roi;
+    float value;
+    float xyzw[4];
+} mvsv_obstacle;   /* 24 bytes */
+#define MVSV_MAX_DETECTORS 8
+/* The detection table for the ROIs of mvsv_set_mean_rois.  n must equal their count (MVSV_ERR_STATE otherwise: set the
+ * ROIs first).  detector_of_roi[i] in [-1, ndet): the detector ROI i belongs to, -1 for a ROI that is not tested.
+ * centers_xy[2i], centers_xy[2i+1]: the image_x, image_y calcCoordinate takes for ROI i, in dMapWork coordinates (the
+ * map without the dMapROI x offset): Subimage::roi_center, Samplepoint::center.  min_max_distance[2d], [2d+1]: the
+ * min_distance / max_distance of detector d in metres (the init() arguments), ndet in [1, MVSV_MAX_DETECTORS].  The
+ * disparity range of every (rig, detector) is computed on the host, again whenever a Q or the table changes.
+ * mvsv_set_mean_rois and every geometry change (which drops the ROIs) drop the table, and with it the obstacle lists
+ * the I/O slots hold.  A compute with MVSV_STAGE_DETECT fails before it takes an I/O slot, with the results of earlier
+ * computes still downloadable: MVSV_ERR_INVALID without MVSV_STAGE_MEANS; MVSV_ERR_STATE without a table, with a
+ * table whose length no longer matches the ROIs, or when a frame names a rig without Q.
+ * Multi-device ctx: repeated on every part, like the other setters.  No reference counterpart (the reference runs the
+ * detectors on the CPU, trgt/demo.cpp:271-276). */
+int mvsv_set_detection(mvsv_ctx* ctx, const int* detector_of_roi, const float* centers_xy, int n,
+                       const float* min_max_distance, int ndet);
+
 /* One pass of the hot path over `batch` stereo pairs held in HOST memory (pair i at base + i*frame_stride).
  * Asynchronous when the host buffers are pinned (mvsv_host_alloc): the copies run on the ctx's copy stream and the
  * call returns at once.  Pageable buffers are accepted too, but the CUDA driver then stages them itself and the call
@@ -316,6 +352,22 @@ int mvsv_download_points_device(mvsv_ctx* ctx, int age, int64_t* offsets, float*
  * takes the slot next, and the setters that free slot buffers, wait for them. */
 int mvsv_download_points_stream(mvsv_ctx* ctx, int age, int64_t* offsets, float* points, size_t capacity_points,
                                 void* stream);
+/* The found obstacles of MVSV_STAGE_DETECT of the compute in I/O slot `age`, copied to host memory; synchronous.  As
+ * mvsv_download_points with records for points: offsets[0 .. batch] (frame f's records are out[offsets[f] ..
+ * offsets[f+1]), offsets[batch] the total), then exactly offsets[batch] records into `out`, which holds `capacity`.
+ *   out == NULL: only the offsets (the size query).
+ *   capacity < offsets[batch]: MVSV_ERR_INVALID, with the offsets written and `out` untouched.
+ *   the compute did not run MVSV_STAGE_DETECT: MVSV_ERR_STATE.  Ages, the rebase of a multi-device ctx and the other
+ *   rejections are those of mvsv_download_points. */
+int mvsv_download_obstacles(mvsv_ctx* ctx, int age, int64_t* offsets, mvsv_obstacle* out, size_t capacity);
+/* The found obstacles in DEVICE memory with no host wait, as mvsv_download_points_stream gives the point list: offsets
+ * (device or managed memory, not NULL) receive the batch + 1 values of mvsv_download_obstacles; out (device or managed
+ * memory, or NULL for the offsets only) receives out[0 .. min(total, capacity)), cut off at the capacity, nothing past it;
+ * offsets[batch] > capacity tells a consumer on the device that the list was cut.  Ordering on `stream`,
+ * stream == NULL, peer access on a multi-device ctx (the parts' totals summed on the device), the slot lifetime and the
+ * rejections are those of mvsv_download_points_stream, with MVSV_STAGE_DETECT in place of MVSV_STAGE_POINTS. */
+int mvsv_download_obstacles_stream(mvsv_ctx* ctx, int age, int64_t* offsets, mvsv_obstacle* out, size_t capacity,
+                                   void* stream);
 /* Utility::calcMinMaxDisparity (src/utility.cpp:287-304) of the last computed maps as a GPU reduction: for every
  * frame the smallest and largest disparity value > 0, minmax[2*i], minmax[2*i+1]; (0, 0) when a map has none (the
  * reference dereferences an end iterator there).  Consumed by the PLY writer's grey ramp (src/ply.cpp:62-95). */
@@ -378,9 +430,9 @@ long long mvsv_debug_read(mvsv_ctx* ctx, int which, void* host, size_t capacity_
  * maps + b*height*stride) become the raw disparity (mvsv_debug_read which=2); then, in the order cv::StereoSGBM applies
  * them, medianBlur(3) when median != 0 and filterSpeckles(newVal, maxSpeckleSize, maxDiff) when maxSpeckleSize > 0
  * (maxDiff in x16 units, as filterSpeckles takes it; neither: a plain copy) leave the final map in the next I/O slot,
- * and `stages` (MVSV_STAGE_XYZ, MVSV_STAGE_POINTS and / or MVSV_STAGE_MEANS only) run on it.  The slot is then read like
- * that of a compute (mvsv_download, mvsv_download_age, mvsv_download_points, mvsv_download_minmax, mvsv_debug_read 2 and
- * 4).  Argument and state
+ * and `stages` (MVSV_STAGE_XYZ, MVSV_STAGE_POINTS, MVSV_STAGE_MEANS and / or MVSV_STAGE_DETECT with MVSV_STAGE_MEANS
+ * only) run on it.  The slot is then read like that of a compute (mvsv_download, mvsv_download_age,
+ * mvsv_download_points, mvsv_download_obstacles, mvsv_download_minmax, mvsv_debug_read 2 and 4).  Argument and state
  * checks, and the handling of a failure, are those of mvsv_compute. */
 int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int batch, int median, int newVal,
                           int maxSpeckleSize, int maxDiff, unsigned stages);

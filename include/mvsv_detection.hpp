@@ -11,6 +11,9 @@
 // Differences, all deliberate: build() takes the means computed on the GPU instead of a cv::Mat; detectObstacles()
 // returns the found points and leaves writing the PLY file to the caller (`ply::write`), the reference hard-codes
 // "pcl/subimage_detection/pcl_NNNN.ply"; Q is a row-major float[16] instead of a CV_32F cv::Mat.
+// The same detection runs on the device as MVSV_STAGE_DETECT (include/mvsv.h): detectionTable() gives a detector's part of
+// the table mvsv_set_detection takes, and buildFromObstacles() turns a frame's records of mvsv_download_obstacles into
+// the found lists and counter that build() + detectObstacles() leave on the same means.
 #pragma once
 #include <cmath>
 #include <fstream>
@@ -18,6 +21,8 @@
 #include <string>
 #include <utility>
 #include <vector>
+
+#include "mvsv.h"
 
 namespace mvsv {
 
@@ -124,19 +129,53 @@ public:
     // ROIs (x, y, w, h in RAW disparity-map coordinates) to hand to mvsv_set_mean_rois, in build() order
     const std::vector<int>& rois() const { return mRois; }
     const std::vector<Vec4>& getFoundPoints() const { return mFoundPoints; }
+    // image_x, image_y of every ROI (in rois() order) as detectObstacles() hands them to calcCoordinate
+    const std::vector<float>& centers() const { return mCenters; }
+    // min_distance, max_distance of init(), in metres
+    std::pair<float, float> getDistance() const { return mDistance; }
 
 protected:
     void initRangeDisparity(const float* Q, float min_distance, float max_distance)
     {
+        mDistance = std::make_pair(min_distance, max_distance);
         for (int i = 0; i < 16; ++i) mQ[i] = Q[i];
         const float lower[3] = {0, 0, min_distance * 1000}, upper[3] = {0, 0, max_distance * 1000};
         mRangeDisparity = std::make_pair(Utility::calcDMapValues(lower, mQ).dValue, Utility::calcDMapValues(upper, mQ).dValue);
     }
-    std::pair<float, float> mRange{0.f, 0.f}, mRangeDisparity{0.f, 0.f};
+    // the found lists from the records of one frame (mvsv_download_obstacles) whose ROI index lies in [first_roi,
+    // first_roi + ROI count): found(i, value) adds ROI i's entry; records of other detectors are skipped
+    template <class Found>
+    void takeObstacles(const mvsv_obstacle* records, size_t count, int first_roi, Found found)
+    {
+        mFoundPoints.clear();
+        const int n = (int)mCenters.size() / 2;
+        for (size_t k = 0; k < count; ++k) {
+            const int i = records[k].roi - first_roi;
+            if (i < 0 || i >= n) continue;
+            found(i, records[k].value);
+            Vec4 p;
+            for (int r = 0; r < 4; ++r) p.v[r] = records[k].xyzw[r];
+            mFoundPoints.push_back(p);
+        }
+    }
+    std::pair<float, float> mRange{0.f, 0.f}, mRangeDisparity{0.f, 0.f}, mDistance{0.f, 0.f};
     float mQ[16];
     std::vector<int> mRois;
+    std::vector<float> mCenters;
     std::vector<Vec4> mFoundPoints;
 };
+
+// Appends detector d's part to the table of mvsv_set_detection: its ROIs (d.rois(), to be appended to the ROIs of
+// mvsv_set_mean_rois in the same order) get detector id min_max_distance.size() / 2, their centers, and its distances.
+inline void detectionTable(const ObstacleDetection& d, std::vector<int>& detector_of_roi, std::vector<float>& centers_xy,
+                           std::vector<float>& min_max_distance)
+{
+    const int id = (int)min_max_distance.size() / 2;
+    detector_of_roi.insert(detector_of_roi.end(), d.centers().size() / 2, id);
+    centers_xy.insert(centers_xy.end(), d.centers().begin(), d.centers().end());
+    min_max_distance.push_back(d.getDistance().first);
+    min_max_distance.push_back(d.getDistance().second);
+}
 
 // src/MeanDisparityDetection.cpp
 class MeanDisparityDetection : public ObstacleDetection {
@@ -148,6 +187,7 @@ public:
     {
         mSubimageVec.clear();
         mRois.clear();
+        mCenters.clear();
         const int distanceX = cols / 9, distanceY = rows / 9;
         for (int r = 0; r < 9; ++r)
             for (int c = 0; c < 9; ++c) {
@@ -155,6 +195,7 @@ public:
                 mSubimageVec.push_back(Subimage(tl, br));
                 mFoundObstacles.push_back(Subimage(tl, br));       // sic: the reference pre-fills the found list too
                 mRois.push_back(x_offset + tl.x); mRois.push_back(tl.y); mRois.push_back(distanceX); mRois.push_back(distanceY);
+                mCenters.push_back((float)mSubimageVec.back().roi_center.x); mCenters.push_back((float)mSubimageVec.back().roi_center.y);
             }
         initRangeDisparity(Q, min_distance, max_distance);
     }
@@ -208,6 +249,19 @@ public:
         if (!mFoundPoints.empty()) ++mObstacleCounter;   // the reference writes pcl_NNNN.ply here
     }
 
+    // detectObstacles() done on the device: the found Subimages (value = the record's mean), found points and counter
+    // from one frame's records; this detector's ROIs start at index first_roi of the table
+    void buildFromObstacles(const mvsv_obstacle* records, size_t count, int first_roi = 0)
+    {
+        mFoundObstacles.clear();
+        takeObstacles(records, count, first_roi, [&](int i, float value) {
+            Subimage s = mSubimageVec[i];
+            s.value = value;
+            mFoundObstacles.push_back(s);
+        });
+        if (!mFoundPoints.empty()) ++mObstacleCounter;
+    }
+
 private:
     std::vector<Subimage> mSubimageVec, mFoundObstacles;
     std::vector<float> mMeanMap, mMeanDistanceMap;
@@ -221,6 +275,7 @@ public:
     {
         mSPVec.clear();
         mRois.clear();
+        mCenters.clear();
         const int distanceX = cols / 8, distanceY = rows / 8;
         for (int c = 1; c < distanceX; ++c)
             for (int r = 1; r < distanceY; ++r) {
@@ -228,6 +283,7 @@ public:
                 mSPVec.push_back(sp);
                 mFoundObstacles.push_back(sp);
                 mRois.push_back(x_offset + sp.roi[0]); mRois.push_back(sp.roi[1]); mRois.push_back(sp.roi[2]); mRois.push_back(sp.roi[3]);
+                mCenters.push_back((float)sp.center.x); mCenters.push_back((float)sp.center.y);
             }
         initRangeDisparity(Q, min_distance, max_distance);
     }
@@ -255,6 +311,18 @@ public:
                 mFoundPoints.push_back(Utility::calcCoordinate(m, mQ));
             }
         }
+        if (!mFoundPoints.empty()) ++mObstacleCounter;
+    }
+
+    // detectObstacles() done on the device, as MeanDisparityDetection::buildFromObstacles
+    void buildFromObstacles(const mvsv_obstacle* records, size_t count, int first_roi = 0)
+    {
+        mFoundObstacles.clear();
+        takeObstacles(records, count, first_roi, [&](int i, float value) {
+            Samplepoint s = mSPVec[i];
+            s.value = value;
+            mFoundObstacles.push_back(s);
+        });
         if (!mFoundPoints.empty()) ++mObstacleCounter;
     }
 

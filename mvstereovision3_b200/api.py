@@ -12,7 +12,10 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmvsv.so")
 
-STAGE_RECTIFY, STAGE_SGBM, STAGE_BM, STAGE_XYZ, STAGE_MEANS, STAGE_POINTS = 1, 2, 4, 8, 16, 32
+STAGE_RECTIFY, STAGE_SGBM, STAGE_BM, STAGE_XYZ, STAGE_MEANS, STAGE_POINTS, STAGE_DETECT = 1, 2, 4, 8, 16, 32, 64
+MAX_DETECTORS = 8   # MVSV_MAX_DETECTORS
+# struct mvsv_obstacle: one found obstacle of STAGE_DETECT (24 bytes)
+OBSTACLE_DTYPE = np.dtype([("roi", "<i4"), ("value", "<f4"), ("xyzw", "<f4", (4,))])
 CUDA_STREAM_LEGACY = 1      # cudaStreamLegacy: the legacy default stream of the current device
 
 
@@ -33,6 +36,7 @@ ABI_SYMBOLS = (
     "mvsv_init_devices", "mvsv_get_devices", "mvsv_download_points",
     "mvsv_compute_device_stream", "mvsv_download_device", "mvsv_download_points_device",
     "mvsv_download_points_stream", "mvsv_download_minmax_device",
+    "mvsv_set_detection", "mvsv_download_obstacles", "mvsv_download_obstacles_stream",
 )
 MAX_RIGS = 64       # MVSV_MAX_RIGS
 
@@ -104,6 +108,9 @@ def load_library():
     lib.mvsv_download_points_device.argtypes = [vp, ci, vp, vp, sz, vp]
     lib.mvsv_download_points_stream.argtypes = [vp, ci, vp, vp, sz, vp]
     lib.mvsv_download_minmax_device.argtypes = [vp, ci, vp, vp]
+    lib.mvsv_set_detection.argtypes = [vp, vp, vp, ci, vp, ci]
+    lib.mvsv_download_obstacles.argtypes = [vp, ci, vp, vp, sz]
+    lib.mvsv_download_obstacles_stream.argtypes = [vp, ci, vp, vp, sz, vp]
     lib.mvsv_set_io_slots.argtypes = [vp, ci]
     lib.mvsv_sync.argtypes = [vp]
     lib.mvsv_download_minmax.argtypes = [vp, vp]
@@ -277,6 +284,18 @@ class Engine:
     def set_mean_rois(self, rois):
         r = np.ascontiguousarray(rois, np.int32).reshape(-1, 4)
         self._ck(self._lib.mvsv_set_mean_rois(self._ctx, r.ctypes.data, len(r)))
+
+    def set_detection(self, detector_of_roi, centers, ranges):
+        """The detection table of STAGE_DETECT (mvsv_set_detection) for the ROIs of set_mean_rois: detector_of_roi [n]
+        (-1: not tested), centers [n, 2] (calcCoordinate's image_x, image_y of each ROI, without the dMapROI x offset),
+        ranges [ndet, 2] (each detector's min_distance, max_distance in metres)."""
+        d = np.ascontiguousarray(detector_of_roi, np.int32).ravel()
+        xy = np.ascontiguousarray(centers, np.float32).reshape(-1, 2)
+        rg = np.ascontiguousarray(ranges, np.float32).reshape(-1, 2)
+        if len(xy) != len(d):
+            raise ValueError("detector_of_roi and centers must have one entry per ROI")
+        self._ck(self._lib.mvsv_set_detection(self._ctx, d.ctypes.data if d.size else None, xy.ctypes.data if xy.size else None,
+                                              int(d.size), rg.ctypes.data if rg.size else None, len(rg)))
 
     # -- compute --------------------------------------------------------------------------------
     @staticmethod
@@ -496,6 +515,46 @@ class Engine:
             self._ctx, age, offs.data_ptr(), pts.data_ptr() if pts.numel() else None, pts.shape[0], h)))
         return offs, pts
 
+    def download_obstacles(self, batch, age=0):
+        """The found obstacles of STAGE_DETECT of the compute `age` calls back (mvsv_download_obstacles): (offsets int64
+        [batch + 1], records [n] of OBSTACLE_DTYPE: roi, value, xyzw); frame f's records are records[offsets[f]:offsets[f + 1]],
+        in ascending ROI order."""
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        offs = np.empty(i.max_batch + 1, np.int64)         # the C call writes the compute's frames + 1 entries
+        self._ck(self._lib.mvsv_download_obstacles(self._ctx, age, offs.ctypes.data, None, 0))
+        out = np.empty(int(offs[batch]), OBSTACLE_DTYPE)
+        self._ck(self._lib.mvsv_download_obstacles(self._ctx, age, offs.ctypes.data, out.ctypes.data if out.size else None,
+                                                   out.size))
+        return offs[:batch + 1], out
+
+    def download_obstacles_stream(self, batch, age=0, out=None, stream=None, device=None):
+        """The found obstacles of download_obstacles() entirely in device memory, with no host wait
+        (mvsv_download_obstacles_stream): (offsets int64 tensor [batch + 1], records float32 tensor [capacity, 6]), a
+        record being roi (int32 bits: records.view(torch.int32)[:, 0]), value, x, y, z, w.  Without `out` both are
+        allocated on `device` (default: the engine's first device) with capacity batch * num_rois, so the list is never cut
+        off.  `out`: (offsets, records) contiguous CUDA tensors; records past its capacity are not written, and
+        offsets[batch] > capacity tells so.  `stream` as in download_points_stream."""
+        torch = _torch()
+        i = self.info
+        if age == 0:
+            self._check_batch(batch, i)
+        if out is None:
+            dev, on_stream = self._device_out(stream, device)
+            with on_stream:
+                offs = torch.empty(batch + 1, dtype=torch.int64, device=dev)
+                rec = torch.empty((batch * i.num_rois, 6), dtype=torch.float32, device=dev)
+        else:
+            offs, rec = out
+            if offs.dtype != torch.int64 or tuple(offs.shape) != (batch + 1,) or not offs.is_cuda or not offs.is_contiguous():
+                raise ValueError("out[0] must be a contiguous int64 CUDA tensor of shape (%d,)" % (batch + 1))
+            if rec.dtype != torch.float32 or rec.dim() != 2 or rec.shape[1] != 6 or not rec.is_cuda or not rec.is_contiguous():
+                raise ValueError("out[1] must be a contiguous float32 CUDA tensor [capacity, 6]")
+        self._on_stream(stream, lambda h: self._ck(self._lib.mvsv_download_obstacles_stream(
+            self._ctx, age, offs.data_ptr(), rec.data_ptr() if rec.numel() else None, rec.shape[0], h)))
+        return offs, rec
+
     def download_minmax_device(self, batch, age=0, out=None, stream=None, device=None):
         """download_minmax() of the compute `age` calls back as an int16 CUDA tensor [batch, 2]
         (mvsv_download_minmax_device), allocated on `device` (default: the engine's first device) or taken from `out`
@@ -547,7 +606,7 @@ class Engine:
     def debug_postfilter(self, maps, median=True, new_val=0, speckle_size=0, speckle_diff=0, stages=0):
         """mvsv_debug_postfilter: int16 maps [B,]H,W (row stride may exceed W) through medianBlur(3) when `median`, then
         filterSpeckles(new_val, speckle_size, speckle_diff) when speckle_size > 0, then `stages` (STAGE_XYZ |
-        STAGE_POINTS | STAGE_MEANS); the results are fetched with download / download_minmax / debug_read like those of a compute."""
+        STAGE_POINTS | STAGE_MEANS | STAGE_DETECT); the results are fetched with download / download_minmax / debug_read like those of a compute."""
         m = np.asarray(maps)
         if m.ndim == 2:
             m = m[None]

@@ -1,5 +1,6 @@
 // C-ABI glue of libmvsv.so (include/mvsv.h): context, device buffers, parameter normalisation, stage sequencing.
 #include "mvsv_internal.h"
+#include "../../include/mvsv_detection.hpp"
 #include <cmath>
 
 #include <algorithm>
@@ -14,7 +15,7 @@
 const char* const kKernelNames[KID_COUNT] = {
     "remap", "sgbm_prefilter", "sgbm_vsum", "sgbm_h1", "sgbm_vdir", "sgbm_td", "sgbm_h2_wta", "median3", "ccl_rows", "ccl_vmerge",
     "ccl_flatten", "ccl_apply", "bm_prefilter", "bm_tex", "bm_colsum", "bm_wta", "xyz", "means", "fill", "minmax", "tm",
-    "bm_lrcheck", "points"};
+    "bm_lrcheck", "points", "detect"};
 
 cudaError_t smem_limit(const void* kernel, int bytes)
 {
@@ -79,6 +80,7 @@ int upload_rig_tables(Engine* c)
         for (int cam = 0; cam < 2; ++cam) t.map[cam][r] = c->map_xy[r][cam];
         for (int i = 0; i < 16; ++i) t.Q[r][i] = (double)c->Q[r][i];
     }
+    std::memcpy(t.det_range, c->det_range, sizeof(t.det_range));
     MVSV_CK(c, cudaMemcpyAsync(c->rig_tables, &t, sizeof(t), cudaMemcpyHostToDevice, c->stream));   // pageable: staged before it returns
     c->rig_tables_dirty = false;
     return MVSV_OK;
@@ -94,7 +96,38 @@ void release_slot(IoSlot& s, bool staging)
     }
     if (staging) { s.minmax.reset(); s.minmax16.reset(); }
     s.disp.reset(); s.xyz.reset(); s.points.reset(); s.offsets.reset(); s.means.reset();
+    s.obstacles.reset(); s.det_offsets.reset();
     s.B = 0; s.stages = 0;
+}
+
+// The (first, second) disparity range of every (rig, detector) of the detection table: Utility::calcDMapValues of the
+// detector's distances with the rig's Q, exactly as the host detectors' init() computes it.  Rigs without Q get none
+// (a compute whose frames name such a rig is rejected).
+void update_det_ranges(Engine* c)
+{
+    std::memset(c->det_range, 0, sizeof(c->det_range));
+    for (int r = 0; r < MVSV_MAX_RIGS; ++r)
+        if (c->has_Q[r])
+            for (int d = 0; d < c->ndet; ++d) {
+                const float lower[3] = {0, 0, c->det_dist[d][0] * 1000}, upper[3] = {0, 0, c->det_dist[d][1] * 1000};
+                c->det_range[r][d][0] = mvsv::Utility::calcDMapValues(lower, c->Q[r]).dValue;
+                c->det_range[r][d][1] = mvsv::Utility::calcDMapValues(upper, c->Q[r]).dValue;
+            }
+    c->rig_tables_dirty = true;
+}
+
+// The detection table goes with the ROIs it describes (mvsv_set_mean_rois, geometry changes), and with it the obstacle
+// lists of the slots.  Called with the engine's streams synchronised.
+void drop_detection(Engine* c)
+{
+    c->has_det = false;
+    c->det_n = 0;
+    c->det_rois.reset();
+    for (IoSlot& s : c->slot) {
+        s.obstacles.reset();
+        s.det_offsets.reset();
+        s.stages &= ~(unsigned)MVSV_STAGE_DETECT;
+    }
 }
 
 // Allocates what each live slot needs in the engine's present state and does not have yet: the rectified images and
@@ -261,6 +294,7 @@ int apply_geometry(Engine* c, const Geometry& g)
         // mean-disparity ROIs are coordinates of the old map: drop them (run() asks for new ones)
         c->rois.reset();
         c->nrois = 0;
+        drop_detection(c);
         for (IoSlot& s : c->slot) release_slot(s, false);
         for (auto& b : c->bm_pre) b.reset();
         c->recL.reset(); c->d2.reset(); c->disp_raw.reset(); c->disp_med.reset(); c->labels.reset(); c->sizes.reset();
@@ -353,12 +387,19 @@ void take_slot(Engine* c)
 // frames
 int check_consumers(Engine* c, const IoSlot& slot, unsigned stages, uint64_t rigs)
 {
-    if (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS))
+    if ((stages & MVSV_STAGE_DETECT) && !(stages & MVSV_STAGE_MEANS))
+        return fail(c, MVSV_ERR_INVALID, "MVSV_STAGE_DETECT needs MVSV_STAGE_MEANS in the same compute");
+    if (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS | MVSV_STAGE_DETECT))
         for (int r = 0; r < MVSV_MAX_RIGS; ++r)
             if (((rigs >> r) & 1) && !c->has_Q[r])
                 return fail(c, MVSV_ERR_STATE, r == 0 ? "mvsv_set_Q not called" : "no Q for rig " + std::to_string(r) + " (mvsv_set_Q_rig)");
     if ((stages & MVSV_STAGE_MEANS) && (c->nrois < 1 || !c->rois || !slot.means))
         return fail(c, MVSV_ERR_STATE, "no mean-disparity ROIs (mvsv_set_mean_rois; a geometry change drops them)");
+    if ((stages & MVSV_STAGE_DETECT) && (!c->has_det || !c->det_rois))
+        return fail(c, MVSV_ERR_STATE, "no detection table (mvsv_set_detection; mvsv_set_mean_rois and geometry changes drop it)");
+    if ((stages & MVSV_STAGE_DETECT) && c->det_n != c->nrois)
+        return fail(c, MVSV_ERR_STATE, "the detection table does not match the ROIs (" + std::to_string(c->det_n) + " against " +
+                                           std::to_string(c->nrois) + ")");
     return MVSV_OK;
 }
 
@@ -371,6 +412,11 @@ int ensure_consumers(Engine* c, IoSlot& slot, unsigned stages)
         MVSV_CK(c, slot.points.ensure(npx * 3));
         MVSV_CK(c, slot.offsets.ensure((size_t)c->maxB + 1));
         MVSV_CK(c, c->pt_tiles.ensure(points_tiles(c->W, c->H, c->maxB)));
+    }
+    if (stages & MVSV_STAGE_DETECT) {
+        MVSV_CK(c, slot.obstacles.ensure((size_t)c->maxB * c->nrois));
+        MVSV_CK(c, slot.det_offsets.ensure((size_t)c->maxB + 1));
+        MVSV_CK(c, c->det_counts.ensure((size_t)c->maxB));
     }
     return MVSV_OK;
 }
@@ -432,7 +478,7 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     if (!rc) rc = inputs_uploaded(c, device_src);
     if (rc) return rc;
     if (signal_read) MVSV_CK(c, cudaEventRecord(c->ev_h2d, device_src ? c->stream : c->copy_stream));
-    if (multi && (rectify || (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS)))) {
+    if (multi && (rectify || (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS | MVSV_STAGE_DETECT)))) {
         rc = upload_rig_tables(c);
         if (rc) return rc;
     }
@@ -446,6 +492,7 @@ int compute_submit(Engine* c, const uint8_t* left, size_t lstride, const uint8_t
     if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
     if (stages & MVSV_STAGE_POINTS) MVSV_CK(c, launch_points(c, batch, multi));
     if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
+    if (stages & MVSV_STAGE_DETECT) MVSV_CK(c, launch_detect(c, batch, multi));
     MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
     MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
     return MVSV_OK;
@@ -497,28 +544,43 @@ int download_wait(Engine* c)
     return MVSV_OK;
 }
 
-// mvsv_download_points, first phase: the frame offsets of the point list in I/O slot `k` (B + 1 values) into `offsets`.
-// The copy is a few bytes to pageable memory, which the CUDA runtime completes before it returns.
-int points_offsets(Engine* c, int k, std::vector<long long>& offsets)
+// The packed lists a compute leaves in an I/O slot, frame offsets first: the point list of MVSV_STAGE_POINTS and the
+// found obstacles of MVSV_STAGE_DETECT
+struct SlotList {
+    const long long* offsets;
+    const void* data;
+    size_t elem;       // bytes per element
+};
+SlotList slot_list(const IoSlot& s, unsigned stage)
+{
+    if (stage == MVSV_STAGE_DETECT) return {s.det_offsets, s.obstacles, sizeof(mvsv_obstacle)};
+    return {s.offsets, s.points, 3 * sizeof(float)};
+}
+
+// mvsv_download_points, first phase: the frame offsets of the list (`stage`) in I/O slot `k` (B + 1 values) into
+// `offsets`.  The copy is a few bytes to pageable memory, which the CUDA runtime completes before it returns.
+int points_offsets(Engine* c, int k, std::vector<long long>& offsets, unsigned stage)
 {
     int rc = bind(c);
     if (rc) return rc;
     const IoSlot& s = c->slot[k];
     offsets.resize((size_t)s.B + 1);
     MVSV_CK(c, cudaStreamWaitEvent(c->dl_stream, s.done, 0));
-    MVSV_CK(c, cudaMemcpyAsync(offsets.data(), s.offsets, offsets.size() * sizeof(long long), cudaMemcpyDeviceToHost, c->dl_stream));
+    MVSV_CK(c, cudaMemcpyAsync(offsets.data(), slot_list(s, stage).offsets, offsets.size() * sizeof(long long),
+                               cudaMemcpyDeviceToHost, c->dl_stream));
     return download_wait(c);
 }
 
-// second phase: queues the copy of the slot's n points to `points` on the download stream, as download_enqueue does
-// (download_wait waits for it)
-int points_enqueue(Engine* c, int k, float* points, long long n, cudaMemcpyKind kind, cudaEvent_t caller_ready)
+// second phase: queues the copy of the list's first n elements to `out` on the download stream, as download_enqueue
+// does (download_wait waits for it)
+int points_enqueue(Engine* c, int k, void* out, long long n, cudaMemcpyKind kind, cudaEvent_t caller_ready, unsigned stage)
 {
     int rc = bind(c);
     if (rc) return rc;
     IoSlot& s = c->slot[k];
+    const SlotList l = slot_list(s, stage);
     if (caller_ready) MVSV_CK(c, cudaStreamWaitEvent(c->dl_stream, caller_ready, 0));
-    if (n > 0) MVSV_CK(c, cudaMemcpyAsync(points, s.points, (size_t)n * 3 * sizeof(float), kind, c->dl_stream));
+    if (n > 0) MVSV_CK(c, cudaMemcpyAsync(out, l.data, (size_t)n * l.elem, kind, c->dl_stream));
     MVSV_CK(c, cudaEventRecord(s.dl_done, c->dl_stream));
     return MVSV_OK;
 }
@@ -1188,6 +1250,7 @@ int mvsv_set_Q_rig(mvsv_ctx* ctx, int rig, const float q[16])
         std::memcpy(c->Q[rig], q, sizeof(float) * 16);
         c->has_Q[rig] = true;
         c->rig_tables_dirty = true;
+        update_det_ranges(c);
         return MVSV_OK;
     });
 }
@@ -1230,12 +1293,43 @@ int mvsv_set_mean_rois(mvsv_ctx* ctx, const int* xywh, int n)
             s.means.reset();
             s.stages &= ~(unsigned)MVSV_STAGE_MEANS;
         }
+        drop_detection(c);
         c->nrois = n;
         if (n == 0) return MVSV_OK;
         MVSV_CK(c, c->rois.alloc((size_t)n * 4));
         rc = ensure_slots(c);
         if (rc) return rc;
         MVSV_CK(c, cudaMemcpy(c->rois, xywh, (size_t)n * 4 * sizeof(int), cudaMemcpyHostToDevice));
+        return MVSV_OK;
+    });
+}
+
+int mvsv_set_detection(mvsv_ctx* ctx, const int* detector_of_roi, const float* centers_xy, int n, const float* min_max_distance,
+                       int ndet)
+{
+    return each(ctx, true, [&](Engine* c) -> int {
+        if (n < 1 || !detector_of_roi || !centers_xy || !min_max_distance) return fail(c, MVSV_ERR_INVALID, "empty detection table");
+        if (ndet < 1 || ndet > MVSV_MAX_DETECTORS) return fail(c, MVSV_ERR_INVALID, "ndet must be in [1, MVSV_MAX_DETECTORS]");
+        if (n != c->nrois)
+            return fail(c, MVSV_ERR_STATE, "the detection table has " + std::to_string(n) + " ROIs, mvsv_set_mean_rois set " +
+                                               std::to_string(c->nrois));
+        std::vector<DetRoi> t((size_t)n);
+        for (int i = 0; i < n; ++i) {
+            if (detector_of_roi[i] < -1 || detector_of_roi[i] >= ndet)
+                return fail(c, MVSV_ERR_INVALID, "detector of ROI " + std::to_string(i) + " outside [-1, ndet)");
+            t[i] = DetRoi{detector_of_roi[i], centers_xy[2 * i], centers_xy[2 * i + 1], 0};
+        }
+        int rc = bind(c);
+        if (rc) return rc;
+        MVSV_CK(c, cudaStreamSynchronize(c->stream));   // computes already submitted read the table they were submitted with
+        c->has_det = false;
+        MVSV_CK(c, c->det_rois.ensure((size_t)n));
+        MVSV_CK(c, cudaMemcpy(c->det_rois, t.data(), (size_t)n * sizeof(DetRoi), cudaMemcpyHostToDevice));
+        c->det_n = n;
+        c->ndet = ndet;
+        for (int d = 0; d < ndet; ++d) { c->det_dist[d][0] = min_max_distance[2 * d]; c->det_dist[d][1] = min_max_distance[2 * d + 1]; }
+        update_det_ranges(c);
+        c->has_det = true;
         return MVSV_OK;
     });
 }
@@ -1320,9 +1414,22 @@ int mvsv_download_device(mvsv_ctx* c, int age, int16_t* disp, size_t dstride, ui
     return download(c, age, disp, dstride, rectL, rectR, rstride, xyz, means, cudaMemcpyDefault, stream);
 }
 
-// mvsv_download_points and mvsv_download_points_device, as download() above
-static int download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points, cudaMemcpyKind kind,
-                           void* stream)
+// The list of `stage` (slot_list) of slot s is there on every part with frames; "<stage> stage was not computed" otherwise
+static int check_list(mvsv_ctx* c, int s, const std::vector<int>& first, unsigned stage)
+{
+    for (size_t k = 0; k + 1 < first.size(); ++k)
+        if (first[k] < first[k + 1]) {
+            const IoSlot& sl = c->parts[k]->slot[s];
+            if (!slot_list(sl, stage).offsets || !(sl.stages & stage))
+                return fail(c, MVSV_ERR_STATE, stage == MVSV_STAGE_DETECT ? "DETECT stage was not computed" : "POINTS stage was not computed");
+        }
+    return MVSV_OK;
+}
+
+// mvsv_download_points, mvsv_download_points_device and mvsv_download_obstacles (`stage`: the list, slot_list), as
+// download() above.  `points`: the destination, `capacity_points` elements of the list.
+static int download_points(mvsv_ctx* c, int age, int64_t* offsets, void* points, size_t capacity_points, cudaMemcpyKind kind,
+                           void* stream, unsigned stage = MVSV_STAGE_POINTS)
 {
     int rc = usable(c);
     if (rc) return rc;
@@ -1337,15 +1444,14 @@ static int download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points
     const int s = (p0->cur + p0->nslots - age) % p0->nslots, n = (int)c->parts.size();
     const std::vector<int> first = firsts(c, s);
     if (first[n] < 1) return fail(c, MVSV_ERR_STATE, "nothing computed yet");
-    for (int k = 0; k < n; ++k)
-        if (first[k] < first[k + 1] && (!c->parts[k]->slot[s].offsets || !(c->parts[k]->slot[s].stages & MVSV_STAGE_POINTS)))
-            return fail(c, MVSV_ERR_STATE, "POINTS stage was not computed");
+    rc = check_list(c, s, first, stage);
+    if (rc) return rc;
     // phase 1: every part's frame offsets; part k's list goes after the points of the parts before it
     std::vector<std::vector<long long>> part(n);
     std::vector<long long> base(n + 1, 0);
     for (int k = 0; k < n; ++k) {
         if (first[k] < first[k + 1]) {
-            rc = on_part(c, k, [&](Engine* p) { return points_offsets(p, s, part[k]); });
+            rc = on_part(c, k, [&](Engine* p) { return points_offsets(p, s, part[k], stage); });
             if (rc) return rc;
         }
         base[k + 1] = base[k] + (part[k].empty() ? 0 : part[k].back());
@@ -1355,8 +1461,9 @@ static int download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points
     offsets[first[n]] = base[n];
     if (!points) return MVSV_OK;
     if (capacity_points < (size_t)base[n])
-        return fail(c, MVSV_ERR_INVALID, "points buffer holds " + std::to_string(capacity_points) + " points, the list has " +
-                                             std::to_string(base[n]));
+        return fail(c, MVSV_ERR_INVALID, (stage == MVSV_STAGE_DETECT ? "obstacle buffer holds " + std::to_string(capacity_points) + " records"
+                                                                     : "points buffer holds " + std::to_string(capacity_points) + " points") +
+                                             ", the list has " + std::to_string(base[n]));
     cudaEvent_t ready = nullptr;
     rc = caller_ready(c, caller, &ready);
     if (rc) return rc;
@@ -1365,7 +1472,9 @@ static int download_points(mvsv_ctx* c, int age, int64_t* offsets, float* points
     for (; queued < n && !rc; ++queued)
         if (first[queued] < first[queued + 1]) {
             rc = on_part(c, queued, [&](Engine* p) {
-                return points_enqueue(p, s, points + 3 * (size_t)base[queued], base[queued + 1] - base[queued], kind, ready);
+                const size_t elem = slot_list(p->slot[s], stage).elem;
+                return points_enqueue(p, s, (char*)points + elem * (size_t)base[queued], base[queued + 1] - base[queued], kind,
+                                      ready, stage);
             });
             if (!rc && caller.st) rc = caller_wait(c, caller, c->parts[queued]->slot[s].dl_done);
         }
@@ -1388,7 +1497,14 @@ int mvsv_download_points_device(mvsv_ctx* c, int age, int64_t* offsets, float* p
     return download_points(c, age, offsets, points, capacity_points, cudaMemcpyDefault, stream);
 }
 
-int mvsv_download_points_stream(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points, void* stream)
+int mvsv_download_obstacles(mvsv_ctx* c, int age, int64_t* offsets, mvsv_obstacle* out, size_t capacity)
+{
+    return download_points(c, age, offsets, out, capacity, cudaMemcpyDeviceToHost, nullptr, MVSV_STAGE_DETECT);
+}
+
+// mvsv_download_points_stream and mvsv_download_obstacles_stream (`stage`: the list, slot_list)
+static int download_list_stream(mvsv_ctx* c, int age, int64_t* offsets, void* points, size_t capacity_points, void* stream,
+                                unsigned stage)
 {
     int rc = usable(c);
     if (rc) return rc;
@@ -1404,13 +1520,11 @@ int mvsv_download_points_stream(mvsv_ctx* c, int age, int64_t* offsets, float* p
     rc = results_slot(c, age, &s, &first);
     if (rc) return rc;
     const int n = (int)c->parts.size();
+    rc = check_list(c, s, first, stage);
+    if (rc) return rc;
     int last = 0;   // the part holding the last frame writes offsets[batch]
     for (int k = 0; k < n; ++k)
-        if (first[k] < first[k + 1]) {
-            last = k;
-            if (!c->parts[k]->slot[s].offsets || !(c->parts[k]->slot[s].stages & MVSV_STAGE_POINTS))
-                return fail(c, MVSV_ERR_STATE, "POINTS stage was not computed");
-        }
+        if (first[k] < first[k + 1]) last = k;
     // k_points_out writes the destinations from the part's device: one on another device needs peer access there
     for (int pass = 0; pass < 2; ++pass)
         for (int k = 0; k < n; ++k) {
@@ -1454,12 +1568,16 @@ int mvsv_download_points_stream(mvsv_ctx* c, int age, int64_t* offsets, float* p
                 const Engine* q = c->parts[j];
                 MVSV_CK(p, cudaStreamWaitEvent(st, q->slot[s].done, 0));
                 MVSV_CK(p, cudaMemcpyPeerAsync((long long*)p->pt_base + nb, p->device,
-                                               (const long long*)q->slot[s].offsets + q->slot[s].B, q->device, sizeof(long long), st));
+                                               slot_list(q->slot[s], stage).offsets + q->slot[s].B, q->device, sizeof(long long), st));
                 ++nb;
             }
-        MVSV_CK(p, launch_points_out(p, sl, nb ? (const long long*)p->pt_base : nullptr, nb,
-                                     reinterpret_cast<long long*>(offsets) + first[k], first[k + 1] - first[k] + (k == last ? 1 : 0),
-                                     points, cap));
+        const long long* bases = nb ? (const long long*)p->pt_base : nullptr;
+        long long* dst_offs = reinterpret_cast<long long*>(offsets) + first[k];
+        const int nout = first[k + 1] - first[k] + (k == last ? 1 : 0);
+        if (stage == MVSV_STAGE_DETECT)
+            MVSV_CK(p, launch_obstacles_out(p, sl, bases, nb, dst_offs, nout, (mvsv_obstacle*)points, cap));
+        else
+            MVSV_CK(p, launch_points_out(p, sl, bases, nb, dst_offs, nout, (float*)points, cap));
         MVSV_CK(p, cudaEventRecord(sl.dl_done, st));
         // the parts before hold their slot until this part has read their totals: their dl_done covers that read
         for (int j = 0; j < k; ++j)
@@ -1471,6 +1589,16 @@ int mvsv_download_points_stream(mvsv_ctx* c, int age, int64_t* offsets, float* p
             }
         return MVSV_OK;
     });
+}
+
+int mvsv_download_points_stream(mvsv_ctx* c, int age, int64_t* offsets, float* points, size_t capacity_points, void* stream)
+{
+    return download_list_stream(c, age, offsets, points, capacity_points, stream, MVSV_STAGE_POINTS);
+}
+
+int mvsv_download_obstacles_stream(mvsv_ctx* c, int age, int64_t* offsets, mvsv_obstacle* out, size_t capacity, void* stream)
+{
+    return download_list_stream(c, age, offsets, out, capacity, stream, MVSV_STAGE_DETECT);
 }
 
 int mvsv_set_io_slots(mvsv_ctx* ctx, int n)
@@ -1662,8 +1790,8 @@ int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int
         if (rc) return rc;
         if (!maps || batch < 1 || batch > c->maxB) return fail(c, MVSV_ERR_INVALID, "bad map pointer or batch size");
         if (stride < (size_t)c->W * sizeof(int16_t)) return fail(c, MVSV_ERR_INVALID, "stride smaller than the map width");
-        if (stages & ~(unsigned)(MVSV_STAGE_XYZ | MVSV_STAGE_POINTS | MVSV_STAGE_MEANS))
-            return fail(c, MVSV_ERR_INVALID, "post-filter hook: only MVSV_STAGE_XYZ, MVSV_STAGE_POINTS and MVSV_STAGE_MEANS");
+        if (stages & ~(unsigned)(MVSV_STAGE_XYZ | MVSV_STAGE_POINTS | MVSV_STAGE_MEANS | MVSV_STAGE_DETECT))
+            return fail(c, MVSV_ERR_INVALID, "post-filter hook: only MVSV_STAGE_XYZ, MVSV_STAGE_POINTS, MVSV_STAGE_MEANS and MVSV_STAGE_DETECT");
         if (maxSpeckleSize > 0 && (newVal < -32768 || newVal > 32767)) return fail(c, MVSV_ERR_INVALID, "newVal does not fit CV_16S");
         const uint64_t rigs = rigs_of_batch(c, batch);
         const bool multi = rigs != 1;
@@ -1683,13 +1811,14 @@ int mvsv_debug_postfilter(mvsv_ctx* ctx, const int16_t* maps, size_t stride, int
             MVSV_CK(c, launch_speckle(c, median ? c->disp_med : c->disp_raw, slot.disp, batch, newVal, maxSpeckleSize, maxDiff));
         if (!median && !speckle)
             MVSV_CK(c, cudaMemcpyAsync(slot.disp, c->disp_raw, npx * sizeof(int16_t), cudaMemcpyDeviceToDevice, c->stream));
-        if (multi && (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS))) {
+        if (multi && (stages & (MVSV_STAGE_XYZ | MVSV_STAGE_POINTS | MVSV_STAGE_DETECT))) {
             rc = upload_rig_tables(c);
             if (rc) return rc;
         }
         if (stages & MVSV_STAGE_XYZ) MVSV_CK(c, multi ? launch_xyz_rigs(c, batch) : launch_xyz(c, batch));
         if (stages & MVSV_STAGE_POINTS) MVSV_CK(c, launch_points(c, batch, multi));
         if (stages & MVSV_STAGE_MEANS) MVSV_CK(c, launch_means(c, batch));
+        if (stages & MVSV_STAGE_DETECT) MVSV_CK(c, launch_detect(c, batch, multi));
         MVSV_CK(c, cudaEventRecord(slot.done, c->stream));
         MVSV_CK(c, cudaEventRecord(c->ev_done, c->stream));
         slot.B = batch;

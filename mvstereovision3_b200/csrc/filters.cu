@@ -5,6 +5,7 @@
 #include <cstdint>
 #include <cfloat>
 #include <cmath>
+#include <cstring>
 
 namespace {
 
@@ -722,6 +723,159 @@ k_points_out(const long long* __restrict__ offs, int nfr, int nout, const long l
     for (long long i = head + tid; i < nf; i += nthr) d[i] = src[i];
 }
 
+// ------------------------------------------------------------------------------------------------
+// MVSV_STAGE_DETECT: MeanDisparityDetection / SamplepointDetection::detectObstacles (include/mvsv_detection.hpp) over
+// the ROI means of a batch.  Ordered compaction in three kernels: count the hits of every frame, scan the counts
+// (k_points_scan with one tile per frame), then re-test every frame and write its records at the frame's base.
+// ------------------------------------------------------------------------------------------------
+constexpr int DET_THREADS = 256;
+
+// Q and the (first, second) ranges of the detectors, of rig 0 (passed by value) or of every rig (RigTables)
+struct DetRig0 { double Q[16]; float range[MVSV_MAX_DETECTORS][2]; };
+
+// The range test of ROI i with mean `value`: the reference's `value < first && value > second`
+__device__ __forceinline__ bool det_hit(const float (*range)[2], int d, float value)
+{
+    return d >= 0 && value < range[d][0] && value > range[d][1];
+}
+
+// Utility::calcCoordinate({value, x, y}, Q) of the header: the products of two floats are exact in double, each add
+// rounds once in the order k = 0..3 from 0 (explicitly rounded: no contraction into an FMA, and 0 + -0 = +0 as on the
+// host), every component rounds to float, then is multiplied by the double reciprocal of the fourth.
+__device__ __forceinline__ void det_coordinate(const double* Q, float x, float y, float value, float (&out)[4])
+{
+    const double in[4] = {(double)x, (double)y, (double)__fdiv_rn(value, 16.f), 1.0};
+    float c[4];
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+        double acc = 0.0;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) acc = __dadd_rn(acc, __dmul_rn(Q[r * 4 + k], in[k]));
+        c[r] = (float)acc;
+    }
+    const double inv = __ddiv_rn(1.0, (double)c[3]);
+#pragma unroll
+    for (int r = 0; r < 4; ++r) out[r] = (float)__dmul_rn((double)c[r], inv);
+    if (isinf(__fdiv_rn(out[2], 1000.f))) out[2] = 0.f;
+}
+
+// One CTA per frame: its number of hits
+template <class RangeOf>
+__device__ __forceinline__ void detect_count(const float* __restrict__ means, const DetRoi* __restrict__ rois, int n,
+                                             long long* __restrict__ counts, RangeOf rangeOf)
+{
+    __shared__ int s_warp[DET_THREADS / 32];
+    const int f = blockIdx.x;
+    const float (*range)[2] = rangeOf(f);
+    const float* m = means + (size_t)f * n;
+    int cnt = 0;
+    for (int i = threadIdx.x; i < n; i += DET_THREADS) cnt += det_hit(range, rois[i].det, m[i]) ? 1 : 0;
+    cnt = __reduce_add_sync(0xffffffffu, cnt);
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = cnt;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int total = 0;
+#pragma unroll
+        for (int w = 0; w < DET_THREADS / 32; ++w) total += s_warp[w];
+        counts[f] = total;
+    }
+}
+
+// One CTA per frame, DET_THREADS ROIs at a time: a ballot ranks the hits within each warp, the warps' counts give their
+// bases, and each hit writes its record at the frame's base (bases[f], scanned) + the hits before it
+template <class RangeOf, class QOf>
+__device__ __forceinline__ void detect_emit(const float* __restrict__ means, const DetRoi* __restrict__ rois, int n,
+                                            const long long* __restrict__ bases, mvsv_obstacle* __restrict__ out,
+                                            RangeOf rangeOf, QOf qOf)
+{
+    __shared__ int s_warp[DET_THREADS / 32];
+    const int f = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const float (*range)[2] = rangeOf(f);
+    const double* Q = qOf(f);
+    const float* m = means + (size_t)f * n;
+    long long run = bases[f];
+    for (int i0 = 0; i0 < n; i0 += DET_THREADS) {
+        const int i = i0 + threadIdx.x;
+        DetRoi r = {-1, 0.f, 0.f, 0};
+        float value = 0.f;
+        if (i < n) { r = rois[i]; value = m[i]; }
+        const bool hit = i < n && det_hit(range, r.det, value);
+        const unsigned ball = __ballot_sync(0xffffffffu, hit);
+        if (lane == 0) s_warp[warp] = __popc(ball);
+        __syncthreads();
+        int before = 0, total = 0;
+#pragma unroll
+        for (int w = 0; w < DET_THREADS / 32; ++w) {
+            const int s = s_warp[w];
+            before += w < warp ? s : 0;
+            total += s;
+        }
+        if (hit) {
+            mvsv_obstacle o;
+            o.roi = i;
+            o.value = value;
+            det_coordinate(Q, r.x, r.y, value, o.xyzw);
+            out[run + before + __popc(ball & ((1u << lane) - 1u))] = o;
+        }
+        run += total;
+        __syncthreads();      // s_warp is rewritten by the next chunk
+    }
+}
+
+__global__ void __launch_bounds__(DET_THREADS)
+k_detect_count(const float* __restrict__ means, const DetRoi* __restrict__ rois, int n, long long* __restrict__ counts, DetRig0 p)
+{
+    detect_count(means, rois, n, counts, [&](int) { return (const float (*)[2])p.range; });
+}
+
+__global__ void __launch_bounds__(DET_THREADS)
+k_detect_count_rigs(const float* __restrict__ means, const DetRoi* __restrict__ rois, int n, long long* __restrict__ counts,
+                    const RigTables* __restrict__ rigs, const int* __restrict__ rig_of_frame)
+{
+    detect_count(means, rois, n, counts, [&](int f) { return (const float (*)[2])rigs->det_range[rig_of_frame[f]]; });
+}
+
+__global__ void __launch_bounds__(DET_THREADS)
+k_detect_emit(const float* __restrict__ means, const DetRoi* __restrict__ rois, int n, const long long* __restrict__ bases,
+              mvsv_obstacle* __restrict__ out, DetRig0 p)
+{
+    detect_emit(means, rois, n, bases, out, [&](int) { return (const float (*)[2])p.range; },
+                [&](int) { return (const double*)p.Q; });
+}
+
+__global__ void __launch_bounds__(DET_THREADS)
+k_detect_emit_rigs(const float* __restrict__ means, const DetRoi* __restrict__ rois, int n, const long long* __restrict__ bases,
+                   mvsv_obstacle* __restrict__ out, const RigTables* __restrict__ rigs, const int* __restrict__ rig_of_frame)
+{
+    detect_emit(means, rois, n, bases, out, [&](int f) { return (const float (*)[2])rigs->det_range[rig_of_frame[f]]; },
+                [&](int f) { return (const double*)rigs->Q[rig_of_frame[f]]; });
+}
+
+// mvsv_download_obstacles_stream, one part: k_points_out for records of six 4-byte words (24 bytes: 8-byte accesses
+// where the destination is 8-byte aligned, as a cudaMalloc source always is)
+__global__ void __launch_bounds__(256)
+k_obstacles_out(const long long* __restrict__ offs, int nfr, int nout, const long long* __restrict__ bases, int nbases,
+                const mvsv_obstacle* __restrict__ src, long long* __restrict__ dst_offs, mvsv_obstacle* __restrict__ dst,
+                long long capacity)
+{
+    long long base = 0;
+    for (int j = 0; j < nbases; ++j) base += bases[j];
+    const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x, nthr = (long long)gridDim.x * blockDim.x;
+    for (long long i = tid; i < nout; i += nthr) dst_offs[i] = base + offs[i];
+    const long long n = dst ? min(offs[nfr], capacity - base) : 0;
+    if (n <= 0) return;
+    mvsv_obstacle* d = dst + base;
+    if ((reinterpret_cast<uintptr_t>(d) & 7) == 0) {
+        const uint2* s2 = reinterpret_cast<const uint2*>(src);
+        uint2* d2 = reinterpret_cast<uint2*>(d);
+        for (long long i = tid; i < 3 * n; i += nthr) d2[i] = s2[i];
+    } else {
+        const unsigned* s1 = reinterpret_cast<const unsigned*>(src);
+        unsigned* d1 = reinterpret_cast<unsigned*>(d);
+        for (long long i = tid; i < 6 * n; i += nthr) d1[i] = s1[i];
+    }
+}
+
 }  // namespace
 
 cudaError_t launch_minmax(Engine* c, const IoSlot& s, int* mm, cudaStream_t st)
@@ -876,6 +1030,42 @@ cudaError_t launch_points(Engine* c, int B, bool rigs)
         for (int i = 0; i < 16; ++i) Q.q[i] = (double)c->Q[0][i];
         k_points_emit<<<ntiles, PT_THREADS, 0, c->stream>>>(disp, c->W, HW, tpf, c->pt_tiles, io(c).points, Q);
     }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_detect(Engine* c, int B, bool rigs)
+{
+    const int n = c->nrois;
+    IoSlot& s = io(c);
+    if (rigs) {
+        { KernelTimer kt(c, KID_DETECT); k_detect_count_rigs<<<B, DET_THREADS, 0, c->stream>>>(s.means, c->det_rois, n, c->det_counts, c->rig_tables, c->rig_frames.rig); }
+    } else {
+        DetRig0 p;
+        for (int i = 0; i < 16; ++i) p.Q[i] = (double)c->Q[0][i];
+        std::memcpy(p.range, c->det_range[0], sizeof(p.range));
+        { KernelTimer kt(c, KID_DETECT); k_detect_count<<<B, DET_THREADS, 0, c->stream>>>(s.means, c->det_rois, n, c->det_counts, p); }
+    }
+    { KernelTimer kt(c, KID_DETECT); k_points_scan<<<1, PT_SCAN_THREADS, 0, c->stream>>>(c->det_counts, B, 1, s.det_offsets, B); }
+    KernelTimer kt(c, KID_DETECT);
+    if (rigs) {
+        k_detect_emit_rigs<<<B, DET_THREADS, 0, c->stream>>>(s.means, c->det_rois, n, c->det_counts, s.obstacles, c->rig_tables,
+                                                           c->rig_frames.rig);
+    } else {
+        DetRig0 p;
+        for (int i = 0; i < 16; ++i) p.Q[i] = (double)c->Q[0][i];
+        std::memcpy(p.range, c->det_range[0], sizeof(p.range));
+        k_detect_emit<<<B, DET_THREADS, 0, c->stream>>>(s.means, c->det_rois, n, c->det_counts, s.obstacles, p);
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_obstacles_out(Engine* c, const IoSlot& s, const long long* bases, int nbases, long long* dst_offs, int nout,
+                                 mvsv_obstacle* dst, long long capacity)
+{
+    const long long work = dst ? 3LL * s.B * c->nrois : nout;
+    const int blocks = (int)std::max(1LL, std::min((work + 255) / 256, 8LL * c->num_sms));
+    KernelTimer kt(c, KID_UNTIMED, c->dl_stream);
+    k_obstacles_out<<<blocks, 256, 0, c->dl_stream>>>(s.det_offsets, s.B, nout, bases, nbases, s.obstacles, dst_offs, dst, capacity);
     return cudaGetLastError();
 }
 

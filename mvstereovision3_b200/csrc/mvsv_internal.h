@@ -32,7 +32,7 @@ struct BmNorm {
 enum KernelId {
     KID_REMAP = 0, KID_SGBM_PREFILTER, KID_SGBM_VSUM, KID_SGBM_H1, KID_SGBM_VDIR, KID_SGBM_TD, KID_SGBM_H2_WTA, KID_MEDIAN,
     KID_CCL_ROWS, KID_CCL_VMERGE, KID_CCL_FLATTEN, KID_CCL_APPLY, KID_BM_PREFILTER, KID_BM_TEX, KID_BM_COLSUM,
-    KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_BM_LRCHECK, KID_POINTS, KID_COUNT
+    KID_BM_WTA, KID_XYZ, KID_MEANS, KID_FILL, KID_MINMAX, KID_TM, KID_BM_LRCHECK, KID_POINTS, KID_DETECT, KID_COUNT
 };
 // a launch counted in mvsv_launch_count but never timed: the per-kernel timing brackets the engine's stream only
 // (mvsv_profile_read waits for that stream), and the device downloads launch on the download stream
@@ -93,6 +93,10 @@ struct IoSlot {
     DeviceBuffer<float> points;
     DeviceBuffer<long long> offsets;
     DeviceBuffer<float> means;                // [B][nrois], once mean-disparity ROIs are set
+    // MVSV_STAGE_DETECT, allocated by the first compute with it: the packed found obstacles ([B*nrois] at most) and the
+    // frame offsets into them ([B+1]); in the slot for the same reason as the points
+    DeviceBuffer<mvsv_obstacle> obstacles;
+    DeviceBuffer<long long> det_offsets;
     cudaEvent_t done = nullptr;               // all kernels of the slot's last compute have finished
     // recorded on dl_stream after every download of the slot's results: a device download (mvsv_download_device) may
     // still be copying when its call returns, so whatever writes the slot next waits for it
@@ -122,7 +126,12 @@ struct RigFrames {
 struct RigTables {
     const int2* map[2][MVSV_MAX_RIGS];
     double Q[MVSV_MAX_RIGS][16];
+    // MVSV_STAGE_DETECT: (first, second) disparity range of every (rig, detector), Engine::det_range
+    float det_range[MVSV_MAX_RIGS][MVSV_MAX_DETECTORS][2];
 };
+
+// one ROI of the detection table (mvsv_set_detection): its detector (-1: not tested) and calcCoordinate's image_x, image_y
+struct DetRoi { int det; float x, y; int pad; };
 
 // One engine on one device: its streams, events, volumes and I/O slots.  An mvsv_ctx (csrc/api.cu) splits every batch
 // across one or more of them.
@@ -218,6 +227,16 @@ struct Engine {
     // mvsv_download_points_stream on a multi-device ctx: the point totals of the parts before this one, copied from
     // their slots on dl_stream (one entry per part of the ctx); k_points_out adds them up into this part's base
     DeviceBuffer<long long> pt_base;
+
+    // mvsv_set_detection: the table (device copy of det_rois_h) of the nrois ROIs, the detectors' distances and the
+    // disparity ranges they give with each rig's Q (recomputed when a Q or the table changes)
+    bool has_det = false;
+    int det_n = 0, ndet = 0;
+    std::vector<DetRoi> det_rois_h;
+    float det_dist[MVSV_MAX_DETECTORS][2] = {};
+    float det_range[MVSV_MAX_RIGS][MVSV_MAX_DETECTORS][2] = {};
+    DeviceBuffer<DetRoi> det_rois;
+    DeviceBuffer<long long> det_counts;       // per frame: its number of hits, then its base (launch_detect)
 };
 
 // the I/O slot of the compute in progress (or of the last one)
@@ -273,6 +292,9 @@ cudaError_t launch_means(Engine* c, int B);
 // launch; `rigs`: frames of several rigs (mvsv_set_frame_rigs)
 size_t points_tiles(int W, int H, int B);
 cudaError_t launch_points(Engine* c, int B, bool rigs);
+// MVSV_STAGE_DETECT of the current I/O slot, after launch_means: the found obstacles of B frames and their offsets;
+// `rigs`: frames of several rigs (Q and ranges from Engine::rig_tables)
+cudaError_t launch_detect(Engine* c, int B, bool rigs);
 // Utility::calcMinMaxDisparity of slot s's disparities into mm ([s.B][2] int: lo, hi) on stream st; the fold turns B
 // such pairs into the int16 pairs of mvsv_download_minmax
 cudaError_t launch_minmax(Engine* c, const IoSlot& s, int* mm, cudaStream_t st);
@@ -281,6 +303,9 @@ cudaError_t launch_minmax_fold(Engine* c, const int* mm, int16_t* out, int B, cu
 // into dst_offs, and the points that fit below `capacity` into dst (NULL: the offsets only), on dl_stream
 cudaError_t launch_points_out(Engine* c, const IoSlot& s, const long long* bases, int nbases, long long* dst_offs, int nout,
                               float* dst, long long capacity);
+// mvsv_download_obstacles_stream, one part: launch_points_out for slot s's found obstacles
+cudaError_t launch_obstacles_out(Engine* c, const IoSlot& s, const long long* bases, int nbases, long long* dst_offs, int nout,
+                                 mvsv_obstacle* dst, long long capacity);
 cudaError_t launch_median(Engine* c, const int16_t* in, int16_t* out, int B);
 cudaError_t launch_speckle(Engine* c, const int16_t* img, int16_t* out, int B, int newVal, int maxSize, int maxDiff);
 // fused previous-row sweep (csrc/sweep.cu): strip decomposition of a batch, scratch sizes, launch
